@@ -21,12 +21,15 @@ strands, per-haplotype counts, min/max row filter) over the whole block.
 on the same GPU: the blocks of consecutive steps alternate between two sets of streams and scratch and overlap on the device).
 `--workload configs3` prints the line of BASELINE.json configs[3] instead: 200,000 haplotypes in SAMPLE BLOCKS, merged on the host by
 tfbs_merge_sample_blocks (min != max over all samples after the gather), with `roofline_k1` for grouping + build.
+`--dump-outputs DIR` writes the rows of the last timed step as .npy files (dump_outputs): the inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -39,6 +42,8 @@ UNIT = "cells/s"
 SM_COUNT = 148
 CELLS_PER_LDS64 = 6          # 3 packed patterns x 2 columns per 64-bit shared-memory read
 LDS64_PER_CLK_PER_SM = 16    # 128 B/clk/SM of shared-memory bandwidth
+DUMP_BYTES = 64 << 20        # --dump-outputs writes at most this much
+DUMP_KEYS = ("region", "inner", "pattern_id", "vmin", "vmax")
 
 
 def parse_args():
@@ -61,7 +66,13 @@ def parse_args():
     ap.add_argument("--no-full-scan", action="store_true", help="skip the delta=0 pass that measures the scan kernel on the reference's full work")
     ap.add_argument("--no-driver", action="store_true", help="skip the wall time of the C++ driver on files")
     ap.add_argument("--option", action="append", default=[], help="library option key=value")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the rows of the last timed step to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times a sample of the block sized by the clock")
+    return args
 
 
 def peaks():
@@ -297,12 +308,13 @@ def main():
         return float(t.item())
 
     def pipelined(ctx, start, collect, steps):
-        """`steps` blocks with two in flight: the next one is enqueued before the previous one is collected."""
+        """`steps` blocks with two in flight: the next one is enqueued before the previous one is collected.  Returns what the last
+        collect returned."""
         start()
         for _ in range(steps - 1):
             start()
             collect()
-        collect()
+        return collect()
 
     def timed(ctx, stream, fn):
         """fn() bracketed by barrier + synchronize on both sides; device time from CUDA events on the library's kernel stream (they are
@@ -342,7 +354,10 @@ def main():
     # the first two blocks size the scratch (each may be repeated once or twice); the third is the first one enqueued with the
     # capacities the device asked for (new shared-memory sizes, buffers): steady state starts with the fourth
     pipelined(ctx, run, coll, max(4, args.warmup))
-    ms_total = timed(ctx, stream, lambda: pipelined(ctx, run, coll, args.steps))
+    last = []
+    ms_total = timed(ctx, stream, lambda: last.append(pipelined(ctx, run, coll, args.steps)))
+    if args.dump_outputs:  # before the next collect reuses the buffers the rows point into
+        dump_outputs(args.dump_outputs, {"rank%d_" % rank if world > 1 else "": last[0]}, DUMP_BYTES // world)
     st = ctx.stats()
     launches = st["total_launches"] * args.steps
     ms_step = ms_total / args.steps
@@ -461,7 +476,7 @@ def main():
             out["secondary"] = {"skipped": str(exc)[:300]}
     if not args.no_driver:
         try:
-            out["wall_s"] = driver_wall_time(args, world)
+            out["wall_s"] = driver_wall_time(args, world, pats, blk)
         except Exception as exc:
             out["wall_s"] = {"skipped": str(exc)[:300]}
     if not args.no_cpu_baseline and world == 1:
@@ -600,7 +615,10 @@ def configs3_line(args, binding, sharding, device, ClockSampler, pk):
     sampler.start()
     for _ in range(max(3, args.warmup)):
         step()
-    ms_step = timed(stream, lambda: [step() for _ in range(args.steps)]) / args.steps
+    last = []
+    ms_step = timed(stream, lambda: last.append([step() for _ in range(args.steps)][-1])) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"block%d_" % i: g for i, g in enumerate(last[0])}, DUMP_BYTES)
     clocks = sampler.stop()
     sts = [c.stats() for c in ctxs]
     tot = lambda k: sum(st[k] for st in sts)
@@ -670,6 +688,42 @@ def configs3_line(args, binding, sharding, device, ClockSampler, pk):
     return out
 
 
+def dump_outputs(out_dir, parts, budget):
+    """--dump-outputs: the rows the timed path handed its caller in its last step, as .npy files by which two builds can be compared.
+    `parts` maps a file-name prefix to the grouped rows of one context (collect_grouped).  Per part, in the library's row order
+    (deterministic, include/tfbs.h): DUMP_KEYS of the rows and `n_groups` of the regions as float64, and the per-sample counts
+    `left` / `right` as float32 (exact: a count is bounded by the window length) for the rows listed in `dense_rows`.  The group
+    labels of the grouped form are not results, so its packed arrays are written decoded (tfbs_expand_rows) rather than as they
+    are.  Whatever exceeds the part's share of `budget` is a fixed, seeded sample of the rows."""
+    import ctypes as C
+    import numpy as np
+    from find_tfbs_b200 import binding
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // max(1, len(parts)) - (1 << 12)  # room for the .npy headers
+
+    def pick(n, k, rng):
+        return np.arange(n) if k >= n else np.sort(rng.choice(n, max(0, k), replace=False))
+
+    for prefix, g in parts.items():
+        rng = np.random.default_rng(0)
+        n, S = int(g["n_rows"]), int(g["n_samples"])
+        out = {"n_groups": np.asarray(g["n_groups"], dtype=np.float64)}
+        rows = pick(n, (share // 2 - out["n_groups"].nbytes) // (8 * (len(DUMP_KEYS) + 1)), rng)
+        out["rows"] = rows.astype(np.float64)
+        for k in DUMP_KEYS:
+            out[k] = np.asarray(g[k], dtype=np.float64)[rows]
+        dense = rows[pick(len(rows), (share // 2) // (8 * max(1, S) + 8), rng)]
+        left, right = np.zeros((len(dense), S), np.uint32), np.zeros((len(dense), S), np.uint32)
+        for j, r in enumerate(dense):
+            rc = binding.lib().tfbs_expand_rows(C.byref(g["_c"]), int(r), 1, left[j].ctypes.data_as(C.POINTER(C.c_uint32)),
+                                                right[j].ctypes.data_as(C.POINTER(C.c_uint32)))
+            if rc != binding.TFBS_OK:
+                raise binding.TfbsError(rc, "tfbs_expand_rows failed")
+        out.update({"dense_rows": dense.astype(np.float64), "left": left.astype(np.float32), "right": right.astype(np.float32)})
+        for k, a in out.items():
+            np.save(os.path.join(out_dir, prefix + k + ".npy"), a)
+
+
 def np_xor(a):
     import numpy as np
     return np.bitwise_xor.reduce(a) if len(a) else 0
@@ -679,28 +733,33 @@ def stream_of(torch, ctx, device):
     return torch.cuda.ExternalStream(ctx.stream(), device=torch.device("cuda", device))
 
 
-def driver_wall_time(args, world):
+def driver_wall_time(args, world, pats, blk):
     """Chromosome wall time: the C++ driver (the reference's command line on top of the library) on the cohort written as files
-    (BCF + CSI, FASTA + .fai, two BED files, PWM + threshold files), one context per GPU (--devices 0..N-1).  The file set is
-    written once by scripts/make_cohort_files.py; without it the measurement is skipped."""
+    (BCF + CSI, FASTA + .fai, two BED files, PWM + threshold files), one context per GPU (--devices 0..N-1).  The file set is read
+    from scratch_data/ when scripts/make_cohort_files.py has written it there; otherwise it is written into a temporary directory
+    first (about half a minute for configs[2], not timed)."""
     name = "cfg2" if args.workload == "configs2" else "cfg1"
     d = os.path.join(ROOT, "scratch_data", name if args.scale == 1.0 else "%s_%g" % (name, args.scale))
     argfile = os.path.join(d, "args.txt")
     exe = os.path.join(ROOT, "find_tfbs_b200", "find-tfbs-b200")
-    if not os.path.exists(argfile) or not os.path.exists(exe):
-        return {"skipped": "no file set at %s (scripts/make_cohort_files.py writes it) or no driver binary" % d}
-    cli = open(argfile).read().split()
-    cli = [a if not a.startswith("scratch_data/") else os.path.join(ROOT, a) for a in cli]
-    outp = "/tmp/tfbs_bench_%d.vcf.gz" % os.getpid()
-    threads = os.cpu_count() or 8
-    cmd = [exe] + cli + ["--output", outp, "--threads", str(threads), "--devices", ",".join(str(k) for k in range(world))]
-    t = time.perf_counter()
-    r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=1500)
-    dt = time.perf_counter() - t
-    tail = [ln for ln in r.stdout.strip().split("\n")[-4:]]
-    size = os.path.getsize(outp) if os.path.exists(outp) else 0
-    if os.path.exists(outp):
-        os.unlink(outp)
+    if not os.path.exists(exe):
+        return {"skipped": "no driver binary at %s" % exe}
+    with tempfile.TemporaryDirectory(prefix="tfbs_bench_") as tmp:
+        if os.path.exists(argfile):
+            cli = open(argfile).read().split()
+            cli = [a if not a.startswith("scratch_data/") else os.path.join(ROOT, a) for a in cli]
+        else:
+            sys.path.insert(0, os.path.join(ROOT, "scripts"))
+            import make_cohort_files
+            cli = make_cohort_files.write_file_set(pats, blk, tmp, tmp)
+        outp = os.path.join(tmp, "out.vcf.gz")
+        threads = os.cpu_count() or 8
+        cmd = [exe] + cli + ["--output", outp, "--threads", str(threads), "--devices", ",".join(str(k) for k in range(world))]
+        t = time.perf_counter()
+        r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=1500)
+        dt = time.perf_counter() - t
+        tail = [ln for ln in r.stdout.strip().split("\n")[-4:]]
+        size = os.path.getsize(outp) if os.path.exists(outp) else 0
     if r.returncode != 0:
         return {"skipped": "driver failed: " + " | ".join(tail)[-300:]}
     return {"value": dt, "unit": "s", "devices": world, "host_threads": threads, "output_bytes": size, "command": "find-tfbs-b200 <file set of the same cohort> --devices 0..N-1",

@@ -78,14 +78,18 @@ CONTRACT_KEYS = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per
                  "config", "roofline", "e2e", "gpu_launches", "clocks", "cpu_baseline")
 
 
-def test_bench_control_flow_dry_run(emu_env):
+def test_bench_control_flow_dry_run(emu_env, tmp_path):
     """bench.py end to end with torch.cuda stubbed and the emulated library (tests/cuda_emu/run_bench_emulated.py): the one JSON
     line carries every contract key and internally consistent counters: the north-star workload (configs[2], strong scaling), the
-    shared-memory gather of the grouped rows, the sustained run, the configs[1] secondary object.  The numbers themselves mean nothing."""
+    shared-memory gather of the grouped rows, the sustained run, the configs[1] secondary object, and --dump-outputs writes the
+    oracle's rows of the same seeded block.  The numbers themselves mean nothing."""
     import json
+    import numpy as np
+    import parity_helpers as hp
+    from find_tfbs_b200 import binding, synth
     r = subprocess.run([sys.executable, os.path.join(EMU, "run_bench_emulated.py"), "--scale", "0.0004", "--steps", "2", "--warmup", "1",
-                        "--cpu-seconds", "0.2", "--no-full-scan", "--sustain-seconds", "0.01", "--no-driver"], cwd=ROOT, env=emu_env,
-                       stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+                        "--cpu-seconds", "0.2", "--no-full-scan", "--sustain-seconds", "0.01", "--no-driver", "--dump-outputs", str(tmp_path)],
+                       cwd=ROOT, env=emu_env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
     assert r.returncode == 0, r.stderr[-3000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, lines
@@ -103,6 +107,17 @@ def test_bench_control_flow_dry_run(emu_env):
     assert d["e2e"]["gathered_on_rank0"]["rows_last_step"] == d["rows_per_step"]
     assert d["sustained"]["steps"] >= 2 and d["secondary"]["config"]["workload"].startswith("configs[1]")
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
+    dump = {f[:-len(".npy")]: np.load(str(tmp_path / f)) for f in os.listdir(str(tmp_path))}
+    assert all(a.dtype in (np.float32, np.float64) for a in dump.values())
+    assert sum(os.path.getsize(str(tmp_path / f)) for f in os.listdir(str(tmp_path))) <= 64 << 20
+    pats, blk = synth.config3(scale=0.0004, seed=3)
+    o = hp.run_oracle(binding.PatternSet(pats), blk)
+    assert len(o["region"]) == d["rows_per_step"] > 0 and np.array_equal(dump["rows"], np.arange(len(o["region"])))
+    for k in ("region", "inner", "pattern_id", "vmin", "vmax"):
+        assert np.array_equal(dump[k], o[k]), k
+    dense = dump["dense_rows"].astype(np.int64)
+    assert np.array_equal(dump["left"], o["left"][dense]) and np.array_equal(dump["right"], o["right"][dense])
+    assert len(dump["n_groups"]) == blk.n_regions and dump["n_groups"].min() >= 1
 
 
 def test_bench_reference_arm():
