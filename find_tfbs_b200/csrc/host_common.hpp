@@ -148,6 +148,7 @@ struct tfbs_ctx {
     int audit = 0;              // set by tfbs_audit_block: per-haplotype flags are kept
     int64_t tiny_caps = 0;      // testing: start the configuration path with minimal scratch so that every growth path runs
     int64_t test_reseed = 0;    // testing: the first attempt of every block is treated as a hash collision (repeated with another seed)
+    int fan_vector = 0;         // 0: the fan-out's count vectors live in shared memory unless a region has too many groups; 1: always in device memory (testing)
 
     // patterns
     bool have_patterns = false;
@@ -181,6 +182,7 @@ struct tfbs_ctx {
     DevBuf d_vq_region, d_vq_leader, d_vq_nd, d_vq_doff, d_vq_dlist, d_vq_segs, d_vq_nseg, d_vq_len, d_vq_flags, d_vq_ntake, d_vq_nitems,
         d_vq_item_off;
     DevBuf d_vmin, d_vmax, d_flag, d_rowwords, d_kbits, d_rowidx, d_rowoff;
+    DevBuf d_fan_vec;  // k_fanout<true>: one count vector per CTA
     // full-scan path
     std::vector<uint32_t> h_ngroups, h_sum_nd;
     std::vector<uint64_t> h_gbase, h_cbase, h_kbase;

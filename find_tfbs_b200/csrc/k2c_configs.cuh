@@ -26,7 +26,7 @@ struct DevPlan {
     u64 unused;
     u64 rowwords_alloc;  // packed row words handed out by the fan-out (an atomic cursor)
     u64 fan_keys;        // keys the fan-out built a count vector for
-    u64 fan_dbg[4];      // -DTFBS_FAN_STATS: pairs, member updates, groups with a non-zero difference, samples with one
+    u64 fan_dbg[5];      // -DTFBS_FAN_STATS: pairs, member updates, groups with a non-zero difference, samples with one, keys of the dense pass
 };
 
 // A count becomes known: total (+ add) against the capacity its consumers were launched for.  Behind an earlier overflow nothing

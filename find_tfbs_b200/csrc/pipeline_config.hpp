@@ -51,9 +51,13 @@ struct ConfigPipeline {
     DevPlan* plan = nullptr;
     DevBlock db{};
     uint64_t ref_items = 0;  // work-list items of the reference haplotypes (pieces of REF_PIECE window starts)
+    // groups a count vector of k_fanout<false> holds in dynamic shared memory next to the pairs and the staging buffer: the device's
+    // per-block limit less the kernel's static shared memory, at most 220 KB (53,120 groups on sm_100: 227 KB - 7.5 KB - 12 KB)
+    const uint32_t smem_groups;
 
     ConfigPipeline(tfbs_ctx* c, Slot* s)
-        : ctx(c), slot(s), B(*s->in), st(c->stream), R(s->in->R), S(s->in->S), H(s->in->H), RH((uint64_t)s->in->R * s->in->H) {}
+        : ctx(c), slot(s), B(*s->in), st(c->stream), R(s->in->R), S(s->in->S), H(s->in->H), RH((uint64_t)s->in->R * s->in->H),
+          smem_groups((uint32_t)((std::min<size_t>(c->prop.sharedMemPerBlockOptin - FAN_STATIC_SMEM, 220 * 1024) - fan_smem_bytes(0, s->in->H, false)) / 4)) {}
 
     uint32_t& launches() { return slot->stats.total_launches; }
     int scan(const uint32_t* d_in, uint64_t n_cap, const u64* n_ptr, u64* d_out) { return device_scan(ctx, d_in, n_cap, n_ptr, d_out, &launches()); }
@@ -65,6 +69,12 @@ struct ConfigPipeline {
 
     // ---- capacities ------------------------------------------------------------------------------------------------
     static uint64_t up(uint64_t need) { return need + need / 4 + 16; }
+    // count vector for `need` groups: with the usual slack, but a need that fits shared memory is not pushed out of it by the slack
+    uint32_t groups_for(uint64_t need) const {
+        uint64_t cap = std::min<uint64_t>((uint64_t)H + 1, up(need));
+        if (need <= smem_groups) cap = std::min<uint64_t>(cap, smem_groups);
+        return (uint32_t)cap;
+    }
     void choose_caps(bool first_attempt) {
         Caps& c = slot->caps;
         const Caps& h = ctx->hint;
@@ -97,7 +107,7 @@ struct ConfigPipeline {
         c.rows = std::min<uint64_t>(std::max<uint64_t>(1, n_keys), pick(h.rows, std::max<uint64_t>(4096, n_keys / 4)));
         c.rowwords = pick(h.rowwords, c.rows * ((uint64_t)(H + 1) / 32 + 1));
         c.capr = ctx->refhit_cap_opt ? (uint32_t)std::max<int64_t>(1, ctx->refhit_cap_opt / std::max<uint32_t>(1, R)) : (uint32_t)pick(h.capr, 512);
-        c.groups = (uint32_t)std::min<uint64_t>((uint64_t)H + 1, pick(h.groups, 2048));
+        c.groups = h.groups ? groups_for(h.groups) : (uint32_t)std::min<uint64_t>((uint64_t)H + 1, 2048);
     }
     uint64_t scratch_bytes_needed() const {
         const Caps& c = slot->caps;
@@ -106,8 +116,22 @@ struct ConfigPipeline {
         while (seg < 2 * ((uint64_t)H + 1)) seg <<= 1;
         tbl = std::max<uint64_t>(tbl, (uint64_t)R * seg);
         return RH * 20 + tbl * 12 + c.seq * 50 + c.d * (4 + 32 + 20 + 4) + c.seq * 32 + c.cfg * 32 + (R + c.cfg) * 60 + c.vd * 36 + c.items * 28 +
-               c.units * 12 + c.dwords * 4 + n_keys * 36 + (uint64_t)c.capr * R * sizeof(RefHit) + c.rows * 34 + c.rowwords * 4;
+               c.units * 12 + c.dwords * 4 + n_keys * 36 + (uint64_t)c.capr * R * sizeof(RefHit) + c.rows * 34 + c.rowwords * 4 + fan_vec_bytes();
     }
+
+    // ---- fan-out: the count vectors in shared memory (k_fanout<false>, one CTA per unit) or in device memory (k_fanout<true>) ----
+    // Device memory when a region may have more groups than shared memory holds, or when option fan_vector asks for it (testing).
+    bool fan_vec() const { return ctx->fan_vector == 1 || slot->caps.groups > smem_groups; }
+    // CTAs per region: FAN_SPLIT when there are many regions, more when few regions would leave SMs idle (sample blocks of a biobank
+    // cohort: few regions, tens of thousands of groups each)
+    uint32_t fan_split() const {
+        return (uint32_t)std::min<uint64_t>(32, std::max<uint64_t>(FAN_SPLIT, (8ull * ctx->prop.multiProcessorCount + R - 1) / std::max<uint32_t>(1, R)));
+    }
+    uint32_t fan_vec_grid() const {
+        return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)ctx->prop.multiProcessorCount * FAN_VEC_CTAS_PER_SM, (uint64_t)R * fan_split()));
+    }
+    uint64_t fan_vec_stride() const { return ((uint64_t)slot->caps.groups + 31) & ~31ull; }  // words of a CTA's slice, 128-byte aligned
+    uint64_t fan_vec_bytes() const { return (n_keys && fan_vec()) ? (uint64_t)fan_vec_grid() * fan_vec_stride() * 4 : 0; }
 
     // ---- scratch -------------------------------------------------------------------------------------------------------
     int reserve() {
@@ -200,6 +224,7 @@ struct ConfigPipeline {
         RS(slot->d_o_bits, c.rows);
         RS(slot->d_o_off, c.rows * 8);
         RS(slot->d_o_packed, c.rowwords * 4);
+        if (fan_vec_bytes()) RS(ctx->d_fan_vec, fan_vec_bytes());
 #undef RS
         CK(slot->h_status.reserve(sizeof(DevStatus), false));
         CK(slot->h_plan.reserve(sizeof(DevPlan), false));
@@ -250,11 +275,16 @@ struct ConfigPipeline {
         slot->res.have_dense = slot->res.have_grouped = false;
         choose_caps(first_attempt);
         const Caps& c = slot->caps;
+        if (fan_vec_bytes() > ctx->scratch_bytes)
+            return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "the fan-out's count vectors for " + std::to_string(c.groups) + " distinct haplotypes per region need about " +
+                                                            std::to_string(fan_vec_bytes() >> 20) + " MB of device scratch, option scratch_mb allows " +
+                                                            std::to_string(ctx->scratch_bytes >> 20));
         if (scratch_bytes_needed() > ctx->scratch_bytes)
             return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "the block needs about " + std::to_string(scratch_bytes_needed() >> 20) +
                                                             " MB of device scratch, option scratch_mb allows " + std::to_string(ctx->scratch_bytes >> 20) +
                                                             ": submit fewer regions per block");
-        if (c.seq > 0x7fffffffull || c.d > 0xfffffff0ull || R + c.cfg > 0x7fffffffull || c.items > 0xfffffff0ull)
+        if (c.seq > 0x7fffffffull || c.d > 0xfffffff0ull || R + c.cfg > 0x7fffffffull || c.items > 0xfffffff0ull ||
+            (fan_vec() && (uint64_t)R * fan_split() > 0xffffffffull))
             return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "block too large for 32-bit work-list indices: submit fewer regions per block");
         if ((rc = reserve())) return rc;
         dst = slot->d_status.as<DevStatus>();
@@ -510,19 +540,26 @@ struct ConfigPipeline {
             fn.o_packed = slot->d_o_packed.as<u32>();
             fn.pid_list = ctx->d_pid_list.as<u16>();
             fn.max_count = &dst->max_count;
-            // one count vector per CTA in shared memory, next to the pairs of a round, the staged rows and (when it fits) the haplotype -> group map
-            const size_t max_smem = std::min<size_t>(ctx->prop.sharedMemPerBlockOptin, 220 * 1024);
-            fn.hg16 = ((uint64_t)H + 1 <= 65536 && fan_smem_bytes(c.groups, H, true) <= 64 * 1024) ? 1u : 0u;
-            const size_t fan_smem = fan_smem_bytes(c.groups, H, fn.hg16 != 0);
-            if (fan_smem > max_smem)
-                return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "a region has more distinct haplotypes than the fan-out kernel holds in shared memory (" +
-                                                                std::to_string(c.groups) + "): use sample blocks");
-            CK(cudaFuncSetAttribute(k_fanout, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fan_smem));
-            CK(cudaFuncSetAttribute(k_fanout, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-            // CTAs per region: FAN_SPLIT when there are many regions, more when few regions would leave SMs idle (sample blocks of a
-            // biobank cohort: few regions, tens of thousands of groups each)
-            const uint32_t split = (uint32_t)std::min<uint64_t>(32, std::max<uint64_t>(FAN_SPLIT, (8ull * slot->stats.sm_count + R - 1) / R));
-            TFBS_LAUNCH(k_fanout, dim3(R, split), FAN_THREADS, fan_smem, st)(db, cf, fn);
+            // shared memory: the pairs of a round, the staged rows, (when it fits) the haplotype -> group map and, unless the count
+            // vectors are in device memory, one count vector per CTA (c.groups <= smem_groups there)
+            const bool vec = fan_vec();
+            const uint32_t smem_vec_groups = vec ? 0u : c.groups;
+            fn.hg16 = ((uint64_t)H + 1 <= 65536 && fan_smem_bytes(smem_vec_groups, H, true) <= 64 * 1024) ? 1u : 0u;
+            const size_t fan_smem = fan_smem_bytes(smem_vec_groups, H, fn.hg16 != 0);
+            const uint32_t split = fan_split();
+            if (vec) {
+                fn.vec = ctx->d_fan_vec.as<u32>();
+                fn.vec_stride = fan_vec_stride();
+                fn.split = split;
+                // the kernel leaves every slice all zero, a fresh or regrown allocation is not: zeroed on every run, repeats included
+                CK(cudaMemsetAsync(ctx->d_fan_vec.p, 0, fan_vec_bytes(), st));
+                CK(cudaFuncSetAttribute(k_fanout<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fan_smem));
+                TFBS_LAUNCH(k_fanout<true>, fan_vec_grid(), FAN_THREADS, fan_smem, st)(db, cf, fn);
+            } else {
+                CK(cudaFuncSetAttribute(k_fanout<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fan_smem));
+                CK(cudaFuncSetAttribute(k_fanout<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+                TFBS_LAUNCH(k_fanout<false>, dim3(R, split), FAN_THREADS, fan_smem, st)(db, cf, fn);
+            }
             ++launches();
             if ((rc = scan(fn.flag, n_keys, nullptr, ctx->d_rowidx.as<u64>()))) return rc;
             gate(ctx->d_rowidx.as<u64>() + n_keys, 0, c.rows, &plan->n_rows, &plan->need_rows);
@@ -605,7 +642,7 @@ struct ConfigPipeline {
         g(c.rows, hp.need_rows);
         g(c.rowwords, hp.need_rowwords);
         if (hp.need_capr > c.capr) c.capr = (uint32_t)up(hp.need_capr);
-        if (hp.need_groups > c.groups) c.groups = (uint32_t)std::min<uint64_t>((uint64_t)H + 1, up(hp.need_groups));
+        if (hp.need_groups > c.groups) c.groups = groups_for(hp.need_groups);
     }
     void note_needs(const DevPlan& hp) {
         Caps& h = ctx->hint;
@@ -645,9 +682,9 @@ struct ConfigPipeline {
         s.n_truncated = hs.n_truncated;
         s.reserved = (uint32_t)std::min<uint64_t>(hp.fan_keys, 0xffffffffu);
         if (getenv("TFBS_DEBUG") && hp.fan_dbg[0])
-            fprintf(stderr, "tfbs: fan-out: %llu keys with a count vector, %llu pairs, %llu member updates, %llu groups / %llu samples with a non-zero difference\n",
+            fprintf(stderr, "tfbs: fan-out: %llu keys with a count vector, %llu pairs, %llu member updates, %llu groups / %llu samples with a non-zero difference, %llu keys in the dense pass\n",
                     (unsigned long long)hp.fan_keys, (unsigned long long)hp.fan_dbg[0], (unsigned long long)hp.fan_dbg[1], (unsigned long long)hp.fan_dbg[2],
-                    (unsigned long long)hp.fan_dbg[3]);
+                    (unsigned long long)hp.fan_dbg[3], (unsigned long long)hp.fan_dbg[4]);
         uint64_t table_bytes = 0;
         for (const ChunkDesc& cd : ctx->cp.chunks) table_bytes += (uint64_t)cd.tbl_words * 8 * s.scan_ctas;
         s.scan_input_bytes = (R && S) ? hp.n_units * 12 * ctx->cp.chunks.size() + table_bytes : 0;

@@ -243,6 +243,10 @@ int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value) {
     else if (k == "refhit_cap") ctx->refhit_cap_opt = std::max<int64_t>(0, value);
     else if (k == "tiny_caps") ctx->tiny_caps = value;
     else if (k == "test_reseed") ctx->test_reseed = value;
+    else if (k == "fan_vector") {
+        if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "fan_vector must be 0 (automatic) or 1 (device memory)");
+        ctx->fan_vector = (int)value;
+    }
     else if (k == "rows_width") {
         if (value != 0 && value != 32) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "rows_width must be 32 or 0 (automatic)");
         ctx->rows_width = (int)value;

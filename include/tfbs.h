@@ -272,7 +272,10 @@ const char* tfbs_last_error(const tfbs_ctx* ctx);
  * every distinct haplotype in full like the reference does; forced to 0 while "record_matches" is on), "scratch_mb" (upper bound of
  * the device scratch a block may use; a block that needs more fails with TFBS_ERR_INVALID_ARGUMENT: submit fewer regions at a time),
  * "table_budget_kb", "rows_width" (32 = counts come back as uint32_t, the reference's Vec<u32>; 0 = the narrowest of 8/16/32 bits
- * that holds every count of the block, see tfbs_rows.count_bytes -- result rows are the dominant PCIe traffic of large cohorts). */
+ * that holds every count of the block, see tfbs_rows.count_bytes -- result rows are the dominant PCIe traffic of large cohorts),
+ * "fan_vector" (0 = automatic, the default: the fan-out keeps its per-group count vectors in shared memory and switches to device
+ * memory when a region of the block may have more distinct haplotypes than shared memory holds, 53,120; 1 = always in device
+ * memory, for tests -- results are the same either way). */
 int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value);
 
 /* Replace the pattern list (the reference's pwm_list, src/main.rs:237). */
