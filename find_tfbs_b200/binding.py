@@ -23,7 +23,7 @@ DIR_P, DIR_N = 0, 1
 EXPORTS = ["tfbs_abi_version", "tfbs_create", "tfbs_destroy", "tfbs_last_error", "tfbs_set_option", "tfbs_set_patterns",
            "tfbs_submit_block", "tfbs_collect", "tfbs_get_matches", "tfbs_upload_block", "tfbs_run_resident", "tfbs_get_stats",
            "tfbs_stream", "tfbs_host_register", "tfbs_host_unregister", "tfbs_audit_block", "tfbs_collect_grouped", "tfbs_expand_rows", "tfbs_set_result_arena",
-           "tfbs_merge_sample_blocks", "tfbs_merge_regions"]
+           "tfbs_merge_sample_blocks", "tfbs_merge_regions", "tfbs_fanout_info"]
 
 
 class TfbsPattern(C.Structure):
@@ -249,6 +249,7 @@ def lib():
                                          C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.tfbs_get_matches.argtypes = [C.c_void_p, C.POINTER(TfbsMatches)]
         L.tfbs_get_stats.argtypes = [C.c_void_p, C.POINTER(TfbsStats)]
+        L.tfbs_fanout_info.argtypes = [C.c_void_p] + [C.POINTER(C.c_uint32)] * 4
         L.tfbs_audit_block.argtypes = [C.c_void_p, C.POINTER(TfbsAudit)]
         L.tfbs_stream.argtypes = [C.c_void_p]
         L.tfbs_stream.restype = C.c_void_p
@@ -530,6 +531,13 @@ class Context:
         s = TfbsStats()
         self._check(self._lib.tfbs_get_stats(self._h, C.byref(s)))
         return {f: getattr(s, f) for f, _ in TfbsStats._fields_}
+
+    def fanout_info(self):
+        """tfbs_fanout_info: the groups a shared-memory count vector holds on this device; for the most recent run, the capacity of
+        the count vectors, the CTAs of the fan-out launch and whether the vectors were in device memory."""
+        v = [C.c_uint32(0) for _ in range(4)]
+        self._check(self._lib.tfbs_fanout_info(self._h, *[C.byref(x) for x in v]))
+        return {"smem_groups": v[0].value, "groups_cap": v[1].value, "ctas": v[2].value, "in_device_memory": bool(v[3].value)}
 
     def stream(self):
         return self._lib.tfbs_stream(self._h)

@@ -121,6 +121,7 @@ struct Slot {
     int attempts = 0;
     cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_t[8]{};
     tfbs_stats stats{};
+    uint32_t fan_groups_cap = 0, fan_ctas = 0, fan_in_device_memory = 0;  // the fan-out of the last run (tfbs_fanout_info)
 };
 
 }  // namespace

@@ -38,6 +38,12 @@ int patch_panic(tfbs_ctx* ctx, uint64_t err_key, uint32_t r, int64_t region_star
     return fail(ctx, TFBS_ERR_MISSING_CASE, "Missing case in haplotype patcher (ref_position=" + std::to_string(pos) + " region=" + std::to_string(r) + ")");
 }
 
+// groups a count vector of k_fanout<false> holds in dynamic shared memory next to the pairs and the staging buffer: the device's
+// per-block limit less the kernel's static shared memory, at most 220 KB (53,120 groups on sm_100: 227 KB - 7.5 KB - 12 KB)
+uint32_t fan_smem_groups(const cudaDeviceProp& prop) {
+    return (uint32_t)((std::min<size_t>(prop.sharedMemPerBlockOptin - FAN_STATIC_SMEM, 220 * 1024) - fan_smem_bytes(0, 0, false)) / 4);
+}
+
 struct ConfigPipeline {
     tfbs_ctx* ctx;
     Slot* slot;
@@ -51,13 +57,11 @@ struct ConfigPipeline {
     DevPlan* plan = nullptr;
     DevBlock db{};
     uint64_t ref_items = 0;  // work-list items of the reference haplotypes (pieces of REF_PIECE window starts)
-    // groups a count vector of k_fanout<false> holds in dynamic shared memory next to the pairs and the staging buffer: the device's
-    // per-block limit less the kernel's static shared memory, at most 220 KB (53,120 groups on sm_100: 227 KB - 7.5 KB - 12 KB)
-    const uint32_t smem_groups;
+    const uint32_t smem_groups;  // fan_smem_groups()
 
     ConfigPipeline(tfbs_ctx* c, Slot* s)
         : ctx(c), slot(s), B(*s->in), st(c->stream), R(s->in->R), S(s->in->S), H(s->in->H), RH((uint64_t)s->in->R * s->in->H),
-          smem_groups((uint32_t)((std::min<size_t>(c->prop.sharedMemPerBlockOptin - FAN_STATIC_SMEM, 220 * 1024) - fan_smem_bytes(0, s->in->H, false)) / 4)) {}
+          smem_groups(fan_smem_groups(c->prop)) {}
 
     uint32_t& launches() { return slot->stats.total_launches; }
     int scan(const uint32_t* d_in, uint64_t n_cap, const u64* n_ptr, u64* d_out) { return device_scan(ctx, d_in, n_cap, n_ptr, d_out, &launches()); }
@@ -275,6 +279,10 @@ struct ConfigPipeline {
         slot->res.have_dense = slot->res.have_grouped = false;
         choose_caps(first_attempt);
         const Caps& c = slot->caps;
+        const bool fans = n_keys && R && S;
+        slot->fan_groups_cap = fans ? c.groups : 0;
+        slot->fan_ctas = fans ? (fan_vec() ? fan_vec_grid() : (uint32_t)std::min<uint64_t>(0xffffffffu, (uint64_t)R * fan_split())) : 0;
+        slot->fan_in_device_memory = (fans && fan_vec()) ? 1 : 0;
         if (fan_vec_bytes() > ctx->scratch_bytes)
             return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "the fan-out's count vectors for " + std::to_string(c.groups) + " distinct haplotypes per region need about " +
                                                             std::to_string(fan_vec_bytes() >> 20) + " MB of device scratch, option scratch_mb allows " +

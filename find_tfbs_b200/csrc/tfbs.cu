@@ -691,6 +691,18 @@ int tfbs_get_stats(const tfbs_ctx* ctx, tfbs_stats* out) {
     return TFBS_OK;
 }
 
+int tfbs_fanout_info(const tfbs_ctx* ctx, uint32_t* smem_groups, uint32_t* groups_cap, uint32_t* ctas, uint32_t* in_device_memory) {
+    if (!ctx || !smem_groups || !groups_cap || !ctas || !in_device_memory) return TFBS_ERR_INVALID_ARGUMENT;
+    if (ctx->twin && ctx->last_target == 1) return tfbs_fanout_info(ctx->twin, smem_groups, groups_cap, ctas, in_device_memory);
+    *smem_groups = fan_smem_groups(ctx->prop);
+    const Slot* s = ctx->last < 0 ? nullptr : &ctx->slot[ctx->last];
+    const bool ran = s && !s->full_mode;
+    *groups_cap = ran ? s->fan_groups_cap : 0;
+    *ctas = ran ? s->fan_ctas : 0;
+    *in_device_memory = ran ? s->fan_in_device_memory : 0;
+    return TFBS_OK;
+}
+
 int tfbs_host_register(void* ptr, size_t bytes) {
     if (!ptr || !bytes) return TFBS_OK;
     return cudaHostRegister(ptr, bytes, cudaHostRegisterDefault) == cudaSuccess ? TFBS_OK : TFBS_ERR_CUDA;

@@ -170,7 +170,8 @@ typedef struct tfbs_grouped_rows {
     uint64_t packed_words;
     const uint32_t* n_groups;      /* [n_regions] distinct haplotypes of the region incl. the reference haplotype (group 0) */
     const void* hap_group;         /* [n_regions * 2 * n_samples] group of haplotype h = 2 * sample + side in its region, as uint16_t
-                                      or uint32_t (hap_group_bytes); 0 = the reference haplotype (main.rs:103-105,129-131) */
+                                      or uint32_t (hap_group_bytes); 0 = the reference haplotype (main.rs:103-105,129-131), the
+                                      other groups numbered 1.. in order of their smallest haplotype */
     uint32_t hap_group_bytes;      /* 2 or 4 */
     uint32_t reserved;
 } tfbs_grouped_rows;
@@ -365,6 +366,15 @@ int tfbs_upload_block(tfbs_ctx* ctx, const tfbs_block* block);
 int tfbs_run_resident(tfbs_ctx* ctx);
 
 int tfbs_get_stats(const tfbs_ctx* ctx, tfbs_stats* out);
+
+/* Where the fan-out keeps its per-group count vectors (option "fan_vector").  *smem_groups: how many groups (distinct haplotypes of
+ * a region, the reference haplotype included) a count vector in shared memory holds on this context's device; a block whose count
+ * vector needs more capacity runs the fan-out with its vectors in device memory.  For the most recent run of the default path
+ * (zeros before the first one, after a full scan, and for a block without keys): *groups_cap = the capacity of its count vector,
+ * *ctas = the CTAs of the fan-out launch (in device memory: a fixed grid whose CTAs each own one count vector and walk the
+ * region's units in turn, so a block with more regions than CTAs reuses every vector), *in_device_memory = 1 when the vectors were
+ * in device memory, 0 when in shared memory. */
+int tfbs_fanout_info(const tfbs_ctx* ctx, uint32_t* smem_groups, uint32_t* groups_cap, uint32_t* ctas, uint32_t* in_device_memory);
 
 /* Page-lock / unlock caller buffers (cudaHostRegister) so that tfbs_submit_block copies them at full PCIe speed.
  * Optional: pageable buffers work, only slower. */
