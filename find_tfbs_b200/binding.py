@@ -23,7 +23,7 @@ DIR_P, DIR_N = 0, 1
 EXPORTS = ["tfbs_abi_version", "tfbs_create", "tfbs_destroy", "tfbs_last_error", "tfbs_set_option", "tfbs_set_patterns",
            "tfbs_submit_block", "tfbs_collect", "tfbs_get_matches", "tfbs_upload_block", "tfbs_run_resident", "tfbs_get_stats",
            "tfbs_stream", "tfbs_host_register", "tfbs_host_unregister", "tfbs_audit_block", "tfbs_collect_grouped", "tfbs_expand_rows", "tfbs_set_result_arena",
-           "tfbs_merge_sample_blocks", "tfbs_merge_regions", "tfbs_fanout_info"]
+           "tfbs_merge_sample_blocks", "tfbs_merge_regions", "tfbs_fanout_info", "tfbs_get_attribution"]
 
 
 class TfbsPattern(C.Structure):
@@ -191,6 +191,17 @@ class TfbsAudit(C.Structure):
 HAP_TRUNCATED, HAP_OVERWRITTEN = 1, 2
 
 
+class TfbsAttribution(C.Structure):
+    _fields_ = [("n_rows", C.c_uint64), ("ref_count", C.POINTER(C.c_uint32)), ("term_off", C.POINTER(C.c_uint64)),
+                ("term_cfg", C.POINTER(C.c_uint32)), ("term_diff", C.POINTER(C.c_int32)), ("n_cfgs", C.c_uint64),
+                ("cfg_region", C.POINTER(C.c_uint32)), ("cfg_flags", C.POINTER(C.c_uint8)), ("cfg_rec_off", C.POINTER(C.c_uint64)),
+                ("cfg_rec", C.POINTER(C.c_uint32)), ("n_groups_total", C.c_uint64), ("group_cfg_off", C.POINTER(C.c_uint64)),
+                ("group_cfg", C.POINTER(C.c_uint32))]
+
+
+CFG_TRUNCATES = 1
+
+
 class TfbsStats(C.Structure):
     _fields_ = [("n_regions", C.c_uint64), ("n_groups", C.c_uint64), ("executed_cells", C.c_uint64), ("nominal_cells", C.c_uint64),
                 ("n_hits", C.c_uint64), ("n_keys", C.c_uint64), ("n_rows", C.c_uint64), ("h2d_bytes", C.c_uint64),
@@ -251,6 +262,7 @@ def lib():
         L.tfbs_get_stats.argtypes = [C.c_void_p, C.POINTER(TfbsStats)]
         L.tfbs_fanout_info.argtypes = [C.c_void_p] + [C.POINTER(C.c_uint32)] * 4
         L.tfbs_audit_block.argtypes = [C.c_void_p, C.POINTER(TfbsAudit)]
+        L.tfbs_get_attribution.argtypes = [C.c_void_p, C.POINTER(TfbsAttribution)]
         L.tfbs_stream.argtypes = [C.c_void_p]
         L.tfbs_stream.restype = C.c_void_p
         L.tfbs_host_register.argtypes = [C.c_void_p, C.c_size_t]
@@ -526,6 +538,28 @@ class Context:
                 "group": arr(a.tie_group, n, np.uint32), "start": arr(a.tie_start, n, np.int64),
                 "hap_group": arr(a.hap_group, nh, np.uint32), "hap_flags": arr(a.hap_flags, nh, np.uint8),
                 "truncated": bool(a.truncated)}
+
+    def attribution(self):
+        """tfbs_get_attribution: for the block the last collect returned, per row the reference haplotype's count and the non-zero
+        count differences of the configurations (term_off / term_cfg / term_diff), per configuration its region, flags and records
+        (indices into the block's variants), per group (block-wide numbering) the configurations its count includes.  NumPy copies."""
+        a = TfbsAttribution()
+        self._check(self._lib.tfbs_get_attribution(self._h, C.byref(a)))
+        n, nc, ng = a.n_rows, a.n_cfgs, a.n_groups_total
+
+        def arr(p, cnt, dt):
+            if cnt == 0:
+                return np.zeros(0, dtype=dt)
+            return np.ctypeslib.as_array(p, shape=(cnt,)).astype(dt, copy=True)
+
+        term_off = arr(a.term_off, n + 1, np.uint64)
+        cfg_rec_off = arr(a.cfg_rec_off, nc + 1, np.uint64)
+        group_cfg_off = arr(a.group_cfg_off, ng + 1, np.uint64)
+        nt, nr, nl = int(term_off[-1]), int(cfg_rec_off[-1]), int(group_cfg_off[-1])
+        return {"n_rows": n, "ref_count": arr(a.ref_count, n, np.uint32), "term_off": term_off, "term_cfg": arr(a.term_cfg, nt, np.uint32),
+                "term_diff": arr(a.term_diff, nt, np.int32), "n_cfgs": nc, "cfg_region": arr(a.cfg_region, nc, np.uint32),
+                "cfg_flags": arr(a.cfg_flags, nc, np.uint8), "cfg_rec_off": cfg_rec_off, "cfg_rec": arr(a.cfg_rec, nr, np.uint32),
+                "n_groups_total": ng, "group_cfg_off": group_cfg_off, "group_cfg": arr(a.group_cfg, nl, np.uint32)}
 
     def stats(self):
         s = TfbsStats()

@@ -104,6 +104,7 @@ int main(int argc, char** argv) {
             if (tfbs_create(o.devices[k], &ctx) != TFBS_OK) die(std::string(tfbs_last_error(nullptr)));
             TF(tfbs_set_patterns(ctx, cpat.data(), (uint32_t)cpat.size()));
             TF(tfbs_set_option(ctx, "rows_width", 0));
+            if (!o.attribution_file.empty()) TF(tfbs_set_option(ctx, "attribution", 1));
             ctxs[k] = ctx;
             us_create += now_us() - tc;
         });
@@ -155,11 +156,22 @@ int main(int argc, char** argv) {
     // The writer (main.rs:264-290 has a writer thread fed through a channel): chunks finish in any order on the devices and are
     // written in chunk order as soon as every earlier chunk is there; a finished chunk's text is freed once written, so the
     // memory in flight is a few chunks, not the chromosome.  POS is the reference's running counter (main.rs:329,424-425).
-    struct ChunkText { std::vector<std::string> rows; };
+    struct ChunkText { std::vector<std::string> rows; std::string attribution; };
     std::mutex out_mu;
     std::condition_variable out_cv;
     std::map<size_t, ChunkText> done_chunks;
     std::vector<std::string> audit_text(o.audit_file.empty() ? 0 : n_chunks);
+    // --attribution: per written row (after --min_maf), in the VCF's order, the configurations -- records of one cluster of nearby
+    // records that haplotypes carry together -- whose count difference to the reference haplotype is not 0.  A haplotype counts
+    // REF_COUNT plus the DIFF of every line whose configuration it carries; HAPLOTYPES = how many selected haplotypes carry it.
+    // TRUNCATES = 1: the configuration runs into patch_haplotype's truncation exit (haplotype.rs:144-149), DIFF includes the hits lost
+    // behind it.  The writer thread appends a chunk's lines with its rows, so they are held for a few chunks at a time.
+    std::ofstream attribution_out;
+    if (!o.attribution_file.empty()) {
+        attribution_out.open(o.attribution_file, std::ios::binary);
+        if (!attribution_out) die("Could not create attribution file");
+        attribution_out << "#ID\tREF_COUNT\tRECORDS\tDIFF\tHAPLOTYPES\tTRUNCATES\n";
+    }
     size_t next_to_write = 0;
     uint64_t fake_position = 1;
     double secs_write = 0;
@@ -209,6 +221,7 @@ int main(int argc, char** argv) {
                 if (gz) gz->write_blocks(pc);
                 else plain << pc;
             }
+            if (attribution_out.is_open()) attribution_out << t.attribution;
             secs_write += std::chrono::duration<double>(std::chrono::steady_clock::now() - tw).count();
             {
                 std::lock_guard<std::mutex> lk(out_mu);
@@ -265,9 +278,12 @@ int main(int argc, char** argv) {
             return true;
         };
         // rows of one block -> text, in the canonical order inside a region: (bed file, inner range, pattern_id); the reference's
-        // order is HashMap::drain().  `counts(i, l, r)` fills the (left, right) vectors of row i.
+        // order is HashMap::drain().  `counts(i, l, r)` fills the (left, right) vectors of row i; `attribution(i, id, text)`, when
+        // given, appends the --attribution lines of a written row i with VCF ID `id`.
+        using AttributionLines = std::function<void(uint64_t, const std::string&, std::string&)>;
         auto rows_to_text = [&](size_t c, const BlockData& bd, uint64_t n_rows, const uint32_t* region, const uint32_t* inner, const uint16_t* pid,
-                                const uint32_t* vmin, const uint32_t* vmax, const std::function<void(uint64_t, uint32_t*, uint32_t*)>& counts) {
+                                const uint32_t* vmin, const uint32_t* vmax, const std::function<void(uint64_t, uint32_t*, uint32_t*)>& counts,
+                                const AttributionLines& attribution = nullptr) {
             uint64_t ts = now_us();
             std::vector<uint64_t> order(n_rows);
             for (uint64_t i = 0; i < n_rows; ++i) order[i] = i;
@@ -283,7 +299,7 @@ int main(int argc, char** argv) {
             us_sort += now_us() - ts;
             uint64_t tf = now_us();
             // row text on --threads host threads (the reference formats inside its worker threads, main.rs:415-425)
-            std::vector<std::string> text(order.size());
+            std::vector<std::string> text(order.size()), att(attribution ? order.size() : 0);
             auto format_range = [&](size_t a, size_t b) {
                 std::vector<uint32_t> l(S), r(S);
                 for (size_t k = a; k < b; ++k) {
@@ -292,9 +308,10 @@ int main(int argc, char** argv) {
                     RowText t = finalise_row(l.data(), r.data(), S, vmin[i], vmax[i], o.min_maf);
                     if (!t.keep) continue;
                     const tfbs_inner_region& ir = bd.inner[inner[i]];
+                    const std::string id = bed_names[ir.bed_index] + "," + pwm_name.at(pid[i]) + "," + std::to_string(ir.start) + "-" + std::to_string(ir.end);
                     // POS is filled in by the writer (a running counter, main.rs:329,424-425)
-                    text[k] = "\t" + bed_names[ir.bed_index] + "," + pwm_name.at(pid[i]) + "," + std::to_string(ir.start) + "-" +
-                              std::to_string(ir.end) + "\t.\t.\t.\tPASS\t" + t.info + "\tGT:DS" + t.genotypes + "\n";
+                    text[k] = "\t" + id + "\t.\t.\t.\tPASS\t" + t.info + "\tGT:DS" + t.genotypes + "\n";
+                    if (attribution) attribution(i, id, att[k]);
                 }
             };
             const size_t nt = std::max<size_t>(1, std::min<size_t>(o.threads, order.size() / 64 + 1));
@@ -307,6 +324,7 @@ int main(int argc, char** argv) {
             ChunkText ct;
             for (std::string& row : text)
                 if (!row.empty()) ct.rows.push_back(std::move(row));
+            for (const std::string& a : att) ct.attribution += a;
             us_format += now_us() - tf;
             chunk_finished(c, std::move(ct));
         };
@@ -341,7 +359,38 @@ int main(int argc, char** argv) {
                     g.n_groups = n_groups.data(); g.hap_group = hap_group.data();
                 }
             };
-            struct Collected { size_t c; std::unique_ptr<BlockData> bd; std::unique_ptr<OwnedRows> rows; };
+            // --attribution: the block's attribution, copied like the rows, and per configuration the haplotypes whose group lists it
+            struct OwnedAttribution {
+                std::vector<uint32_t> ref_count, term_cfg, cfg_rec;
+                std::vector<int32_t> term_diff;
+                std::vector<uint64_t> term_off, cfg_rec_off, haplotypes;
+                std::vector<uint8_t> cfg_flags;
+                OwnedAttribution(const tfbs_attribution& a, const tfbs_grouped_rows& g) {
+                    const uint64_t n = a.n_rows, nt = a.term_off[n], nc = a.n_cfgs;
+                    ref_count.assign(a.ref_count, a.ref_count + n);
+                    term_off.assign(a.term_off, a.term_off + n + 1);
+                    term_cfg.assign(a.term_cfg, a.term_cfg + nt);
+                    term_diff.assign(a.term_diff, a.term_diff + nt);
+                    cfg_flags.assign(a.cfg_flags, a.cfg_flags + nc);
+                    cfg_rec_off.assign(a.cfg_rec_off, a.cfg_rec_off + nc + 1);
+                    cfg_rec.assign(a.cfg_rec, a.cfg_rec + cfg_rec_off[nc]);
+                    // haplotypes per group (block-wide group index), then per configuration over the groups that list it
+                    const uint64_t H = 2ull * g.n_samples;
+                    std::vector<uint64_t> members(a.n_groups_total, 0);
+                    uint64_t gb = 0;
+                    for (uint32_t r = 0; r < g.n_regions && a.n_groups_total; ++r) {
+                        for (uint64_t h = 0; h < H; ++h) {
+                            const uint64_t x = r * H + h;
+                            ++members[gb + (g.hap_group_bytes == 2 ? ((const uint16_t*)g.hap_group)[x] : ((const uint32_t*)g.hap_group)[x])];
+                        }
+                        gb += g.n_groups[r];
+                    }
+                    haplotypes.assign(nc, 0);
+                    for (uint64_t G = 0; G < a.n_groups_total; ++G)
+                        for (uint64_t k = a.group_cfg_off[G]; k < a.group_cfg_off[G + 1]; ++k) haplotypes[a.group_cfg[k]] += members[G];
+                }
+            };
+            struct Collected { size_t c; std::unique_ptr<BlockData> bd; std::unique_ptr<OwnedRows> rows; std::unique_ptr<OwnedAttribution> att; };
             std::mutex fmu;
             std::condition_variable fcv;
             std::deque<Collected> to_format;
@@ -358,8 +407,25 @@ int main(int argc, char** argv) {
                         fcv.notify_all();
                     }
                     const tfbs_grouped_rows& g = it.rows->g;
-                    rows_to_text(it.c, *it.bd, g.n_rows, g.region, g.inner, g.pattern_id, g.vmin, g.vmax,
-                                 [&](uint64_t i, uint32_t* l, uint32_t* r) { tfbs_expand_rows(&g, i, 1, l, r); });
+                    const OwnedAttribution* at = it.att.get();
+                    const BlockData& bd = *it.bd;
+                    // ID, REF_COUNT, RECORDS (POS:REF:ALT, 1-based POS), DIFF, HAPLOTYPES, TRUNCATES: one line per term of the row
+                    auto lines = [&](uint64_t i, const std::string& id, std::string& out) {
+                        for (uint64_t t = at->term_off[i]; t < at->term_off[i + 1]; ++t) {
+                            const uint32_t cfg = at->term_cfg[t];
+                            std::string recs;
+                            for (uint64_t k = at->cfg_rec_off[cfg]; k < at->cfg_rec_off[cfg + 1]; ++k) {
+                                const tfbs_variant& v = bd.variants[at->cfg_rec[k]];
+                                if (!recs.empty()) recs += ';';
+                                recs += std::to_string(v.pos + 1) + ":" + std::string((const char*)bd.alleles.data() + v.ref_off, v.ref_len) + ":" +
+                                        std::string((const char*)bd.alleles.data() + v.alt_off, v.alt_len);
+                            }
+                            out += id + "\t" + std::to_string(at->ref_count[i]) + "\t" + recs + "\t" + std::to_string(at->term_diff[t]) + "\t" +
+                                   std::to_string(at->haplotypes[cfg]) + "\t" + ((at->cfg_flags[cfg] & TFBS_CFG_TRUNCATES) ? "1" : "0") + "\n";
+                        }
+                    };
+                    rows_to_text(it.c, bd, g.n_rows, g.region, g.inner, g.pattern_id, g.vmin, g.vmax,
+                                 [&](uint64_t i, uint32_t* l, uint32_t* r) { tfbs_expand_rows(&g, i, 1, l, r); }, at ? AttributionLines(lines) : nullptr);
                 }
             });
             // two blocks in flight per device: the copies and the host work of one overlap the kernels of the other
@@ -383,9 +449,15 @@ int main(int argc, char** argv) {
                 us_gpu += now_us() - tg;
                 note_stats(item.c);
                 std::unique_ptr<OwnedRows> own(new OwnedRows(g));
+                std::unique_ptr<OwnedAttribution> att;
+                if (!o.attribution_file.empty()) {
+                    tfbs_attribution a;
+                    TF(tfbs_get_attribution(ctx, &a));
+                    att.reset(new OwnedAttribution(a, g));
+                }
                 std::unique_lock<std::mutex> lk(fmu);
                 fcv.wait(lk, [&] { return to_format.size() < 2; });  // bounded: at most two collected blocks wait for their text
-                to_format.push_back(Collected{item.c, std::move(item.bd), std::move(own)});
+                to_format.push_back(Collected{item.c, std::move(item.bd), std::move(own), std::move(att)});
                 fcv.notify_all();
             }
             {
@@ -461,6 +533,10 @@ int main(int argc, char** argv) {
         if (!af) die("Could not create audit file");
         af << "#tie\tCHROM\tREGION\tPWM\tSTRAND\tSTART\tMIN_SCORE\tGROUP\tHAPLOTYPES\n#truncated|overwritten\tCHROM\tREGION\tHAPLOTYPE\n";
         for (const std::string& t : audit_text) af << t;
+    }
+    if (attribution_out.is_open()) {
+        attribution_out.close();
+        if (!attribution_out) die("Could not write attribution file");
     }
     if (rename(part.c_str(), o.output.c_str()) != 0) die("Could not rename " + part + " into " + o.output);
     if (o.tabix) {

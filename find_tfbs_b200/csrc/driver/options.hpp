@@ -11,6 +11,7 @@ namespace {
 struct Options {
     std::string chromosome, bcf, output, reference, pwm_file, threshold_dir, samples_file;
     std::string audit_file;  // --audit: threshold ties, truncated and overwritten haplotypes (tfbs_audit_block), tab-separated
+    std::string attribution_file;  // --attribution: per written row, the configurations of records that change its count (tfbs_get_attribution)
     std::vector<std::string> beds, pwm_names;
     float pwm_threshold = 0;
     bool forward_only = false, tabix = false, verbose = false, has_samples = false, plain_text = false;
@@ -41,6 +42,7 @@ void usage() {
          "         --pwm_names NAME[,NAME] --pwm_file PWM.txt --pwm_threshold_directory DIR --pwm_threshold P\n"
          "         [--forward_only] [--threads N] [--min_maf N] [--after_position POS] [--samples FILE] [--tabix] [--verbose]\n"
          "         [--devices 0,1,...] [--chunk REGIONS_PER_BLOCK] [--plain] [--audit AUDIT.tsv] [--no_index] [--compression_level 1..9]\n"
+         "         [--attribution ATTRIBUTION.tsv]\n"
          "       find-tfbs-b200 --write_thresholds DIR --pwm_file PWM.txt [--pwm_names NAME[,NAME]] [--pvalues P[,P]]   (exact .thr files)");
 }
 
@@ -117,6 +119,8 @@ Options parse_args(int argc, char** argv) {
     o.compression_level = (int)std::min<uint64_t>(9, std::max<uint64_t>(1, num("compression_level", 3, "Cannot parse compression_level")));
     if (kv.count("samples")) { o.has_samples = true; o.samples_file = kv["samples"]; }
     if (kv.count("audit")) o.audit_file = kv["audit"];
+    if (kv.count("attribution")) o.attribution_file = kv["attribution"];
+    if (!o.audit_file.empty() && !o.attribution_file.empty()) die("error: --attribution cannot be used with --audit");
     if (kv.count("devices")) {
         o.devices.clear();
         for (auto& d : split(kv["devices"], ',')) o.devices.push_back(atoi(d.c_str()));

@@ -96,12 +96,16 @@ struct Results {
     uint64_t packed_words = 0;
     uint32_t hg_bytes = 4;
     bool have_grouped = false;
+    // attribution (option "attribution", tfbs_get_attribution)
+    HostBuf h_a_ref, h_a_toff, h_a_tcfg, h_a_tdiff, h_a_creg, h_a_cflags, h_a_croff, h_a_crec, h_a_goff, h_a_gcfg;
+    bool have_attribution = false;
 };
 
 // Capacities a run of the configuration path was enqueued with (see DevPlan): sizes that only the device learns.
 struct Caps {
     uint64_t seq = 0, d = 0, cfg = 0, vd = 0, items = 0, units = 0, dwords = 0, rows = 0, rowwords = 0;
     uint32_t capr = 0, groups = 0;
+    uint64_t terms = 0;  // option "attribution": non-zero (row, configuration) differences
 };
 
 struct Slot {
@@ -112,6 +116,7 @@ struct Slot {
     // device results of the configuration path: they outlive the shared scratch, which the next block reuses at once
     DevBuf d_status, d_plan, d_hap_group, d_gbase, d_hg_narrow;
     DevBuf d_o_region, d_o_inner, d_o_pid, d_o_vmin, d_o_vmax, d_o_base, d_o_bits, d_o_off, d_o_packed, d_left, d_right;
+    DevBuf d_a_ref, d_a_toff, d_a_tcfg, d_a_tdiff, d_a_creg, d_a_cflags, d_a_croff, d_a_crec, d_a_goff, d_a_gcfg;  // attribution
     HostBuf h_status, h_plan;
     Results res;
     Caps caps;
@@ -122,6 +127,8 @@ struct Slot {
     cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_t[8]{};
     tfbs_stats stats{};
     uint32_t fan_groups_cap = 0, fan_ctas = 0, fan_in_device_memory = 0;  // the fan-out of the last run (tfbs_fanout_info)
+    bool attribution = false;                        // the run enqueued the attribution launches
+    uint64_t att_cfgs = 0, att_seqs = 0, att_terms = 0;  // their sizes (configurations, distinct haplotypes, terms)
 };
 
 }  // namespace
@@ -150,6 +157,11 @@ struct tfbs_ctx {
     int64_t tiny_caps = 0;      // testing: start the configuration path with minimal scratch so that every growth path runs
     int64_t test_reseed = 0;    // testing: the first attempt of every block is treated as a hash collision (repeated with another seed)
     int fan_vector = 0;         // 0: the fan-out's count vectors live in shared memory unless a region has too many groups; 1: always in device memory (testing)
+    int attribution = 0;        // 1: the default path keeps the per-row configuration differences (tfbs_get_attribution)
+    // attribution of the block the last tfbs_collect / tfbs_collect_grouped returned, copied to the host by that collect
+    enum { ATT_NONE = 0, ATT_OFF, ATT_FULL_SCAN, ATT_READY };
+    int att_state = ATT_NONE;
+    tfbs_attribution att{};
 
     // patterns
     bool have_patterns = false;
@@ -184,6 +196,7 @@ struct tfbs_ctx {
         d_vq_item_off;
     DevBuf d_vmin, d_vmax, d_flag, d_rowwords, d_kbits, d_rowidx, d_rowoff;
     DevBuf d_fan_vec;  // k_fanout<true>: one count vector per CTA
+    DevBuf d_att_eflag, d_att_cfgid, d_att_nrec, d_att_col, d_att_gn, d_att_tcnt;  // option "attribution"
     // full-scan path
     std::vector<uint32_t> h_ngroups, h_sum_nd;
     std::vector<uint64_t> h_gbase, h_cbase, h_kbase;

@@ -27,6 +27,7 @@ struct DevPlan {
     u64 rowwords_alloc;  // packed row words handed out by the fan-out (an atomic cursor)
     u64 fan_keys;        // keys the fan-out built a count vector for
     u64 fan_dbg[5];      // -DTFBS_FAN_STATS: pairs, member updates, groups with a non-zero difference, samples with one, keys of the dense pass
+    u64 n_terms, need_terms;  // option "attribution": non-zero (row, configuration) differences (k3_attribution.cuh)
 };
 
 // A count becomes known: total (+ add) against the capacity its consumers were launched for.  Behind an earlier overflow nothing

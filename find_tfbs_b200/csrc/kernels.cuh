@@ -11,6 +11,7 @@
 //   BED merge         k_bed_rank/merge      merged regions of all BED files          (bed.rs:37-45, range.rs:43-87)
 //   K3  count/rows    k_rows_*              count_matches_by_sample fan-out           (main.rs:506-531)
 //                                           + min/max filter of counts_as_genotypes   (main.rs:439-458)
+//       attribution   k_att_*               per row, the configurations that change its count (option "attribution")
 //
 // All arithmetic is integer; results are bit-exact by construction (scores are i32 sums, SURVEY D1).
 #pragma once
@@ -26,4 +27,5 @@
 #include "k2_finish.cuh"
 #include "k3_rows.cuh"
 #include "k3_fanout.cuh"
+#include "k3_attribution.cuh"
 #include "k_bed.cuh"

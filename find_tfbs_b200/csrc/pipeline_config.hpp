@@ -94,7 +94,7 @@ struct ConfigPipeline {
         if (!first_attempt) return;  // a repeated run keeps the capacities finalize() grew
         if (ctx->tiny_caps) {  // testing: every growth path runs
             c = Caps{};
-            c.seq = R; c.d = 1; c.cfg = 1; c.vd = 1; c.items = ref_items + 1; c.units = 1; c.dwords = 1; c.rows = 1; c.rowwords = 1; c.capr = 1; c.groups = 1;
+            c.seq = R; c.d = 1; c.cfg = 1; c.vd = 1; c.items = ref_items + 1; c.units = 1; c.dwords = 1; c.rows = 1; c.rowwords = 1; c.capr = 1; c.groups = 1; c.terms = 1;
             return;
         }
         // what the previous blocks needed (+ 25 %) when there is a history, else a guess from the shape of the block; a wrong guess
@@ -112,6 +112,7 @@ struct ConfigPipeline {
         c.rowwords = pick(h.rowwords, c.rows * ((uint64_t)(H + 1) / 32 + 1));
         c.capr = ctx->refhit_cap_opt ? (uint32_t)std::max<int64_t>(1, ctx->refhit_cap_opt / std::max<uint32_t>(1, R)) : (uint32_t)pick(h.capr, 512);
         c.groups = h.groups ? groups_for(h.groups) : (uint32_t)std::min<uint64_t>((uint64_t)H + 1, 2048);
+        c.terms = pick(h.terms, 4 * c.rows);
     }
     uint64_t scratch_bytes_needed() const {
         const Caps& c = slot->caps;
@@ -120,7 +121,12 @@ struct ConfigPipeline {
         while (seg < 2 * ((uint64_t)H + 1)) seg <<= 1;
         tbl = std::max<uint64_t>(tbl, (uint64_t)R * seg);
         return RH * 20 + tbl * 12 + c.seq * 50 + c.d * (4 + 32 + 20 + 4) + c.seq * 32 + c.cfg * 32 + (R + c.cfg) * 60 + c.vd * 36 + c.items * 28 +
-               c.units * 12 + c.dwords * 4 + n_keys * 36 + (uint64_t)c.capr * R * sizeof(RefHit) + c.rows * 34 + c.rowwords * 4 + fan_vec_bytes();
+               c.units * 12 + c.dwords * 4 + n_keys * 36 + (uint64_t)c.capr * R * sizeof(RefHit) + c.rows * 34 + c.rowwords * 4 + fan_vec_bytes() + attribution_bytes();
+    }
+    // option "attribution": scratch per diff-list entry, configuration, distinct haplotype and row, the per-slot results, the terms
+    uint64_t attribution_bytes() const {
+        const Caps& c = slot->caps;
+        return ctx->attribution ? c.d * 20 + c.cfg * 21 + c.seq * 12 + c.rows * 16 + c.terms * 8 : 0;
     }
 
     // ---- fan-out: the count vectors in shared memory (k_fanout<false>, one CTA per unit) or in device memory (k_fanout<true>) ----
@@ -229,6 +235,24 @@ struct ConfigPipeline {
         RS(slot->d_o_off, c.rows * 8);
         RS(slot->d_o_packed, c.rowwords * 4);
         if (fan_vec_bytes()) RS(ctx->d_fan_vec, fan_vec_bytes());
+        if (ctx->attribution) {
+            RS(ctx->d_att_eflag, c.d * 4);
+            RS(ctx->d_att_cfgid, (c.d + 1) * 8);
+            RS(ctx->d_att_nrec, c.cfg * 4);
+            RS(ctx->d_att_col, c.cfg * 4);
+            RS(ctx->d_att_gn, c.seq * 4);
+            RS(ctx->d_att_tcnt, c.rows * 4);
+            RS(slot->d_a_ref, c.rows * 4);
+            RS(slot->d_a_toff, (c.rows + 1) * 8);
+            RS(slot->d_a_tcfg, c.terms * 4);
+            RS(slot->d_a_tdiff, c.terms * 4);
+            RS(slot->d_a_creg, c.cfg * 4);
+            RS(slot->d_a_cflags, c.cfg);
+            RS(slot->d_a_croff, (c.cfg + 1) * 8);
+            RS(slot->d_a_crec, c.d * 4);
+            RS(slot->d_a_goff, (c.seq + 1) * 8);
+            RS(slot->d_a_gcfg, c.d * 4);
+        }
 #undef RS
         CK(slot->h_status.reserve(sizeof(DevStatus), false));
         CK(slot->h_plan.reserve(sizeof(DevPlan), false));
@@ -276,7 +300,8 @@ struct ConfigPipeline {
         slot->stats.scan_launches = 0;
         slot->stats.scan_input_bytes = 0;
         slot->res.n_rows = 0;
-        slot->res.have_dense = slot->res.have_grouped = false;
+        slot->res.have_dense = slot->res.have_grouped = slot->res.have_attribution = false;
+        slot->attribution = ctx->attribution != 0;
         choose_caps(first_attempt);
         const Caps& c = slot->caps;
         const bool fans = n_keys && R && S;
@@ -574,8 +599,58 @@ struct ConfigPipeline {
             gate(&plan->rowwords_alloc, 0, c.rowwords, &plan->n_rowwords, &plan->need_rowwords);
             TFBS_LAUNCH(k_row_headers, R, 128, 0, st)(db, cf, fn, &plan->n_rows);
             ++launches();
+            if (ctx->attribution && (rc = enqueue_attribution(sq, cf, vq, &fn))) return rc;
+        } else if (ctx->attribution && (rc = enqueue_attribution(sq, cf, vq, nullptr))) {
+            return rc;
         }
         return finish_enqueue();
+    }
+
+    // ---- option "attribution" (k3_attribution.cuh): behind the row headers, while D, C0, the diff lists and the runs are this block's ----
+    // 6 launches, 4 more for the terms when the block has keys
+    int enqueue_attribution(const DevSeqs& sq, const DevConfigs& cf, const DevSeqs& vq, const DevFan* fn) {
+        const Caps& c = slot->caps;
+        int rc;
+        DevAttr at{};
+        at.e_flag = ctx->d_att_eflag.as<u32>();
+        at.cfg_id = ctx->d_att_cfgid.as<u64>();
+        at.cfg_nrec = ctx->d_att_nrec.as<u32>();
+        at.cfg_col = ctx->d_att_col.as<u32>();
+        at.glist_n = ctx->d_att_gn.as<u32>();
+        at.t_cnt = ctx->d_att_tcnt.as<u32>();
+        at.cfg_region = slot->d_a_creg.as<u32>();
+        at.cfg_flags = slot->d_a_cflags.as<u8>();
+        at.cfg_rec_off = slot->d_a_croff.as<u64>();
+        at.cfg_rec = slot->d_a_crec.as<u32>();
+        at.group_off = slot->d_a_goff.as<u64>();
+        at.group_cfg = slot->d_a_gcfg.as<u32>();
+        at.ref_count = slot->d_a_ref.as<u32>();
+        at.term_off = slot->d_a_toff.as<u64>();
+        at.term_cfg = slot->d_a_tcfg.as<u32>();
+        at.term_diff = slot->d_a_tdiff.as<int>();
+        at.cfg_cap = c.cfg;
+        at.d_cap = c.d;
+        at.terms_cap = c.terms;
+        // 1. output ids: the rank of the representative entries in diff-list order
+        TFBS_LAUNCH(k_att_flags, slot->stats.sm_count * 8, 256, 0, st)(cf, at, &plan->n_d);
+        ++launches();
+        if ((rc = scan(at.e_flag, c.d, &plan->n_d, at.cfg_id))) return rc;
+        // 2. configurations and group lists: describe + count, two scans, fill
+        TFBS_LAUNCH(k_att_configs<false>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, vq, at);
+        ++launches();
+        if ((rc = scan(at.cfg_nrec, c.cfg, &plan->n_cfg, at.cfg_rec_off))) return rc;
+        if ((rc = scan(at.glist_n, c.seq, &plan->n_seq, at.group_off))) return rc;
+        TFBS_LAUNCH(k_att_configs<true>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, vq, at);
+        ++launches();
+        if (!fn) return TFBS_OK;
+        // 3. terms: count, scan, gate, fill
+        TFBS_LAUNCH(k_att_terms<false>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
+        ++launches();
+        if ((rc = scan(at.t_cnt, c.rows, &plan->n_rows, at.term_off))) return rc;
+        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(at.term_off, &plan->n_rows, (u64)c.terms, &plan->n_terms, &plan->need_terms, &plan->abort);
+        TFBS_LAUNCH(k_att_terms<true>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
+        launches() += 2;
+        return TFBS_OK;
     }
 
     int finish_enqueue() {
@@ -649,6 +724,7 @@ struct ConfigPipeline {
         g(c.dwords, hp.need_dwords);
         g(c.rows, hp.need_rows);
         g(c.rowwords, hp.need_rowwords);
+        g(c.terms, hp.need_terms);
         if (hp.need_capr > c.capr) c.capr = (uint32_t)up(hp.need_capr);
         if (hp.need_groups > c.groups) c.groups = groups_for(hp.need_groups);
     }
@@ -662,6 +738,7 @@ struct ConfigPipeline {
         h.dwords = std::max<uint64_t>(h.dwords, hp.need_dwords);
         h.rows = std::max<uint64_t>(h.rows, hp.need_rows);
         h.rowwords = std::max<uint64_t>(h.rowwords, hp.need_rowwords);
+        h.terms = std::max<uint64_t>(h.terms, hp.need_terms);
         h.capr = std::max<uint32_t>(h.capr, hp.need_capr);
         h.groups = std::max<uint32_t>(h.groups, hp.need_groups);
     }
@@ -697,6 +774,9 @@ struct ConfigPipeline {
         for (const ChunkDesc& cd : ctx->cp.chunks) table_bytes += (uint64_t)cd.tbl_words * 8 * s.scan_ctas;
         s.scan_input_bytes = (R && S) ? hp.n_units * 12 * ctx->cp.chunks.size() + table_bytes : 0;
         slot->res.n_rows = hp.n_rows;
+        slot->att_cfgs = hp.n_cfg;
+        slot->att_seqs = hp.n_seq;
+        slot->att_terms = hp.n_terms;
         slot->res.packed_words = hp.n_rowwords;
         slot->res.row_bytes = 4;
         if (ctx->rows_width == 0) slot->res.row_bytes = hs.max_count < 256 ? 1 : (hs.max_count < 65536 ? 2 : 4);
@@ -817,6 +897,48 @@ struct ConfigPipeline {
             hdr->sequence = hdr->sequence + 1;
         }
         res.have_grouped = true;
+        return TFBS_OK;
+    }
+
+    // attribution -> host (stream_out), the offset arrays first: they give the sizes of the others.  Counted in d2h_bytes.  Called by the
+    // collect that returns the block, while the slot's device buffers are still this block's.
+    int fetch_attribution() {
+        Results& res = slot->res;
+        if (res.have_attribution) return TFBS_OK;
+        cudaStream_t so = ctx->stream_out;
+        const uint64_t n = res.n_rows, nc = slot->att_cfgs, ng = slot->att_seqs;
+        CK(res.h_a_toff.reserve((n + 1) * 8, false));
+        CK(res.h_a_croff.reserve((nc + 1) * 8, false));
+        CK(res.h_a_goff.reserve((ng + 1) * 8, false));
+        uint64_t* toff = res.h_a_toff.as<uint64_t>();
+        uint64_t* croff = res.h_a_croff.as<uint64_t>();
+        uint64_t* goff = res.h_a_goff.as<uint64_t>();
+        uint64_t bytes = 0;
+        auto offsets = [&](uint64_t* h, const DevBuf& d, uint64_t cnt) -> int {  // cnt = 0: the scan may not have run
+            if (!cnt) { h[0] = 0; return TFBS_OK; }
+            CK(cudaMemcpyAsync(h, d.p, (cnt + 1) * 8, cudaMemcpyDeviceToHost, so));
+            bytes += (cnt + 1) * 8;
+            return TFBS_OK;
+        };
+        int rc;
+        if ((rc = offsets(toff, slot->d_a_toff, n)) || (rc = offsets(croff, slot->d_a_croff, nc)) || (rc = offsets(goff, slot->d_a_goff, ng))) return rc;
+        CK(cudaStreamSynchronize(so));
+        const uint64_t nt = toff[n], nr = croff[nc], nl = goff[ng];
+        if (nt != slot->att_terms) return fail(ctx, TFBS_ERR_INTERNAL, "attribution: the term count disagrees with the gate");
+        auto copy = [&](HostBuf& h, const DevBuf& d, uint64_t b) -> int {
+            CK(h.reserve(std::max<uint64_t>(1, b), false));
+            if (b) CK(cudaMemcpyAsync(h.p, d.p, b, cudaMemcpyDeviceToHost, so));
+            bytes += b;
+            return TFBS_OK;
+        };
+        if ((rc = copy(res.h_a_ref, slot->d_a_ref, n * 4)) || (rc = copy(res.h_a_tcfg, slot->d_a_tcfg, nt * 4)) ||
+            (rc = copy(res.h_a_tdiff, slot->d_a_tdiff, nt * 4)) || (rc = copy(res.h_a_creg, slot->d_a_creg, nc * 4)) ||
+            (rc = copy(res.h_a_cflags, slot->d_a_cflags, nc)) || (rc = copy(res.h_a_crec, slot->d_a_crec, nr * 4)) ||
+            (rc = copy(res.h_a_gcfg, slot->d_a_gcfg, nl * 4)))
+            return rc;
+        CK(cudaStreamSynchronize(so));
+        slot->stats.d2h_bytes += bytes;
+        res.have_attribution = true;
         return TFBS_OK;
     }
 

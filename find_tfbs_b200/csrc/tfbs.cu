@@ -60,6 +60,33 @@ int finish_oldest(tfbs_ctx* ctx, Slot** out) {
     return TFBS_OK;
 }
 
+// The collect that returns a block also brings its attribution to the host (option "attribution"): a later block may take the slot's
+// device buffers before tfbs_get_attribution is called.
+int take_attribution(tfbs_ctx* ctx, Slot* slot) {
+    if (slot->full_mode) { ctx->att_state = tfbs_ctx::ATT_FULL_SCAN; return TFBS_OK; }
+    if (!slot->attribution) { ctx->att_state = tfbs_ctx::ATT_OFF; return TFBS_OK; }
+    int rc = ConfigPipeline(ctx, slot).fetch_attribution();
+    if (rc) return rc;
+    const Results& res = slot->res;
+    tfbs_attribution& out = ctx->att;
+    memset(&out, 0, sizeof out);
+    out.n_rows = res.n_rows;
+    out.ref_count = res.h_a_ref.as<uint32_t>();
+    out.term_off = res.h_a_toff.as<uint64_t>();
+    out.term_cfg = res.h_a_tcfg.as<uint32_t>();
+    out.term_diff = res.h_a_tdiff.as<int32_t>();
+    out.n_cfgs = slot->att_cfgs;
+    out.cfg_region = res.h_a_creg.as<uint32_t>();
+    out.cfg_flags = res.h_a_cflags.as<uint8_t>();
+    out.cfg_rec_off = res.h_a_croff.as<uint64_t>();
+    out.cfg_rec = res.h_a_crec.as<uint32_t>();
+    out.n_groups_total = slot->att_seqs;
+    out.group_cfg_off = res.h_a_goff.as<uint64_t>();
+    out.group_cfg = res.h_a_gcfg.as<uint32_t>();
+    ctx->att_state = tfbs_ctx::ATT_READY;
+    return TFBS_OK;
+}
+
 void retire_oldest(tfbs_ctx* ctx) {
     ctx->last = ctx->head;
     ctx->slot[ctx->head].state = 0;
@@ -127,7 +154,7 @@ void share_hints(tfbs_ctx* a, tfbs_ctx* b) {  // what one twin learnt about the 
     Caps& y = b->hint;
 #define TFBS_BOTH(f) x.f = y.f = std::max(x.f, y.f)
     TFBS_BOTH(seq); TFBS_BOTH(d); TFBS_BOTH(cfg); TFBS_BOTH(vd); TFBS_BOTH(items); TFBS_BOTH(units); TFBS_BOTH(dwords); TFBS_BOTH(rows);
-    TFBS_BOTH(rowwords); TFBS_BOTH(capr); TFBS_BOTH(groups);
+    TFBS_BOTH(rowwords); TFBS_BOTH(capr); TFBS_BOTH(groups); TFBS_BOTH(terms);
 #undef TFBS_BOTH
 }
 int twin_failed(tfbs_ctx* ctx, int rc) {
@@ -247,6 +274,10 @@ int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value) {
         if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "fan_vector must be 0 (automatic) or 1 (device memory)");
         ctx->fan_vector = (int)value;
     }
+    else if (k == "attribution") {
+        if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "attribution must be 0 or 1");
+        ctx->attribution = (int)value;
+    }
     else if (k == "rows_width") {
         if (value != 0 && value != 32) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "rows_width must be 32 or 0 (automatic)");
         ctx->rows_width = (int)value;
@@ -358,10 +389,13 @@ int tfbs_collect(tfbs_ctx* ctx, tfbs_rows* out) {
         return rc;
     }
     CK(cudaSetDevice(ctx->device));
+    if (!ctx->bypass) ctx->last_target = 0;  // (a twin's results are not this block's)
+    ctx->att_state = tfbs_ctx::ATT_NONE;
     Slot* slot = nullptr;
     int rc = finish_oldest(ctx, &slot);
     if (rc) return rc;
     if (!slot->full_mode && (rc = ConfigPipeline(ctx, slot).fetch_dense())) { retire_oldest(ctx); return rc; }
+    if ((rc = take_attribution(ctx, slot))) { retire_oldest(ctx); return rc; }
     const Results& res = slot->res;
     out->n_rows = res.n_rows;
     out->n_samples = slot->in->S;
@@ -390,14 +424,17 @@ int tfbs_collect_grouped(tfbs_ctx* ctx, tfbs_grouped_rows* out) {
         return rc;
     }
     CK(cudaSetDevice(ctx->device));
+    if (!ctx->bypass) ctx->last_target = 0;
+    ctx->att_state = tfbs_ctx::ATT_NONE;
     Slot* slot = nullptr;
     int rc = finish_oldest(ctx, &slot);
     if (rc) return rc;
     if (slot->full_mode) {
+        ctx->att_state = tfbs_ctx::ATT_FULL_SCAN;
         retire_oldest(ctx);
         return fail(ctx, TFBS_ERR_STATE, "grouped rows come from the default scoring mode (delta = 1, record_matches off): use tfbs_collect");
     }
-    if ((rc = ConfigPipeline(ctx, slot).fetch_grouped())) { retire_oldest(ctx); return rc; }
+    if ((rc = ConfigPipeline(ctx, slot).fetch_grouped()) || (rc = take_attribution(ctx, slot))) { retire_oldest(ctx); return rc; }
     const Results& res = slot->res;
     memset(out, 0, sizeof *out);
     out->n_rows = res.n_rows;
@@ -569,6 +606,20 @@ int tfbs_merge_regions(tfbs_ctx* ctx, const uint64_t* start, const uint64_t* end
     CK(cudaMemcpyAsync(out_end, d_out.as<u64>() + n, misc[0] * 8, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     *n_out = misc[0];
+    return TFBS_OK;
+}
+
+int tfbs_get_attribution(tfbs_ctx* ctx, tfbs_attribution* out) {
+    if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
+    if (ctx->twin && !ctx->bypass && ctx->last_target == 1) return twin_failed(ctx, tfbs_get_attribution(ctx->twin, out));
+    switch (ctx->att_state) {
+    case tfbs_ctx::ATT_NONE: return fail(ctx, TFBS_ERR_STATE, "no block has been collected yet (tfbs_collect / tfbs_collect_grouped first)");
+    case tfbs_ctx::ATT_OFF: return fail(ctx, TFBS_ERR_STATE, "option attribution was off for the last block: set it to 1 before the run");
+    case tfbs_ctx::ATT_FULL_SCAN:
+        return fail(ctx, TFBS_ERR_STATE, "the last block was a full scan (delta = 0 or record_matches): attribution comes from the default path only");
+    default: break;
+    }
+    *out = ctx->att;
     return TFBS_OK;
 }
 

@@ -215,6 +215,38 @@ typedef struct tfbs_audit {
     uint32_t reserved;
 } tfbs_audit;
 
+/*
+ * Attribution of one block's rows (option "attribution" = 1, default path only; tfbs_get_attribution): which CONFIGURATIONS -- the
+ * records of one cluster of nearby records that a haplotype carries together -- change each row's count, and by how much.  For row j
+ * (row j of the tfbs_collect / tfbs_collect_grouped that returned the block) and every haplotype h of its region, the count h gets
+ * (left or right) is exactly
+ *     ref_count[j] + sum of term_diff[t] over t in [term_off[j], term_off[j + 1]) with term_cfg[t] in the list of group(h)
+ * where group(h) = hap_group of h in its region and the list of group g of region r is group_cfg[group_cfg_off[G] ..
+ * group_cfg_off[G + 1]), G = (sum of n_groups over the regions before r) + g.  Counts are integers: the equality has no tolerance.
+ * Configuration ids are numbered block-wide, by region, then by their first carrier group and position: they do not depend on hash
+ * seeds or on the order threads ran in.
+ */
+enum { TFBS_CFG_TRUNCATES = 1 };
+typedef struct tfbs_attribution {
+    uint64_t n_rows;               /* == n_rows of the collect */
+    const uint32_t* ref_count;     /* [n_rows] count of the region's reference haplotype for the row's key */
+    const uint64_t* term_off;      /* [n_rows + 1] */
+    const uint32_t* term_cfg;      /* [term_off[n_rows]] configurations whose count difference for the key is not 0, ascending */
+    const int32_t* term_diff;      /* [term_off[n_rows]] the configuration's count minus the reference haplotype's count */
+    uint64_t n_cfgs;               /* configurations of the block */
+    const uint32_t* cfg_region;    /* [n_cfgs] merged region of the configuration */
+    const uint8_t* cfg_flags;      /* [n_cfgs] TFBS_CFG_TRUNCATES: its walk reached patch_haplotype's truncation exit (haplotype.rs:144-149),
+                                      its difference includes the reference hits lost behind it */
+    const uint64_t* cfg_rec_off;   /* [n_cfgs + 1] */
+    const uint32_t* cfg_rec;       /* records of the configuration as indices into tfbs_block.variants, in the order the walk applies
+                                      them (position order) */
+    uint64_t n_groups_total;       /* sum of n_groups over the regions */
+    const uint64_t* group_cfg_off; /* [n_groups_total + 1] */
+    const uint32_t* group_cfg;     /* configurations whose difference the group's count includes, in the order of the group's records.
+                                      Empty for group 0 and for groups overwritten in the sequence-keyed map (counted as the reference
+                                      haplotype); behind a truncation only what the haplotype still applies */
+} tfbs_attribution;
+
 /* Row filter: which keys tfbs_collect returns. */
 enum {
     TFBS_ROWS_VARYING = 0, /* only keys with min != max, i.e. those counts_as_genotypes keeps (main.rs:456-458) */
@@ -276,7 +308,8 @@ const char* tfbs_last_error(const tfbs_ctx* ctx);
  * that holds every count of the block, see tfbs_rows.count_bytes -- result rows are the dominant PCIe traffic of large cohorts),
  * "fan_vector" (0 = automatic, the default: the fan-out keeps its per-group count vectors in shared memory and switches to device
  * memory when a region of the block may have more distinct haplotypes than shared memory holds, 53,120; 1 = always in device
- * memory, for tests -- results are the same either way). */
+ * memory, for tests -- results are the same either way), "attribution" (0 = off, the default; 1 = the default path also keeps the
+ * per-row count differences of every configuration for tfbs_get_attribution: the rows themselves do not change). */
 int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value);
 
 /* Replace the pattern list (the reference's pwm_list, src/main.rs:237). */
@@ -349,6 +382,12 @@ int tfbs_merge_sample_blocks(const tfbs_grouped_rows* const* parts, uint32_t n_p
  */
 int tfbs_merge_regions(tfbs_ctx* ctx, const uint64_t* start, const uint64_t* end, uint64_t n, uint64_t* out_start, uint64_t* out_end,
                        uint64_t* n_out);
+
+/* Attribution (see tfbs_attribution) of the block the last tfbs_collect or tfbs_collect_grouped returned; both forms give the same
+ * rows in the same order.  That collect already copied it to the host (option "attribution" on for the run), so blocks submitted
+ * since do not affect it.  Fails with TFBS_ERR_STATE when nothing has been collected, when option "attribution" was off for that run,
+ * or when the run was a full scan ("delta" = 0 or "record_matches").  Pointers stay valid as those of tfbs_rows do. */
+int tfbs_get_attribution(tfbs_ctx* ctx, tfbs_attribution* out);
 
 /* Matches of the last run when "record_matches" was on (call after tfbs_collect). */
 int tfbs_get_matches(tfbs_ctx* ctx, tfbs_matches* out);
