@@ -1,7 +1,6 @@
-// host_common.hpp -- the context behind the C ABI: device / pinned buffers, a block on the device, the two slots of blocks in flight
+// host_common.hpp -- the context behind the C ABI: device / pinned buffers, a block on the device, the two slots of blocks in flight, the two lanes they run on
 // Host side of libtfbs_b200.so (tfbs.cu is the map); one translation unit.
 #pragma once
-#include <deque>
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -111,6 +110,7 @@ struct Caps {
 struct Slot {
     int state = 0;  // 0 free, 1 enqueued (nothing has been waited for), 2 finished (results final)
     bool full_mode = false;
+    int lane = 0;   // tfbs_ctx::lane the block runs on (start_block)
     BlockDev own;
     BlockDev* in = nullptr;
     // device results of the configuration path: they outlive the shared scratch, which the next block reuses at once
@@ -131,13 +131,42 @@ struct Slot {
     uint64_t att_cfgs = 0, att_seqs = 0, att_terms = 0;  // their sizes (configurations, distinct haplotypes, terms)
 };
 
+// The streams a block's work is enqueued on and the scratch its kernels share with the blocks before and after it on the same lane.
+// Every block runs on lane 0 unless option "dual_stream" gives slot 1 a lane of its own (start_block): the kernels of consecutive
+// blocks then overlap on the device instead of queueing on one stream.
+struct Lane {
+    cudaStream_t stream = nullptr;      // kernels
+    cudaStream_t stream_in = nullptr;   // host -> device copies of the next block
+    cudaStream_t stream_out = nullptr;  // device -> host copies of finished rows
+
+    // scratch shared by consecutive blocks of the lane (their kernels are serialised on `stream`)
+    DevBuf d_ref_codes, d_allele_codes, d_var_class, d_var_inwin, d_var_althash, d_ref_prefix;
+    DevBuf d_sig, d_nd_in, d_leader, d_hap_group, d_ngroups, d_sum_nd, d_ref_used;
+    DevBuf d_keys, d_vals, d_scanwork;
+    DevBuf d_kbase, d_hap_mask, d_mask_base, d_region_dups, d_var_row;
+    // distinct haplotypes ("sequences")
+    DevBuf d_seq_region, d_seq_leader, d_seq_nd, d_seq_doff, d_dlist, d_segs, d_seq_nseg, d_seq_len, d_seq_hash, d_seq_flags, d_seq_ntake,
+        d_seq_nitems, d_item_off, d_items, d_list, d_ent_units, d_ent_uoff, d_pk, d_nm, d_refhits, d_refcnt;
+    // configuration path
+    DevBuf d_var_cluster, d_var_sorted, d_ncfg, d_cfgbase, d_dwords, d_dbase, d_run_len, d_run_key, d_run_rep, d_run_cfg, d_cfg_src,
+        d_cfg_net, d_mcount, d_moff, d_mfill, d_members, d_D, d_C0;
+    DevBuf d_vq_region, d_vq_leader, d_vq_nd, d_vq_doff, d_vq_dlist, d_vq_segs, d_vq_nseg, d_vq_len, d_vq_flags, d_vq_ntake, d_vq_nitems,
+        d_vq_item_off;
+    DevBuf d_vmin, d_vmax, d_flag, d_rowwords, d_kbits, d_rowidx, d_rowoff;
+    DevBuf d_fan_vec;  // k_fanout<true>: one count vector per CTA
+    DevBuf d_att_eflag, d_att_cfgid, d_att_nrec, d_att_col, d_att_gn, d_att_tcnt;  // option "attribution"
+    // full-scan path (lane 0 only)
+    DevBuf d_gbase, d_cbase, d_C;
+    DevBuf d_rows_region, d_rows_inner, d_rows_pid, d_rows_vmin, d_rows_vmax, d_rows_left, d_rows_right;
+    DevBuf d_m_region, d_m_pattern, d_m_group, d_m_start;
+    DevBuf d_hap_flags;
+};
+
 }  // namespace
 
 struct tfbs_ctx {
     int device = 0;
-    cudaStream_t stream = nullptr;      // kernels
-    cudaStream_t stream_in = nullptr;   // host -> device copies of the next block
-    cudaStream_t stream_out = nullptr;  // device -> host copies of finished rows
+    Lane lane[2];
     cudaDeviceProp prop{};
     std::string err;
 
@@ -158,6 +187,7 @@ struct tfbs_ctx {
     int64_t test_reseed = 0;    // testing: the first attempt of every block is treated as a hash collision (repeated with another seed)
     int fan_vector = 0;         // 0: the fan-out's count vectors live in shared memory unless a region has too many groups; 1: always in device memory (testing)
     int attribution = 0;        // 1: the default path keeps the per-row configuration differences (tfbs_get_attribution)
+    int dual_stream = 0;        // 1: a block in slot 1 of the default path runs on lane 1
     // attribution of the block the last tfbs_collect / tfbs_collect_grouped returned, copied to the host by that collect
     enum { ATT_NONE = 0, ATT_OFF, ATT_FULL_SCAN, ATT_READY };
     int att_state = ATT_NONE;
@@ -181,29 +211,9 @@ struct tfbs_ctx {
     uint8_t* arena = nullptr;      // tfbs_set_result_arena: grouped rows are copied straight into the caller's memory
     size_t arena_bytes = 0;
 
-    // scratch shared by consecutive blocks (their kernels are serialised on `stream`)
-    DevBuf d_ref_codes, d_allele_codes, d_var_class, d_var_inwin, d_var_althash, d_ref_prefix;
-    DevBuf d_sig, d_nd_in, d_leader, d_hap_group, d_ngroups, d_sum_nd, d_ref_used;
-    DevBuf d_keys, d_vals, d_scanwork;
-    DevBuf d_kbase, d_hap_mask, d_mask_base, d_region_dups, d_var_row;
-    // distinct haplotypes ("sequences")
-    DevBuf d_seq_region, d_seq_leader, d_seq_nd, d_seq_doff, d_dlist, d_segs, d_seq_nseg, d_seq_len, d_seq_hash, d_seq_flags, d_seq_ntake,
-        d_seq_nitems, d_item_off, d_items, d_list, d_ent_units, d_ent_uoff, d_pk, d_nm, d_refhits, d_refcnt;
-    // configuration path
-    DevBuf d_var_cluster, d_var_sorted, d_ncfg, d_cfgbase, d_dwords, d_dbase, d_run_len, d_run_key, d_run_rep, d_run_cfg, d_cfg_src,
-        d_cfg_net, d_mcount, d_moff, d_mfill, d_members, d_D, d_C0;
-    DevBuf d_vq_region, d_vq_leader, d_vq_nd, d_vq_doff, d_vq_dlist, d_vq_segs, d_vq_nseg, d_vq_len, d_vq_flags, d_vq_ntake, d_vq_nitems,
-        d_vq_item_off;
-    DevBuf d_vmin, d_vmax, d_flag, d_rowwords, d_kbits, d_rowidx, d_rowoff;
-    DevBuf d_fan_vec;  // k_fanout<true>: one count vector per CTA
-    DevBuf d_att_eflag, d_att_cfgid, d_att_nrec, d_att_col, d_att_gn, d_att_tcnt;  // option "attribution"
     // full-scan path
     std::vector<uint32_t> h_ngroups, h_sum_nd;
     std::vector<uint64_t> h_gbase, h_cbase, h_kbase;
-    DevBuf d_gbase, d_cbase, d_C, d_tile_sums;
-    DevBuf d_rows_region, d_rows_inner, d_rows_pid, d_rows_vmin, d_rows_vmax, d_rows_left, d_rows_right;
-    DevBuf d_m_region, d_m_pattern, d_m_group, d_m_start;
-    DevBuf d_hap_flags;
     HostBuf h_m_region, h_m_pattern, h_m_group, h_m_start, h_hap_group;
     HostBuf h_totals;
     HostBuf h_hap_flags;
@@ -214,16 +224,6 @@ struct tfbs_ctx {
     bool matches_truncated = false;
 
     cudaEvent_t ev[10]{};
-
-    // option "dual_stream": a second, complete context on the same device (own streams and scratch); blocks alternate between the
-    // two, so the kernels of consecutive blocks overlap on the device instead of queueing on one stream
-    tfbs_ctx* twin = nullptr;
-    bool is_twin = false, bypass = false;
-    int dual = 0;
-    int next_target = 0, last_target = 0;   // 0 = this context, 1 = the twin
-    std::deque<int> order;                  // targets of the blocks in flight, oldest first
-    int fixed_half = -1;                    // result arena: this context always writes this half (blocks alternate between the twins)
-    std::vector<std::pair<std::string, int64_t>> opt_log;
 };
 
 namespace {
@@ -244,9 +244,11 @@ int fail(tfbs_ctx* ctx, int code, const std::string& msg) {
 
 // Everything enqueued so far has finished (needed before an allocation that enqueued work may still use is replaced).
 int quiesce(tfbs_ctx* ctx) {
-    CK(cudaStreamSynchronize(ctx->stream_in));
-    CK(cudaStreamSynchronize(ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream_out));
+    for (const Lane& L : ctx->lane) {
+        CK(cudaStreamSynchronize(L.stream_in));
+        CK(cudaStreamSynchronize(L.stream));
+        CK(cudaStreamSynchronize(L.stream_out));
+    }
     return TFBS_OK;
 }
 
@@ -358,18 +360,19 @@ int upload_block(tfbs_ctx* ctx, const tfbs_block* b, BlockDev* B, cudaStream_t s
 }
 
 // Scratch the input encoding of a block needs (shared by both pipelines).
-int reserve_encoding(tfbs_ctx* ctx, const BlockDev& B) {
+int reserve_encoding(tfbs_ctx* ctx, Lane& L, const BlockDev& B) {
     int rc;
-    if ((rc = grow(ctx, ctx->d_ref_codes, std::max<uint64_t>(1, B.n_ref_bytes)))) return rc;
-    if ((rc = grow(ctx, ctx->d_allele_codes, std::max<uint64_t>(1, B.n_allele_bytes)))) return rc;
-    if ((rc = grow(ctx, ctx->d_var_class, std::max<uint64_t>(1, B.n_var) * 4))) return rc;
-    if ((rc = grow(ctx, ctx->d_var_inwin, std::max<uint64_t>(1, B.n_var)))) return rc;
-    if ((rc = grow(ctx, ctx->d_var_althash, std::max<uint64_t>(1, B.n_var) * 8))) return rc;
-    if ((rc = grow(ctx, ctx->d_ref_prefix, (B.n_ref_bytes + B.R + 1) * 8))) return rc;
+    if ((rc = grow(ctx, L.d_ref_codes, std::max<uint64_t>(1, B.n_ref_bytes)))) return rc;
+    if ((rc = grow(ctx, L.d_allele_codes, std::max<uint64_t>(1, B.n_allele_bytes)))) return rc;
+    if ((rc = grow(ctx, L.d_var_class, std::max<uint64_t>(1, B.n_var) * 4))) return rc;
+    if ((rc = grow(ctx, L.d_var_inwin, std::max<uint64_t>(1, B.n_var)))) return rc;
+    if ((rc = grow(ctx, L.d_var_althash, std::max<uint64_t>(1, B.n_var) * 8))) return rc;
+    if ((rc = grow(ctx, L.d_ref_prefix, (B.n_ref_bytes + B.R + 1) * 8))) return rc;
     return TFBS_OK;
 }
 
-DevBlock dev_block(const tfbs_ctx* ctx, const BlockDev& B) {
+// The block's arrays are only read: both lanes may run the resident block at once.  Its encoding is the lane's scratch.
+DevBlock dev_block(const Lane& L, const BlockDev& B) {
     DevBlock b{};
     b.R = B.R;
     b.S = B.S;
@@ -377,35 +380,35 @@ DevBlock dev_block(const tfbs_ctx* ctx, const BlockDev& B) {
     b.region_start = B.d_region_start.as<i64>();
     b.region_end = B.d_region_end.as<i64>();
     b.ref_off = B.d_ref_off.as<u64>();
-    b.ref_codes = ctx->d_ref_codes.as<u8>();
+    b.ref_codes = L.d_ref_codes.as<u8>();
     b.inner_off = B.d_inner_off.as<u32>();
     b.inner = B.d_inner.as<tfbs_inner_region>();
     b.var_off = B.d_var_off.as<u32>();
     b.variants = B.d_variants.as<tfbs_variant>();
-    b.allele_codes = ctx->d_allele_codes.as<u8>();
+    b.allele_codes = L.d_allele_codes.as<u8>();
     b.carriers = B.d_carriers.as<u32>();
     b.pitch = B.pitch;
-    b.var_class = ctx->d_var_class.as<u32>();
-    b.var_inwin = ctx->d_var_inwin.as<u8>();
-    b.var_althash = ctx->d_var_althash.as<u64>();
-    b.ref_prefix = ctx->d_ref_prefix.as<u64>();
+    b.var_class = L.d_var_class.as<u32>();
+    b.var_inwin = L.d_var_inwin.as<u8>();
+    b.var_althash = L.d_var_althash.as<u64>();
+    b.ref_prefix = L.d_ref_prefix.as<u64>();
     return b;
 }
 
 // exclusive scan of d_in[0, n) into d_out[0, n], total into d_out[n]; n = n_ptr ? min(*n_ptr, n_cap) : n_cap (one launch)
-int device_scan(tfbs_ctx* ctx, const uint32_t* d_in, uint64_t n_cap, const u64* n_ptr, u64* d_out, uint32_t* launches) {
-    cudaStream_t st = ctx->stream;
+int device_scan(tfbs_ctx* ctx, Lane& L, const uint32_t* d_in, uint64_t n_cap, const u64* n_ptr, u64* d_out, uint32_t* launches) {
+    cudaStream_t st = L.stream;
     const uint64_t tiles = (n_cap + SCAN_TILE - 1) / SCAN_TILE;
     if (tiles == 0) {
         CK(cudaMemsetAsync(d_out, 0, sizeof(u64), st));
         return TFBS_OK;
     }
-    if (!ctx->d_scanwork.fits((tiles + 1) * 8)) {
-        int rc = grow(ctx, ctx->d_scanwork, (tiles + 1) * 8);
+    if (!L.d_scanwork.fits((tiles + 1) * 8)) {
+        int rc = grow(ctx, L.d_scanwork, (tiles + 1) * 8);
         if (rc) return rc;
     }
-    CK(cudaMemsetAsync(ctx->d_scanwork.p, 0, (tiles + 1) * 8, st));
-    TFBS_LAUNCH(k_exclusive_scan, (unsigned)tiles, SCAN_THREADS, 0, st)(d_in, n_cap, n_ptr, d_out, ctx->d_scanwork.as<u64>());
+    CK(cudaMemsetAsync(L.d_scanwork.p, 0, (tiles + 1) * 8, st));
+    TFBS_LAUNCH(k_exclusive_scan, (unsigned)tiles, SCAN_THREADS, 0, st)(d_in, n_cap, n_ptr, d_out, L.d_scanwork.as<u64>());
     if (launches) ++*launches;
     CK(cudaGetLastError());
     return TFBS_OK;

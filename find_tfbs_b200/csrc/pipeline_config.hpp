@@ -1,7 +1,7 @@
 // pipeline_config.hpp -- the default path: configurations (k2c_configs.cuh), fan-out into grouped rows (k3_fanout.cuh), no host round trip
 // Host side of libtfbs_b200.so (tfbs.cu is the map); one translation unit.
 //
-// enqueue() launches the whole pipeline of a block on the context's kernel stream and returns: every size that only the device
+// enqueue() launches the whole pipeline of a block on the kernel stream of its lane and returns: every size that only the device
 // learns (distinct haplotypes, carried records, configurations, work-list items, packed bases, rows) is met with a CAPACITY chosen
 // from the previous blocks (tfbs_ctx::hint) and a gate kernel that publishes the real count; a count above its capacity raises
 // DevPlan::abort, the later stages skip, and finalize() -- called from tfbs_collect, the only place the host waits -- repeats the
@@ -47,6 +47,7 @@ uint32_t fan_smem_groups(const cudaDeviceProp& prop) {
 struct ConfigPipeline {
     tfbs_ctx* ctx;
     Slot* slot;
+    Lane& L;  // the slot's streams and scratch
     BlockDev& B;
     cudaStream_t st;
     const uint32_t R, S, H;
@@ -60,11 +61,11 @@ struct ConfigPipeline {
     const uint32_t smem_groups;  // fan_smem_groups()
 
     ConfigPipeline(tfbs_ctx* c, Slot* s)
-        : ctx(c), slot(s), B(*s->in), st(c->stream), R(s->in->R), S(s->in->S), H(s->in->H), RH((uint64_t)s->in->R * s->in->H),
+        : ctx(c), slot(s), L(c->lane[s->lane]), B(*s->in), st(L.stream), R(s->in->R), S(s->in->S), H(s->in->H), RH((uint64_t)s->in->R * s->in->H),
           smem_groups(fan_smem_groups(c->prop)) {}
 
     uint32_t& launches() { return slot->stats.total_launches; }
-    int scan(const uint32_t* d_in, uint64_t n_cap, const u64* n_ptr, u64* d_out) { return device_scan(ctx, d_in, n_cap, n_ptr, d_out, &launches()); }
+    int scan(const uint32_t* d_in, uint64_t n_cap, const u64* n_ptr, u64* d_out) { return device_scan(ctx, L, d_in, n_cap, n_ptr, d_out, &launches()); }
     int gate(const u64* total, uint64_t add, uint64_t cap, u64* n_out, u64* need_out) {
         TFBS_LAUNCH(k_gate, 1, 1, 0, st)(total, (u64)add, (u64)cap, n_out, need_out, &plan->abort);
         ++launches();
@@ -148,83 +149,83 @@ struct ConfigPipeline {
         const Caps& c = slot->caps;
         int rc;
 #define RS(buf, bytes) if ((rc = grow(ctx, buf, std::max<uint64_t>(1, (uint64_t)(bytes))))) return rc
-        if ((rc = reserve_encoding(ctx, B))) return rc;
+        if ((rc = reserve_encoding(ctx, L, B))) return rc;
         RS(slot->d_status, sizeof(DevStatus));
         RS(slot->d_plan, sizeof(DevPlan));
         RS(slot->d_hap_group, RH * 4);
         RS(slot->d_gbase, (uint64_t)(R + 1) * 8);
-        RS(ctx->d_sig, RH * 8);
-        RS(ctx->d_nd_in, RH * 4);
-        RS(ctx->d_leader, RH * 4);
-        RS(ctx->d_ngroups, (uint64_t)R * 4);
-        RS(ctx->d_sum_nd, (uint64_t)R * 4);
-        RS(ctx->d_ref_used, (uint64_t)R * 4);
-        RS(ctx->d_kbase, (uint64_t)(R + 1) * 8);
+        RS(L.d_sig, RH * 8);
+        RS(L.d_nd_in, RH * 4);
+        RS(L.d_leader, RH * 4);
+        RS(L.d_ngroups, (uint64_t)R * 4);
+        RS(L.d_sum_nd, (uint64_t)R * 4);
+        RS(L.d_ref_used, (uint64_t)R * 4);
+        RS(L.d_kbase, (uint64_t)(R + 1) * 8);
         {
             uint64_t mask_words = 0;  // H * sum over the regions of ceil(V / 32)
             for (uint32_t r = 0; r < R; ++r) mask_words += (uint64_t)H * ((B.h_var_off[r + 1] - B.h_var_off[r] + 31) / 32);
-            RS(ctx->d_hap_mask, mask_words * 4);
-            RS(ctx->d_mask_base, (uint64_t)(R + 1) * 8);
-            RS(ctx->d_region_dups, (uint64_t)R * 4);
-            RS(ctx->d_var_row, B.n_var * 4);
+            RS(L.d_hap_mask, mask_words * 4);
+            RS(L.d_mask_base, (uint64_t)(R + 1) * 8);
+            RS(L.d_region_dups, (uint64_t)R * 4);
+            RS(L.d_var_row, B.n_var * 4);
         }
-        RS(ctx->d_seq_region, c.seq * 4);
-        RS(ctx->d_seq_leader, c.seq * 4);
-        RS(ctx->d_seq_nd, c.seq * 4);
-        RS(ctx->d_seq_doff, (c.seq + 1) * 8);
-        RS(ctx->d_seq_nseg, c.seq * 4);
-        RS(ctx->d_seq_len, c.seq * 4);
-        RS(ctx->d_seq_hash, c.seq * 8);
-        RS(ctx->d_seq_flags, c.seq);
-        RS(ctx->d_seq_ntake, c.seq * 4);
-        RS(ctx->d_dlist, c.d * 4);
-        RS(ctx->d_segs, (2 * c.d + 2 * c.seq) * sizeof(Seg));
-        RS(ctx->d_var_cluster, B.n_var * 4);
-        RS(ctx->d_var_sorted, B.n_var * 4);
-        RS(ctx->d_ncfg, (uint64_t)R * 4);
-        RS(ctx->d_dwords, (uint64_t)R * 4);
-        RS(ctx->d_cfgbase, (uint64_t)(R + 1) * 8);
-        RS(ctx->d_dbase, (uint64_t)(R + 1) * 8);
-        RS(ctx->d_run_len, c.d * 4);
-        RS(ctx->d_run_key, c.d * 8);
-        RS(ctx->d_run_rep, c.d * 4);
-        RS(ctx->d_run_cfg, c.d * 4);
-        RS(ctx->d_cfg_src, c.cfg * 4);
-        RS(ctx->d_cfg_net, c.cfg * 4);
-        RS(ctx->d_mcount, c.cfg * 4);
-        RS(ctx->d_moff, (c.cfg + 1) * 8);
-        RS(ctx->d_mfill, c.cfg * 4);
-        RS(ctx->d_members, c.d * 4);
+        RS(L.d_seq_region, c.seq * 4);
+        RS(L.d_seq_leader, c.seq * 4);
+        RS(L.d_seq_nd, c.seq * 4);
+        RS(L.d_seq_doff, (c.seq + 1) * 8);
+        RS(L.d_seq_nseg, c.seq * 4);
+        RS(L.d_seq_len, c.seq * 4);
+        RS(L.d_seq_hash, c.seq * 8);
+        RS(L.d_seq_flags, c.seq);
+        RS(L.d_seq_ntake, c.seq * 4);
+        RS(L.d_dlist, c.d * 4);
+        RS(L.d_segs, (2 * c.d + 2 * c.seq) * sizeof(Seg));
+        RS(L.d_var_cluster, B.n_var * 4);
+        RS(L.d_var_sorted, B.n_var * 4);
+        RS(L.d_ncfg, (uint64_t)R * 4);
+        RS(L.d_dwords, (uint64_t)R * 4);
+        RS(L.d_cfgbase, (uint64_t)(R + 1) * 8);
+        RS(L.d_dbase, (uint64_t)(R + 1) * 8);
+        RS(L.d_run_len, c.d * 4);
+        RS(L.d_run_key, c.d * 8);
+        RS(L.d_run_rep, c.d * 4);
+        RS(L.d_run_cfg, c.d * 4);
+        RS(L.d_cfg_src, c.cfg * 4);
+        RS(L.d_cfg_net, c.cfg * 4);
+        RS(L.d_mcount, c.cfg * 4);
+        RS(L.d_moff, (c.cfg + 1) * 8);
+        RS(L.d_mfill, c.cfg * 4);
+        RS(L.d_members, c.d * 4);
         const uint64_t nv = R + c.cfg;
-        RS(ctx->d_vq_region, nv * 4);
-        RS(ctx->d_vq_leader, nv * 4);
-        RS(ctx->d_vq_nd, nv * 4);
-        RS(ctx->d_vq_doff, (nv + 1) * 8);
-        RS(ctx->d_vq_nseg, nv * 4);
-        RS(ctx->d_vq_len, nv * 4);
-        RS(ctx->d_vq_flags, nv);
-        RS(ctx->d_vq_ntake, nv * 4);
-        RS(ctx->d_vq_nitems, nv * 4);
-        RS(ctx->d_vq_item_off, (nv + 1) * 8);
-        RS(ctx->d_vq_dlist, c.vd * 4);
-        RS(ctx->d_vq_segs, (2 * c.vd + 2 * nv) * sizeof(Seg));
-        RS(ctx->d_items, c.items * sizeof(ScanItem));
-        RS(ctx->d_list, c.items * 4);
-        RS(ctx->d_ent_units, c.items * 4);
-        RS(ctx->d_ent_uoff, (c.items + 1) * 8);
-        RS(ctx->d_pk, c.units * 8);
-        RS(ctx->d_nm, c.units * 4);
-        RS(ctx->d_D, c.dwords * 4);
-        RS(ctx->d_C0, n_keys * 4);
-        RS(ctx->d_refhits, (uint64_t)c.capr * R * sizeof(RefHit));
-        RS(ctx->d_refcnt, (uint64_t)R * 4);
-        RS(ctx->d_vmin, n_keys * 4);
-        RS(ctx->d_vmax, n_keys * 4);
-        RS(ctx->d_flag, n_keys * 4);
-        RS(ctx->d_rowwords, n_keys * 4);
-        RS(ctx->d_kbits, n_keys);
-        RS(ctx->d_rowidx, (n_keys + 1) * 8);
-        RS(ctx->d_rowoff, (n_keys + 1) * 8);
+        RS(L.d_vq_region, nv * 4);
+        RS(L.d_vq_leader, nv * 4);
+        RS(L.d_vq_nd, nv * 4);
+        RS(L.d_vq_doff, (nv + 1) * 8);
+        RS(L.d_vq_nseg, nv * 4);
+        RS(L.d_vq_len, nv * 4);
+        RS(L.d_vq_flags, nv);
+        RS(L.d_vq_ntake, nv * 4);
+        RS(L.d_vq_nitems, nv * 4);
+        RS(L.d_vq_item_off, (nv + 1) * 8);
+        RS(L.d_vq_dlist, c.vd * 4);
+        RS(L.d_vq_segs, (2 * c.vd + 2 * nv) * sizeof(Seg));
+        RS(L.d_items, c.items * sizeof(ScanItem));
+        RS(L.d_list, c.items * 4);
+        RS(L.d_ent_units, c.items * 4);
+        RS(L.d_ent_uoff, (c.items + 1) * 8);
+        RS(L.d_pk, c.units * 8);
+        RS(L.d_nm, c.units * 4);
+        RS(L.d_D, c.dwords * 4);
+        RS(L.d_C0, n_keys * 4);
+        RS(L.d_refhits, (uint64_t)c.capr * R * sizeof(RefHit));
+        RS(L.d_refcnt, (uint64_t)R * 4);
+        RS(L.d_vmin, n_keys * 4);
+        RS(L.d_vmax, n_keys * 4);
+        RS(L.d_flag, n_keys * 4);
+        RS(L.d_rowwords, n_keys * 4);
+        RS(L.d_kbits, n_keys);
+        RS(L.d_rowidx, (n_keys + 1) * 8);
+        RS(L.d_rowoff, (n_keys + 1) * 8);
         RS(slot->d_o_region, c.rows * 4);
         RS(slot->d_o_inner, c.rows * 4);
         RS(slot->d_o_pid, c.rows * 2);
@@ -234,14 +235,14 @@ struct ConfigPipeline {
         RS(slot->d_o_bits, c.rows);
         RS(slot->d_o_off, c.rows * 8);
         RS(slot->d_o_packed, c.rowwords * 4);
-        if (fan_vec_bytes()) RS(ctx->d_fan_vec, fan_vec_bytes());
+        if (fan_vec_bytes()) RS(L.d_fan_vec, fan_vec_bytes());
         if (ctx->attribution) {
-            RS(ctx->d_att_eflag, c.d * 4);
-            RS(ctx->d_att_cfgid, (c.d + 1) * 8);
-            RS(ctx->d_att_nrec, c.cfg * 4);
-            RS(ctx->d_att_col, c.cfg * 4);
-            RS(ctx->d_att_gn, c.seq * 4);
-            RS(ctx->d_att_tcnt, c.rows * 4);
+            RS(L.d_att_eflag, c.d * 4);
+            RS(L.d_att_cfgid, (c.d + 1) * 8);
+            RS(L.d_att_nrec, c.cfg * 4);
+            RS(L.d_att_col, c.cfg * 4);
+            RS(L.d_att_gn, c.seq * 4);
+            RS(L.d_att_tcnt, c.rows * 4);
             RS(slot->d_a_ref, c.rows * 4);
             RS(slot->d_a_toff, (c.rows + 1) * 8);
             RS(slot->d_a_tcfg, c.terms * 4);
@@ -261,10 +262,10 @@ struct ConfigPipeline {
 
     int table_slots(uint64_t slots) {  // the shared open-addressing table with room for `slots` slots, emptied
         int rc;
-        if ((rc = grow(ctx, ctx->d_keys, slots * 8))) return rc;
-        if ((rc = grow(ctx, ctx->d_vals, slots * 4))) return rc;
-        CK(cudaMemsetAsync(ctx->d_keys.p, 0, slots * 8, st));
-        CK(cudaMemsetAsync(ctx->d_vals.p, 0xff, slots * 4, st));
+        if ((rc = grow(ctx, L.d_keys, slots * 8))) return rc;
+        if ((rc = grow(ctx, L.d_vals, slots * 4))) return rc;
+        CK(cudaMemsetAsync(L.d_keys.p, 0, slots * 8, st));
+        CK(cudaMemsetAsync(L.d_vals.p, 0xff, slots * 4, st));
         return TFBS_OK;
     }
     int table(uint64_t entries, uint32_t* mask) {  // the same as one table of a power-of-two number of slots >= 2 * entries
@@ -272,10 +273,10 @@ struct ConfigPipeline {
         while (cap < 2 * entries) cap <<= 1;
         if (cap > (1ull << 31)) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "block too large for the grouping table: submit fewer regions at a time");
         int rc;
-        if ((rc = grow(ctx, ctx->d_keys, cap * 8))) return rc;
-        if ((rc = grow(ctx, ctx->d_vals, cap * 4))) return rc;
-        CK(cudaMemsetAsync(ctx->d_keys.p, 0, cap * 8, st));
-        CK(cudaMemsetAsync(ctx->d_vals.p, 0xff, cap * 4, st));
+        if ((rc = grow(ctx, L.d_keys, cap * 8))) return rc;
+        if ((rc = grow(ctx, L.d_vals, cap * 4))) return rc;
+        CK(cudaMemsetAsync(L.d_keys.p, 0, cap * 8, st));
+        CK(cudaMemsetAsync(L.d_vals.p, 0xff, cap * 4, st));
         *mask = (uint32_t)(cap - 1);
         return TFBS_OK;
     }
@@ -331,27 +332,27 @@ struct ConfigPipeline {
         // ---- inputs: ASCII -> codes, Diff classes, prefix hashes of the reference windows, keys per region ----
         const unsigned enc_grid = slot->stats.sm_count * 16;
         if (B.n_ref_bytes) {
-            TFBS_LAUNCH(k_encode, std::min<unsigned>(grid_for(B.n_ref_bytes, 256), enc_grid), 256, 0, st)(B.d_ref_ascii.as<u8>(), ctx->d_ref_codes.as<u8>(), B.n_ref_bytes, &dst->bad_ref_base);
+            TFBS_LAUNCH(k_encode, std::min<unsigned>(grid_for(B.n_ref_bytes, 256), enc_grid), 256, 0, st)(B.d_ref_ascii.as<u8>(), L.d_ref_codes.as<u8>(), B.n_ref_bytes, &dst->bad_ref_base);
             ++launches();
         }
         if (B.n_allele_bytes) {
-            TFBS_LAUNCH(k_encode, std::min<unsigned>(grid_for(B.n_allele_bytes, 256), enc_grid), 256, 0, st)(B.d_allele_ascii.as<u8>(), ctx->d_allele_codes.as<u8>(), B.n_allele_bytes, &dst->bad_allele_base);
+            TFBS_LAUNCH(k_encode, std::min<unsigned>(grid_for(B.n_allele_bytes, 256), enc_grid), 256, 0, st)(B.d_allele_ascii.as<u8>(), L.d_allele_codes.as<u8>(), B.n_allele_bytes, &dst->bad_allele_base);
             ++launches();
         }
-        db = dev_block(ctx, B);
-        db.hap_mask = ctx->d_hap_mask.as<u32>();
-        db.mask_base = ctx->d_mask_base.as<u64>();
-        db.region_dups = ctx->d_region_dups.as<u32>();
-        db.var_row = db.var_row_out = ctx->d_var_row.as<u32>();
+        db = dev_block(L, B);
+        db.hap_mask = L.d_hap_mask.as<u32>();
+        db.mask_base = L.d_mask_base.as<u64>();
+        db.region_dups = L.d_region_dups.as<u32>();
+        db.var_row = db.var_row_out = L.d_var_row.as<u32>();
         db.hash_seed = slot->seed;
-        TFBS_LAUNCH(k_mask_words, grid_for(R, 256), 256, 0, st)(db, ctx->d_dwords.as<u32>());
+        TFBS_LAUNCH(k_mask_words, grid_for(R, 256), 256, 0, st)(db, L.d_dwords.as<u32>());
         ++launches();
-        if ((rc = scan(ctx->d_dwords.as<u32>(), R, nullptr, ctx->d_mask_base.as<u64>()))) return rc;
-        TFBS_LAUNCH(k_variant_prep, R, 128, 0, st)(db, 0, ctx->d_var_class.as<u32>(), ctx->d_var_inwin.as<u8>(), ctx->d_region_dups.as<u32>());
-        TFBS_LAUNCH(k_ref_prefix, R, SCAN_THREADS, 0, st)(db, 0, ctx->d_ref_prefix.as<u64>());
-        TFBS_LAUNCH(k_region_keys, grid_for(R, 256), 256, 0, st)(db, n_pid, ctx->d_dwords.as<u32>());
+        if ((rc = scan(L.d_dwords.as<u32>(), R, nullptr, L.d_mask_base.as<u64>()))) return rc;
+        TFBS_LAUNCH(k_variant_prep, R, 128, 0, st)(db, 0, L.d_var_class.as<u32>(), L.d_var_inwin.as<u8>(), L.d_region_dups.as<u32>());
+        TFBS_LAUNCH(k_ref_prefix, R, SCAN_THREADS, 0, st)(db, 0, L.d_ref_prefix.as<u64>());
+        TFBS_LAUNCH(k_region_keys, grid_for(R, 256), 256, 0, st)(db, n_pid, L.d_dwords.as<u32>());
         launches() += 3;
-        if ((rc = scan(ctx->d_dwords.as<u32>(), R, nullptr, ctx->d_kbase.as<u64>()))) return rc;
+        if ((rc = scan(L.d_dwords.as<u32>(), R, nullptr, L.d_kbase.as<u64>()))) return rc;
 
         // ---- K0: grouping by Vec<Diff> (haplotype.rs:65-75) ----
         u32* hap_group = slot->d_hap_group.as<u32>();
@@ -365,17 +366,17 @@ struct ConfigPipeline {
                 const uint32_t nr = std::min(regions_per_super, R - r0);
                 const uint64_t pairs = (uint64_t)nr * H;
                 if ((rc = table_slots((uint64_t)nr * seg))) return rc;
-                TFBS_LAUNCH(k_signatures, grid_for((uint64_t)nr * ((H + 31) / 32) * 32, 256), 256, 0, st)(db, r0, nr, slot->seed, ctx->d_sig.as<u64>(), ctx->d_nd_in.as<u32>());
-                TFBS_LAUNCH(k_group_insert, grid_for(pairs, 256), 256, 0, st)(H, r0, nr, ctx->d_sig.as<u64>(), ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), 0u, seg);
-                TFBS_LAUNCH(k_group_lookup, grid_for(pairs, 256), 256, 0, st)(db, r0, nr, ctx->d_sig.as<u64>(), ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), 0u, seg,
-                                                                     ctx->d_leader.as<u32>(), dst);
-                TFBS_LAUNCH(k_group_rank, nr, 256, 0, st)(H, r0, ctx->d_leader.as<u32>(), ctx->d_nd_in.as<u32>(), hap_group, ctx->d_ngroups.as<u32>(),
-                                                 ctx->d_sum_nd.as<u32>());
+                TFBS_LAUNCH(k_signatures, grid_for((uint64_t)nr * ((H + 31) / 32) * 32, 256), 256, 0, st)(db, r0, nr, slot->seed, L.d_sig.as<u64>(), L.d_nd_in.as<u32>());
+                TFBS_LAUNCH(k_group_insert, grid_for(pairs, 256), 256, 0, st)(H, r0, nr, L.d_sig.as<u64>(), L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg);
+                TFBS_LAUNCH(k_group_lookup, grid_for(pairs, 256), 256, 0, st)(db, r0, nr, L.d_sig.as<u64>(), L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg,
+                                                                     L.d_leader.as<u32>(), dst);
+                TFBS_LAUNCH(k_group_rank, nr, 256, 0, st)(H, r0, L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), hap_group, L.d_ngroups.as<u32>(),
+                                                 L.d_sum_nd.as<u32>());
                 launches() += 4;
             }
         }
         u64* gbase = slot->d_gbase.as<u64>();
-        if ((rc = scan(ctx->d_ngroups.as<u32>(), R, nullptr, gbase))) return rc;
+        if ((rc = scan(L.d_ngroups.as<u32>(), R, nullptr, gbase))) return rc;
         gate(gbase + R, 0, c.seq, &plan->n_seq, &plan->need_seq);
         CK(cudaEventRecord(slot->ev_t[1], st));
 
@@ -386,18 +387,18 @@ struct ConfigPipeline {
         sq.abort = &plan->abort;
         sq.gbase = gbase;
         sq.gbase0 = 0;
-        sq.seq_region = ctx->d_seq_region.as<u32>();
-        sq.seq_leader = ctx->d_seq_leader.as<u32>();
-        sq.seq_nd = ctx->d_seq_nd.as<u32>();
-        sq.seq_doff = ctx->d_seq_doff.as<u64>();
-        sq.dlist = ctx->d_dlist.as<u32>();
-        sq.segs = ctx->d_segs.as<Seg>();
-        sq.seq_nseg = ctx->d_seq_nseg.as<u32>();
-        sq.seq_len = ctx->d_seq_len.as<u32>();
-        sq.seq_hash = ctx->d_seq_hash.as<u64>();
-        sq.seq_flags = ctx->d_seq_flags.as<u8>();
-        sq.seq_ntake = ctx->d_seq_ntake.as<u32>();
-        TFBS_LAUNCH(k_seq_init, R, 128, 0, st)(H, 0, hap_group, ctx->d_leader.as<u32>(), ctx->d_nd_in.as<u32>(), sq);
+        sq.seq_region = L.d_seq_region.as<u32>();
+        sq.seq_leader = L.d_seq_leader.as<u32>();
+        sq.seq_nd = L.d_seq_nd.as<u32>();
+        sq.seq_doff = L.d_seq_doff.as<u64>();
+        sq.dlist = L.d_dlist.as<u32>();
+        sq.segs = L.d_segs.as<Seg>();
+        sq.seq_nseg = L.d_seq_nseg.as<u32>();
+        sq.seq_len = L.d_seq_len.as<u32>();
+        sq.seq_hash = L.d_seq_hash.as<u64>();
+        sq.seq_flags = L.d_seq_flags.as<u8>();
+        sq.seq_ntake = L.d_seq_ntake.as<u32>();
+        TFBS_LAUNCH(k_seq_init, R, 128, 0, st)(H, 0, hap_group, L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), sq);
         ++launches();
         if ((rc = scan(sq.seq_nd, c.seq, &plan->n_seq, sq.seq_doff))) return rc;
         // the total sits behind the last sequence; k_gate reads it through the clamped count
@@ -407,10 +408,10 @@ struct ConfigPipeline {
         ++launches();
         {
             if ((rc = table_slots((uint64_t)R * seg))) return rc;  // at most H + 1 distinct haplotypes per region
-            CK(cudaMemsetAsync(ctx->d_ref_used.p, 0, (size_t)R * 4, st));
-            TFBS_LAUNCH(k_seq_insert, grid_for(c.seq, 256), 256, 0, st)(sq, ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), 0u, seg, 0u);
-            TFBS_LAUNCH(k_seq_resolve, grid_for(c.seq, 128), 128, 0, st)(db, sq, ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), 0u, seg, 0u, dst, 0u);
-            TFBS_LAUNCH(k_redirect, grid_for(RH, 256), 256, 0, st)(H, 0, R, sq, hap_group, ctx->d_ref_used.as<u32>(), (u8*)nullptr, (u64*)&dst->nominal_cells,
+            CK(cudaMemsetAsync(L.d_ref_used.p, 0, (size_t)R * 4, st));
+            TFBS_LAUNCH(k_seq_insert, grid_for(c.seq, 256), 256, 0, st)(sq, L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg, 0u);
+            TFBS_LAUNCH(k_seq_resolve, grid_for(c.seq, 128), 128, 0, st)(db, sq, L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg, 0u, dst, 0u);
+            TFBS_LAUNCH(k_redirect, grid_for(RH, 256), 256, 0, st)(H, 0, R, sq, hap_group, L.d_ref_used.as<u32>(), (u8*)nullptr, (u64*)&dst->nominal_cells,
                                                                    ctx->dpat.max_len, ctx->dpat.sum_len, (u64)ctx->dpat.sum_len_sq, ctx->dpat.n_patterns, ctx->dpat.pat_len);
             launches() += 3;
         }
@@ -420,25 +421,25 @@ struct ConfigPipeline {
         DevConfigs cf{};
         cf.max_len = cp.max_len;
         cf.n_pid = n_pid;
-        cf.var_cluster = ctx->d_var_cluster.as<u32>();
-        cf.var_sorted = ctx->d_var_sorted.as<u32>();
-        cf.ncfg = ctx->d_ncfg.as<u32>();
-        cf.cfgbase = ctx->d_cfgbase.as<u64>();
-        cf.dwords = ctx->d_dwords.as<u32>();
-        cf.dbase = ctx->d_dbase.as<u64>();
-        cf.kbase = ctx->d_kbase.as<u64>();
-        cf.run_len = ctx->d_run_len.as<u32>();
-        cf.run_key = ctx->d_run_key.as<u64>();
-        cf.run_rep = ctx->d_run_rep.as<u32>();
-        cf.run_cfg = ctx->d_run_cfg.as<u32>();
-        cf.cfg_src = ctx->d_cfg_src.as<u32>();
-        cf.cfg_net = ctx->d_cfg_net.as<int>();
-        cf.mcount = ctx->d_mcount.as<u32>();
-        cf.moff = ctx->d_moff.as<u64>();
-        cf.mfill = ctx->d_mfill.as<u32>();
-        cf.members = ctx->d_members.as<u32>();
-        cf.D = ctx->d_D.as<u32>();
-        cf.C0 = ctx->d_C0.as<u32>();
+        cf.var_cluster = L.d_var_cluster.as<u32>();
+        cf.var_sorted = L.d_var_sorted.as<u32>();
+        cf.ncfg = L.d_ncfg.as<u32>();
+        cf.cfgbase = L.d_cfgbase.as<u64>();
+        cf.dwords = L.d_dwords.as<u32>();
+        cf.dbase = L.d_dbase.as<u64>();
+        cf.kbase = L.d_kbase.as<u64>();
+        cf.run_len = L.d_run_len.as<u32>();
+        cf.run_key = L.d_run_key.as<u64>();
+        cf.run_rep = L.d_run_rep.as<u32>();
+        cf.run_cfg = L.d_run_cfg.as<u32>();
+        cf.cfg_src = L.d_cfg_src.as<u32>();
+        cf.cfg_net = L.d_cfg_net.as<int>();
+        cf.mcount = L.d_mcount.as<u32>();
+        cf.moff = L.d_moff.as<u64>();
+        cf.mfill = L.d_mfill.as<u32>();
+        cf.members = L.d_members.as<u32>();
+        cf.D = L.d_D.as<u32>();
+        cf.C0 = L.d_C0.as<u32>();
         cf.plan = plan;
         TFBS_LAUNCH(k_cluster, R, 128, 0, st)(db, cf);
         ++launches();
@@ -446,8 +447,8 @@ struct ConfigPipeline {
             uint32_t mask;
             if ((rc = table(c.d, &mask))) return rc;
             CK(cudaMemsetAsync(cf.ncfg, 0, (size_t)R * 4, st));
-            TFBS_LAUNCH(k_cfg_runs, grid_for(c.seq, 128), 128, 0, st)(db, sq, cf, (u64)c.d, slot->seed, ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), mask);
-            TFBS_LAUNCH(k_cfg_resolve, grid_for(c.seq, 128), 128, 0, st)(sq, cf, (u64)c.d, ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), mask);
+            TFBS_LAUNCH(k_cfg_runs, grid_for(c.seq, 128), 128, 0, st)(db, sq, cf, (u64)c.d, slot->seed, L.d_keys.as<u64>(), L.d_vals.as<u32>(), mask);
+            TFBS_LAUNCH(k_cfg_resolve, grid_for(c.seq, 128), 128, 0, st)(sq, cf, (u64)c.d, L.d_keys.as<u64>(), L.d_vals.as<u32>(), mask);
             launches() += 2;
         }
         TFBS_LAUNCH(k_region_sizes, grid_for(R, 256), 256, 0, st)(db, cf);
@@ -464,24 +465,24 @@ struct ConfigPipeline {
         vq.n_seq_ptr = &plan->n_vseq;
         vq.abort = &plan->abort;
         vq.n_ref = R;
-        vq.seq_region = ctx->d_vq_region.as<u32>();
-        vq.seq_leader = ctx->d_vq_leader.as<u32>();
-        vq.seq_nd = ctx->d_vq_nd.as<u32>();
-        vq.seq_doff = ctx->d_vq_doff.as<u64>();
-        vq.dlist = ctx->d_vq_dlist.as<u32>();
-        vq.segs = ctx->d_vq_segs.as<Seg>();
-        vq.seq_nseg = ctx->d_vq_nseg.as<u32>();
-        vq.seq_len = ctx->d_vq_len.as<u32>();
-        vq.seq_flags = ctx->d_vq_flags.as<u8>();
-        vq.seq_ntake = ctx->d_vq_ntake.as<u32>();
-        vq.seq_nitems = ctx->d_vq_nitems.as<u32>();
-        vq.item_off = ctx->d_vq_item_off.as<u64>();
-        vq.items = ctx->d_items.as<ScanItem>();
+        vq.seq_region = L.d_vq_region.as<u32>();
+        vq.seq_leader = L.d_vq_leader.as<u32>();
+        vq.seq_nd = L.d_vq_nd.as<u32>();
+        vq.seq_doff = L.d_vq_doff.as<u64>();
+        vq.dlist = L.d_vq_dlist.as<u32>();
+        vq.segs = L.d_vq_segs.as<Seg>();
+        vq.seq_nseg = L.d_vq_nseg.as<u32>();
+        vq.seq_len = L.d_vq_len.as<u32>();
+        vq.seq_flags = L.d_vq_flags.as<u8>();
+        vq.seq_ntake = L.d_vq_ntake.as<u32>();
+        vq.seq_nitems = L.d_vq_nitems.as<u32>();
+        vq.item_off = L.d_vq_item_off.as<u64>();
+        vq.items = L.d_items.as<ScanItem>();
         vq.n_items_cap = (u32)c.items;
-        vq.ent_units = ctx->d_ent_units.as<u32>();
-        vq.ent_uoff = ctx->d_ent_uoff.as<u64>();
-        vq.pk = ctx->d_pk.as<u64>();
-        vq.nm = ctx->d_nm.as<u32>();
+        vq.ent_units = L.d_ent_units.as<u32>();
+        vq.ent_uoff = L.d_ent_uoff.as<u64>();
+        vq.pk = L.d_pk.as<u64>();
+        vq.nm = L.d_nm.as<u32>();
         vq.units_cap = c.units;
         TFBS_LAUNCH(k_vseq_init, grid_for(R, 256), 256, 0, st)(R, vq);
         TFBS_LAUNCH(k_cfg_fill, grid_for(c.seq, 128), 128, 0, st)(sq, cf, vq, (u64)c.d);
@@ -498,20 +499,20 @@ struct ConfigPipeline {
         if ((rc = scan(vq.seq_nitems, R + c.cfg, &plan->n_vseq, vq.item_off))) return rc;
         TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(vq.item_off, &plan->n_vseq, (u64)c.items, &plan->n_items, &plan->need_items, &plan->abort);
         TFBS_LAUNCH(k_vitems<true>, grid_for(R + c.cfg, 128), 128, 0, st)(vq, cp.max_len, &plan->abort);
-        TFBS_LAUNCH(k_vitem_units, grid_for(c.items, 256), 256, 0, st)(vq, &plan->n_items, ctx->d_list.as<u32>());
+        TFBS_LAUNCH(k_vitem_units, grid_for(c.items, 256), 256, 0, st)(vq, &plan->n_items, L.d_list.as<u32>());
         launches() += 3;
         if ((rc = scan(vq.ent_units, c.items, &plan->n_items, vq.ent_uoff))) return rc;
         TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(vq.ent_uoff, &plan->n_items, (u64)c.units, &plan->n_units, &plan->need_units, &plan->abort);
-        TFBS_LAUNCH(k_emit_list, grid_for(c.items * EMIT_LANES, 256), 256, 0, st)(db, vq, ctx->d_list.as<u32>(), &plan->n_items);
-        TFBS_LAUNCH(k_item_stats, grid_for(c.items, 256), 256, 0, st)(vq, ctx->dpat, ctx->d_list.as<u32>(), &plan->n_items, dst);
+        TFBS_LAUNCH(k_emit_list, grid_for(c.items * EMIT_LANES, 256), 256, 0, st)(db, vq, L.d_list.as<u32>(), &plan->n_items);
+        TFBS_LAUNCH(k_item_stats, grid_for(c.items, 256), 256, 0, st)(vq, ctx->dpat, L.d_list.as<u32>(), &plan->n_items, dst);
         launches() += 3;
 
         // ---- the scan: one launch per pattern chunk ----
         TFBS_LAUNCH(k_zero_words, slot->stats.sm_count * 8, 256, 0, st)(cf.D, &plan->n_dwords, (u64)c.dwords);
         ++launches();
         if (n_keys) CK(cudaMemsetAsync(cf.C0, 0, n_keys * 4, st));
-        CK(cudaMemsetAsync(ctx->d_refcnt.p, 0, (size_t)R * 4, st));
-        DevRefHits drh{ctx->d_refhits.as<RefHit>(), ctx->d_refcnt.as<u32>(), c.capr, 0};
+        CK(cudaMemsetAsync(L.d_refcnt.p, 0, (size_t)R * 4, st));
+        DevRefHits drh{L.d_refhits.as<RefHit>(), L.d_refcnt.as<u32>(), c.capr, 0};
         DevCounts dc{cf.C0, cf.kbase, 0};
         DevMatches dm{};
         const int smem_bytes = (int)(sizeof(CtaShared) + SCAN_WARPS * sizeof(WarpShared) + ((cp.max_chunk_bytes + 15) & ~15u));
@@ -524,8 +525,8 @@ struct ConfigPipeline {
         CK(cudaEventRecord(slot->ev_t[3], st));
         for (uint32_t ch = 0; ch < cp.chunks.size(); ++ch) {
             CK(cudaMemsetAsync(&dst->work_counter, 0, 4, st));
-            if (wide) TFBS_LAUNCH(k_scan<2>, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, ctx->d_list.as<u32>(), &plan->n_items, (u32)SCAN_PER_GRAB, dst, ch);
-            else TFBS_LAUNCH(k_scan<3>, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, ctx->d_list.as<u32>(), &plan->n_items, (u32)SCAN_PER_GRAB, dst, ch);
+            if (wide) TFBS_LAUNCH(k_scan<2>, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, L.d_list.as<u32>(), &plan->n_items, (u32)SCAN_PER_GRAB, dst, ch);
+            else TFBS_LAUNCH(k_scan<3>, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, L.d_list.as<u32>(), &plan->n_items, (u32)SCAN_PER_GRAB, dst, ch);
             ++launches();
             ++slot->stats.scan_launches;
         }
@@ -537,11 +538,11 @@ struct ConfigPipeline {
         launches() += 2;
         CK(cudaMemsetAsync(cf.mcount, 0, c.cfg * 4, st));
         CK(cudaMemsetAsync(cf.mfill, 0, c.cfg * 4, st));
-        TFBS_LAUNCH(k_members<false>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, drh, ctx->d_ref_used.as<u32>(), (u64)c.d, ctx->dpat, dst);
+        TFBS_LAUNCH(k_members<false>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, drh, L.d_ref_used.as<u32>(), (u64)c.d, ctx->dpat, dst);
         ++launches();
         if ((rc = scan(cf.mcount, c.cfg, &plan->n_cfg, cf.moff))) return rc;
         TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(cf.moff, &plan->n_cfg, (u64)c.d, &plan->n_members, &plan->need_members, &plan->abort);
-        TFBS_LAUNCH(k_members<true>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, drh, ctx->d_ref_used.as<u32>(), (u64)c.d, ctx->dpat, dst);
+        TFBS_LAUNCH(k_members<true>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, drh, L.d_ref_used.as<u32>(), (u64)c.d, ctx->dpat, dst);
         launches() += 2;
         CK(cudaEventRecord(slot->ev_t[5], st));
 
@@ -553,13 +554,13 @@ struct ConfigPipeline {
             fn.n_pid = n_pid;
             fn.rows_mode = ctx->rows_mode;
             fn.groups_cap = c.groups;
-            fn.vmin = ctx->d_vmin.as<u32>();
-            fn.vmax = ctx->d_vmax.as<u32>();
-            fn.flag = ctx->d_flag.as<u32>();
-            fn.k_base = ctx->d_rowwords.as<u32>();
-            fn.k_bits = ctx->d_kbits.as<u8>();
-            fn.k_off = ctx->d_rowoff.as<u64>();
-            fn.rowidx = ctx->d_rowidx.as<u64>();
+            fn.vmin = L.d_vmin.as<u32>();
+            fn.vmax = L.d_vmax.as<u32>();
+            fn.flag = L.d_flag.as<u32>();
+            fn.k_base = L.d_rowwords.as<u32>();
+            fn.k_bits = L.d_kbits.as<u8>();
+            fn.k_off = L.d_rowoff.as<u64>();
+            fn.rowidx = L.d_rowidx.as<u64>();
             fn.rows_cap = c.rows;
             fn.words_cap = c.rowwords;
             fn.o_region = slot->d_o_region.as<u32>();
@@ -581,11 +582,11 @@ struct ConfigPipeline {
             const size_t fan_smem = fan_smem_bytes(smem_vec_groups, H, fn.hg16 != 0);
             const uint32_t split = fan_split();
             if (vec) {
-                fn.vec = ctx->d_fan_vec.as<u32>();
+                fn.vec = L.d_fan_vec.as<u32>();
                 fn.vec_stride = fan_vec_stride();
                 fn.split = split;
                 // the kernel leaves every slice all zero, a fresh or regrown allocation is not: zeroed on every run, repeats included
-                CK(cudaMemsetAsync(ctx->d_fan_vec.p, 0, fan_vec_bytes(), st));
+                CK(cudaMemsetAsync(L.d_fan_vec.p, 0, fan_vec_bytes(), st));
                 CK(cudaFuncSetAttribute(k_fanout<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fan_smem));
                 TFBS_LAUNCH(k_fanout<true>, fan_vec_grid(), FAN_THREADS, fan_smem, st)(db, cf, fn);
             } else {
@@ -594,8 +595,8 @@ struct ConfigPipeline {
                 TFBS_LAUNCH(k_fanout<false>, dim3(R, split), FAN_THREADS, fan_smem, st)(db, cf, fn);
             }
             ++launches();
-            if ((rc = scan(fn.flag, n_keys, nullptr, ctx->d_rowidx.as<u64>()))) return rc;
-            gate(ctx->d_rowidx.as<u64>() + n_keys, 0, c.rows, &plan->n_rows, &plan->need_rows);
+            if ((rc = scan(fn.flag, n_keys, nullptr, L.d_rowidx.as<u64>()))) return rc;
+            gate(L.d_rowidx.as<u64>() + n_keys, 0, c.rows, &plan->n_rows, &plan->need_rows);
             gate(&plan->rowwords_alloc, 0, c.rowwords, &plan->n_rowwords, &plan->need_rowwords);
             TFBS_LAUNCH(k_row_headers, R, 128, 0, st)(db, cf, fn, &plan->n_rows);
             ++launches();
@@ -612,12 +613,12 @@ struct ConfigPipeline {
         const Caps& c = slot->caps;
         int rc;
         DevAttr at{};
-        at.e_flag = ctx->d_att_eflag.as<u32>();
-        at.cfg_id = ctx->d_att_cfgid.as<u64>();
-        at.cfg_nrec = ctx->d_att_nrec.as<u32>();
-        at.cfg_col = ctx->d_att_col.as<u32>();
-        at.glist_n = ctx->d_att_gn.as<u32>();
-        at.t_cnt = ctx->d_att_tcnt.as<u32>();
+        at.e_flag = L.d_att_eflag.as<u32>();
+        at.cfg_id = L.d_att_cfgid.as<u64>();
+        at.cfg_nrec = L.d_att_nrec.as<u32>();
+        at.cfg_col = L.d_att_col.as<u32>();
+        at.glist_n = L.d_att_gn.as<u32>();
+        at.t_cnt = L.d_att_tcnt.as<u32>();
         at.cfg_region = slot->d_a_creg.as<u32>();
         at.cfg_flags = slot->d_a_cflags.as<u8>();
         at.cfg_rec_off = slot->d_a_croff.as<u64>();
@@ -808,14 +809,14 @@ struct ConfigPipeline {
     int fetch_grouped() {
         Results& res = slot->res;
         if (res.have_grouped) return TFBS_OK;
-        cudaStream_t so = ctx->stream_out;
+        cudaStream_t so = L.stream_out;
         const uint64_t n = res.n_rows, w = res.packed_words;
         res.hg_bytes = (uint64_t)H + 1 <= 65536 ? 2 : 4;
         const bool maps = R && S;
         tfbs_arena_header* hdr = nullptr;
         slot->stats.d2h_bytes = 0;
         if (ctx->arena) {
-            uint8_t* half = ctx->arena + (size_t)(ctx->fixed_half >= 0 ? ctx->fixed_half : (int)(slot - ctx->slot)) * (ctx->arena_bytes / 2);
+            uint8_t* half = ctx->arena + (size_t)(slot - ctx->slot) * (ctx->arena_bytes / 2);
             hdr = reinterpret_cast<tfbs_arena_header*>(half);
             tfbs_arena_header h = *hdr;
             if (h.magic != TFBS_ARENA_MAGIC) { memset(&h, 0, sizeof h); h.magic = TFBS_ARENA_MAGIC; }
@@ -905,7 +906,7 @@ struct ConfigPipeline {
     int fetch_attribution() {
         Results& res = slot->res;
         if (res.have_attribution) return TFBS_OK;
-        cudaStream_t so = ctx->stream_out;
+        cudaStream_t so = L.stream_out;
         const uint64_t n = res.n_rows, nc = slot->att_cfgs, ng = slot->att_seqs;
         CK(res.h_a_toff.reserve((n + 1) * 8, false));
         CK(res.h_a_croff.reserve((nc + 1) * 8, false));
@@ -946,7 +947,7 @@ struct ConfigPipeline {
     int fetch_dense() {
         Results& res = slot->res;
         if (res.have_dense) return TFBS_OK;
-        cudaStream_t so = ctx->stream_out;
+        cudaStream_t so = L.stream_out;
         const uint64_t n = res.n_rows;
         const uint32_t eb = res.row_bytes;
         int rc;

@@ -13,6 +13,7 @@ namespace {
 struct FullPipeline {
     tfbs_ctx* ctx;
     Slot* slot;
+    Lane& L;  // lane 0: the full scan owns the device
     BlockDev& B;
     Results& res;
     cudaStream_t st;
@@ -43,7 +44,7 @@ struct FullPipeline {
     };
 
     FullPipeline(tfbs_ctx* c, Slot* s)
-        : ctx(c), slot(s), B(*s->in), res(s->res), st(c->stream), R(s->in->R), S(s->in->S), H(s->in->H), RH((uint64_t)s->in->R * s->in->H) {}
+        : ctx(c), slot(s), L(c->lane[s->lane]), B(*s->in), res(s->res), st(L.stream), R(s->in->R), S(s->in->S), H(s->in->H), RH((uint64_t)s->in->R * s->in->H) {}
 
     int run() {
         int rc;
@@ -77,7 +78,7 @@ private:
     tfbs_stats& stats() { return slot->stats; }
     uint32_t& launches() { return slot->stats.total_launches; }
 
-    int scan(const uint32_t* d_in, uint64_t n, u64* d_out) { return device_scan(ctx, d_in, n, nullptr, d_out, &launches()); }
+    int scan(const uint32_t* d_in, uint64_t n, u64* d_out) { return device_scan(ctx, L, d_in, n, nullptr, d_out, &launches()); }
 
     int read_status(DevStatus* hs) {
         CK(cudaMemcpyAsync(slot->h_status.p, dst, sizeof(DevStatus), cudaMemcpyDeviceToHost, st));
@@ -98,7 +99,7 @@ private:
         ctx->matches_truncated = false;
         int rc;
         if ((rc = quiesce(ctx))) return rc;  // this pipeline owns the device for the duration of the call
-        if ((rc = reserve_encoding(ctx, B))) return rc;
+        if ((rc = reserve_encoding(ctx, L, B))) return rc;
         CK(slot->d_status.reserve(sizeof(DevStatus)));
         CK(slot->h_status.reserve(sizeof(DevStatus), false));
         CK(ctx->h_totals.reserve(64, false));
@@ -116,32 +117,32 @@ private:
     // ASCII -> nucleotide codes, Diff classes, prefix hashes of the reference windows
     int encode_inputs() {
         if (B.n_ref_bytes) {
-            TFBS_LAUNCH(k_encode, std::min<unsigned>(grid_for(B.n_ref_bytes, 256), stats().sm_count * 16), 256, 0, st)(B.d_ref_ascii.as<u8>(), ctx->d_ref_codes.as<u8>(),
+            TFBS_LAUNCH(k_encode, std::min<unsigned>(grid_for(B.n_ref_bytes, 256), stats().sm_count * 16), 256, 0, st)(B.d_ref_ascii.as<u8>(), L.d_ref_codes.as<u8>(),
                                                                                                      B.n_ref_bytes, &dst->bad_ref_base);
             ++launches();
         }
         if (B.n_allele_bytes) {
             TFBS_LAUNCH(k_encode, std::min<unsigned>(grid_for(B.n_allele_bytes, 256), stats().sm_count * 16), 256, 0, st)(
-                B.d_allele_ascii.as<u8>(), ctx->d_allele_codes.as<u8>(), B.n_allele_bytes, &dst->bad_allele_base);
+                B.d_allele_ascii.as<u8>(), L.d_allele_codes.as<u8>(), B.n_allele_bytes, &dst->bad_allele_base);
             ++launches();
         }
-        db = dev_block(ctx, B);
-        TFBS_LAUNCH(k_variant_prep, R, 128, 0, st)(db, 0, ctx->d_var_class.as<u32>(), ctx->d_var_inwin.as<u8>(), (u32*)nullptr);
-        TFBS_LAUNCH(k_ref_prefix, R, SCAN_THREADS, 0, st)(db, 0, ctx->d_ref_prefix.as<u64>());
+        db = dev_block(L, B);
+        TFBS_LAUNCH(k_variant_prep, R, 128, 0, st)(db, 0, L.d_var_class.as<u32>(), L.d_var_inwin.as<u8>(), (u32*)nullptr);
+        TFBS_LAUNCH(k_ref_prefix, R, SCAN_THREADS, 0, st)(db, 0, L.d_ref_prefix.as<u64>());
         launches() += 2;
         return TFBS_OK;
     }
 
     // ---- phase 1: grouping (K0), over super-batches bounded by the hash table; a signature collision retries with another seed ----
     int group_haplotypes() {
-        CK(ctx->d_sig.reserve(RH * 8));
-        CK(ctx->d_nd_in.reserve(RH * 4));
-        CK(ctx->d_leader.reserve(RH * 4));
-        CK(ctx->d_hap_group.reserve(RH * 4));
-        CK(ctx->d_ngroups.reserve((size_t)R * 4));
-        CK(ctx->d_sum_nd.reserve((size_t)R * 4));
-        CK(ctx->d_ref_used.reserve((size_t)R * 4));
-        if (ctx->audit) CK(ctx->d_hap_flags.reserve(RH));
+        CK(L.d_sig.reserve(RH * 8));
+        CK(L.d_nd_in.reserve(RH * 4));
+        CK(L.d_leader.reserve(RH * 4));
+        CK(L.d_hap_group.reserve(RH * 4));
+        CK(L.d_ngroups.reserve((size_t)R * 4));
+        CK(L.d_sum_nd.reserve((size_t)R * 4));
+        CK(L.d_ref_used.reserve((size_t)R * 4));
+        if (ctx->audit) CK(L.d_hap_flags.reserve(RH));
         const uint64_t max_pairs = 1ull << 25;
         uint32_t regions_per_super = (uint32_t)std::max<uint64_t>(1, max_pairs / std::max<uint32_t>(1, H));
         uint64_t seed = 0x243f6a8885a308d3ull;
@@ -151,23 +152,23 @@ private:
                 uint64_t pairs = (uint64_t)nr * H;
                 uint32_t cap = 1024;
                 while (cap < 2 * pairs) cap <<= 1;
-                CK(ctx->d_keys.reserve((size_t)cap * 8));
-                CK(ctx->d_vals.reserve((size_t)cap * 4));
-                CK(cudaMemsetAsync(ctx->d_keys.p, 0, (size_t)cap * 8, st));
-                CK(cudaMemsetAsync(ctx->d_vals.p, 0xff, (size_t)cap * 4, st));
-                TFBS_LAUNCH(k_signatures, grid_for((uint64_t)nr * ((H + 31) / 32) * 32, 256), 256, 0, st)(db, r0, nr, seed, ctx->d_sig.as<u64>(), ctx->d_nd_in.as<u32>());
-                TFBS_LAUNCH(k_group_insert, grid_for(pairs, 256), 256, 0, st)(H, r0, nr, ctx->d_sig.as<u64>(), ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), cap - 1, 0u);
-                TFBS_LAUNCH(k_group_lookup, grid_for(pairs, 256), 256, 0, st)(db, r0, nr, ctx->d_sig.as<u64>(), ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), cap - 1, 0u,
-                                                                     ctx->d_leader.as<u32>(), dst);
-                TFBS_LAUNCH(k_group_rank, nr, 256, 0, st)(H, r0, ctx->d_leader.as<u32>(), ctx->d_nd_in.as<u32>(), ctx->d_hap_group.as<u32>(),
-                                                 ctx->d_ngroups.as<u32>(), ctx->d_sum_nd.as<u32>());
+                CK(L.d_keys.reserve((size_t)cap * 8));
+                CK(L.d_vals.reserve((size_t)cap * 4));
+                CK(cudaMemsetAsync(L.d_keys.p, 0, (size_t)cap * 8, st));
+                CK(cudaMemsetAsync(L.d_vals.p, 0xff, (size_t)cap * 4, st));
+                TFBS_LAUNCH(k_signatures, grid_for((uint64_t)nr * ((H + 31) / 32) * 32, 256), 256, 0, st)(db, r0, nr, seed, L.d_sig.as<u64>(), L.d_nd_in.as<u32>());
+                TFBS_LAUNCH(k_group_insert, grid_for(pairs, 256), 256, 0, st)(H, r0, nr, L.d_sig.as<u64>(), L.d_keys.as<u64>(), L.d_vals.as<u32>(), cap - 1, 0u);
+                TFBS_LAUNCH(k_group_lookup, grid_for(pairs, 256), 256, 0, st)(db, r0, nr, L.d_sig.as<u64>(), L.d_keys.as<u64>(), L.d_vals.as<u32>(), cap - 1, 0u,
+                                                                     L.d_leader.as<u32>(), dst);
+                TFBS_LAUNCH(k_group_rank, nr, 256, 0, st)(H, r0, L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), L.d_hap_group.as<u32>(),
+                                                 L.d_ngroups.as<u32>(), L.d_sum_nd.as<u32>());
                 launches() += 4;
             }
             CK(cudaGetLastError());
             ctx->h_ngroups.resize(R);
             ctx->h_sum_nd.resize(R);
-            CK(cudaMemcpyAsync(ctx->h_ngroups.data(), ctx->d_ngroups.p, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
-            CK(cudaMemcpyAsync(ctx->h_sum_nd.data(), ctx->d_sum_nd.p, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(ctx->h_ngroups.data(), L.d_ngroups.p, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(ctx->h_sum_nd.data(), L.d_sum_nd.p, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
             DevStatus hs;
             int rc = read_status(&hs);
             if (rc) return rc;
@@ -200,26 +201,26 @@ private:
             ctx->h_kbase[r + 1] = ctx->h_kbase[r] + (uint64_t)n_pid * nk;
         }
         int rc;
-        if ((rc = upload_on(ctx, st, ctx->d_gbase, ctx->h_gbase.data(), R + 1, nullptr))) return rc;
-        if ((rc = upload_on(ctx, st, ctx->d_cbase, ctx->h_cbase.data(), R + 1, nullptr))) return rc;
-        if ((rc = upload_on(ctx, st, ctx->d_kbase, ctx->h_kbase.data(), R + 1, nullptr))) return rc;
+        if ((rc = upload_on(ctx, st, L.d_gbase, ctx->h_gbase.data(), R + 1, nullptr))) return rc;
+        if ((rc = upload_on(ctx, st, L.d_cbase, ctx->h_cbase.data(), R + 1, nullptr))) return rc;
+        if ((rc = upload_on(ctx, st, L.d_kbase, ctx->h_kbase.data(), R + 1, nullptr))) return rc;
         return TFBS_OK;
     }
 
     // match buffer, shared-memory size and grid of the scan kernel
     int setup_scan() {
         if (ctx->record_matches) {
-            CK(ctx->d_m_region.reserve(ctx->max_matches * 4));
-            CK(ctx->d_m_pattern.reserve(ctx->max_matches * 4));
-            CK(ctx->d_m_group.reserve(ctx->max_matches * 4));
-            CK(ctx->d_m_start.reserve(ctx->max_matches * 8));
+            CK(L.d_m_region.reserve(ctx->max_matches * 4));
+            CK(L.d_m_pattern.reserve(ctx->max_matches * 4));
+            CK(L.d_m_group.reserve(ctx->max_matches * 4));
+            CK(L.d_m_start.reserve(ctx->max_matches * 8));
         }
         dm.enabled = ctx->record_matches ? 1u : 0u;
         dm.cap = (u32)std::min<uint64_t>(ctx->max_matches, 0xffffffffu);
-        dm.region = ctx->d_m_region.as<u32>();
-        dm.pattern_index = ctx->d_m_pattern.as<u32>();
-        dm.group = ctx->d_m_group.as<u32>();
-        dm.start = ctx->d_m_start.as<i64>();
+        dm.region = L.d_m_region.as<u32>();
+        dm.pattern_index = L.d_m_pattern.as<u32>();
+        dm.group = L.d_m_group.as<u32>();
+        dm.start = L.d_m_start.as<i64>();
         smem_bytes = (int)(sizeof(CtaShared) + SCAN_WARPS * sizeof(WarpShared) + ((ctx->cp.max_chunk_bytes + 15) & ~15u));
         wide = ctx->cp.fields == 2;
         if (wide) CK(cudaFuncSetAttribute(k_scan<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
@@ -268,60 +269,60 @@ private:
     int reserve_batch(Batch* b) {
         const uint64_t n_seq = b->n_seq, n_d = b->n_d, n_c = b->n_c, n_keys = b->n_keys;
         const uint64_t ic = std::max<uint64_t>(1, n_seq);  // at most one item per sequence
-        CK(ctx->d_seq_region.reserve(n_seq * 4));
-        CK(ctx->d_seq_leader.reserve(n_seq * 4));
-        CK(ctx->d_seq_nd.reserve(n_seq * 4));
-        CK(ctx->d_seq_doff.reserve((n_seq + 1) * 8));
-        CK(ctx->d_dlist.reserve(std::max<uint64_t>(1, n_d) * 4));
-        CK(ctx->d_segs.reserve((2 * n_d + 2 * n_seq) * sizeof(Seg)));
-        CK(ctx->d_seq_nseg.reserve(n_seq * 4));
-        CK(ctx->d_seq_len.reserve(n_seq * 4));
-        CK(ctx->d_seq_hash.reserve(n_seq * 8));
-        CK(ctx->d_seq_flags.reserve(n_seq));
-        CK(ctx->d_seq_ntake.reserve(n_seq * 4));
-        CK(ctx->d_C.reserve(std::max<uint64_t>(1, n_c) * 4));
-        CK(ctx->d_vmin.reserve(std::max<uint64_t>(1, n_keys) * 4));
-        CK(ctx->d_vmax.reserve(std::max<uint64_t>(1, n_keys) * 4));
-        CK(ctx->d_flag.reserve(std::max<uint64_t>(1, n_keys) * 4));
-        CK(ctx->d_rowidx.reserve((n_keys + 1) * 8));
-        CK(ctx->d_refcnt.reserve((size_t)b->nr * 4));
-        CK(ctx->d_seq_nitems.reserve(n_seq * 4));
-        CK(ctx->d_item_off.reserve((n_seq + 1) * 8));
-        CK(ctx->d_items.reserve(ic * sizeof(ScanItem)));
-        CK(ctx->d_list.reserve(ic * 4));
-        CK(ctx->d_ent_units.reserve(ic * 4));
-        CK(ctx->d_ent_uoff.reserve((ic + 1) * 8));
-        CK(ctx->d_pk.reserve(std::max<uint64_t>(1, b->n_units) * 8));
-        CK(ctx->d_nm.reserve(std::max<uint64_t>(1, b->n_units) * 4));
+        CK(L.d_seq_region.reserve(n_seq * 4));
+        CK(L.d_seq_leader.reserve(n_seq * 4));
+        CK(L.d_seq_nd.reserve(n_seq * 4));
+        CK(L.d_seq_doff.reserve((n_seq + 1) * 8));
+        CK(L.d_dlist.reserve(std::max<uint64_t>(1, n_d) * 4));
+        CK(L.d_segs.reserve((2 * n_d + 2 * n_seq) * sizeof(Seg)));
+        CK(L.d_seq_nseg.reserve(n_seq * 4));
+        CK(L.d_seq_len.reserve(n_seq * 4));
+        CK(L.d_seq_hash.reserve(n_seq * 8));
+        CK(L.d_seq_flags.reserve(n_seq));
+        CK(L.d_seq_ntake.reserve(n_seq * 4));
+        CK(L.d_C.reserve(std::max<uint64_t>(1, n_c) * 4));
+        CK(L.d_vmin.reserve(std::max<uint64_t>(1, n_keys) * 4));
+        CK(L.d_vmax.reserve(std::max<uint64_t>(1, n_keys) * 4));
+        CK(L.d_flag.reserve(std::max<uint64_t>(1, n_keys) * 4));
+        CK(L.d_rowidx.reserve((n_keys + 1) * 8));
+        CK(L.d_refcnt.reserve((size_t)b->nr * 4));
+        CK(L.d_seq_nitems.reserve(n_seq * 4));
+        CK(L.d_item_off.reserve((n_seq + 1) * 8));
+        CK(L.d_items.reserve(ic * sizeof(ScanItem)));
+        CK(L.d_list.reserve(ic * 4));
+        CK(L.d_ent_units.reserve(ic * 4));
+        CK(L.d_ent_uoff.reserve((ic + 1) * 8));
+        CK(L.d_pk.reserve(std::max<uint64_t>(1, b->n_units) * 8));
+        CK(L.d_nm.reserve(std::max<uint64_t>(1, b->n_units) * 4));
 
         DevSeqs& sq = b->sq;
         sq = DevSeqs{};
         sq.n_seq = (u32)n_seq;
-        sq.gbase = ctx->d_gbase.as<u64>();
+        sq.gbase = L.d_gbase.as<u64>();
         sq.gbase0 = ctx->h_gbase[b->r0];
-        sq.seq_region = ctx->d_seq_region.as<u32>();
-        sq.seq_leader = ctx->d_seq_leader.as<u32>();
-        sq.seq_nd = ctx->d_seq_nd.as<u32>();
-        sq.seq_doff = ctx->d_seq_doff.as<u64>();
-        sq.dlist = ctx->d_dlist.as<u32>();
-        sq.segs = ctx->d_segs.as<Seg>();
-        sq.seq_nseg = ctx->d_seq_nseg.as<u32>();
-        sq.seq_len = ctx->d_seq_len.as<u32>();
-        sq.ent_units = ctx->d_ent_units.as<u32>();
-        sq.ent_uoff = ctx->d_ent_uoff.as<u64>();
-        sq.pk = ctx->d_pk.as<u64>();
-        sq.nm = ctx->d_nm.as<u32>();
-        sq.seq_hash = ctx->d_seq_hash.as<u64>();
-        sq.seq_flags = ctx->d_seq_flags.as<u8>();
-        sq.seq_ntake = ctx->d_seq_ntake.as<u32>();
-        sq.seq_nitems = ctx->d_seq_nitems.as<u32>();
-        sq.item_off = ctx->d_item_off.as<u64>();
-        sq.items = ctx->d_items.as<ScanItem>();
+        sq.seq_region = L.d_seq_region.as<u32>();
+        sq.seq_leader = L.d_seq_leader.as<u32>();
+        sq.seq_nd = L.d_seq_nd.as<u32>();
+        sq.seq_doff = L.d_seq_doff.as<u64>();
+        sq.dlist = L.d_dlist.as<u32>();
+        sq.segs = L.d_segs.as<Seg>();
+        sq.seq_nseg = L.d_seq_nseg.as<u32>();
+        sq.seq_len = L.d_seq_len.as<u32>();
+        sq.ent_units = L.d_ent_units.as<u32>();
+        sq.ent_uoff = L.d_ent_uoff.as<u64>();
+        sq.pk = L.d_pk.as<u64>();
+        sq.nm = L.d_nm.as<u32>();
+        sq.seq_hash = L.d_seq_hash.as<u64>();
+        sq.seq_flags = L.d_seq_flags.as<u8>();
+        sq.seq_ntake = L.d_seq_ntake.as<u32>();
+        sq.seq_nitems = L.d_seq_nitems.as<u32>();
+        sq.item_off = L.d_item_off.as<u64>();
+        sq.items = L.d_items.as<ScanItem>();
         sq.n_items_cap = (u32)std::min<uint64_t>(ic, 0xffffffffu);
         sq.units_cap = b->n_units;
-        b->drh = DevRefHits{nullptr, ctx->d_refcnt.as<u32>(), 0, b->r0};
-        b->dc.C = ctx->d_C.as<u32>();
-        b->dc.cbase = ctx->d_cbase.as<u64>();
+        b->drh = DevRefHits{nullptr, L.d_refcnt.as<u32>(), 0, b->r0};
+        b->dc.C = L.d_C.as<u32>();
+        b->dc.cbase = L.d_cbase.as<u64>();
         b->dc.cbase0 = ctx->h_cbase[b->r0];
         b->d_n_items = sq.item_off + n_seq;
         return TFBS_OK;
@@ -331,22 +332,22 @@ private:
     int build_sequences(Batch& b) {
         int rc;
         const uint64_t n_seq = b.n_seq;
-        TFBS_LAUNCH(k_seq_init, b.nr, 128, 0, st)(H, b.r0, ctx->d_hap_group.as<u32>(), ctx->d_leader.as<u32>(), ctx->d_nd_in.as<u32>(), b.sq);
+        TFBS_LAUNCH(k_seq_init, b.nr, 128, 0, st)(H, b.r0, L.d_hap_group.as<u32>(), L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), b.sq);
         ++launches();
         if ((rc = scan(b.sq.seq_nd, n_seq, b.sq.seq_doff))) return rc;
         TFBS_LAUNCH(k_walk, grid_for(n_seq, 128), 128, 0, st)(db, b.sq, ~0ull, dst, 1u);
         ++launches();
         uint32_t cap = 1024;
         while (cap < 2 * n_seq) cap <<= 1;
-        CK(ctx->d_keys.reserve((size_t)cap * 8));
-        CK(ctx->d_vals.reserve((size_t)cap * 4));
-        CK(cudaMemsetAsync(ctx->d_keys.p, 0, (size_t)cap * 8, st));
-        CK(cudaMemsetAsync(ctx->d_vals.p, 0xff, (size_t)cap * 4, st));
-        CK(cudaMemsetAsync(ctx->d_ref_used.as<u32>() + b.r0, 0, (size_t)b.nr * 4, st));
-        TFBS_LAUNCH(k_seq_insert, grid_for(n_seq, 256), 256, 0, st)(b.sq, ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), cap - 1, 0u, 0u);
-        TFBS_LAUNCH(k_seq_resolve, grid_for(n_seq, 128), 128, 0, st)(db, b.sq, ctx->d_keys.as<u64>(), ctx->d_vals.as<u32>(), cap - 1, 0u, 0u, dst, 1u);
-        TFBS_LAUNCH(k_redirect, grid_for((uint64_t)b.nr * H, 256), 256, 0, st)(H, b.r0, b.nr, b.sq, ctx->d_hap_group.as<u32>(), ctx->d_ref_used.as<u32>(),
-                                                                        ctx->audit ? ctx->d_hap_flags.as<u8>() : nullptr, (u64*)nullptr, 0u, 0u, 0ull, 0u, (const u32*)nullptr);
+        CK(L.d_keys.reserve((size_t)cap * 8));
+        CK(L.d_vals.reserve((size_t)cap * 4));
+        CK(cudaMemsetAsync(L.d_keys.p, 0, (size_t)cap * 8, st));
+        CK(cudaMemsetAsync(L.d_vals.p, 0xff, (size_t)cap * 4, st));
+        CK(cudaMemsetAsync(L.d_ref_used.as<u32>() + b.r0, 0, (size_t)b.nr * 4, st));
+        TFBS_LAUNCH(k_seq_insert, grid_for(n_seq, 256), 256, 0, st)(b.sq, L.d_keys.as<u64>(), L.d_vals.as<u32>(), cap - 1, 0u, 0u);
+        TFBS_LAUNCH(k_seq_resolve, grid_for(n_seq, 128), 128, 0, st)(db, b.sq, L.d_keys.as<u64>(), L.d_vals.as<u32>(), cap - 1, 0u, 0u, dst, 1u);
+        TFBS_LAUNCH(k_redirect, grid_for((uint64_t)b.nr * H, 256), 256, 0, st)(H, b.r0, b.nr, b.sq, L.d_hap_group.as<u32>(), L.d_ref_used.as<u32>(),
+                                                                        ctx->audit ? L.d_hap_flags.as<u8>() : nullptr, (u64*)nullptr, 0u, 0u, 0ull, 0u, (const u32*)nullptr);
         launches() += 3;
         return TFBS_OK;
     }
@@ -357,28 +358,28 @@ private:
         DevSeqs& sq = b.sq;
         int rc;
         const uint64_t n_seq = b.n_seq;
-        if (b.n_c) CK(cudaMemsetAsync(ctx->d_C.p, 0, b.n_c * 4, st));
-        TFBS_LAUNCH(k_full_items<false>, grid_for(n_seq, 128), 128, 0, st)(sq, ctx->d_ref_used.as<u32>());
+        if (b.n_c) CK(cudaMemsetAsync(L.d_C.p, 0, b.n_c * 4, st));
+        TFBS_LAUNCH(k_full_items<false>, grid_for(n_seq, 128), 128, 0, st)(sq, L.d_ref_used.as<u32>());
         ++launches();
         if ((rc = scan(sq.seq_nitems, n_seq, sq.item_off))) return rc;
-        TFBS_LAUNCH(k_full_items<true>, grid_for(n_seq, 128), 128, 0, st)(sq, ctx->d_ref_used.as<u32>());
-        TFBS_LAUNCH(k_vitem_units, grid_for(n_seq, 256), 256, 0, st)(sq, b.d_n_items, ctx->d_list.as<u32>());
+        TFBS_LAUNCH(k_full_items<true>, grid_for(n_seq, 128), 128, 0, st)(sq, L.d_ref_used.as<u32>());
+        TFBS_LAUNCH(k_vitem_units, grid_for(n_seq, 256), 256, 0, st)(sq, b.d_n_items, L.d_list.as<u32>());
         launches() += 2;
-        if ((rc = device_scan(ctx, sq.ent_units, n_seq, b.d_n_items, sq.ent_uoff, &launches()))) return rc;
+        if ((rc = device_scan(ctx, L, sq.ent_units, n_seq, b.d_n_items, sq.ent_uoff, &launches()))) return rc;
         CK(cudaMemcpyAsync((char*)ctx->h_totals.p + 24, b.d_n_items, 8, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         b.n_list_host = ctx->h_totals.as<uint64_t>()[3];
         uint64_t table_bytes = 0;
         if (b.n_list_host) {
-            TFBS_LAUNCH(k_emit_list, grid_for(b.n_list_host * EMIT_LANES, 256), 256, 0, st)(db, sq, ctx->d_list.as<u32>(), b.d_n_items);
-            TFBS_LAUNCH(k_item_stats, grid_for(b.n_list_host, 256), 256, 0, st)(sq, ctx->dpat, ctx->d_list.as<u32>(), b.d_n_items, dst);
+            TFBS_LAUNCH(k_emit_list, grid_for(b.n_list_host * EMIT_LANES, 256), 256, 0, st)(db, sq, L.d_list.as<u32>(), b.d_n_items);
+            TFBS_LAUNCH(k_item_stats, grid_for(b.n_list_host, 256), 256, 0, st)(sq, ctx->dpat, L.d_list.as<u32>(), b.d_n_items, dst);
             launches() += 2;
         }
         CK(cudaEventRecord(ctx->ev[8], st));
         for (uint32_t c = 0; c < ctx->cp.chunks.size() && b.n_list_host; ++c) {
             CK(cudaMemsetAsync(&dst->work_counter, 0, 4, st));
-            if (wide) TFBS_LAUNCH(k_scan<2>, scan_grid, SCAN_CTA, smem_bytes, st)(db, sq, ctx->dpat, b.dc, dm, b.drh, no_cf, 0, ctx->d_list.as<u32>(), b.d_n_items, 1u, dst, c);
-            else TFBS_LAUNCH(k_scan<3>, scan_grid, SCAN_CTA, smem_bytes, st)(db, sq, ctx->dpat, b.dc, dm, b.drh, no_cf, 0, ctx->d_list.as<u32>(), b.d_n_items, 1u, dst, c);
+            if (wide) TFBS_LAUNCH(k_scan<2>, scan_grid, SCAN_CTA, smem_bytes, st)(db, sq, ctx->dpat, b.dc, dm, b.drh, no_cf, 0, L.d_list.as<u32>(), b.d_n_items, 1u, dst, c);
+            else TFBS_LAUNCH(k_scan<3>, scan_grid, SCAN_CTA, smem_bytes, st)(db, sq, ctx->dpat, b.dc, dm, b.drh, no_cf, 0, L.d_list.as<u32>(), b.d_n_items, 1u, dst, c);
             ++launches();
             ++stats().scan_launches;
             table_bytes += (uint64_t)ctx->cp.chunks[c].tbl_words * 8 * scan_grid;
@@ -396,12 +397,12 @@ private:
     int rows_pass(Batch& b) {
         if (!b.n_keys) return TFBS_OK;
         int rc;
-        TFBS_LAUNCH(k_rows_minmax, b.nr, 128, 0, st)(db, b.r0, ctx->d_hap_group.as<u32>(), b.dc, ctx->d_gbase.as<u64>(), n_pid, ctx->d_kbase.as<u64>(),
-                                          ctx->h_kbase[b.r0], ctx->rows_mode, ctx->d_vmin.as<u32>(), ctx->d_vmax.as<u32>(), ctx->d_flag.as<u32>(),
+        TFBS_LAUNCH(k_rows_minmax, b.nr, 128, 0, st)(db, b.r0, L.d_hap_group.as<u32>(), b.dc, L.d_gbase.as<u64>(), n_pid, L.d_kbase.as<u64>(),
+                                          ctx->h_kbase[b.r0], ctx->rows_mode, L.d_vmin.as<u32>(), L.d_vmax.as<u32>(), L.d_flag.as<u32>(),
                                           &dst->max_count);
         ++launches();
-        if ((rc = scan(ctx->d_flag.as<u32>(), b.n_keys, ctx->d_rowidx.as<u64>()))) return rc;
-        CK(cudaMemcpyAsync(ctx->h_totals.p, ctx->d_rowidx.as<u64>() + b.n_keys, 8, cudaMemcpyDeviceToHost, st));
+        if ((rc = scan(L.d_flag.as<u32>(), b.n_keys, L.d_rowidx.as<u64>()))) return rc;
+        CK(cudaMemcpyAsync(ctx->h_totals.p, L.d_rowidx.as<u64>() + b.n_keys, 8, cudaMemcpyDeviceToHost, st));
         return TFBS_OK;
     }
 
@@ -409,8 +410,8 @@ private:
     int count_and_filter(Batch* bp) {
         Batch& b = *bp;
         int rc;
-        TFBS_LAUNCH(k_nominal, grid_for((uint64_t)b.nr * H, 256), 256, 0, st)(db, b.r0, b.nr, ctx->d_hap_group.as<u32>(), b.sq, ctx->dpat, dst);
-        TFBS_LAUNCH(k_seq_stats, grid_for(b.n_seq, 256), 256, 0, st)(b.sq, ctx->dpat, ctx->d_ref_used.as<u32>(), dst);
+        TFBS_LAUNCH(k_nominal, grid_for((uint64_t)b.nr * H, 256), 256, 0, st)(db, b.r0, b.nr, L.d_hap_group.as<u32>(), b.sq, ctx->dpat, dst);
+        TFBS_LAUNCH(k_seq_stats, grid_for(b.n_seq, 256), 256, 0, st)(b.sq, ctx->dpat, L.d_ref_used.as<u32>(), dst);
         launches() += 2;
         if ((rc = rows_pass(b))) return rc;
         if ((rc = read_status(&b.hs))) return rc;
@@ -450,13 +451,13 @@ private:
                 res.row_bytes = eb;
             }
             eb = res.row_bytes;
-            CK(ctx->d_rows_region.reserve(batch_rows * 4));
-            CK(ctx->d_rows_inner.reserve(batch_rows * 4));
-            CK(ctx->d_rows_pid.reserve(batch_rows * 2));
-            CK(ctx->d_rows_vmin.reserve(batch_rows * 4));
-            CK(ctx->d_rows_vmax.reserve(batch_rows * 4));
-            CK(ctx->d_rows_left.reserve(batch_rows * S * eb));
-            CK(ctx->d_rows_right.reserve(batch_rows * S * eb));
+            CK(L.d_rows_region.reserve(batch_rows * 4));
+            CK(L.d_rows_inner.reserve(batch_rows * 4));
+            CK(L.d_rows_pid.reserve(batch_rows * 2));
+            CK(L.d_rows_vmin.reserve(batch_rows * 4));
+            CK(L.d_rows_vmax.reserve(batch_rows * 4));
+            CK(L.d_rows_left.reserve(batch_rows * S * eb));
+            CK(L.d_rows_right.reserve(batch_rows * S * eb));
             CK(res.h_region.reserve(tot * 4, true));
             CK(res.h_inner.reserve(tot * 4, true));
             CK(res.h_pid.reserve(tot * 2, true));
@@ -464,12 +465,12 @@ private:
             CK(res.h_vmax.reserve(tot * 4, true));
             CK(res.h_left.reserve(tot * S * eb, true));
             CK(res.h_right.reserve(tot * S * eb, true));
-            DevRows dr{ctx->d_rows_region.as<u32>(), ctx->d_rows_inner.as<u32>(), ctx->d_rows_pid.as<u16>(), ctx->d_rows_vmin.as<u32>(),
-                       ctx->d_rows_vmax.as<u32>(), ctx->d_rows_left.p, ctx->d_rows_right.p};
+            DevRows dr{L.d_rows_region.as<u32>(), L.d_rows_inner.as<u32>(), L.d_rows_pid.as<u16>(), L.d_rows_vmin.as<u32>(),
+                       L.d_rows_vmax.as<u32>(), L.d_rows_left.p, L.d_rows_right.p};
 #define TFBS_ROWS_WRITE(T)                                                                                                              \
-    TFBS_LAUNCH(k_rows_write<T>, grid_for(n_keys * 32, 256), 256, 0, st)(db, b.r0, b.nr, ctx->d_hap_group.as<u32>(), b.dc, n_pid, ctx->d_pid_list.as<u16>(), \
-                                                                ctx->d_kbase.as<u64>(), ctx->h_kbase[b.r0], n_keys, ctx->d_vmin.as<u32>(),   \
-                                                                ctx->d_vmax.as<u32>(), ctx->d_flag.as<u32>(), ctx->d_rowidx.as<u64>(), dr, 0)
+    TFBS_LAUNCH(k_rows_write<T>, grid_for(n_keys * 32, 256), 256, 0, st)(db, b.r0, b.nr, L.d_hap_group.as<u32>(), b.dc, n_pid, ctx->d_pid_list.as<u16>(), \
+                                                                L.d_kbase.as<u64>(), ctx->h_kbase[b.r0], n_keys, L.d_vmin.as<u32>(),   \
+                                                                L.d_vmax.as<u32>(), L.d_flag.as<u32>(), L.d_rowidx.as<u64>(), dr, 0)
             if (eb == 1) TFBS_ROWS_WRITE(u8);
             else if (eb == 2) TFBS_ROWS_WRITE(u16);
             else TFBS_ROWS_WRITE(u32);
@@ -509,11 +510,11 @@ private:
         CK(cudaEventRecord(ctx->ev[6], st));
         if (ctx->record_matches) {
             CK(ctx->h_hap_group.reserve(RH * 4, false));
-            CK(cudaMemcpyAsync(ctx->h_hap_group.p, ctx->d_hap_group.p, RH * 4, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(ctx->h_hap_group.p, L.d_hap_group.p, RH * 4, cudaMemcpyDeviceToHost, st));
         }
         if (ctx->audit) {
             CK(ctx->h_hap_flags.reserve(RH, false));
-            CK(cudaMemcpyAsync(ctx->h_hap_flags.p, ctx->d_hap_flags.p, RH, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(ctx->h_hap_flags.p, L.d_hap_flags.p, RH, cudaMemcpyDeviceToHost, st));
         }
         DevStatus hs;
         int rc = read_status(&hs);

@@ -1,11 +1,13 @@
 // tfbs.cu -- C ABI (include/tfbs.h) over the sm_100a kernels in kernels.cuh.
 //
-//   host_common.hpp      the context: device / pinned buffers, a block on the device, two slots of blocks in flight, three streams
+//   host_common.hpp      the context: device / pinned buffers, a block on the device, two slots of blocks in flight, two lanes of
+//                        streams and scratch
 //   pipeline_config.hpp  the default path: configurations + fan-out into grouped rows, enqueued without a single host round trip
 //   pipeline_full.hpp    every distinct haplotype scored in full like the reference ("delta" = 0, the hit list, the audit)
 //
-// One context = one CUDA device.  tfbs_submit_block copies a block on the copy-in stream and enqueues its kernels on the kernel
-// stream; tfbs_collect waits for the oldest block, fetches its rows on the copy-out stream and is the only place the host waits.
+// One context = one CUDA device.  tfbs_submit_block copies a block on the copy-in stream of its lane and enqueues its kernels on the
+// lane's kernel stream; tfbs_collect waits for the oldest block, fetches its rows on the lane's copy-out stream and is the only place
+// the host waits.
 // There is no CPU fallback: every entry point that computes fails with TFBS_ERR_CUDA when no device is usable.
 #include "host_common.hpp"
 #include "pipeline_config.hpp"
@@ -15,21 +17,28 @@ namespace {
 
 bool wants_full(const tfbs_ctx* ctx) { return !ctx->delta || ctx->record_matches || ctx->audit; }
 
-// Run (full path) or enqueue (configuration path) the block `in` on the next free slot.
-int start_block(tfbs_ctx* ctx, BlockDev* in, bool copies_pending) {
+// Run (full path) or enqueue (configuration path) a block on the next free slot: the block `in` that is on the device already, or
+// (in == NULL) the caller's block `b`, copied into the slot first.
+int start_block(tfbs_ctx* ctx, BlockDev* in, const tfbs_block* b) {
     if (!ctx->have_patterns) return fail(ctx, TFBS_ERR_STATE, "tfbs_set_patterns has not been called");
-    if (!in->valid) return fail(ctx, TFBS_ERR_STATE, "no block has been uploaded");
     if (ctx->in_flight >= 2) return fail(ctx, TFBS_ERR_STATE, "two blocks are already in flight on this context: call tfbs_collect first");
     const int k = (ctx->head + ctx->in_flight) % 2;
     Slot* slot = &ctx->slot[k];
+    slot->lane = ctx->dual_stream && !wants_full(ctx) ? k : 0;  // option "dual_stream": consecutive blocks run on different lanes
+    Lane& L = ctx->lane[slot->lane];
+    const bool copies_pending = !in;
+    int rc;
+    if (copies_pending) {
+        if ((rc = upload_block(ctx, b, &slot->own, L.stream_in))) return rc;
+        in = &slot->own;
+    }
+    if (!in->valid) return fail(ctx, TFBS_ERR_STATE, "no block has been uploaded");
     slot->in = in;
     slot->state = 0;
-    if (copies_pending) CK(cudaEventRecord(slot->ev_in, ctx->stream_in));
-    else CK(cudaEventRecord(slot->ev_in, ctx->stream));
-    int rc;
+    CK(cudaEventRecord(slot->ev_in, copies_pending ? L.stream_in : L.stream));
     if (wants_full(ctx)) {
         if (ctx->in_flight) return fail(ctx, TFBS_ERR_STATE, "the full scan (delta = 0, record_matches, audit) runs one block at a time: call tfbs_collect first");
-        CK(cudaStreamWaitEvent(ctx->stream, slot->ev_in, 0));
+        CK(cudaStreamWaitEvent(L.stream, slot->ev_in, 0));
         slot->full_mode = true;
         rc = FullPipeline(ctx, slot).run();
         if (rc) return rc;
@@ -112,7 +121,7 @@ int install_patterns(tfbs_ctx* ctx, const tfbs_pattern* patterns, uint32_t n_pat
     const CompiledPatterns& c = ctx->cp;
     std::vector<uint64_t> table = c.table;
     table.resize(table.size() + 2, 0);  // 128-bit loads may read one word past the end
-    cudaStream_t st = ctx->stream;
+    cudaStream_t st = ctx->lane[0].stream;
     if ((rc = upload_on(ctx, st, ctx->d_table, table.data(), table.size(), nullptr))) return rc;
     if ((rc = upload_on(ctx, st, ctx->d_chunks, c.chunks.data(), c.chunks.size(), nullptr))) return rc;
     if ((rc = upload_on(ctx, st, ctx->d_runs, c.runs.data(), c.runs.size(), nullptr))) return rc;
@@ -147,26 +156,6 @@ int drain(tfbs_ctx* ctx) {
     return rc;
 }
 
-// ---- option "dual_stream": routing between a context and its twin ----
-bool dual_active(const tfbs_ctx* ctx) { return ctx->dual && ctx->twin && !ctx->bypass && !wants_full(ctx); }
-void share_hints(tfbs_ctx* a, tfbs_ctx* b) {  // what one twin learnt about the blocks' sizes serves the other
-    Caps& x = a->hint;
-    Caps& y = b->hint;
-#define TFBS_BOTH(f) x.f = y.f = std::max(x.f, y.f)
-    TFBS_BOTH(seq); TFBS_BOTH(d); TFBS_BOTH(cfg); TFBS_BOTH(vd); TFBS_BOTH(items); TFBS_BOTH(units); TFBS_BOTH(dwords); TFBS_BOTH(rows);
-    TFBS_BOTH(rowwords); TFBS_BOTH(capr); TFBS_BOTH(groups); TFBS_BOTH(terms);
-#undef TFBS_BOTH
-}
-int twin_failed(tfbs_ctx* ctx, int rc) {
-    if (rc != TFBS_OK) ctx->err = ctx->twin->err;
-    return rc;
-}
-struct Bypass {  // the public entry points call themselves once more for "this context itself"
-    tfbs_ctx* c;
-    explicit Bypass(tfbs_ctx* ctx) : c(ctx) { c->bypass = true; }
-    ~Bypass() { c->bypass = false; }
-};
-
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------
@@ -196,20 +185,18 @@ int tfbs_create(int device, tfbs_ctx** out) {
     }
     tfbs_ctx* ctx = new tfbs_ctx();
     ctx->device = device;
-    if ((e = cudaGetDeviceProperties(&ctx->prop, device)) != cudaSuccess ||
-        (e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess ||
-        (e = cudaStreamCreateWithFlags(&ctx->stream_in, cudaStreamNonBlocking)) != cudaSuccess ||
-        (e = cudaStreamCreateWithFlags(&ctx->stream_out, cudaStreamNonBlocking)) != cudaSuccess) {
+    e = cudaGetDeviceProperties(&ctx->prop, device);
+    for (Lane& L : ctx->lane)
+        for (cudaStream_t* s : {&L.stream, &L.stream_in, &L.stream_out})
+            if (e == cudaSuccess) e = cudaStreamCreateWithFlags(s, cudaStreamNonBlocking);
+    if (e != cudaSuccess) {
         g_create_error = std::string("CUDA initialisation failed: ") + cudaGetErrorString(e);
-        delete ctx;
+        tfbs_destroy(ctx);
         return TFBS_ERR_CUDA;
     }
     if (ctx->prop.major < 10) {
         g_create_error = std::string("device ") + ctx->prop.name + " is not sm_100-class; this library carries sm_100a code only";
-        cudaStreamDestroy(ctx->stream);
-        cudaStreamDestroy(ctx->stream_in);
-        cudaStreamDestroy(ctx->stream_out);
-        delete ctx;
+        tfbs_destroy(ctx);
         return TFBS_ERR_CUDA;
     }
     for (auto& ev : ctx->ev) cudaEventCreate(&ev);
@@ -218,8 +205,9 @@ int tfbs_create(int device, tfbs_ctx** out) {
         cudaEventCreate(&s.ev_done);
         for (auto& ev : s.ev_t) cudaEventCreate(&ev);
     }
-    TFBS_LAUNCH(k_hash_pow_init, 1, 32, 0, ctx->stream)();  // ordered before every pipeline: they are enqueued on the same stream
-    if ((e = cudaGetLastError()) != cudaSuccess) {
+    // every pipeline reads its table; lane 1's streams are not ordered after lane 0's, so the table is complete before the call returns
+    TFBS_LAUNCH(k_hash_pow_init, 1, 32, 0, ctx->lane[0].stream)();
+    if ((e = cudaGetLastError()) != cudaSuccess || (e = cudaStreamSynchronize(ctx->lane[0].stream)) != cudaSuccess) {
         g_create_error = std::string("CUDA initialisation failed: ") + cudaGetErrorString(e);
         tfbs_destroy(ctx);
         return TFBS_ERR_CUDA;
@@ -230,12 +218,10 @@ int tfbs_create(int device, tfbs_ctx** out) {
 
 void tfbs_destroy(tfbs_ctx* ctx) {
     if (!ctx) return;
-    if (ctx->twin) { tfbs_destroy(ctx->twin); ctx->twin = nullptr; }
-    if (ctx->is_twin) ctx->arena = nullptr;  // the arena is page-locked by the owner of the pair
     cudaSetDevice(ctx->device);
-    cudaStreamSynchronize(ctx->stream_in);
-    cudaStreamSynchronize(ctx->stream);
-    cudaStreamSynchronize(ctx->stream_out);
+    for (Lane& L : ctx->lane)
+        for (cudaStream_t s : {L.stream_in, L.stream, L.stream_out})
+            if (s) cudaStreamSynchronize(s);
     for (auto& ev : ctx->ev)
         if (ev) cudaEventDestroy(ev);
     for (Slot& s : ctx->slot) {
@@ -245,9 +231,9 @@ void tfbs_destroy(tfbs_ctx* ctx) {
             if (ev) cudaEventDestroy(ev);
     }
     if (ctx->arena) cudaHostUnregister(ctx->arena);
-    cudaStreamDestroy(ctx->stream);
-    cudaStreamDestroy(ctx->stream_in);
-    cudaStreamDestroy(ctx->stream_out);
+    for (Lane& L : ctx->lane)
+        for (cudaStream_t s : {L.stream, L.stream_in, L.stream_out})
+            if (s) cudaStreamDestroy(s);
     delete ctx;
 }
 
@@ -283,25 +269,10 @@ int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value) {
         ctx->rows_width = (int)value;
     }
     else if (k == "dual_stream") {
-        if (ctx->is_twin) return TFBS_OK;
-        if (!ctx->order.empty() || ctx->in_flight) return fail(ctx, TFBS_ERR_STATE, "dual_stream with blocks in flight: call tfbs_collect first");
-        if (value && !ctx->twin) {
-            tfbs_ctx* t = nullptr;
-            int rc = tfbs_create(ctx->device, &t);
-            if (rc != TFBS_OK) return fail(ctx, rc, g_create_error);
-            t->is_twin = true;
-            for (const auto& kv : ctx->opt_log) tfbs_set_option(t, kv.first.c_str(), kv.second);
-            ctx->twin = t;
-            if (ctx->have_patterns && (rc = twin_failed(ctx, tfbs_set_patterns(t, ctx->orig_patterns.data(), (uint32_t)ctx->orig_patterns.size())))) return rc;
-            if (ctx->arena) return fail(ctx, TFBS_ERR_STATE, "set dual_stream before tfbs_set_result_arena");
-        }
-        ctx->dual = value != 0;
-        ctx->next_target = 0;
-        return TFBS_OK;
+        if (ctx->in_flight) return fail(ctx, TFBS_ERR_STATE, "dual_stream with blocks in flight: call tfbs_collect first");
+        ctx->dual_stream = value != 0;
     }
     else return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "unknown option " + k);
-    ctx->opt_log.emplace_back(k, value);
-    if (ctx->twin) return twin_failed(ctx, tfbs_set_option(ctx->twin, key, value));
     return TFBS_OK;
 }
 
@@ -319,7 +290,6 @@ int tfbs_set_patterns(tfbs_ctx* ctx, const tfbs_pattern* patterns, uint32_t n_pa
         } else {
             ctx->orig_patterns[i].weights = nullptr;
         }
-    if (ctx->twin) return twin_failed(ctx, tfbs_set_patterns(ctx->twin, patterns, n_patterns));
     return TFBS_OK;
 }
 
@@ -328,68 +298,29 @@ int tfbs_upload_block(tfbs_ctx* ctx, const tfbs_block* block) {
     CK(cudaSetDevice(ctx->device));
     int rc = drain(ctx);  // the resident block may still be read by runs in flight
     if (rc) return rc;
-    rc = upload_block(ctx, block, &ctx->resident, ctx->stream_in);
+    rc = upload_block(ctx, block, &ctx->resident, ctx->lane[0].stream_in);
     if (rc) return rc;
-    CK(cudaStreamSynchronize(ctx->stream_in));
+    CK(cudaStreamSynchronize(ctx->lane[0].stream_in));
     ctx->last_block = &ctx->resident;
-    if (ctx->twin && ctx->dual) return twin_failed(ctx, tfbs_upload_block(ctx->twin, block));
     return TFBS_OK;
 }
 
 int tfbs_run_resident(tfbs_ctx* ctx) {
     if (!ctx) return TFBS_ERR_INVALID_ARGUMENT;
-    if (dual_active(ctx)) {
-        if (ctx->order.size() >= 2) return fail(ctx, TFBS_ERR_STATE, "two blocks are already in flight on this context: call tfbs_collect first");
-        const int tgt = ctx->next_target;
-        int rc;
-        if (tgt) rc = twin_failed(ctx, tfbs_run_resident(ctx->twin));
-        else { Bypass by(ctx); rc = tfbs_run_resident(ctx); }
-        if (rc) return rc;
-        ctx->order.push_back(tgt);
-        ctx->next_target ^= 1;
-        return TFBS_OK;
-    }
     CK(cudaSetDevice(ctx->device));
     if (!ctx->resident.valid) return fail(ctx, TFBS_ERR_STATE, "no block has been uploaded");
-    return start_block(ctx, &ctx->resident, false);
+    return start_block(ctx, &ctx->resident, nullptr);
 }
 
 int tfbs_submit_block(tfbs_ctx* ctx, const tfbs_block* block) {
     if (!ctx) return TFBS_ERR_INVALID_ARGUMENT;
-    if (dual_active(ctx)) {
-        if (ctx->order.size() >= 2) return fail(ctx, TFBS_ERR_STATE, "two blocks are already in flight on this context: call tfbs_collect first");
-        const int tgt = ctx->next_target;
-        int rc;
-        if (tgt) rc = twin_failed(ctx, tfbs_submit_block(ctx->twin, block));
-        else { Bypass by(ctx); rc = tfbs_submit_block(ctx, block); }
-        if (rc) return rc;
-        ctx->order.push_back(tgt);
-        ctx->next_target ^= 1;
-        return TFBS_OK;
-    }
     CK(cudaSetDevice(ctx->device));
-    if (!ctx->have_patterns) return fail(ctx, TFBS_ERR_STATE, "tfbs_set_patterns has not been called");
-    if (ctx->in_flight >= 2) return fail(ctx, TFBS_ERR_STATE, "two blocks are already in flight on this context: call tfbs_collect first");
-    Slot* slot = &ctx->slot[(ctx->head + ctx->in_flight) % 2];
-    int rc = upload_block(ctx, block, &slot->own, ctx->stream_in);
-    if (rc) return rc;
-    return start_block(ctx, &slot->own, true);
+    return start_block(ctx, nullptr, block);
 }
 
 int tfbs_collect(tfbs_ctx* ctx, tfbs_rows* out) {
     if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
-    if (ctx->twin && !ctx->bypass && !ctx->order.empty()) {  // the oldest block in flight, whichever twin has it
-        const int tgt = ctx->order.front();
-        ctx->order.pop_front();
-        ctx->last_target = tgt;
-        int rc;
-        if (tgt) rc = twin_failed(ctx, tfbs_collect(ctx->twin, out));
-        else { Bypass by(ctx); rc = tfbs_collect(ctx, out); }
-        share_hints(ctx, ctx->twin);
-        return rc;
-    }
     CK(cudaSetDevice(ctx->device));
-    if (!ctx->bypass) ctx->last_target = 0;  // (a twin's results are not this block's)
     ctx->att_state = tfbs_ctx::ATT_NONE;
     Slot* slot = nullptr;
     int rc = finish_oldest(ctx, &slot);
@@ -413,18 +344,7 @@ int tfbs_collect(tfbs_ctx* ctx, tfbs_rows* out) {
 
 int tfbs_collect_grouped(tfbs_ctx* ctx, tfbs_grouped_rows* out) {
     if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
-    if (ctx->twin && !ctx->bypass && !ctx->order.empty()) {
-        const int tgt = ctx->order.front();
-        ctx->order.pop_front();
-        ctx->last_target = tgt;
-        int rc;
-        if (tgt) rc = twin_failed(ctx, tfbs_collect_grouped(ctx->twin, out));
-        else { Bypass by(ctx); rc = tfbs_collect_grouped(ctx, out); }
-        share_hints(ctx, ctx->twin);
-        return rc;
-    }
     CK(cudaSetDevice(ctx->device));
-    if (!ctx->bypass) ctx->last_target = 0;
     ctx->att_state = tfbs_ctx::ATT_NONE;
     Slot* slot = nullptr;
     int rc = finish_oldest(ctx, &slot);
@@ -462,19 +382,8 @@ int tfbs_set_result_arena(tfbs_ctx* ctx, void* base, size_t bytes) {
     CK(cudaSetDevice(ctx->device));
     int rc = quiesce(ctx);
     if (rc) return rc;
-    if (ctx->in_flight || !ctx->order.empty()) return fail(ctx, TFBS_ERR_STATE, "tfbs_set_result_arena with blocks in flight: call tfbs_collect first");
-    if (ctx->twin) {  // the twin writes the second half of the same arena (page-locked once, by this context)
-        tfbs_ctx* t = ctx->twin;
-        if ((rc = quiesce(t))) return twin_failed(ctx, rc);
-        for (Slot& s : t->slot)
-            for (HostBuf* hb : {&s.res.h_region, &s.res.h_inner, &s.res.h_pid, &s.res.h_vmin, &s.res.h_vmax, &s.res.h_base, &s.res.h_bits, &s.res.h_off,
-                                &s.res.h_packed, &s.res.h_ngroups, &s.res.h_hg})
-                if (!hb->owned) hb->bind(nullptr, 0);
-        t->arena = nullptr;
-        t->arena_bytes = 0;
-        t->fixed_half = ctx->fixed_half = -1;
-        ctx->next_target = 0;
-    }
+    if (ctx->in_flight) return fail(ctx, TFBS_ERR_STATE, "tfbs_set_result_arena with blocks in flight: call tfbs_collect first");
+    ctx->head = 0;  // a block's rows go to the half of its slot: the next block to the first half
     if (ctx->arena) {
         cudaHostUnregister(ctx->arena);
         for (Slot& s : ctx->slot)
@@ -491,12 +400,6 @@ int tfbs_set_result_arena(tfbs_ctx* ctx, void* base, size_t bytes) {
     ctx->arena_bytes = bytes;
     memset(base, 0, sizeof(tfbs_arena_header));
     memset((uint8_t*)base + bytes / 2, 0, sizeof(tfbs_arena_header));
-    if (ctx->twin && ctx->dual) {
-        ctx->twin->arena = ctx->arena;
-        ctx->twin->arena_bytes = bytes;
-        ctx->twin->fixed_half = 1;
-        ctx->fixed_half = 0;
-    }
     return TFBS_OK;
 }
 
@@ -584,7 +487,7 @@ int tfbs_merge_regions(tfbs_ctx* ctx, const uint64_t* start, const uint64_t* end
     if (n == 0) return TFBS_OK;
     if (n > 0x7fffffffull) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "too many ranges");
     CK(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
+    cudaStream_t st = ctx->lane[0].stream;
     DevBuf d_in, d_out, d_order, d_misc;
     CK(d_in.reserve(n * 16));
     CK(d_out.reserve(n * 16));
@@ -611,7 +514,6 @@ int tfbs_merge_regions(tfbs_ctx* ctx, const uint64_t* start, const uint64_t* end
 
 int tfbs_get_attribution(tfbs_ctx* ctx, tfbs_attribution* out) {
     if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
-    if (ctx->twin && !ctx->bypass && ctx->last_target == 1) return twin_failed(ctx, tfbs_get_attribution(ctx->twin, out));
     switch (ctx->att_state) {
     case tfbs_ctx::ATT_NONE: return fail(ctx, TFBS_ERR_STATE, "no block has been collected yet (tfbs_collect / tfbs_collect_grouped first)");
     case tfbs_ctx::ATT_OFF: return fail(ctx, TFBS_ERR_STATE, "option attribution was off for the last block: set it to 1 before the run");
@@ -678,7 +580,7 @@ int tfbs_audit_block(tfbs_ctx* ctx, tfbs_audit* out) {
     auto run_once = [&]() -> int {
         ctx->in_flight = 0;
         ctx->head = 0;
-        return start_block(ctx, blk, false);
+        return start_block(ctx, blk, nullptr);
     };
     // a run that overflows the match buffer says how many hits there were: run it once more with a buffer of that size
     auto run_recorded = [&]() -> int {
@@ -736,7 +638,6 @@ int tfbs_audit_block(tfbs_ctx* ctx, tfbs_audit* out) {
 
 int tfbs_get_stats(const tfbs_ctx* ctx, tfbs_stats* out) {
     if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
-    if (ctx->twin && ctx->last_target == 1) return tfbs_get_stats(ctx->twin, out);
     if (ctx->last < 0) memset(out, 0, sizeof *out);
     else *out = ctx->slot[ctx->last].stats;
     return TFBS_OK;
@@ -744,7 +645,6 @@ int tfbs_get_stats(const tfbs_ctx* ctx, tfbs_stats* out) {
 
 int tfbs_fanout_info(const tfbs_ctx* ctx, uint32_t* smem_groups, uint32_t* groups_cap, uint32_t* ctas, uint32_t* in_device_memory) {
     if (!ctx || !smem_groups || !groups_cap || !ctas || !in_device_memory) return TFBS_ERR_INVALID_ARGUMENT;
-    if (ctx->twin && ctx->last_target == 1) return tfbs_fanout_info(ctx->twin, smem_groups, groups_cap, ctas, in_device_memory);
     *smem_groups = fan_smem_groups(ctx->prop);
     const Slot* s = ctx->last < 0 ? nullptr : &ctx->slot[ctx->last];
     const bool ran = s && !s->full_mode;
@@ -763,6 +663,6 @@ int tfbs_host_unregister(void* ptr) {
     return cudaHostUnregister(ptr) == cudaSuccess ? TFBS_OK : TFBS_ERR_CUDA;
 }
 
-void* tfbs_stream(const tfbs_ctx* ctx) { return ctx ? (void*)ctx->stream : nullptr; }
+void* tfbs_stream(const tfbs_ctx* ctx) { return ctx ? (void*)ctx->lane[0].stream : nullptr; }
 
 }  // extern "C"

@@ -309,7 +309,10 @@ const char* tfbs_last_error(const tfbs_ctx* ctx);
  * "fan_vector" (0 = automatic, the default: the fan-out keeps its per-group count vectors in shared memory and switches to device
  * memory when a region of the block may have more distinct haplotypes than shared memory holds, 53,120; 1 = always in device
  * memory, for tests -- results are the same either way), "attribution" (0 = off, the default; 1 = the default path also keeps the
- * per-row count differences of every configuration for tfbs_get_attribution: the rows themselves do not change). */
+ * per-row count differences of every configuration for tfbs_get_attribution: the rows themselves do not change), "dual_stream"
+ * (0 = off, the default; 1 = consecutive blocks of the default scoring mode alternate between two lanes, each with its own kernel
+ * and copy streams and its own device scratch, so that the kernels of the two blocks in flight overlap on the device: worth it when
+ * blocks are small, while a second lane doubles the scratch of large blocks; fails with TFBS_ERR_STATE while blocks are in flight). */
 int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value);
 
 /* Replace the pattern list (the reference's pwm_list, src/main.rs:237). */
@@ -420,7 +423,8 @@ int tfbs_fanout_info(const tfbs_ctx* ctx, uint32_t* smem_groups, uint32_t* group
 int tfbs_host_register(void* ptr, size_t bytes);
 int tfbs_host_unregister(void* ptr);
 
-/* The CUDA stream (cudaStream_t) all work of this context is enqueued on. */
+/* The kernel stream (cudaStream_t) of the context's first lane: the pipelines of its blocks run on it, except, with option
+ * "dual_stream", those of every other block of the default scoring mode, which run on the second lane's own kernel stream. */
 void* tfbs_stream(const tfbs_ctx* ctx);
 
 #ifdef __cplusplus

@@ -353,7 +353,7 @@ def test_small_deterministic_across_contexts_repeats_and_fanout():
 
 @pytest.mark.gpu
 def test_small_two_blocks_in_flight_dual_stream():
-    """Blocks alternate between two streams, two in flight: each block's attribution equals the one of a context of its own."""
+    """Blocks alternate between the two lanes, two in flight: each block's attribution equals the one of a context of its own."""
     ps, b1 = small_cohort(1)
     b2 = small_cohort(2)[1]
     want = [run(ps, b, binding.ROWS_VARYING)[1] for b in (b1, b2, b1)]
@@ -369,7 +369,7 @@ def test_small_two_blocks_in_flight_dual_stream():
         ctx.submit_block(b1)
         got.append((ctx.collect(), ctx.attribution()))
         got.append((own(ctx.collect_grouped()), ctx.attribution()))
-        # a full scan on the context itself after the last block came from the second stream: refused, not the older attribution
+        # a full scan (always on lane 0) after blocks on both lanes: refused, not the older attribution
         ctx.set_option("delta", 0)
         ctx.submit_block(b2)
         ctx.collect()

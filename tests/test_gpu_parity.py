@@ -234,20 +234,25 @@ def test_threshold_boundary_ties():
     assert counts[0] >= counts[1] >= counts[2] >= counts[3] and counts[0] > counts[3]
 
 
-def test_audit_enumerates_ties_and_flags():
-    """tfbs_audit_block: the windows scoring exactly min_score (strict >, pattern.rs:151) and the truncated / overwritten haplotypes
-    (haplotype.rs:144-149, :84) are the same sets the oracle finds; the context is left with a normal run of the block."""
+def tie_patterns_and_block():
+    """Patterns with coarse weights (many attainable ties) and a cohort with dense indels, overwrites and truncations."""
     rng = np.random.default_rng(3)
-    w = rng.integers(-3, 4, size=(8, 4)).astype(np.int32) * 100   # coarse weights: many attainable ties
+    w = rng.integers(-3, 4, size=(8, 4)).astype(np.int32) * 100
     best = int(w.max(axis=1).sum())
     pats = [{"weights": w, "min_score": best - 400, "pattern_id": 1, "direction": 0},
             {"weights": w[::-1, ::-1].copy(), "min_score": best - 400, "pattern_id": 1, "direction": 1}]
     pats += synth.make_pwms(2, seed=77, lmin=6, lmax=14)
     for p in pats[2:]:
         p["pattern_id"] += 2
-    ps = PatternSet(pats)
     blk = synth.make_cohort(12, 24, seed=13, lmax_pattern=14, region_len=(100, 500), variant_rate=1 / 10.0, frac_ins=0.15, frac_del=0.2,
                             same_pos_frac=0.1, n_runs=3, two_beds=True)
+    return PatternSet(pats), blk
+
+
+def test_audit_enumerates_ties_and_flags():
+    """tfbs_audit_block: the windows scoring exactly min_score (strict >, pattern.rs:151) and the truncated / overwritten haplotypes
+    (haplotype.rs:144-149, :84) are the same sets the oracle finds; the context is left with a normal run of the block."""
+    ps, blk = tie_patterns_and_block()
     oa = hp.oracle_audit(ps, blk)
     au, rows, st = hp.gpu_audit(ps, blk)
     assert not au["truncated"]
@@ -564,7 +569,7 @@ def test_grouped_rows_two_blocks_in_flight_and_scratch_growth():
             d = hp.run_gpu(ps, blk, mode, False, {"tiny_caps": 1})
             hp.assert_rows_equal(d, o)
             hp.check_stats(d["stats"], o)
-            for dual in (0, 1):  # option dual_stream: the blocks alternate between the context and its twin (own streams and scratch)
+            for dual in (0, 1):  # option dual_stream: slot 1 runs on a second lane (own streams and scratch)
                 ctx = binding.Context(0)
                 try:
                     ctx.set_option("rows_mode", mode)
@@ -590,7 +595,7 @@ def test_grouped_rows_two_blocks_in_flight_and_scratch_growth():
                     hp.assert_rows_equal(ctx.collect_grouped(expand=True), o)
                     with pytest.raises(binding.TfbsError):
                         ctx.collect()  # nothing in flight any more
-                    if dual:  # result arena: the context writes the first half, its twin the second
+                    if dual:  # result arena: the block of slot 0 (lane 0) writes the first half, that of slot 1 (lane 1) the second
                         raw = np.zeros((4 << 20) + 64, dtype=np.uint8)
                         arena = raw[(-raw.ctypes.data) % 64:][:4 << 20]  # 64-byte aligned
                         ctx.set_result_arena(arena)
@@ -605,6 +610,52 @@ def test_grouped_rows_two_blocks_in_flight_and_scratch_growth():
                         assert ctx.stats()["n_regions"] == b1.n_regions
                 finally:
                     ctx.close()
+
+
+def test_dual_stream_set_after_upload():
+    """Option dual_stream set after tfbs_upload_block: two runs of the resident block in flight, one on each lane, both read the
+    one copy of the block on the device and return the oracle's rows."""
+    pats = synth.make_pwms(5, seed=43)
+    lmax = max(p["weights"].shape[0] for p in pats)
+    blk = synth.make_cohort(12, 10, seed=43, lmax_pattern=lmax, region_len=(100, 600), frac_ins=0.15, frac_del=0.15)
+    ps = PatternSet(pats)
+    o = hp.run_oracle(ps, blk)
+    ctx = binding.Context(0)
+    try:
+        ctx.set_patterns(ps)
+        ctx.upload_block(blk)
+        ctx.set_option("dual_stream", 1)
+        ctx.run_resident()
+        ctx.run_resident()
+        hp.assert_rows_equal(ctx.collect(), o)
+        hp.assert_rows_equal(ctx.collect(), o)
+    finally:
+        ctx.close()
+
+
+def test_dual_stream_audit_takes_the_last_block():
+    """With dual_stream on, tfbs_audit_block audits the block most recently submitted, whichever lane ran it: after b1 and b2 (of
+    different region counts) are collected, the audit is that of b2 -- the same ties and flags as a single-stream context's audit of
+    b2 -- and the normal run it leaves behind returns b2's rows."""
+    ps, blk = tie_patterns_and_block()
+    b1, b2 = blk.slice(0, 16), blk.slice(16, blk.n_regions)
+    ref, _, _ = hp.gpu_audit(ps, b2)
+    assert len(ref["region"]) > 0
+    ctx = binding.Context(0)
+    try:
+        ctx.set_patterns(ps)
+        ctx.set_option("dual_stream", 1)
+        ctx.submit_block(b1)
+        ctx.submit_block(b2)
+        ctx.collect()
+        ctx.collect()
+        au = ctx.audit()
+        assert len(au["hap_group"]) == b2.n_regions * 2 * b2.n_samples  # tfbs_audit.n_regions is b2's
+        for k in ("region", "pattern_index", "group", "start", "hap_group", "hap_flags"):
+            assert np.array_equal(au[k], ref[k]), k
+        hp.assert_rows_equal(ctx.collect(), hp.run_oracle(ps, b2))
+    finally:
+        ctx.close()
 
 
 def test_bed_merge_on_device():

@@ -275,8 +275,8 @@ def test_forced_device_vector_tiny_caps_and_narrow_rows():
 
 @pytest.mark.gpu
 def test_forced_device_vector_in_flight_twin_and_arena():
-    """Two blocks in flight on one context and on a dual_stream pair (the twin has its own count vectors), grouped rows expanded on
-    the host, and a result arena written by both twins."""
+    """Two blocks in flight on one lane and, with option dual_stream, on two lanes (each with its own count vectors), grouped rows
+    expanded on the host, and a result arena whose halves are written by the two lanes."""
     pats = synth.make_pwms(6, seed=3)
     lmax = max(p["weights"].shape[0] for p in pats)
     blk = synth.make_cohort(12, 10, seed=3, lmax_pattern=lmax, region_len=(200, 600), two_beds=True, frac_ins=0.15, frac_del=0.15)
