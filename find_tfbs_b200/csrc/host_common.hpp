@@ -7,7 +7,10 @@
 #include <climits>
 #include <cstdio>
 #include <cstring>
+#include <map>
+#include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "kernels.cuh"
@@ -240,6 +243,22 @@ namespace {
 int fail(tfbs_ctx* ctx, int code, const std::string& msg) {
     ctx->err = msg;
     return code;
+}
+
+// A kernel's dynamic shared-memory limit (cudaFuncAttributeMaxDynamicSharedMemorySize) belongs to the function on the device, not to
+// a context: every context and thread of the process that uses the device shares it.  Contexts on one device that set it to their
+// own block's need would lower it under one another, and a launch that needs more than the value left behind fails with "invalid
+// argument".  So the limit is only ever raised, under one lock per kernel signature.
+template <typename F>
+cudaError_t raise_smem_limit(F kernel, int device, int bytes) {
+    static std::mutex mu;
+    static std::map<std::pair<const void*, int>, int> limit;
+    std::lock_guard<std::mutex> lock(mu);
+    int& cur = limit[{reinterpret_cast<const void*>(kernel), device}];
+    if (bytes <= cur) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess) cur = bytes;
+    return e;
 }
 
 // Everything enqueued so far has finished (needed before an allocation that enqueued work may still use is replaced).

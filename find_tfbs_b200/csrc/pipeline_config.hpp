@@ -517,8 +517,8 @@ struct ConfigPipeline {
         DevMatches dm{};
         const int smem_bytes = (int)(sizeof(CtaShared) + SCAN_WARPS * sizeof(WarpShared) + ((cp.max_chunk_bytes + 15) & ~15u));
         const bool wide = cp.fields == 2;
-        if (wide) CK(cudaFuncSetAttribute(k_scan<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-        else CK(cudaFuncSetAttribute(k_scan<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+        if (wide) CK(raise_smem_limit(k_scan<2>, ctx->device, smem_bytes));
+        else CK(raise_smem_limit(k_scan<3>, ctx->device, smem_bytes));
         uint32_t scan_grid = (uint32_t)ctx->prop.multiProcessorCount;  // persistent: one CTA per SM shares one copy of the tables
         if (ctx->scan_ctas_per_sm < 0) scan_grid = (uint32_t)std::max(1, -ctx->scan_ctas_per_sm);
         slot->stats.scan_ctas = scan_grid;
@@ -587,10 +587,10 @@ struct ConfigPipeline {
                 fn.split = split;
                 // the kernel leaves every slice all zero, a fresh or regrown allocation is not: zeroed on every run, repeats included
                 CK(cudaMemsetAsync(L.d_fan_vec.p, 0, fan_vec_bytes(), st));
-                CK(cudaFuncSetAttribute(k_fanout<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fan_smem));
+                CK(raise_smem_limit(k_fanout<true>, ctx->device, (int)fan_smem));
                 TFBS_LAUNCH(k_fanout<true>, fan_vec_grid(), FAN_THREADS, fan_smem, st)(db, cf, fn);
             } else {
-                CK(cudaFuncSetAttribute(k_fanout<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fan_smem));
+                CK(raise_smem_limit(k_fanout<false>, ctx->device, (int)fan_smem));
                 CK(cudaFuncSetAttribute(k_fanout<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
                 TFBS_LAUNCH(k_fanout<false>, dim3(R, split), FAN_THREADS, fan_smem, st)(db, cf, fn);
             }

@@ -223,8 +223,8 @@ private:
         dm.start = L.d_m_start.as<i64>();
         smem_bytes = (int)(sizeof(CtaShared) + SCAN_WARPS * sizeof(WarpShared) + ((ctx->cp.max_chunk_bytes + 15) & ~15u));
         wide = ctx->cp.fields == 2;
-        if (wide) CK(cudaFuncSetAttribute(k_scan<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-        else CK(cudaFuncSetAttribute(k_scan<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+        if (wide) CK(raise_smem_limit(k_scan<2>, ctx->device, smem_bytes));
+        else CK(raise_smem_limit(k_scan<3>, ctx->device, smem_bytes));
         scan_grid = (uint32_t)ctx->prop.multiProcessorCount;  // persistent: one CTA per SM shares one copy of the tables
         if (ctx->scan_ctas_per_sm < 0) scan_grid = (uint32_t)std::max(1, -ctx->scan_ctas_per_sm);  // debugging: fixed grid size
         stats().scan_ctas = scan_grid;

@@ -11,7 +11,8 @@
 
 using namespace tfbs;
 
-static int check(const std::vector<tfbs_pattern>& pats, uint32_t budget, int force_wide, std::mt19937_64& rng, const char* what) {
+static int check(const std::vector<tfbs_pattern>& pats, uint32_t budget, int force_wide, std::mt19937_64& rng, const char* what,
+                 const std::vector<std::vector<uint8_t>>& plant = {}) {
     CompiledPatterns cp;
     std::string err;
     int rc = compile_patterns(pats.data(), (uint32_t)pats.size(), budget, force_wide, &cp, &err);
@@ -19,6 +20,8 @@ static int check(const std::vector<tfbs_pattern>& pats, uint32_t budget, int for
     const int bits = cp.fields == 3 ? 21 : 32;
     std::vector<uint8_t> seq(600);
     for (auto& c : seq) c = (rng() % 23 == 0) ? 4 : (uint8_t)(rng() % 4);
+    for (size_t k = 0; k < plant.size(); ++k)  // windows placed on purpose, 40 bases apart
+        for (size_t c = 0; c < plant[k].size(); ++c) seq[40 + 40 * k + c] = plant[k][c];
     std::vector<int> seen(pats.size(), 0);
     long long n_hits = 0;
     for (const ChunkDesc& cd : cp.chunks) {
@@ -107,6 +110,53 @@ int main() {
         bad += check(pats, 96 * 1024, 0, rng, name);
         snprintf(name, sizeof name, "round %d (wide, 12 KB chunks)", round);
         bad += check(pats, 12 * 1024, 1, rng, name);
+    }
+    // the format decision at the field capacity: slot 0 of three length-4 patterns has bmax = 2^20 + 2^19 (21-bit set) or
+    // 2^31 + 2^29 (32-bit set); the best window B (bmax) and the worst window W (score M) are placed in the sequence, and slot 1
+    // scores exactly its min_score on B, so that a carry out of slot 0's field would flag it.
+    {
+        const int best[4] = {0, 1, 2, 3}, worst[4] = {3, 2, 0, 1};
+        const std::vector<std::vector<uint8_t>> plant = {{0, 1, 2, 3}, {3, 2, 0, 1}, {0, 1, 2, 3, 3, 2, 0, 1}};
+        struct Case { int64_t span_lo, span_hi, thr; int fields; const char* what; };
+        const int64_t F21 = 1 << 20, F32 = int64_t(1) << 31;
+        const Case cases[] = {
+            {-196608, 196608, F21 / 2, 3, "bmax - thr = 2^20 (21-bit field exactly full)"},
+            {-196608, 196608, F21 - 1, 3, "thr = 2^20 - 1 (bias 0)"},
+            {-196608, 196608, F21 / 2 - 1, 2, "bmax - thr = 2^20 + 1"},
+            {-196608, 196608, F21, 2, "thr = 2^20"},
+            {-402653184, 268435456, F32 / 4, 2, "bmax - thr = 2^31 (32-bit field exactly full)"},
+            {-402653184, 268435456, F32 / 4 - 1, 0, "bmax - thr = 2^31 + 1"},
+            {-402653184, 268435456, F32, 0, "thr = 2^31"},
+        };
+        for (const Case& k : cases) {
+            std::vector<int32_t> w0(16, 1000), w1(16), w2(16);
+            for (int c = 0; c < 4; ++c) { w0[4 * c + best[c]] = (int32_t)k.span_hi; w0[4 * c + worst[c]] = (int32_t)k.span_lo; }
+            for (int i = 0; i < 16; ++i) { w1[i] = (int32_t)(rng() % 121) - 60; w2[i] = (int32_t)(rng() % 121) - 60; }
+            int s1b = 0, s1w = 0, s2b = 0;
+            for (int c = 0; c < 4; ++c) { s1b += w1[4 * c + best[c]]; s1w += w1[4 * c + worst[c]]; s2b += w2[4 * c + best[c]]; }
+            w1[worst[0]] += s1b + 1 - s1w;  // slot 1: min_score on B, min_score + 1 on W
+            const int64_t M = 4 * k.span_lo;
+            const int64_t ms0 = M + k.thr;
+            if (ms0 > INT32_MAX || ms0 < INT32_MIN) { printf("FAIL %s: min_score outside int32\n", k.what); ++bad; continue; }
+            std::vector<tfbs_pattern> pats(3);
+            const std::vector<int32_t>* ws[3] = {&w0, &w1, &w2};
+            const int32_t ms[3] = {(int32_t)ms0, s1b, s2b - 1};
+            for (int f = 0; f < 3; ++f) pats[f] = tfbs_pattern{ws[f]->data(), 4, ms[f], (uint16_t)(f + 1), 0, TFBS_PATTERN_PWM};
+            CompiledPatterns cp;
+            std::string err;
+            int rc = compile_patterns(pats.data(), 3, 96 * 1024, 0, &cp, &err);
+            if (k.fields == 0) {
+                if (rc != TFBS_ERR_SCORE_RANGE) { printf("FAIL %s: accepted (rc %d, fields %u)\n", k.what, rc, cp.fields); ++bad; }
+                else printf("ok %s: TFBS_ERR_SCORE_RANGE\n", k.what);
+                continue;
+            }
+            if (rc != TFBS_OK || (int)cp.fields != k.fields) {
+                printf("FAIL %s: rc %d, fields %u, expected %d\n", k.what, rc, cp.fields, k.fields);
+                ++bad;
+                continue;
+            }
+            bad += check(pats, 96 * 1024, 0, rng, k.what, plant);
+        }
     }
     // error paths
     {

@@ -10,7 +10,8 @@ every window of every pattern, count the windows whose hit range overlaps an inn
   position, a deletion keeps its first ALT base and skips the rest of REF;
 * a window of length L starting at sequence index i scores sum_c w[c][base(i + c)], N scoring 0, in float64; its hit range is
   (pos(i), pos(i) + L - 1) (pattern.rs:119-171);
-* an inner region counts a hit when the hit's start or end lies inside it (range.rs:18-21, main.rs:500-534);
+* an inner region counts a hit when the hit's start or end lies inside it (range.rs:18-21, main.rs:500-534), `multiplicity` times
+  (a BED line listed that many times);
 * haplotypes carrying the same records form one group; group 0 is the reference haplotype, the others are numbered in order of
   their smallest haplotype (the numbering tfbs_collect_grouped returns).
 
@@ -43,11 +44,13 @@ COMPLEMENT = np.array([3, 2, 1, 0])  # A<->T, C<->G
 # ---- inputs ----------------------------------------------------------------------------------------------------------------------
 
 class Region:
-    """One window: reference bases (str) starting at `start`, inner regions [(first, last)] (inclusive), records [(pos, REF, ALT)]
-    and carriers[v, h] = haplotype h carries record v."""
+    """One window: reference bases (str) starting at `start`, inner regions [(first, last)] or [(first, last, multiplicity)]
+    (inclusive; multiplicity 1 when left out), records [(pos, REF, ALT)] and carriers[v, h] = haplotype h carries record v."""
 
     def __init__(self, start, ref, inner, records=(), carriers=None, n_haps=0):
-        self.start, self.ref, self.inner, self.records = start, ref, list(inner), list(records)
+        self.start, self.ref, self.records = start, ref, list(records)
+        self.inner = [(x[0], x[1]) for x in inner]
+        self.mult = [x[2] if len(x) > 2 else 1 for x in inner]
         self.carriers = np.zeros((len(self.records), n_haps), bool) if carriers is None else np.asarray(carriers, bool)
         self.codes = np.array([CODE[b] for b in ref.upper()], np.int64)
         assert self.carriers.shape[0] == len(self.records)
@@ -64,7 +67,7 @@ def make_block(regions, n_samples):
     inner = np.zeros(int(inner_off[-1]), INNER_DTYPE)
     inner["start"] = [a for r in regions for a, _ in r.inner]
     inner["end"] = [b for r in regions for _, b in r.inner]
-    inner["multiplicity"] = 1
+    inner["multiplicity"] = [m for r in regions for m in r.mult]
     var_off = np.concatenate([[0], np.cumsum([len(r.records) for r in regions])]).astype(np.uint32)
     variants = np.zeros(int(var_off[-1]), VARIANT_DTYPE)
     alleles, rows = bytearray(), []
@@ -177,6 +180,8 @@ def region_counts(region, patterns, pids, ge=False):
         batches = [(gs, np.stack([seqs[g][0] for g in gs]), np.stack([seqs[g][1] for g in gs])) for gs in by_len.values()]
     for gs, S, P in batches:
         for pat in patterns:
+            if pat.get("kind", binding.PATTERN_PWM) != binding.PATTERN_PWM:  # OtherPattern never matches (pattern.rs:166-168)
+                continue
             sc = window_scores(S, pat["weights"])
             if sc.shape[1] == 0:
                 continue
@@ -189,11 +194,11 @@ def region_counts(region, patterns, pids, ge=False):
             if (P == P[0]).all():  # one set of hit ranges for the whole batch: count by a product with the overlap matrix
                 f, l = first[0][:, None], last[0][:, None]
                 over = ((f >= a) & (f <= b)) | ((l >= a) & (l <= b))
-                counts[gs, k0:k0 + n_inner] += hit.astype(np.int64) @ over.astype(np.int64)
+                counts[gs, k0:k0 + n_inner] += (hit.astype(np.int64) @ over.astype(np.int64)) * np.array(region.mult, np.int64)
                 continue
             for i in range(n_inner):
                 over = ((first >= a[i]) & (first <= b[i])) | ((last >= a[i]) & (last <= b[i]))
-                counts[gs, k0 + i] += (hit & over).sum(axis=1)
+                counts[gs, k0 + i] += (hit & over).sum(axis=1) * region.mult[i]
     return hap_group, counts
 
 
