@@ -23,7 +23,7 @@ DIR_P, DIR_N = 0, 1
 EXPORTS = ["tfbs_abi_version", "tfbs_create", "tfbs_destroy", "tfbs_last_error", "tfbs_set_option", "tfbs_set_patterns",
            "tfbs_submit_block", "tfbs_collect", "tfbs_get_matches", "tfbs_upload_block", "tfbs_run_resident", "tfbs_get_stats",
            "tfbs_stream", "tfbs_host_register", "tfbs_host_unregister", "tfbs_audit_block", "tfbs_collect_grouped", "tfbs_expand_rows", "tfbs_set_result_arena",
-           "tfbs_merge_sample_blocks", "tfbs_merge_regions", "tfbs_fanout_info", "tfbs_get_attribution"]
+           "tfbs_merge_sample_blocks", "tfbs_merge_regions", "tfbs_fanout_info", "tfbs_get_attribution", "tfbs_get_sites"]
 
 
 class TfbsPattern(C.Structure):
@@ -202,6 +202,11 @@ class TfbsAttribution(C.Structure):
 CFG_TRUNCATES = 1
 
 
+class TfbsSites(C.Structure):
+    _fields_ = [("n_cfgs", C.c_uint64), ("site_off", C.POINTER(C.c_uint64)), ("pattern_index", C.POINTER(C.c_uint32)),
+                ("start", C.POINTER(C.c_int64)), ("score", C.POINTER(C.c_int32)), ("change", C.POINTER(C.c_int8))]
+
+
 class TfbsStats(C.Structure):
     _fields_ = [("n_regions", C.c_uint64), ("n_groups", C.c_uint64), ("executed_cells", C.c_uint64), ("nominal_cells", C.c_uint64),
                 ("n_hits", C.c_uint64), ("n_keys", C.c_uint64), ("n_rows", C.c_uint64), ("h2d_bytes", C.c_uint64),
@@ -263,6 +268,7 @@ def lib():
         L.tfbs_fanout_info.argtypes = [C.c_void_p] + [C.POINTER(C.c_uint32)] * 4
         L.tfbs_audit_block.argtypes = [C.c_void_p, C.POINTER(TfbsAudit)]
         L.tfbs_get_attribution.argtypes = [C.c_void_p, C.POINTER(TfbsAttribution)]
+        L.tfbs_get_sites.argtypes = [C.c_void_p, C.POINTER(TfbsSites)]
         L.tfbs_stream.argtypes = [C.c_void_p]
         L.tfbs_stream.restype = C.c_void_p
         L.tfbs_host_register.argtypes = [C.c_void_p, C.c_size_t]
@@ -560,6 +566,23 @@ class Context:
                 "term_diff": arr(a.term_diff, nt, np.int32), "n_cfgs": nc, "cfg_region": arr(a.cfg_region, nc, np.uint32),
                 "cfg_flags": arr(a.cfg_flags, nc, np.uint8), "cfg_rec_off": cfg_rec_off, "cfg_rec": arr(a.cfg_rec, nr, np.uint32),
                 "n_groups_total": ng, "group_cfg_off": group_cfg_off, "group_cfg": arr(a.group_cfg, nl, np.uint32)}
+
+    def sites(self):
+        """tfbs_get_sites: for the block the last collect returned, per configuration (the ids of attribution()) the hits it gains
+        (change +1) and loses (change -1) against the reference haplotype: site_off / pattern_index / start / score / change.  NumPy copies."""
+        a = TfbsSites()
+        self._check(self._lib.tfbs_get_sites(self._h, C.byref(a)))
+        nc = a.n_cfgs
+
+        def arr(p, cnt, dt):
+            if cnt == 0:
+                return np.zeros(0, dtype=dt)
+            return np.ctypeslib.as_array(p, shape=(cnt,)).astype(dt, copy=True)
+
+        site_off = arr(a.site_off, nc + 1, np.uint64)
+        ns = int(site_off[-1])
+        return {"n_cfgs": nc, "site_off": site_off, "pattern_index": arr(a.pattern_index, ns, np.uint32), "start": arr(a.start, ns, np.int64),
+                "score": arr(a.score, ns, np.int32), "change": arr(a.change, ns, np.int8)}
 
     def stats(self):
         s = TfbsStats()

@@ -104,7 +104,8 @@ int main(int argc, char** argv) {
             if (tfbs_create(o.devices[k], &ctx) != TFBS_OK) die(std::string(tfbs_last_error(nullptr)));
             TF(tfbs_set_patterns(ctx, cpat.data(), (uint32_t)cpat.size()));
             TF(tfbs_set_option(ctx, "rows_width", 0));
-            if (!o.attribution_file.empty()) TF(tfbs_set_option(ctx, "attribution", 1));
+            if (!o.attribution_file.empty() || !o.sites_file.empty()) TF(tfbs_set_option(ctx, "attribution", 1));
+            if (!o.sites_file.empty()) TF(tfbs_set_option(ctx, "sites", 1));
             ctxs[k] = ctx;
             us_create += now_us() - tc;
         });
@@ -156,7 +157,7 @@ int main(int argc, char** argv) {
     // The writer (main.rs:264-290 has a writer thread fed through a channel): chunks finish in any order on the devices and are
     // written in chunk order as soon as every earlier chunk is there; a finished chunk's text is freed once written, so the
     // memory in flight is a few chunks, not the chromosome.  POS is the reference's running counter (main.rs:329,424-425).
-    struct ChunkText { std::vector<std::string> rows; std::string attribution; };
+    struct ChunkText { std::vector<std::string> rows; std::string attribution, sites; };
     std::mutex out_mu;
     std::condition_variable out_cv;
     std::map<size_t, ChunkText> done_chunks;
@@ -171,6 +172,16 @@ int main(int argc, char** argv) {
         attribution_out.open(o.attribution_file, std::ios::binary);
         if (!attribution_out) die("Could not create attribution file");
         attribution_out << "#ID\tREF_COUNT\tRECORDS\tDIFF\tHAPLOTYPES\tTRUNCATES\n";
+    }
+    // --sites: per written row and term (ID and RECORDS as in --attribution), the binding sites of the term's configuration with the
+    // row's pattern_id whose window overlaps the row's inner region (range.rs:18-21): the hits the configuration's records create
+    // (CHANGE +1) or destroy (-1) against the reference haplotype; START / END = the window, SCORE = its exact score.  A haplotype that
+    // carries the configuration counts the sum of CHANGE over the lines (times the BED line's multiplicity) more than REF_COUNT.
+    std::ofstream sites_out;
+    if (!o.sites_file.empty()) {
+        sites_out.open(o.sites_file, std::ios::binary);
+        if (!sites_out) die("Could not create sites file");
+        sites_out << "#ID\tRECORDS\tPATTERN\tSTRAND\tSTART\tEND\tSCORE\tCHANGE\n";
     }
     size_t next_to_write = 0;
     uint64_t fake_position = 1;
@@ -222,6 +233,7 @@ int main(int argc, char** argv) {
                 else plain << pc;
             }
             if (attribution_out.is_open()) attribution_out << t.attribution;
+            if (sites_out.is_open()) sites_out << t.sites;
             secs_write += std::chrono::duration<double>(std::chrono::steady_clock::now() - tw).count();
             {
                 std::lock_guard<std::mutex> lk(out_mu);
@@ -278,9 +290,9 @@ int main(int argc, char** argv) {
             return true;
         };
         // rows of one block -> text, in the canonical order inside a region: (bed file, inner range, pattern_id); the reference's
-        // order is HashMap::drain().  `counts(i, l, r)` fills the (left, right) vectors of row i; `attribution(i, id, text)`, when
-        // given, appends the --attribution lines of a written row i with VCF ID `id`.
-        using AttributionLines = std::function<void(uint64_t, const std::string&, std::string&)>;
+        // order is HashMap::drain().  `counts(i, l, r)` fills the (left, right) vectors of row i; `attribution(i, id, att, sites)`,
+        // when given, appends the --attribution and --sites lines of a written row i with VCF ID `id`.
+        using AttributionLines = std::function<void(uint64_t, const std::string&, std::string&, std::string&)>;
         auto rows_to_text = [&](size_t c, const BlockData& bd, uint64_t n_rows, const uint32_t* region, const uint32_t* inner, const uint16_t* pid,
                                 const uint32_t* vmin, const uint32_t* vmax, const std::function<void(uint64_t, uint32_t*, uint32_t*)>& counts,
                                 const AttributionLines& attribution = nullptr) {
@@ -299,7 +311,7 @@ int main(int argc, char** argv) {
             us_sort += now_us() - ts;
             uint64_t tf = now_us();
             // row text on --threads host threads (the reference formats inside its worker threads, main.rs:415-425)
-            std::vector<std::string> text(order.size()), att(attribution ? order.size() : 0);
+            std::vector<std::string> text(order.size()), att(attribution ? order.size() : 0), sit(attribution ? order.size() : 0);
             auto format_range = [&](size_t a, size_t b) {
                 std::vector<uint32_t> l(S), r(S);
                 for (size_t k = a; k < b; ++k) {
@@ -311,7 +323,7 @@ int main(int argc, char** argv) {
                     const std::string id = bed_names[ir.bed_index] + "," + pwm_name.at(pid[i]) + "," + std::to_string(ir.start) + "-" + std::to_string(ir.end);
                     // POS is filled in by the writer (a running counter, main.rs:329,424-425)
                     text[k] = "\t" + id + "\t.\t.\t.\tPASS\t" + t.info + "\tGT:DS" + t.genotypes + "\n";
-                    if (attribution) attribution(i, id, att[k]);
+                    if (attribution) attribution(i, id, att[k], sit[k]);
                 }
             };
             const size_t nt = std::max<size_t>(1, std::min<size_t>(o.threads, order.size() / 64 + 1));
@@ -325,6 +337,7 @@ int main(int argc, char** argv) {
             for (std::string& row : text)
                 if (!row.empty()) ct.rows.push_back(std::move(row));
             for (const std::string& a : att) ct.attribution += a;
+            for (const std::string& a : sit) ct.sites += a;
             us_format += now_us() - tf;
             chunk_finished(c, std::move(ct));
         };
@@ -359,13 +372,24 @@ int main(int argc, char** argv) {
                     g.n_groups = n_groups.data(); g.hap_group = hap_group.data();
                 }
             };
-            // --attribution: the block's attribution, copied like the rows, and per configuration the haplotypes whose group lists it
+            // --attribution / --sites: the block's attribution (and sites), copied like the rows, and per configuration the haplotypes
+            // whose group lists it
             struct OwnedAttribution {
-                std::vector<uint32_t> ref_count, term_cfg, cfg_rec;
-                std::vector<int32_t> term_diff;
-                std::vector<uint64_t> term_off, cfg_rec_off, haplotypes;
+                std::vector<uint32_t> ref_count, term_cfg, cfg_rec, site_pat;
+                std::vector<int32_t> term_diff, site_score;
+                std::vector<uint64_t> term_off, cfg_rec_off, haplotypes, site_off;
+                std::vector<int64_t> site_start;
                 std::vector<uint8_t> cfg_flags;
-                OwnedAttribution(const tfbs_attribution& a, const tfbs_grouped_rows& g) {
+                std::vector<int8_t> site_change;
+                OwnedAttribution(const tfbs_attribution& a, const tfbs_grouped_rows& g, const tfbs_sites* s) {
+                    if (s) {
+                        const uint64_t ns = s->site_off[s->n_cfgs];
+                        site_off.assign(s->site_off, s->site_off + s->n_cfgs + 1);
+                        site_pat.assign(s->pattern_index, s->pattern_index + ns);
+                        site_start.assign(s->start, s->start + ns);
+                        site_score.assign(s->score, s->score + ns);
+                        site_change.assign(s->change, s->change + ns);
+                    }
                     const uint64_t n = a.n_rows, nt = a.term_off[n], nc = a.n_cfgs;
                     ref_count.assign(a.ref_count, a.ref_count + n);
                     term_off.assign(a.term_off, a.term_off + n + 1);
@@ -409,8 +433,11 @@ int main(int argc, char** argv) {
                     const tfbs_grouped_rows& g = it.rows->g;
                     const OwnedAttribution* at = it.att.get();
                     const BlockData& bd = *it.bd;
-                    // ID, REF_COUNT, RECORDS (POS:REF:ALT, 1-based POS), DIFF, HAPLOTYPES, TRUNCATES: one line per term of the row
-                    auto lines = [&](uint64_t i, const std::string& id, std::string& out) {
+                    // --attribution: ID, REF_COUNT, RECORDS (POS:REF:ALT, 1-based POS), DIFF, HAPLOTYPES, TRUNCATES: one line per term of the
+                    // row; --sites: ID, RECORDS, PATTERN, STRAND, START, END, SCORE, CHANGE: one line per site of the term's configuration
+                    // with the row's pattern_id that overlaps the row's inner region
+                    auto lines = [&](uint64_t i, const std::string& id, std::string& out, std::string& sites) {
+                        const tfbs_inner_region& ir = bd.inner[g.inner[i]];
                         for (uint64_t t = at->term_off[i]; t < at->term_off[i + 1]; ++t) {
                             const uint32_t cfg = at->term_cfg[t];
                             std::string recs;
@@ -420,8 +447,19 @@ int main(int argc, char** argv) {
                                 recs += std::to_string(v.pos + 1) + ":" + std::string((const char*)bd.alleles.data() + v.ref_off, v.ref_len) + ":" +
                                         std::string((const char*)bd.alleles.data() + v.alt_off, v.alt_len);
                             }
-                            out += id + "\t" + std::to_string(at->ref_count[i]) + "\t" + recs + "\t" + std::to_string(at->term_diff[t]) + "\t" +
-                                   std::to_string(at->haplotypes[cfg]) + "\t" + ((at->cfg_flags[cfg] & TFBS_CFG_TRUNCATES) ? "1" : "0") + "\n";
+                            if (attribution_out.is_open())
+                                out += id + "\t" + std::to_string(at->ref_count[i]) + "\t" + recs + "\t" + std::to_string(at->term_diff[t]) + "\t" +
+                                       std::to_string(at->haplotypes[cfg]) + "\t" + ((at->cfg_flags[cfg] & TFBS_CFG_TRUNCATES) ? "1" : "0") + "\n";
+                            if (at->site_off.empty()) continue;
+                            for (uint64_t k = at->site_off[cfg]; k < at->site_off[cfg + 1]; ++k) {
+                                const Pwm& pw = pwms[at->site_pat[k]];
+                                if (pw.pattern_id != g.pattern_id[i]) continue;
+                                const int64_t s0 = at->site_start[k], s1 = s0 + (int64_t)(pw.w.size() / 4) - 1;
+                                const int64_t i0 = (int64_t)ir.start, i1 = (int64_t)ir.end;
+                                if (!((s0 >= i0 && s0 <= i1) || (s1 >= i0 && s1 <= i1))) continue;  // Range::overlaps, range.rs:18-21
+                                sites += id + "\t" + recs + "\t" + pw.name + "\t" + (pw.direction == TFBS_DIR_P ? "+" : "-") + "\t" + std::to_string(s0) + "\t" +
+                                         std::to_string(s1) + "\t" + std::to_string(at->site_score[k]) + "\t" + (at->site_change[k] > 0 ? "+1" : "-1") + "\n";
+                            }
                         }
                     };
                     rows_to_text(it.c, bd, g.n_rows, g.region, g.inner, g.pattern_id, g.vmin, g.vmax,
@@ -450,10 +488,12 @@ int main(int argc, char** argv) {
                 note_stats(item.c);
                 std::unique_ptr<OwnedRows> own(new OwnedRows(g));
                 std::unique_ptr<OwnedAttribution> att;
-                if (!o.attribution_file.empty()) {
+                if (!o.attribution_file.empty() || !o.sites_file.empty()) {
                     tfbs_attribution a;
                     TF(tfbs_get_attribution(ctx, &a));
-                    att.reset(new OwnedAttribution(a, g));
+                    tfbs_sites s;
+                    if (!o.sites_file.empty()) TF(tfbs_get_sites(ctx, &s));
+                    att.reset(new OwnedAttribution(a, g, o.sites_file.empty() ? nullptr : &s));
                 }
                 std::unique_lock<std::mutex> lk(fmu);
                 fcv.wait(lk, [&] { return to_format.size() < 2; });  // bounded: at most two collected blocks wait for their text
@@ -537,6 +577,10 @@ int main(int argc, char** argv) {
     if (attribution_out.is_open()) {
         attribution_out.close();
         if (!attribution_out) die("Could not write attribution file");
+    }
+    if (sites_out.is_open()) {
+        sites_out.close();
+        if (!sites_out) die("Could not write sites file");
     }
     if (rename(part.c_str(), o.output.c_str()) != 0) die("Could not rename " + part + " into " + o.output);
     if (o.tabix) {

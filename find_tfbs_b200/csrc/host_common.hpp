@@ -101,6 +101,9 @@ struct Results {
     // attribution (option "attribution", tfbs_get_attribution)
     HostBuf h_a_ref, h_a_toff, h_a_tcfg, h_a_tdiff, h_a_creg, h_a_cflags, h_a_croff, h_a_crec, h_a_goff, h_a_gcfg;
     bool have_attribution = false;
+    // sites (option "sites", tfbs_get_sites)
+    HostBuf h_s_off, h_s_pat, h_s_start, h_s_score, h_s_change;
+    bool have_sites = false;
 };
 
 // Capacities a run of the configuration path was enqueued with (see DevPlan): sizes that only the device learns.
@@ -108,6 +111,7 @@ struct Caps {
     uint64_t seq = 0, d = 0, cfg = 0, vd = 0, items = 0, units = 0, dwords = 0, rows = 0, rowwords = 0;
     uint32_t capr = 0, groups = 0;
     uint64_t terms = 0;  // option "attribution": non-zero (row, configuration) differences
+    uint64_t sites_raw = 0, sites = 0;  // option "sites": gained and lost hits before and after equal pairs cancel
 };
 
 struct Slot {
@@ -120,6 +124,7 @@ struct Slot {
     DevBuf d_status, d_plan, d_hap_group, d_gbase, d_hg_narrow;
     DevBuf d_o_region, d_o_inner, d_o_pid, d_o_vmin, d_o_vmax, d_o_base, d_o_bits, d_o_off, d_o_packed, d_left, d_right;
     DevBuf d_a_ref, d_a_toff, d_a_tcfg, d_a_tdiff, d_a_creg, d_a_cflags, d_a_croff, d_a_crec, d_a_goff, d_a_gcfg;  // attribution
+    DevBuf d_s_off, d_s_pat, d_s_start, d_s_score, d_s_change;  // sites
     HostBuf h_status, h_plan;
     Results res;
     Caps caps;
@@ -132,6 +137,8 @@ struct Slot {
     uint32_t fan_groups_cap = 0, fan_ctas = 0, fan_in_device_memory = 0;  // the fan-out of the last run (tfbs_fanout_info)
     bool attribution = false;                        // the run enqueued the attribution launches
     uint64_t att_cfgs = 0, att_seqs = 0, att_terms = 0;  // their sizes (configurations, distinct haplotypes, terms)
+    bool sites = false;                              // the run enqueued the sites launches
+    uint64_t n_sites = 0;                            // sites after the cancellation
 };
 
 // The streams a block's work is enqueued on and the scratch its kernels share with the blocks before and after it on the same lane.
@@ -158,6 +165,7 @@ struct Lane {
     DevBuf d_vmin, d_vmax, d_flag, d_rowwords, d_kbits, d_rowidx, d_rowoff;
     DevBuf d_fan_vec;  // k_fanout<true>: one count vector per CTA
     DevBuf d_att_eflag, d_att_cfgid, d_att_nrec, d_att_col, d_att_gn, d_att_tcnt;  // option "attribution"
+    DevBuf d_site_refpat, d_site_refscore, d_site_raw, d_site_bucket, d_site_keep, d_site_kpos, d_site_oid, d_site_cnt, d_site_boff;  // option "sites"
     // full-scan path (lane 0 only)
     DevBuf d_gbase, d_cbase, d_C;
     DevBuf d_rows_region, d_rows_inner, d_rows_pid, d_rows_vmin, d_rows_vmax, d_rows_left, d_rows_right;
@@ -190,18 +198,21 @@ struct tfbs_ctx {
     int64_t test_reseed = 0;    // testing: the first attempt of every block is treated as a hash collision (repeated with another seed)
     int fan_vector = 0;         // 0: the fan-out's count vectors live in shared memory unless a region has too many groups; 1: always in device memory (testing)
     int attribution = 0;        // 1: the default path keeps the per-row configuration differences (tfbs_get_attribution)
+    int sites = 0;              // 1: and the hits each configuration gains and loses (tfbs_get_sites; needs attribution = 1)
     int dual_stream = 0;        // 1: a block in slot 1 of the default path runs on lane 1
     // attribution of the block the last tfbs_collect / tfbs_collect_grouped returned, copied to the host by that collect
     enum { ATT_NONE = 0, ATT_OFF, ATT_FULL_SCAN, ATT_READY };
     int att_state = ATT_NONE;
     tfbs_attribution att{};
+    int site_state = ATT_NONE;  // the same states for the sites of that block
+    tfbs_sites site{};
 
     // patterns
     bool have_patterns = false;
     std::vector<tfbs_pattern> orig_patterns;          // the caller's list (tfbs_audit_block re-compiles it with lowered thresholds)
     std::vector<std::vector<int32_t>> orig_weights;
     CompiledPatterns cp;
-    DevBuf d_table, d_chunks, d_runs, d_trip_pat, d_pat_len, d_pat_pid, d_pid_list;
+    DevBuf d_table, d_chunks, d_runs, d_trip_pat, d_pat_len, d_pat_pid, d_pat_w, d_pid_list;
     DevPatterns dpat{};
 
     // blocks in flight: a ring of two slots, plus the resident block of tfbs_upload_block

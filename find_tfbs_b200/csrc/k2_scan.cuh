@@ -6,7 +6,33 @@
 
 namespace tfbs {
 
-// Rare path: a window scored above the threshold in at least one field.
+// Option "sites": the exact score of a hit, from the pattern's weights and the packed bases of the list entry (N scores 0).  On the
+// configuration path the work list is the identity (k_vitem_units), so the item is the entry, and its units hold the bases
+// [p0 & ~31, p1 + 64]: a window [i, i + L) with p0 <= i <= p1 and L <= 32 lies inside.  Then the site is kept: a configuration's hit
+// goes to the raw site list (+1), a hit of the reference haplotype is remembered next to its RefHit slot (k_cfg_lost takes the lost ones).
+__device__ __forceinline__ void keep_site(const ScanEnv* env, u32 mode, u64 at, u32 entry, u32 pi, u32 i, u32 L, int hs) {
+    const DevSeqs& sq = *env->sq;
+    const DevConfigs& cf = *env->cf;
+    const u64* pk = sq.pk + sq.ent_uoff[entry];
+    const u32* nm = sq.nm + sq.ent_uoff[entry];
+    const int* w = env->pt->pat_w + (u64)pi * (kMaxPatternLen * 4);
+    const u32 base = sq.items[entry].p0 & ~31u;
+    int score = 0;
+    for (u32 k = 0; k < L; ++k) {
+        const u32 x = i + k - base;
+        if (!((nm[x >> 5] >> (x & 31)) & 1u)) score += w[4 * k + ((u32)(pk[x >> 5] >> (2 * (x & 31))) & 3u)];
+    }
+    if (mode == 2) {
+        put_site(cf, (u32)at, pi, hs, score, 1);
+    } else {
+        cf.ref_pat[at] = pi;
+        cf.ref_score[at] = score;
+    }
+}
+
+// Rare path: a window scored above the threshold in at least one field.  SITES (a k_scan of its own, so that the registers and the
+// stack of the scan without option "sites" stay as they are): the sites are kept too (keep_site).
+template <bool SITES>
 __device__ __noinline__ u32 scan_on_hit(u64 hit, u32 t, u32 i, u32 item_index, ChunkDesc cd, const ScanEnv* env) {
     u32 counted = 0;  // hits of a full scan: the caller adds them to the statistics once per work grab
     const DevSeqs& sq = *env->sq;
@@ -48,13 +74,18 @@ __device__ __noinline__ u32 scan_on_hit(u64 hit, u32 t, u32 i, u32 item_index, C
             crow = cf.D + cf.dbase[r] + (c - cf.cfgbase[r]);
             cstride = cf.ncfg[r];
             atomicAdd(&cf.cfg_net[c], 1);
+            if (SITES) keep_site(env, 2, c, item_index, (u32)pi, i, L, (int)hs);
         } else {
             crow = env->ct->C + (env->ct->cbase[r] - env->ct->cbase0) + (u64)g * pt.n_pid * nk;
             if (mode == 1) {
                 const u32 rr = r - env->rh->r0;
                 u32 slot = atomicAdd(&env->rh->cnt[rr], 1u);
-                if (slot < env->rh->capr) env->rh->buf[(u64)rr * env->rh->capr + slot] = RefHit{r, (int)hs, L, pl};
-                else st->refhit_overflow = 1;
+                if (slot < env->rh->capr) {
+                    env->rh->buf[(u64)rr * env->rh->capr + slot] = RefHit{r, (int)hs, L, pl};
+                    if (SITES) keep_site(env, 1, (u64)rr * env->rh->capr + slot, item_index, (u32)pi, i, L, (int)hs);
+                } else {
+                    st->refhit_overflow = 1;
+                }
             } else {
                 ++counted;
             }
@@ -89,23 +120,23 @@ __device__ __forceinline__ u64 pair_sum(const u8* tb, const u32 (&idx)[kMaxGroup
 }
 
 // All triples of one run (same number of column pairs G): G LDS.64 + 64-bit adds per triple and lane.
-template <int G, int FIELDS>
+template <int G, int FIELDS, bool SITES>
 __device__ __forceinline__ void scan_run(const u8* tb, u32 n_trip, u32 t0, const u32 (&idx)[kMaxGroups], u32 i, u32 item_index,
                                          const ChunkDesc& cd, const ScanEnv* env, u32& n_counted) {
 #pragma unroll SCAN_UNROLL
     for (u32 t = 0; t < n_trip; ++t) {
         u64 acc = pair_sum<0, G>(tb, idx);
         u64 hit = acc & HitMask<FIELDS>::value;
-        if (hit && i != 0xffffffffu) n_counted += scan_on_hit(hit, t0 + t, i, item_index, cd, env);
+        if (hit && i != 0xffffffffu) n_counted += scan_on_hit<SITES>(hit, t0 + t, i, item_index, cd, env);
         tb += G * (kPairEntries * 8);
     }
 }
 
-template <int FIELDS>
+template <int FIELDS, bool SITES>
 __device__ __forceinline__ void scan_dispatch(u32 G, const u8* tb, u32 n_trip, u32 t0, const u32 (&idx)[kMaxGroups], u32 i, u32 item_index,
                                               const ChunkDesc& cd, const ScanEnv* env, u32& n_counted) {
     switch (G) {
-#define TFBS_CASE(N) case N: scan_run<N, FIELDS>(tb, n_trip, t0, idx, i, item_index, cd, env, n_counted); break;
+#define TFBS_CASE(N) case N: scan_run<N, FIELDS, SITES>(tb, n_trip, t0, idx, i, item_index, cd, env, n_counted); break;
         TFBS_CASE(1) TFBS_CASE(2) TFBS_CASE(3) TFBS_CASE(4) TFBS_CASE(5) TFBS_CASE(6) TFBS_CASE(7) TFBS_CASE(8)
         TFBS_CASE(9) TFBS_CASE(10) TFBS_CASE(11) TFBS_CASE(12) TFBS_CASE(13) TFBS_CASE(14) TFBS_CASE(15) TFBS_CASE(16)
 #undef TFBS_CASE
@@ -122,7 +153,7 @@ __device__ __forceinline__ u32 pair_code_bytes(u32 a, u32 b) {  // pair_entry(a,
 // takes `per_grab` consecutive entries of the list from an atomic counter, stages their packed bases into its private
 // pair-code planes (several short items side by side, long items in tiles) and scans all triples of the chunk, 32 window
 // starts at a time.
-template <int FIELDS>
+template <int FIELDS, bool SITES = false>
 __global__ void __launch_bounds__(SCAN_CTA, 1)
     k_scan(const __grid_constant__ DevBlock b, const __grid_constant__ DevSeqs sq, const __grid_constant__ DevPatterns pt,
            const __grid_constant__ DevCounts ct, const __grid_constant__ DevMatches mt, const __grid_constant__ DevRefHits rh,
@@ -227,7 +258,7 @@ __global__ void __launch_bounds__(SCAN_CTA, 1)
                 u32 t0 = 0;
                 for (u32 rn = 0; rn < n_runs; ++rn) {
                     const RunDesc rd = cs->runs[rn];
-                    scan_dispatch<FIELDS>(rd.groups, tb, rd.n_triples, t0, idx, i, item_index, cd, &env, n_counted);
+                    scan_dispatch<FIELDS, SITES>(rd.groups, tb, rd.n_triples, t0, idx, i, item_index, cd, &env, n_counted);
                     tb += (size_t)rd.n_triples * rd.groups * (kPairEntries * 8);
                     t0 += rd.n_triples;
                 }

@@ -16,6 +16,7 @@ struct DevPatterns {
     const int* trip_pat;
     const u32* pat_len;
     const u32* pat_pid_index;
+    const int* pat_w;  // [n_patterns][kMaxPatternLen][4] weights (option "sites": the rare path scores the windows it keeps)
     u32 n_chunks;
     u32 n_pid;       // distinct pattern ids
     u32 n_patterns;

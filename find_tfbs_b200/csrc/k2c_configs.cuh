@@ -28,6 +28,8 @@ struct DevPlan {
     u64 fan_keys;        // keys the fan-out built a count vector for
     u64 fan_dbg[5];      // -DTFBS_FAN_STATS: pairs, member updates, groups with a non-zero difference, samples with one, keys of the dense pass
     u64 n_terms, need_terms;  // option "attribution": non-zero (row, configuration) differences (k3_attribution.cuh)
+    u64 site_alloc;           // option "sites": raw sites handed out by the rare path and k_cfg_lost (an atomic cursor)
+    u64 n_sraw, need_sraw, n_sites, need_sites;  // raw sites, and those left after gained / lost pairs cancel (k3_sites.cuh)
 };
 
 // A count becomes known: total (+ add) against the capacity its consumers were launched for.  Behind an earlier overflow nothing
@@ -52,6 +54,16 @@ __global__ void k_zero_words(u32* p, const u64* n_ptr, u64 cap) {
     u64 n = *n_ptr < cap ? *n_ptr : cap;
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) p[i] = 0;
 }
+
+// Option "sites": a hit a configuration gains (+1, rare path, mode 2) or a reference hit it loses (-1, k_cfg_lost), before equal
+// (pattern, start, score) pairs cancel (k3_sites.cuh).
+struct RawSite {
+    u32 cfg;     // virtual configuration index (cfgbase[r] + column); the output id once k_site_scatter has grouped them
+    u32 pat;     // pattern index
+    int start;   // window start relative to region_start (pattern.rs:156)
+    int score;   // exact window score
+    int change;  // +1 gained, -1 lost
+};
 
 struct DevConfigs {
     u32 max_len;           // longest pattern (main.rs:404)
@@ -81,7 +93,17 @@ struct DevConfigs {
     u32* D;                // [region][key][configuration of the region]: difference to the reference haplotype's count (wrapping u32)
     u32* C0;               // [key] counts of the region's reference haplotype
     DevPlan* plan;
+    // option "sites" (site_raw NULL when off)
+    RawSite* site_raw;     // [site_cap] in no particular order, behind plan->site_alloc
+    u64 site_cap;
+    u32* ref_pat;          // parallel to DevRefHits::buf: pattern index and score of each reference hit
+    int* ref_score;
 };
+
+__device__ __forceinline__ void put_site(const DevConfigs& cf, u32 c, u32 pat, int start, int score, int change) {
+    const u64 k = atomicAdd(&cf.plan->site_alloc, 1ULL);
+    if (k < cf.site_cap) cf.site_raw[k] = RawSite{c, pat, start, score, change};
+}
 
 // One CTA per region: the in-window records by position, cut into clusters.
 __global__ void k_cluster(DevBlock b, DevConfigs cf) {
@@ -316,6 +338,10 @@ __global__ void k_cfg_lost(DevBlock b, DevSeqs vq, DevConfigs cf, DevRefHits rh)
                      (i64)h.relpos + h.len <= (i64)sg[s].relpos + (i64)(sg[s + 1].out_start - sg[s].out_start);
         if (inside) continue;
         ++lost;
+        if (cf.site_raw) {
+            const u64 x = (u64)(r - rh.r0) * rh.capr + j;
+            put_site(cf, (u32)c, cf.ref_pat[x], h.relpos, cf.ref_score[x], -1);
+        }
         const i64 hs = h.relpos, he = hs + h.len - 1;
         for (u32 k = 0; k < nk; ++k) {
             i64 is = inner[k].start - rs, ie = inner[k].end - rs;

@@ -26,6 +26,7 @@ struct DevAttr {
     u32* cfg_col;     // [cfg] column of the configuration in its region's difference matrix
     u32* glist_n;     // [seq] live runs of the distinct haplotype
     u32* t_cnt;       // [rows] non-zero terms of the row
+    u32* site_oid;    // [cfg] option "sites" (else NULL): output id of the virtual configuration cfgbase[r] + column (k3_sites.cuh)
     // results (per slot)
     u32* cfg_region;  // [cfg]
     u8* cfg_flags;    // [cfg]
@@ -76,6 +77,7 @@ __global__ void k_att_configs(DevSeqs sq, DevConfigs cf, DevSeqs vq, DevAttr at)
             const u32 col = cf.run_cfg[e];
             at.cfg_region[o] = r;
             at.cfg_col[o] = col;
+            if (at.site_oid) at.site_oid[cf.cfgbase[r] + col] = (u32)o;
             at.cfg_nrec[o] = n;
             at.cfg_flags[o] = vq.seq_flags[(u64)vq.n_ref + cf.cfgbase[r] + col] & 1;
         }

@@ -12,6 +12,7 @@
 //   K3  count/rows    k_rows_*              count_matches_by_sample fan-out           (main.rs:506-531)
 //                                           + min/max filter of counts_as_genotypes   (main.rs:439-458)
 //       attribution   k_att_*               per row, the configurations that change its count (option "attribution")
+//       sites         k_site_*              per configuration, the hits it gains and loses (option "sites")
 //
 // All arithmetic is integer; results are bit-exact by construction (scores are i32 sums, SURVEY D1).
 #pragma once
@@ -28,4 +29,5 @@
 #include "k3_rows.cuh"
 #include "k3_fanout.cuh"
 #include "k3_attribution.cuh"
+#include "k3_sites.cuh"
 #include "k_bed.cuh"

@@ -95,7 +95,7 @@ struct ConfigPipeline {
         if (!first_attempt) return;  // a repeated run keeps the capacities finalize() grew
         if (ctx->tiny_caps) {  // testing: every growth path runs
             c = Caps{};
-            c.seq = R; c.d = 1; c.cfg = 1; c.vd = 1; c.items = ref_items + 1; c.units = 1; c.dwords = 1; c.rows = 1; c.rowwords = 1; c.capr = 1; c.groups = 1; c.terms = 1;
+            c.seq = R; c.d = 1; c.cfg = 1; c.vd = 1; c.items = ref_items + 1; c.units = 1; c.dwords = 1; c.rows = 1; c.rowwords = 1; c.capr = 1; c.groups = 1; c.terms = 1; c.sites_raw = 1; c.sites = 1;
             return;
         }
         // what the previous blocks needed (+ 25 %) when there is a history, else a guess from the shape of the block; a wrong guess
@@ -114,6 +114,8 @@ struct ConfigPipeline {
         c.capr = ctx->refhit_cap_opt ? (uint32_t)std::max<int64_t>(1, ctx->refhit_cap_opt / std::max<uint32_t>(1, R)) : (uint32_t)pick(h.capr, 512);
         c.groups = h.groups ? groups_for(h.groups) : (uint32_t)std::min<uint64_t>((uint64_t)H + 1, 2048);
         c.terms = pick(h.terms, 4 * c.rows);
+        c.sites_raw = pick(h.sites_raw, 8 * c.cfg + 1024);
+        c.sites = pick(h.sites, 4 * c.cfg + 1024);
     }
     uint64_t scratch_bytes_needed() const {
         const Caps& c = slot->caps;
@@ -122,12 +124,18 @@ struct ConfigPipeline {
         while (seg < 2 * ((uint64_t)H + 1)) seg <<= 1;
         tbl = std::max<uint64_t>(tbl, (uint64_t)R * seg);
         return RH * 20 + tbl * 12 + c.seq * 50 + c.d * (4 + 32 + 20 + 4) + c.seq * 32 + c.cfg * 32 + (R + c.cfg) * 60 + c.vd * 36 + c.items * 28 +
-               c.units * 12 + c.dwords * 4 + n_keys * 36 + (uint64_t)c.capr * R * sizeof(RefHit) + c.rows * 34 + c.rowwords * 4 + fan_vec_bytes() + attribution_bytes();
+               c.units * 12 + c.dwords * 4 + n_keys * 36 + (uint64_t)c.capr * R * sizeof(RefHit) + c.rows * 34 + c.rowwords * 4 + fan_vec_bytes() + attribution_bytes() + sites_bytes();
     }
     // option "attribution": scratch per diff-list entry, configuration, distinct haplotype and row, the per-slot results, the terms
     uint64_t attribution_bytes() const {
         const Caps& c = slot->caps;
         return ctx->attribution ? c.d * 20 + c.cfg * 21 + c.seq * 12 + c.rows * 16 + c.terms * 8 : 0;
+    }
+    // option "sites": score and pattern of every reference hit, the raw sites twice (+ flag and index), per configuration its output id,
+    // count and offsets, the per-slot results
+    uint64_t sites_bytes() const {
+        const Caps& c = slot->caps;
+        return slot->sites ? (uint64_t)c.capr * R * 8 + c.sites_raw * (2 * sizeof(RawSite) + 12) + c.cfg * 24 + c.sites * 17 : 0;
     }
 
     // ---- fan-out: the count vectors in shared memory (k_fanout<false>, one CTA per unit) or in device memory (k_fanout<true>) ----
@@ -254,6 +262,22 @@ struct ConfigPipeline {
             RS(slot->d_a_goff, (c.seq + 1) * 8);
             RS(slot->d_a_gcfg, c.d * 4);
         }
+        if (slot->sites) {
+            RS(L.d_site_refpat, (uint64_t)c.capr * R * 4);
+            RS(L.d_site_refscore, (uint64_t)c.capr * R * 4);
+            RS(L.d_site_raw, c.sites_raw * sizeof(RawSite));
+            RS(L.d_site_bucket, c.sites_raw * sizeof(RawSite));
+            RS(L.d_site_keep, c.sites_raw * 4);
+            RS(L.d_site_kpos, (c.sites_raw + 1) * 8);
+            RS(L.d_site_oid, c.cfg * 4);
+            RS(L.d_site_cnt, c.cfg * 4);
+            RS(L.d_site_boff, (c.cfg + 1) * 8);
+            RS(slot->d_s_off, (c.cfg + 1) * 8);
+            RS(slot->d_s_pat, c.sites * 4);
+            RS(slot->d_s_start, c.sites * 8);
+            RS(slot->d_s_score, c.sites * 4);
+            RS(slot->d_s_change, c.sites);
+        }
 #undef RS
         CK(slot->h_status.reserve(sizeof(DevStatus), false));
         CK(slot->h_plan.reserve(sizeof(DevPlan), false));
@@ -301,8 +325,9 @@ struct ConfigPipeline {
         slot->stats.scan_launches = 0;
         slot->stats.scan_input_bytes = 0;
         slot->res.n_rows = 0;
-        slot->res.have_dense = slot->res.have_grouped = slot->res.have_attribution = false;
+        slot->res.have_dense = slot->res.have_grouped = slot->res.have_attribution = slot->res.have_sites = false;
         slot->attribution = ctx->attribution != 0;
+        slot->sites = slot->attribution && ctx->sites;
         choose_caps(first_attempt);
         const Caps& c = slot->caps;
         const bool fans = n_keys && R && S;
@@ -441,6 +466,12 @@ struct ConfigPipeline {
         cf.D = L.d_D.as<u32>();
         cf.C0 = L.d_C0.as<u32>();
         cf.plan = plan;
+        if (slot->sites) {
+            cf.site_raw = L.d_site_raw.as<RawSite>();
+            cf.site_cap = c.sites_raw;
+            cf.ref_pat = L.d_site_refpat.as<u32>();
+            cf.ref_score = L.d_site_refscore.as<int>();
+        }
         TFBS_LAUNCH(k_cluster, R, 128, 0, st)(db, cf);
         ++launches();
         {
@@ -517,16 +548,16 @@ struct ConfigPipeline {
         DevMatches dm{};
         const int smem_bytes = (int)(sizeof(CtaShared) + SCAN_WARPS * sizeof(WarpShared) + ((cp.max_chunk_bytes + 15) & ~15u));
         const bool wide = cp.fields == 2;
-        if (wide) CK(raise_smem_limit(k_scan<2>, ctx->device, smem_bytes));
-        else CK(raise_smem_limit(k_scan<3>, ctx->device, smem_bytes));
+        // option "sites": the kernels whose rare path also keeps the sites
+        auto kern = wide ? (slot->sites ? k_scan<2, true> : k_scan<2>) : (slot->sites ? k_scan<3, true> : k_scan<3>);
+        CK(raise_smem_limit(kern, ctx->device, smem_bytes));
         uint32_t scan_grid = (uint32_t)ctx->prop.multiProcessorCount;  // persistent: one CTA per SM shares one copy of the tables
         if (ctx->scan_ctas_per_sm < 0) scan_grid = (uint32_t)std::max(1, -ctx->scan_ctas_per_sm);
         slot->stats.scan_ctas = scan_grid;
         CK(cudaEventRecord(slot->ev_t[3], st));
         for (uint32_t ch = 0; ch < cp.chunks.size(); ++ch) {
             CK(cudaMemsetAsync(&dst->work_counter, 0, 4, st));
-            if (wide) TFBS_LAUNCH(k_scan<2>, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, L.d_list.as<u32>(), &plan->n_items, (u32)SCAN_PER_GRAB, dst, ch);
-            else TFBS_LAUNCH(k_scan<3>, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, L.d_list.as<u32>(), &plan->n_items, (u32)SCAN_PER_GRAB, dst, ch);
+            TFBS_LAUNCH(kern, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, L.d_list.as<u32>(), &plan->n_items, (u32)SCAN_PER_GRAB, dst, ch);
             ++launches();
             ++slot->stats.scan_launches;
         }
@@ -608,7 +639,7 @@ struct ConfigPipeline {
     }
 
     // ---- option "attribution" (k3_attribution.cuh): behind the row headers, while D, C0, the diff lists and the runs are this block's ----
-    // 6 launches, 4 more for the terms when the block has keys
+    // 6 launches, 4 more for the terms when the block has keys, and the 8 of option "sites"
     int enqueue_attribution(const DevSeqs& sq, const DevConfigs& cf, const DevSeqs& vq, const DevFan* fn) {
         const Caps& c = slot->caps;
         int rc;
@@ -619,6 +650,7 @@ struct ConfigPipeline {
         at.cfg_col = L.d_att_col.as<u32>();
         at.glist_n = L.d_att_gn.as<u32>();
         at.t_cnt = L.d_att_tcnt.as<u32>();
+        at.site_oid = slot->sites ? L.d_site_oid.as<u32>() : nullptr;
         at.cfg_region = slot->d_a_creg.as<u32>();
         at.cfg_flags = slot->d_a_cflags.as<u8>();
         at.cfg_rec_off = slot->d_a_croff.as<u64>();
@@ -643,13 +675,52 @@ struct ConfigPipeline {
         if ((rc = scan(at.glist_n, c.seq, &plan->n_seq, at.group_off))) return rc;
         TFBS_LAUNCH(k_att_configs<true>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, vq, at);
         ++launches();
-        if (!fn) return TFBS_OK;
-        // 3. terms: count, scan, gate, fill
-        TFBS_LAUNCH(k_att_terms<false>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
+        if (fn) {
+            // 3. terms: count, scan, gate, fill
+            TFBS_LAUNCH(k_att_terms<false>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
+            ++launches();
+            if ((rc = scan(at.t_cnt, c.rows, &plan->n_rows, at.term_off))) return rc;
+            TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(at.term_off, &plan->n_rows, (u64)c.terms, &plan->n_terms, &plan->need_terms, &plan->abort);
+            TFBS_LAUNCH(k_att_terms<true>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
+            launches() += 2;
+        }
+        return slot->sites ? enqueue_sites() : TFBS_OK;
+    }
+
+    // ---- option "sites" (k3_sites.cuh): behind the attribution, which has written the output id of every virtual configuration ----
+    // 8 launches
+    int enqueue_sites() {
+        const Caps& c = slot->caps;
+        int rc;
+        DevSites s{};
+        s.raw = L.d_site_raw.as<RawSite>();
+        s.bucket = L.d_site_bucket.as<RawSite>();
+        s.keep = L.d_site_keep.as<u32>();
+        s.kpos = L.d_site_kpos.as<u64>();
+        s.oid = L.d_site_oid.as<u32>();
+        s.cnt = L.d_site_cnt.as<u32>();
+        s.boff = L.d_site_boff.as<u64>();
+        s.site_off = slot->d_s_off.as<u64>();
+        s.pat = slot->d_s_pat.as<u32>();
+        s.start = slot->d_s_start.as<i64>();
+        s.score = slot->d_s_score.as<int>();
+        s.change = slot->d_s_change.as<signed char>();
+        s.cfg_region = slot->d_a_creg.as<u32>();
+        const unsigned grid = slot->stats.sm_count * 8;
+        // 1. the raw sites against their capacity, grouped by output id
+        gate(&plan->site_alloc, 0, c.sites_raw, &plan->n_sraw, &plan->need_sraw);
+        CK(cudaMemsetAsync(s.cnt, 0, c.cfg * 4, st));
+        TFBS_LAUNCH(k_site_count, grid, 256, 0, st)(s, &plan->n_sraw, &plan->abort);
         ++launches();
-        if ((rc = scan(at.t_cnt, c.rows, &plan->n_rows, at.term_off))) return rc;
-        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(at.term_off, &plan->n_rows, (u64)c.terms, &plan->n_terms, &plan->need_terms, &plan->abort);
-        TFBS_LAUNCH(k_att_terms<true>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
+        if ((rc = scan(s.cnt, c.cfg, &plan->n_cfg, s.boff))) return rc;
+        TFBS_LAUNCH(k_site_scatter, grid, 256, 0, st)(s, &plan->n_sraw, &plan->abort);
+        // 2. sorted per configuration, survivors flagged
+        TFBS_LAUNCH(k_site_rank, (unsigned)std::min<uint64_t>(std::max<uint64_t>(1, c.cfg), grid), SITE_THREADS, 0, st)(s, &plan->n_cfg, &plan->abort);
+        launches() += 2;
+        // 3. survivors numbered, checked against the result capacity, written
+        if ((rc = scan(s.keep, c.sites_raw, &plan->n_sraw, s.kpos))) return rc;
+        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(s.kpos, &plan->n_sraw, (u64)c.sites, &plan->n_sites, &plan->need_sites, &plan->abort);
+        TFBS_LAUNCH(k_site_emit, grid, 256, 0, st)(db, s, &plan->n_sraw, &plan->n_cfg, &plan->abort);
         launches() += 2;
         return TFBS_OK;
     }
@@ -726,6 +797,8 @@ struct ConfigPipeline {
         g(c.rows, hp.need_rows);
         g(c.rowwords, hp.need_rowwords);
         g(c.terms, hp.need_terms);
+        g(c.sites_raw, hp.need_sraw);
+        g(c.sites, hp.need_sites);
         if (hp.need_capr > c.capr) c.capr = (uint32_t)up(hp.need_capr);
         if (hp.need_groups > c.groups) c.groups = groups_for(hp.need_groups);
     }
@@ -740,6 +813,8 @@ struct ConfigPipeline {
         h.rows = std::max<uint64_t>(h.rows, hp.need_rows);
         h.rowwords = std::max<uint64_t>(h.rowwords, hp.need_rowwords);
         h.terms = std::max<uint64_t>(h.terms, hp.need_terms);
+        h.sites_raw = std::max<uint64_t>(h.sites_raw, hp.need_sraw);
+        h.sites = std::max<uint64_t>(h.sites, hp.need_sites);
         h.capr = std::max<uint32_t>(h.capr, hp.need_capr);
         h.groups = std::max<uint32_t>(h.groups, hp.need_groups);
     }
@@ -778,6 +853,7 @@ struct ConfigPipeline {
         slot->att_cfgs = hp.n_cfg;
         slot->att_seqs = hp.n_seq;
         slot->att_terms = hp.n_terms;
+        slot->n_sites = hp.n_sites;
         slot->res.packed_words = hp.n_rowwords;
         slot->res.row_bytes = 4;
         if (ctx->rows_width == 0) slot->res.row_bytes = hs.max_count < 256 ? 1 : (hs.max_count < 65536 ? 2 : 4);
@@ -940,6 +1016,39 @@ struct ConfigPipeline {
         CK(cudaStreamSynchronize(so));
         slot->stats.d2h_bytes += bytes;
         res.have_attribution = true;
+        return TFBS_OK;
+    }
+
+    // sites -> host (stream_out), behind the attribution: the offsets first, they give the size of the rest.  Counted in d2h_bytes.
+    int fetch_sites() {
+        Results& res = slot->res;
+        if (res.have_sites) return TFBS_OK;
+        cudaStream_t so = L.stream_out;
+        const uint64_t nc = slot->att_cfgs;
+        CK(res.h_s_off.reserve((nc + 1) * 8, false));
+        uint64_t* off = res.h_s_off.as<uint64_t>();
+        uint64_t bytes = 0;
+        off[0] = 0;
+        if (nc) {  // (with no configuration the layout may not have run)
+            CK(cudaMemcpyAsync(off, slot->d_s_off.p, (nc + 1) * 8, cudaMemcpyDeviceToHost, so));
+            CK(cudaStreamSynchronize(so));
+            bytes += (nc + 1) * 8;
+        }
+        const uint64_t ns = off[nc];
+        if (ns != slot->n_sites) return fail(ctx, TFBS_ERR_INTERNAL, "sites: the site count disagrees with the gate");
+        auto copy = [&](HostBuf& h, const DevBuf& d, uint64_t b) -> int {
+            CK(h.reserve(std::max<uint64_t>(1, b), false));
+            if (b) CK(cudaMemcpyAsync(h.p, d.p, b, cudaMemcpyDeviceToHost, so));
+            bytes += b;
+            return TFBS_OK;
+        };
+        int rc;
+        if ((rc = copy(res.h_s_pat, slot->d_s_pat, ns * 4)) || (rc = copy(res.h_s_start, slot->d_s_start, ns * 8)) ||
+            (rc = copy(res.h_s_score, slot->d_s_score, ns * 4)) || (rc = copy(res.h_s_change, slot->d_s_change, ns)))
+            return rc;
+        CK(cudaStreamSynchronize(so));
+        slot->stats.d2h_bytes += bytes;
+        res.have_sites = true;
         return TFBS_OK;
     }
 

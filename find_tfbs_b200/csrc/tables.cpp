@@ -93,6 +93,8 @@ int compile_patterns(const tfbs_pattern* patterns, uint32_t n, uint32_t table_bu
         p.pid_index = pid_index[p.pattern_id];
         cp.pat_len.push_back(p.len);
         cp.pat_pid_index.push_back(p.pid_index);
+        cp.pat_w.insert(cp.pat_w.end(), p.w.begin(), p.w.end());
+        cp.pat_w.resize(cp.pat_w.size() + (4 * (size_t)kMaxPatternLen - p.w.size()), 0);
         cp.max_len = std::max(cp.max_len, p.len);
         if (p.kind == TFBS_PATTERN_PWM) {
             cp.sum_len += p.len;

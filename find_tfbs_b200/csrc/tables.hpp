@@ -69,6 +69,7 @@ struct CompiledPatterns {
     std::vector<int32_t> trip_pat;           // 3 slots per triple (unused slots -1): index into patterns
     std::vector<uint32_t> pat_len;           // per pattern
     std::vector<uint32_t> pat_pid_index;     // per pattern
+    std::vector<int32_t> pat_w;              // per pattern kMaxPatternLen x 4 weights, zero behind its length (option "sites" scores hits)
     uint32_t max_len = 0;                    // max pattern_length over all patterns (main.rs:404)
     uint32_t sum_len = 0;                    // sum of L over PWM patterns
     uint64_t sum_len_sq = 0;                 // sum of L*(L-1)

@@ -22,6 +22,8 @@ bool wants_full(const tfbs_ctx* ctx) { return !ctx->delta || ctx->record_matches
 int start_block(tfbs_ctx* ctx, BlockDev* in, const tfbs_block* b) {
     if (!ctx->have_patterns) return fail(ctx, TFBS_ERR_STATE, "tfbs_set_patterns has not been called");
     if (ctx->in_flight >= 2) return fail(ctx, TFBS_ERR_STATE, "two blocks are already in flight on this context: call tfbs_collect first");
+    if (ctx->sites && !ctx->attribution)
+        return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "option sites needs option attribution = 1: sites refer to its configuration ids");
     const int k = (ctx->head + ctx->in_flight) % 2;
     Slot* slot = &ctx->slot[k];
     slot->lane = ctx->dual_stream && !wants_full(ctx) ? k : 0;  // option "dual_stream": consecutive blocks run on different lanes
@@ -72,10 +74,23 @@ int finish_oldest(tfbs_ctx* ctx, Slot** out) {
 // The collect that returns a block also brings its attribution to the host (option "attribution"): a later block may take the slot's
 // device buffers before tfbs_get_attribution is called.
 int take_attribution(tfbs_ctx* ctx, Slot* slot) {
-    if (slot->full_mode) { ctx->att_state = tfbs_ctx::ATT_FULL_SCAN; return TFBS_OK; }
+    if (slot->full_mode) { ctx->att_state = ctx->site_state = tfbs_ctx::ATT_FULL_SCAN; return TFBS_OK; }
+    ctx->site_state = tfbs_ctx::ATT_OFF;
     if (!slot->attribution) { ctx->att_state = tfbs_ctx::ATT_OFF; return TFBS_OK; }
     int rc = ConfigPipeline(ctx, slot).fetch_attribution();
     if (rc) return rc;
+    if (slot->sites) {
+        if ((rc = ConfigPipeline(ctx, slot).fetch_sites())) return rc;
+        const Results& res = slot->res;
+        tfbs_sites& so = ctx->site;
+        so.n_cfgs = slot->att_cfgs;
+        so.site_off = res.h_s_off.as<uint64_t>();
+        so.pattern_index = res.h_s_pat.as<uint32_t>();
+        so.start = res.h_s_start.as<int64_t>();
+        so.score = res.h_s_score.as<int32_t>();
+        so.change = res.h_s_change.as<int8_t>();
+        ctx->site_state = tfbs_ctx::ATT_READY;
+    }
     const Results& res = slot->res;
     tfbs_attribution& out = ctx->att;
     memset(&out, 0, sizeof out);
@@ -128,6 +143,7 @@ int install_patterns(tfbs_ctx* ctx, const tfbs_pattern* patterns, uint32_t n_pat
     if ((rc = upload_on(ctx, st, ctx->d_trip_pat, c.trip_pat.data(), c.trip_pat.size(), nullptr))) return rc;
     if ((rc = upload_on(ctx, st, ctx->d_pat_len, c.pat_len.data(), c.pat_len.size(), nullptr))) return rc;
     if ((rc = upload_on(ctx, st, ctx->d_pat_pid, c.pat_pid_index.data(), c.pat_pid_index.size(), nullptr))) return rc;
+    if ((rc = upload_on(ctx, st, ctx->d_pat_w, c.pat_w.data(), c.pat_w.size(), nullptr))) return rc;
     if ((rc = upload_on(ctx, st, ctx->d_pid_list, c.pid_list.data(), c.pid_list.size(), nullptr))) return rc;
     CK(cudaStreamSynchronize(st));
     DevPatterns& d = ctx->dpat;
@@ -137,6 +153,7 @@ int install_patterns(tfbs_ctx* ctx, const tfbs_pattern* patterns, uint32_t n_pat
     d.trip_pat = ctx->d_trip_pat.as<int>();
     d.pat_len = ctx->d_pat_len.as<u32>();
     d.pat_pid_index = ctx->d_pat_pid.as<u32>();
+    d.pat_w = ctx->d_pat_w.as<int>();
     d.n_chunks = (u32)c.chunks.size();
     d.n_pid = (u32)c.pid_list.size();
     d.n_patterns = (u32)c.patterns.size();
@@ -264,6 +281,10 @@ int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value) {
         if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "attribution must be 0 or 1");
         ctx->attribution = (int)value;
     }
+    else if (k == "sites") {
+        if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "sites must be 0 or 1");
+        ctx->sites = (int)value;
+    }
     else if (k == "rows_width") {
         if (value != 0 && value != 32) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "rows_width must be 32 or 0 (automatic)");
         ctx->rows_width = (int)value;
@@ -321,7 +342,7 @@ int tfbs_submit_block(tfbs_ctx* ctx, const tfbs_block* block) {
 int tfbs_collect(tfbs_ctx* ctx, tfbs_rows* out) {
     if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
     CK(cudaSetDevice(ctx->device));
-    ctx->att_state = tfbs_ctx::ATT_NONE;
+    ctx->att_state = ctx->site_state = tfbs_ctx::ATT_NONE;
     Slot* slot = nullptr;
     int rc = finish_oldest(ctx, &slot);
     if (rc) return rc;
@@ -345,12 +366,12 @@ int tfbs_collect(tfbs_ctx* ctx, tfbs_rows* out) {
 int tfbs_collect_grouped(tfbs_ctx* ctx, tfbs_grouped_rows* out) {
     if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
     CK(cudaSetDevice(ctx->device));
-    ctx->att_state = tfbs_ctx::ATT_NONE;
+    ctx->att_state = ctx->site_state = tfbs_ctx::ATT_NONE;
     Slot* slot = nullptr;
     int rc = finish_oldest(ctx, &slot);
     if (rc) return rc;
     if (slot->full_mode) {
-        ctx->att_state = tfbs_ctx::ATT_FULL_SCAN;
+        ctx->att_state = ctx->site_state = tfbs_ctx::ATT_FULL_SCAN;
         retire_oldest(ctx);
         return fail(ctx, TFBS_ERR_STATE, "grouped rows come from the default scoring mode (delta = 1, record_matches off): use tfbs_collect");
     }
@@ -522,6 +543,19 @@ int tfbs_get_attribution(tfbs_ctx* ctx, tfbs_attribution* out) {
     default: break;
     }
     *out = ctx->att;
+    return TFBS_OK;
+}
+
+int tfbs_get_sites(tfbs_ctx* ctx, tfbs_sites* out) {
+    if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
+    switch (ctx->site_state) {
+    case tfbs_ctx::ATT_NONE: return fail(ctx, TFBS_ERR_STATE, "no block has been collected yet (tfbs_collect / tfbs_collect_grouped first)");
+    case tfbs_ctx::ATT_OFF: return fail(ctx, TFBS_ERR_STATE, "option sites was off for the last block: set it (and attribution) to 1 before the run");
+    case tfbs_ctx::ATT_FULL_SCAN:
+        return fail(ctx, TFBS_ERR_STATE, "the last block was a full scan (delta = 0, record_matches or the audit): sites come from the default path only");
+    default: break;
+    }
+    *out = ctx->site;
     return TFBS_OK;
 }
 

@@ -247,6 +247,27 @@ typedef struct tfbs_attribution {
                                       haplotype); behind a truncation only what the haplotype still applies */
 } tfbs_attribution;
 
+/*
+ * Binding sites behind the attribution's terms (option "sites" = 1 together with "attribution" = 1; tfbs_get_sites).  For
+ * configuration c (the ids of tfbs_attribution) take two multisets of (pattern_index, start, score) hit triples: A, the hits of the
+ * region's extended window patched with c's records alone (truncation exit included), and R, the hits of the unpatched window.  A hit
+ * is a complete window with score > min_score; start is the position of its first base (pattern.rs:156: bases an insertion adds share
+ * its anchor's position).  The sites of c are A - R with change +1 (gained) and R - A with change -1 (lost), multiset differences: a
+ * hit that survives unchanged is not listed, one whose score moves but stays above the threshold is a lost / gained pair.  For every
+ * row j with pattern_id p and inner region k, multiplicity(k) times the sum of change over c's sites whose pattern has id p and whose
+ * range [start, start + L - 1] overlaps k (range.rs:18-21) is c's term_diff for row j, or 0 when c has no term there.
+ * Sites are ordered by configuration, then by (pattern_index, start, score, change) ascending; they do not depend on hash seeds, on
+ * the order threads ran in or on the stream the block ran on.
+ */
+typedef struct tfbs_sites {
+    uint64_t n_cfgs;                /* == tfbs_attribution.n_cfgs of the same collect */
+    const uint64_t* site_off;       /* [n_cfgs + 1]: sites of configuration c are [site_off[c], site_off[c + 1]) */
+    const uint32_t* pattern_index;  /* index into the array given to tfbs_set_patterns (gives pattern_id, strand, L) */
+    const int64_t* start;           /* as tfbs_matches.start */
+    const int32_t* score;           /* exact window score */
+    const int8_t* change;           /* +1 gained, -1 lost */
+} tfbs_sites;
+
 /* Row filter: which keys tfbs_collect returns. */
 enum {
     TFBS_ROWS_VARYING = 0, /* only keys with min != max, i.e. those counts_as_genotypes keeps (main.rs:456-458) */
@@ -309,7 +330,9 @@ const char* tfbs_last_error(const tfbs_ctx* ctx);
  * "fan_vector" (0 = automatic, the default: the fan-out keeps its per-group count vectors in shared memory and switches to device
  * memory when a region of the block may have more distinct haplotypes than shared memory holds, 53,120; 1 = always in device
  * memory, for tests -- results are the same either way), "attribution" (0 = off, the default; 1 = the default path also keeps the
- * per-row count differences of every configuration for tfbs_get_attribution: the rows themselves do not change), "dual_stream"
+ * per-row count differences of every configuration for tfbs_get_attribution: the rows themselves do not change), "sites" (0 = off,
+ * the default; 1 = the default path also keeps the hits each configuration gains and loses, with their exact scores, for
+ * tfbs_get_sites; needs "attribution" = 1, else tfbs_submit_block / tfbs_run_resident fail with TFBS_ERR_INVALID_ARGUMENT), "dual_stream"
  * (0 = off, the default; 1 = consecutive blocks of the default scoring mode alternate between two lanes, each with its own kernel
  * and copy streams and its own device scratch, so that the kernels of the two blocks in flight overlap on the device: worth it when
  * blocks are small, while a second lane doubles the scratch of large blocks; fails with TFBS_ERR_STATE while blocks are in flight). */
@@ -391,6 +414,11 @@ int tfbs_merge_regions(tfbs_ctx* ctx, const uint64_t* start, const uint64_t* end
  * since do not affect it.  Fails with TFBS_ERR_STATE when nothing has been collected, when option "attribution" was off for that run,
  * or when the run was a full scan ("delta" = 0 or "record_matches").  Pointers stay valid as those of tfbs_rows do. */
 int tfbs_get_attribution(tfbs_ctx* ctx, tfbs_attribution* out);
+
+/* Sites (see tfbs_sites) of the block the last tfbs_collect or tfbs_collect_grouped returned, copied to the host by that collect
+ * right after its attribution.  Fails with TFBS_ERR_STATE when nothing has been collected, when option "sites" was off for that run,
+ * or when the run was a full scan ("delta" = 0, "record_matches" or the audit).  Pointers stay valid as those of tfbs_rows do. */
+int tfbs_get_sites(tfbs_ctx* ctx, tfbs_sites* out);
 
 /* Matches of the last run when "record_matches" was on (call after tfbs_collect). */
 int tfbs_get_matches(tfbs_ctx* ctx, tfbs_matches* out);
