@@ -23,7 +23,8 @@ DIR_P, DIR_N = 0, 1
 EXPORTS = ["tfbs_abi_version", "tfbs_create", "tfbs_destroy", "tfbs_last_error", "tfbs_set_option", "tfbs_set_patterns",
            "tfbs_submit_block", "tfbs_collect", "tfbs_get_matches", "tfbs_upload_block", "tfbs_run_resident", "tfbs_get_stats",
            "tfbs_stream", "tfbs_host_register", "tfbs_host_unregister", "tfbs_audit_block", "tfbs_collect_grouped", "tfbs_expand_rows", "tfbs_set_result_arena",
-           "tfbs_merge_sample_blocks", "tfbs_merge_regions", "tfbs_fanout_info", "tfbs_get_attribution", "tfbs_get_sites"]
+           "tfbs_merge_sample_blocks", "tfbs_merge_regions", "tfbs_fanout_info", "tfbs_get_attribution", "tfbs_get_sites",
+           "tfbs_get_record_sites"]
 
 
 class TfbsPattern(C.Structure):
@@ -207,6 +208,15 @@ class TfbsSites(C.Structure):
                 ("start", C.POINTER(C.c_int64)), ("score", C.POINTER(C.c_int32)), ("change", C.POINTER(C.c_int8))]
 
 
+class TfbsRecordSites(C.Structure):
+    _fields_ = [("n_records", C.c_uint64), ("rec_flags", C.POINTER(C.c_uint8)), ("site_off", C.POINTER(C.c_uint64)),
+                ("pattern_index", C.POINTER(C.c_uint32)), ("start", C.POINTER(C.c_int64)), ("score", C.POINTER(C.c_int32)),
+                ("change", C.POINTER(C.c_int8))]
+
+
+REC_OUTSIDE, REC_REF_MISMATCH, REC_MISSING_CASE = 1, 2, 4
+
+
 class TfbsStats(C.Structure):
     _fields_ = [("n_regions", C.c_uint64), ("n_groups", C.c_uint64), ("executed_cells", C.c_uint64), ("nominal_cells", C.c_uint64),
                 ("n_hits", C.c_uint64), ("n_keys", C.c_uint64), ("n_rows", C.c_uint64), ("h2d_bytes", C.c_uint64),
@@ -269,6 +279,7 @@ def lib():
         L.tfbs_audit_block.argtypes = [C.c_void_p, C.POINTER(TfbsAudit)]
         L.tfbs_get_attribution.argtypes = [C.c_void_p, C.POINTER(TfbsAttribution)]
         L.tfbs_get_sites.argtypes = [C.c_void_p, C.POINTER(TfbsSites)]
+        L.tfbs_get_record_sites.argtypes = [C.c_void_p, C.POINTER(TfbsRecordSites)]
         L.tfbs_stream.argtypes = [C.c_void_p]
         L.tfbs_stream.restype = C.c_void_p
         L.tfbs_host_register.argtypes = [C.c_void_p, C.c_size_t]
@@ -583,6 +594,25 @@ class Context:
         ns = int(site_off[-1])
         return {"n_cfgs": nc, "site_off": site_off, "pattern_index": arr(a.pattern_index, ns, np.uint32), "start": arr(a.start, ns, np.int64),
                 "score": arr(a.score, ns, np.int32), "change": arr(a.change, ns, np.int8)}
+
+    def record_sites(self):
+        """tfbs_get_record_sites: for the block the last collect returned, per record (tfbs_block.variants order) its REC_* flags and the
+        hits it gains (change +1) and loses (change -1) on its own: rec_flags / site_off / pattern_index / start / score / change.
+        NumPy copies."""
+        a = TfbsRecordSites()
+        self._check(self._lib.tfbs_get_record_sites(self._h, C.byref(a)))
+        nv = a.n_records
+
+        def arr(p, cnt, dt):
+            if cnt == 0:
+                return np.zeros(0, dtype=dt)
+            return np.ctypeslib.as_array(p, shape=(cnt,)).astype(dt, copy=True)
+
+        site_off = arr(a.site_off, nv + 1, np.uint64)
+        ns = int(site_off[-1])
+        return {"n_records": nv, "rec_flags": arr(a.rec_flags, nv, np.uint8), "site_off": site_off,
+                "pattern_index": arr(a.pattern_index, ns, np.uint32), "start": arr(a.start, ns, np.int64), "score": arr(a.score, ns, np.int32),
+                "change": arr(a.change, ns, np.int8)}
 
     def stats(self):
         s = TfbsStats()

@@ -106,6 +106,7 @@ int main(int argc, char** argv) {
             TF(tfbs_set_option(ctx, "rows_width", 0));
             if (!o.attribution_file.empty() || !o.sites_file.empty()) TF(tfbs_set_option(ctx, "attribution", 1));
             if (!o.sites_file.empty()) TF(tfbs_set_option(ctx, "sites", 1));
+            if (!o.record_sites_file.empty()) TF(tfbs_set_option(ctx, "record_sites", 1));
             ctxs[k] = ctx;
             us_create += now_us() - tc;
         });
@@ -157,7 +158,7 @@ int main(int argc, char** argv) {
     // The writer (main.rs:264-290 has a writer thread fed through a channel): chunks finish in any order on the devices and are
     // written in chunk order as soon as every earlier chunk is there; a finished chunk's text is freed once written, so the
     // memory in flight is a few chunks, not the chromosome.  POS is the reference's running counter (main.rs:329,424-425).
-    struct ChunkText { std::vector<std::string> rows; std::string attribution, sites; };
+    struct ChunkText { std::vector<std::string> rows; std::string attribution, sites, record_sites; };
     std::mutex out_mu;
     std::condition_variable out_cv;
     std::map<size_t, ChunkText> done_chunks;
@@ -182,6 +183,18 @@ int main(int argc, char** argv) {
         sites_out.open(o.sites_file, std::ios::binary);
         if (!sites_out) die("Could not create sites file");
         sites_out << "#ID\tRECORDS\tPATTERN\tSTRAND\tSTART\tEND\tSCORE\tCHANGE\n";
+    }
+    // --record_sites: per merged region (REGION, as the row IDs write ranges), per record of its window in BCF order (RECORD, as in
+    // RECORDS) and per binding site of that record alone whose window overlaps one of the region's inner regions (range.rs:18-21): the
+    // hits the record creates (CHANGE +1) or destroys (-1) against the reference haplotype, whoever carries it -- the sites that can
+    // move one of the region's counts.  Independent of the rows (--min_maf and the row filter do not thin it); records that
+    // patch_haplotype would not apply alone (outside the window, REF mismatch, missing case) have no lines.
+    std::ofstream record_sites_out;
+    std::atomic<uint64_t> rec_flagged[3] = {{0}, {0}, {0}};  // records without lines: outside, REF mismatch, missing case
+    if (!o.record_sites_file.empty()) {
+        record_sites_out.open(o.record_sites_file, std::ios::binary);
+        if (!record_sites_out) die("Could not create record sites file");
+        record_sites_out << "#RECORD\tREGION\tPATTERN\tSTRAND\tSTART\tEND\tSCORE\tCHANGE\n";
     }
     size_t next_to_write = 0;
     uint64_t fake_position = 1;
@@ -234,6 +247,7 @@ int main(int argc, char** argv) {
             }
             if (attribution_out.is_open()) attribution_out << t.attribution;
             if (sites_out.is_open()) sites_out << t.sites;
+            if (record_sites_out.is_open()) record_sites_out << t.record_sites;
             secs_write += std::chrono::duration<double>(std::chrono::steady_clock::now() - tw).count();
             {
                 std::lock_guard<std::mutex> lk(out_mu);
@@ -295,7 +309,7 @@ int main(int argc, char** argv) {
         using AttributionLines = std::function<void(uint64_t, const std::string&, std::string&, std::string&)>;
         auto rows_to_text = [&](size_t c, const BlockData& bd, uint64_t n_rows, const uint32_t* region, const uint32_t* inner, const uint16_t* pid,
                                 const uint32_t* vmin, const uint32_t* vmax, const std::function<void(uint64_t, uint32_t*, uint32_t*)>& counts,
-                                const AttributionLines& attribution = nullptr) {
+                                const AttributionLines& attribution = nullptr, std::string record_sites = std::string()) {
             uint64_t ts = now_us();
             std::vector<uint64_t> order(n_rows);
             for (uint64_t i = 0; i < n_rows; ++i) order[i] = i;
@@ -334,6 +348,7 @@ int main(int argc, char** argv) {
                 for (auto& t : ft) t.join();
             }
             ChunkText ct;
+            ct.record_sites = std::move(record_sites);
             for (std::string& row : text)
                 if (!row.empty()) ct.rows.push_back(std::move(row));
             for (const std::string& a : att) ct.attribution += a;
@@ -414,7 +429,62 @@ int main(int argc, char** argv) {
                         for (uint64_t k = a.group_cfg_off[G]; k < a.group_cfg_off[G + 1]; ++k) haplotypes[a.group_cfg[k]] += members[G];
                 }
             };
-            struct Collected { size_t c; std::unique_ptr<BlockData> bd; std::unique_ptr<OwnedRows> rows; std::unique_ptr<OwnedAttribution> att; };
+            // --record_sites: the block's record sites, copied like the rows
+            struct OwnedRecordSites {
+                std::vector<uint8_t> flags;
+                std::vector<uint64_t> off;
+                std::vector<uint32_t> pat;
+                std::vector<int64_t> start;
+                std::vector<int32_t> score;
+                std::vector<int8_t> change;
+                explicit OwnedRecordSites(const tfbs_record_sites& s) {
+                    const uint64_t nv = s.n_records, ns = s.site_off[nv];
+                    flags.assign(s.rec_flags, s.rec_flags + nv);
+                    off.assign(s.site_off, s.site_off + nv + 1);
+                    pat.assign(s.pattern_index, s.pattern_index + ns);
+                    start.assign(s.start, s.start + ns);
+                    score.assign(s.score, s.score + ns);
+                    change.assign(s.change, s.change + ns);
+                }
+            };
+            struct Collected {
+                size_t c;
+                std::unique_ptr<BlockData> bd;
+                std::unique_ptr<OwnedRows> rows;
+                std::unique_ptr<OwnedAttribution> att;
+                std::unique_ptr<OwnedRecordSites> rec;
+            };
+            // RECORD, REGION, PATTERN, STRAND, START, END, SCORE, CHANGE of block c: its regions in order, their records in BCF order
+            auto record_lines = [&](size_t c, const BlockData& bd, const OwnedRecordSites& rs) {
+                std::string out;
+                const size_t m0 = c * o.chunk;
+                for (size_t r = 0; r + 1 < bd.var_off.size(); ++r) {
+                    const std::string region = std::to_string(merged[m0 + r].start) + "-" + std::to_string(merged[m0 + r].end);
+                    for (uint32_t v = bd.var_off[r]; v < bd.var_off[r + 1]; ++v) {
+                        const uint8_t fl = rs.flags[v];
+                        if (fl) {
+                            rec_flagged[fl & TFBS_REC_OUTSIDE ? 0 : fl & TFBS_REC_REF_MISMATCH ? 1 : 2] += 1;
+                            continue;
+                        }
+                        const tfbs_variant& x = bd.variants[v];
+                        const std::string rec = std::to_string(x.pos + 1) + ":" + std::string((const char*)bd.alleles.data() + x.ref_off, x.ref_len) + ":" +
+                                                std::string((const char*)bd.alleles.data() + x.alt_off, x.alt_len);
+                        for (uint64_t k = rs.off[v]; k < rs.off[v + 1]; ++k) {
+                            const Pwm& pw = pwms[rs.pat[k]];
+                            const int64_t s0 = rs.start[k], s1 = s0 + (int64_t)(pw.w.size() / 4) - 1;
+                            bool hit = false;
+                            for (uint32_t j = bd.inner_off[r]; j < bd.inner_off[r + 1] && !hit; ++j) {
+                                const int64_t i0 = (int64_t)bd.inner[j].start, i1 = (int64_t)bd.inner[j].end;
+                                hit = (s0 >= i0 && s0 <= i1) || (s1 >= i0 && s1 <= i1);  // Range::overlaps, range.rs:18-21
+                            }
+                            if (!hit) continue;
+                            out += rec + "\t" + region + "\t" + pw.name + "\t" + (pw.direction == TFBS_DIR_P ? "+" : "-") + "\t" + std::to_string(s0) + "\t" +
+                                   std::to_string(s1) + "\t" + std::to_string(rs.score[k]) + "\t" + (rs.change[k] > 0 ? "+1" : "-1") + "\n";
+                        }
+                    }
+                }
+                return out;
+            };
             std::mutex fmu;
             std::condition_variable fcv;
             std::deque<Collected> to_format;
@@ -463,7 +533,8 @@ int main(int argc, char** argv) {
                         }
                     };
                     rows_to_text(it.c, bd, g.n_rows, g.region, g.inner, g.pattern_id, g.vmin, g.vmax,
-                                 [&](uint64_t i, uint32_t* l, uint32_t* r) { tfbs_expand_rows(&g, i, 1, l, r); }, at ? AttributionLines(lines) : nullptr);
+                                 [&](uint64_t i, uint32_t* l, uint32_t* r) { tfbs_expand_rows(&g, i, 1, l, r); }, at ? AttributionLines(lines) : nullptr,
+                                 it.rec ? record_lines(it.c, bd, *it.rec) : std::string());
                 }
             });
             // two blocks in flight per device: the copies and the host work of one overlap the kernels of the other
@@ -495,9 +566,15 @@ int main(int argc, char** argv) {
                     if (!o.sites_file.empty()) TF(tfbs_get_sites(ctx, &s));
                     att.reset(new OwnedAttribution(a, g, o.sites_file.empty() ? nullptr : &s));
                 }
+                std::unique_ptr<OwnedRecordSites> rec;
+                if (!o.record_sites_file.empty()) {
+                    tfbs_record_sites s;
+                    TF(tfbs_get_record_sites(ctx, &s));
+                    rec.reset(new OwnedRecordSites(s));
+                }
                 std::unique_lock<std::mutex> lk(fmu);
                 fcv.wait(lk, [&] { return to_format.size() < 2; });  // bounded: at most two collected blocks wait for their text
-                to_format.push_back(Collected{item.c, std::move(item.bd), std::move(own), std::move(att)});
+                to_format.push_back(Collected{item.c, std::move(item.bd), std::move(own), std::move(att), std::move(rec)});
                 fcv.notify_all();
             }
             {
@@ -581,6 +658,13 @@ int main(int argc, char** argv) {
     if (sites_out.is_open()) {
         sites_out.close();
         if (!sites_out) die("Could not write sites file");
+    }
+    if (record_sites_out.is_open()) {
+        record_sites_out.close();
+        if (!record_sites_out) die("Could not write record sites file");
+        if (o.verbose)
+            printf("Record sites: records without sites: %llu outside their window, %llu REF mismatch, %llu missing case\n",
+                   (unsigned long long)rec_flagged[0].load(), (unsigned long long)rec_flagged[1].load(), (unsigned long long)rec_flagged[2].load());
     }
     if (rename(part.c_str(), o.output.c_str()) != 0) die("Could not rename " + part + " into " + o.output);
     if (o.tabix) {

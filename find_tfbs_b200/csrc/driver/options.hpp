@@ -13,6 +13,7 @@ struct Options {
     std::string audit_file;  // --audit: threshold ties, truncated and overwritten haplotypes (tfbs_audit_block), tab-separated
     std::string attribution_file;  // --attribution: per written row, the configurations of records that change its count (tfbs_get_attribution)
     std::string sites_file;        // --sites: per term of a written row, the binding sites its configuration gains and loses (tfbs_get_sites)
+    std::string record_sites_file; // --record_sites: per merged region and record, the binding sites the record gains and loses alone (tfbs_get_record_sites)
     std::vector<std::string> beds, pwm_names;
     float pwm_threshold = 0;
     bool forward_only = false, tabix = false, verbose = false, has_samples = false, plain_text = false;
@@ -43,7 +44,7 @@ void usage() {
          "         --pwm_names NAME[,NAME] --pwm_file PWM.txt --pwm_threshold_directory DIR --pwm_threshold P\n"
          "         [--forward_only] [--threads N] [--min_maf N] [--after_position POS] [--samples FILE] [--tabix] [--verbose]\n"
          "         [--devices 0,1,...] [--chunk REGIONS_PER_BLOCK] [--plain] [--audit AUDIT.tsv] [--no_index] [--compression_level 1..9]\n"
-         "         [--attribution ATTRIBUTION.tsv] [--sites SITES.tsv]\n"
+         "         [--attribution ATTRIBUTION.tsv] [--sites SITES.tsv] [--record_sites RECORD_SITES.tsv]\n"
          "       find-tfbs-b200 --write_thresholds DIR --pwm_file PWM.txt [--pwm_names NAME[,NAME]] [--pvalues P[,P]]   (exact .thr files)");
 }
 
@@ -124,6 +125,8 @@ Options parse_args(int argc, char** argv) {
     if (!o.audit_file.empty() && !o.attribution_file.empty()) die("error: --attribution cannot be used with --audit");
     if (kv.count("sites")) o.sites_file = kv["sites"];
     if (!o.audit_file.empty() && !o.sites_file.empty()) die("error: --sites cannot be used with --audit");
+    if (kv.count("record_sites")) o.record_sites_file = kv["record_sites"];
+    if (!o.audit_file.empty() && !o.record_sites_file.empty()) die("error: --record_sites cannot be used with --audit");
     if (kv.count("devices")) {
         o.devices.clear();
         for (auto& d : split(kv["devices"], ',')) o.devices.push_back(atoi(d.c_str()));

@@ -104,6 +104,9 @@ struct Results {
     // sites (option "sites", tfbs_get_sites)
     HostBuf h_s_off, h_s_pat, h_s_start, h_s_score, h_s_change;
     bool have_sites = false;
+    // record sites (option "record_sites", tfbs_get_record_sites)
+    HostBuf h_r_flags, h_r_off, h_r_pat, h_r_start, h_r_score, h_r_change;
+    bool have_record_sites = false;
 };
 
 // Capacities a run of the configuration path was enqueued with (see DevPlan): sizes that only the device learns.
@@ -112,6 +115,7 @@ struct Caps {
     uint32_t capr = 0, groups = 0;
     uint64_t terms = 0;  // option "attribution": non-zero (row, configuration) differences
     uint64_t sites_raw = 0, sites = 0;  // option "sites": gained and lost hits before and after equal pairs cancel
+    uint64_t rsites = 0;                // option "record_sites": the records' hits after the cancellation
 };
 
 struct Slot {
@@ -125,6 +129,7 @@ struct Slot {
     DevBuf d_o_region, d_o_inner, d_o_pid, d_o_vmin, d_o_vmax, d_o_base, d_o_bits, d_o_off, d_o_packed, d_left, d_right;
     DevBuf d_a_ref, d_a_toff, d_a_tcfg, d_a_tdiff, d_a_creg, d_a_cflags, d_a_croff, d_a_crec, d_a_goff, d_a_gcfg;  // attribution
     DevBuf d_s_off, d_s_pat, d_s_start, d_s_score, d_s_change;  // sites
+    DevBuf d_r_flags, d_r_off, d_r_pat, d_r_start, d_r_score, d_r_change;  // record sites
     HostBuf h_status, h_plan;
     Results res;
     Caps caps;
@@ -139,6 +144,9 @@ struct Slot {
     uint64_t att_cfgs = 0, att_seqs = 0, att_terms = 0;  // their sizes (configurations, distinct haplotypes, terms)
     bool sites = false;                              // the run enqueued the sites launches
     uint64_t n_sites = 0;                            // sites after the cancellation
+    bool record_sites = false;                       // the run scored every record alone (option "record_sites")
+    bool keep_sites = false;                         // sites || record_sites: the scan keeps sites, the k_site_* launches run
+    uint64_t n_rsites = 0, n_records = 0;            // the records' sites after the cancellation; records of the block
 };
 
 // The streams a block's work is enqueued on and the scratch its kernels share with the blocks before and after it on the same lane.
@@ -165,7 +173,7 @@ struct Lane {
     DevBuf d_vmin, d_vmax, d_flag, d_rowwords, d_kbits, d_rowidx, d_rowoff;
     DevBuf d_fan_vec;  // k_fanout<true>: one count vector per CTA
     DevBuf d_att_eflag, d_att_cfgid, d_att_nrec, d_att_col, d_att_gn, d_att_tcnt;  // option "attribution"
-    DevBuf d_site_refpat, d_site_refscore, d_site_raw, d_site_bucket, d_site_keep, d_site_kpos, d_site_oid, d_site_cnt, d_site_boff;  // option "sites"
+    DevBuf d_site_refpat, d_site_refscore, d_site_raw, d_site_bucket, d_site_keep, d_site_kpos, d_site_oid, d_site_cnt, d_site_boff;  // options "sites", "record_sites"
     // full-scan path (lane 0 only)
     DevBuf d_gbase, d_cbase, d_C;
     DevBuf d_rows_region, d_rows_inner, d_rows_pid, d_rows_vmin, d_rows_vmax, d_rows_left, d_rows_right;
@@ -199,6 +207,7 @@ struct tfbs_ctx {
     int fan_vector = 0;         // 0: the fan-out's count vectors live in shared memory unless a region has too many groups; 1: always in device memory (testing)
     int attribution = 0;        // 1: the default path keeps the per-row configuration differences (tfbs_get_attribution)
     int sites = 0;              // 1: and the hits each configuration gains and loses (tfbs_get_sites; needs attribution = 1)
+    int record_sites = 0;       // 1: the default path also scores every record of the block alone (tfbs_get_record_sites)
     int dual_stream = 0;        // 1: a block in slot 1 of the default path runs on lane 1
     // attribution of the block the last tfbs_collect / tfbs_collect_grouped returned, copied to the host by that collect
     enum { ATT_NONE = 0, ATT_OFF, ATT_FULL_SCAN, ATT_READY };
@@ -206,6 +215,8 @@ struct tfbs_ctx {
     tfbs_attribution att{};
     int site_state = ATT_NONE;  // the same states for the sites of that block
     tfbs_sites site{};
+    int rec_state = ATT_NONE;   // and for its record sites
+    tfbs_record_sites rec{};
 
     // patterns
     bool have_patterns = false;

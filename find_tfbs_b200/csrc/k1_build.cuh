@@ -118,6 +118,7 @@ __device__ __forceinline__ void report(DevStatus* st, u64 q, i64 relpos, u32 cod
 struct WalkOut {
     u32 ns, len, ntake;
     bool trunc;
+    u32 err;  // DEV_* of the panic that ended the walk (reported to st only when st != NULL), else DEV_OK
 };
 template <class Sink>
 __device__ __forceinline__ WalkOut walk_diffs_to(const DevBlock& b, u32 r, const u32* dl, u32 nd, Sink&& put, DevStatus* st, u64 q_report) {
@@ -127,6 +128,7 @@ __device__ __forceinline__ WalkOut walk_diffs_to(const DevBlock& b, u32 r, const
     const i64 avail_end = start + n_ref - 1;
     u32 out = 0, ns = 0;
     bool trunc = false;
+    u32 err = DEV_OK;
     i64 rp = start;
     auto emit_ref = [&](i64 a, i64 e2) {
         if (a < start) a = start;
@@ -148,7 +150,7 @@ __device__ __forceinline__ WalkOut walk_diffs_to(const DevBlock& b, u32 r, const
             rp = d.pos;
         } else if (d.pos == rp && d.ref_len == 1) {  // :115-135 SNV or insertion
             u8 at = (rp >= start && rp <= avail_end) ? b.ref_codes[ro + (u64)(rp - start)] : (u8)4;
-            if (b.allele_codes[d.ref_off] != at) { if (st) report(st, q_report, rp - start, DEV_REF_MISMATCH); break; }
+            if (b.allele_codes[d.ref_off] != at) { err = DEV_REF_MISMATCH; if (st) report(st, q_report, rp - start, err); break; }
             put(ns++, Seg{out, d.alt_off, (int)(rp - start), 1u}, dl[k]);
             out += d.alt_len;
             rp += 1;
@@ -159,7 +161,8 @@ __device__ __forceinline__ WalkOut walk_diffs_to(const DevBlock& b, u32 r, const
             rp += d.ref_len;
             ++k;
         } else if (d.pos == rp) {  // :141-143
-            if (st) report(st, q_report, rp - start, DEV_MISSING_CASE);
+            err = DEV_MISSING_CASE;
+            if (st) report(st, q_report, rp - start, err);
             break;
         } else if (rp >= end) {  // :144-146
             trunc = true;
@@ -173,7 +176,7 @@ __device__ __forceinline__ WalkOut walk_diffs_to(const DevBlock& b, u32 r, const
         }
     }
     put(ns, Seg{out, 0u, 0, 2u}, 0xffffffffu);  // terminator
-    return WalkOut{ns, out, k, trunc};
+    return WalkOut{ns, out, k, trunc, err};
 }
 __device__ __forceinline__ WalkOut walk_diffs(const DevBlock& b, u32 r, const u32* dl, u32 nd, Seg* sg, DevStatus* st, u64 q_report) {
     return walk_diffs_to(b, r, dl, nd, [sg](u32 i, const Seg& x, u32) { sg[i] = x; }, st, q_report);

@@ -8,8 +8,9 @@ namespace tfbs {
 
 // Option "sites": the exact score of a hit, from the pattern's weights and the packed bases of the list entry (N scores 0).  On the
 // configuration path the work list is the identity (k_vitem_units), so the item is the entry, and its units hold the bases
-// [p0 & ~31, p1 + 64]: a window [i, i + L) with p0 <= i <= p1 and L <= 32 lies inside.  Then the site is kept: a configuration's hit
-// goes to the raw site list (+1), a hit of the reference haplotype is remembered next to its RefHit slot (k_cfg_lost takes the lost ones).
+// [p0 & ~31, p1 + 64]: a window [i, i + L) with p0 <= i <= p1 and L <= 32 lies inside.  Then the site is kept: a configuration's or a
+// record's hit goes to the raw site list (+1), a hit of the reference haplotype is remembered next to its RefHit slot (k_cfg_lost takes
+// the lost ones).
 __device__ __forceinline__ void keep_site(const ScanEnv* env, u32 mode, u64 at, u32 entry, u32 pi, u32 i, u32 L, int hs) {
     const DevSeqs& sq = *env->sq;
     const DevConfigs& cf = *env->cf;
@@ -31,7 +32,8 @@ __device__ __forceinline__ void keep_site(const ScanEnv* env, u32 mode, u64 at, 
 }
 
 // Rare path: a window scored above the threshold in at least one field.  SITES (a k_scan of its own, so that the registers and the
-// stack of the scan without option "sites" stay as they are): the sites are kept too (keep_site).
+// stack of the scan without options "sites" and "record_sites" stay as they are): the sites are kept too (keep_site), and the virtual
+// sequences behind the configurations are records alone, whose hits are sites only.
 template <bool SITES>
 __device__ __noinline__ u32 scan_on_hit(u64 hit, u32 t, u32 i, u32 item_index, ChunkDesc cd, const ScanEnv* env) {
     u32 counted = 0;  // hits of a full scan: the caller adds them to the statistics once per work grab
@@ -71,10 +73,14 @@ __device__ __noinline__ u32 scan_on_hit(u64 hit, u32 t, u32 i, u32 item_index, C
         if (mode == 2) {  // a configuration: its column of the region's difference matrix D[key][configuration]
             const DevConfigs& cf = *env->cf;
             const u64 c = (u64)q - sq.n_ref;
+            if (SITES && c >= cf.plan->n_cfg) {  // a record alone (option "record_sites"): nothing is counted
+                keep_site(env, 2, c, item_index, (u32)pi, i, L, (int)hs);
+                continue;
+            }
             crow = cf.D + cf.dbase[r] + (c - cf.cfgbase[r]);
             cstride = cf.ncfg[r];
             atomicAdd(&cf.cfg_net[c], 1);
-            if (SITES) keep_site(env, 2, c, item_index, (u32)pi, i, L, (int)hs);
+            if (SITES && cf.cfg_sites) keep_site(env, 2, c, item_index, (u32)pi, i, L, (int)hs);
         } else {
             crow = env->ct->C + (env->ct->cbase[r] - env->ct->cbase0) + (u64)g * pt.n_pid * nk;
             if (mode == 1) {

@@ -30,6 +30,8 @@ struct DevPlan {
     u64 n_terms, need_terms;  // option "attribution": non-zero (row, configuration) differences (k3_attribution.cuh)
     u64 site_alloc;           // option "sites": raw sites handed out by the rare path and k_cfg_lost (an atomic cursor)
     u64 n_sraw, need_sraw, n_sites, need_sites;  // raw sites, and those left after gained / lost pairs cancel (k3_sites.cuh)
+    u64 n_sid;                // configurations + records alone: the virtual sequences behind the references, the ids the sites are ranked by
+    u64 n_rsites, need_rsites;  // option "record_sites": the records' sites left after the cancellation
 };
 
 // A count becomes known: total (+ add) against the capacity its consumers were launched for.  Behind an earlier overflow nothing
@@ -55,10 +57,10 @@ __global__ void k_zero_words(u32* p, const u64* n_ptr, u64 cap) {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) p[i] = 0;
 }
 
-// Option "sites": a hit a configuration gains (+1, rare path, mode 2) or a reference hit it loses (-1, k_cfg_lost), before equal
-// (pattern, start, score) pairs cancel (k3_sites.cuh).
+// Options "sites" / "record_sites": a hit a configuration or a record alone gains (+1, rare path, mode 2) or a reference hit it loses
+// (-1, k_cfg_lost), before equal (pattern, start, score) pairs cancel (k3_sites.cuh).
 struct RawSite {
-    u32 cfg;     // virtual configuration index (cfgbase[r] + column); the output id once k_site_scatter has grouped them
+    u32 cfg;     // virtual configuration index (cfgbase[r] + column), or n_cfg + v for record v; the output id once k_site_scatter has grouped them
     u32 pat;     // pattern index
     int start;   // window start relative to region_start (pattern.rs:156)
     int score;   // exact window score
@@ -93,11 +95,13 @@ struct DevConfigs {
     u32* D;                // [region][key][configuration of the region]: difference to the reference haplotype's count (wrapping u32)
     u32* C0;               // [key] counts of the region's reference haplotype
     DevPlan* plan;
-    // option "sites" (site_raw NULL when off)
+    // options "sites" / "record_sites" (site_raw NULL when both are off)
     RawSite* site_raw;     // [site_cap] in no particular order, behind plan->site_alloc
     u64 site_cap;
     u32* ref_pat;          // parallel to DevRefHits::buf: pattern index and score of each reference hit
     int* ref_score;
+    u32 cfg_sites;         // option "sites": the configurations keep their sites too (with "record_sites" alone only the records do)
+    u8* rec_flags;         // option "record_sites": [n_var] TFBS_REC_* of every record (k_cfg_walk)
 };
 
 __device__ __forceinline__ void put_site(const DevConfigs& cf, u32 c, u32 pat, int start, int score, int change) {
@@ -205,13 +209,27 @@ __global__ void k_region_sizes(DevBlock b, DevConfigs cf) {
     if (w > 0xffffffffULL) cf.plan->abort = 1;  // a single region with more than 2^32 (configuration, key) pairs: not representable
 }
 
-// Virtual sequences: q < R is the reference haplotype of region q, R + cfgbase[r] + c configuration c of region r.
-__global__ void k_vseq_init(u32 R, DevSeqs vq) {
-    const u32 r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= R || r >= vq.n_seq) return;
-    vq.seq_region[r] = r;
-    vq.seq_leader[r] = 0xffffffffu;
-    vq.seq_nd[r] = 0;
+// Virtual sequences: q < R is the reference haplotype of region q, R + cfgbase[r] + c configuration c of region r, and (option
+// "record_sites", n_rec = the block's records) R + n_cfg + v record v alone: its diff list is [v], empty outside its region's window.
+__global__ void k_vseq_init(DevBlock b, DevConfigs cf, DevSeqs vq, u32 n_rec) {
+    const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t == 0) cf.plan->n_sid = cf.plan->n_cfg + n_rec;
+    if (t < b.R && t < vq.n_seq) {
+        vq.seq_region[t] = t;
+        vq.seq_leader[t] = 0xffffffffu;
+        vq.seq_nd[t] = 0;
+    }
+    if (t >= n_rec || cf.plan->abort) return;
+    const u64 u = (u64)vq.n_ref + cf.plan->n_cfg + t;
+    if (u >= vq.n_seq) return;
+    u32 lo = 0, hi = b.R;  // the region of record t: the last r with var_off[r] <= t
+    while (hi - lo > 1) {
+        const u32 mid = (lo + hi) / 2;
+        if (b.var_off[mid] <= t) lo = mid; else hi = mid;
+    }
+    vq.seq_region[u] = lo;
+    vq.seq_leader[u] = 0xffffffffu;
+    vq.seq_nd[u] = b.var_inwin[t] ? 1u : 0u;
 }
 __global__ void k_cfg_fill(DevSeqs sq, DevConfigs cf, DevSeqs vq, u64 d_cap) {
     if (cf.plan->abort) return;
@@ -236,6 +254,8 @@ __global__ void k_cfg_fill(DevSeqs sq, DevConfigs cf, DevSeqs vq, u64 d_cap) {
 }
 
 // Thread per virtual sequence: the configuration's records walked like patch_haplotype would walk a haplotype that carries only them.
+// A record alone that lies outside the window or meets one of patch_haplotype's panics gets its flag and length 0 (no windows): only
+// a haplotype's own walk (k_walk) fails the block.
 __global__ void k_cfg_walk(DevBlock b, DevSeqs sq, DevConfigs cf, DevSeqs vq, u64 vd_cap) {
     if (cf.plan->abort) return;
     const u32 u = blockIdx.x * blockDim.x + threadIdx.x;
@@ -244,8 +264,12 @@ __global__ void k_cfg_walk(DevBlock b, DevSeqs sq, DevConfigs cf, DevSeqs vq, u6
     const u32 nd = vq.seq_nd[u];
     if (doff + nd > vd_cap) return;
     u32* dl = vq.dlist + doff;
-    if (u >= vq.n_ref) {
-        const u32* src = sq.dlist + cf.cfg_src[u - vq.n_ref];
+    const u64 c = (u64)u - vq.n_ref, n_cfg = cf.plan->n_cfg;
+    const bool rec = u >= vq.n_ref && c >= n_cfg;
+    if (rec) {
+        if (nd) dl[0] = (u32)(c - n_cfg);
+    } else if (u >= vq.n_ref) {
+        const u32* src = sq.dlist + cf.cfg_src[c];
         for (u32 k = 0; k < nd; ++k) dl[k] = src[k];
     }
     Seg* sg = vq.segs + 2 * doff + 2 * (u64)u;
@@ -254,6 +278,12 @@ __global__ void k_cfg_walk(DevBlock b, DevSeqs sq, DevConfigs cf, DevSeqs vq, u6
     vq.seq_len[u] = w.len;
     vq.seq_flags[u] = w.trunc ? 1 : 0;
     vq.seq_ntake[u] = w.ntake;
+    if (rec) {
+        const u8 f = !nd ? (u8)TFBS_REC_OUTSIDE
+                   : w.err == DEV_REF_MISMATCH ? (u8)TFBS_REC_REF_MISMATCH : w.err == DEV_MISSING_CASE ? (u8)TFBS_REC_MISSING_CASE : (u8)0;
+        cf.rec_flags[c - n_cfg] = f;
+        if (f) vq.seq_len[u] = 0;
+    }
 }
 
 // Work list over the virtual sequences: the reference haplotype of a region in full, a configuration only at the window starts
@@ -312,12 +342,15 @@ __global__ void k_vitem_units(DevSeqs vq, const u64* n_items_ptr, u32* list) {
 
 // 8 lanes per configuration: the hits of the region's reference haplotype that the configuration does not inherit (the window is
 // not inside ONE of its reference-copy segments; behind a truncation nothing is) are taken out of its column of the difference matrix.
+// A record alone (option "record_sites") only lists them as lost sites; one without windows (a flag, k_cfg_walk) has none.
 __global__ void k_cfg_lost(DevBlock b, DevSeqs vq, DevConfigs cf, DevRefHits rh) {
     if (cf.plan->abort) return;
     constexpr u32 GS = 8;
     const u32 u = vq.n_ref + (blockIdx.x * blockDim.x + threadIdx.x) / GS;
     const u32 lane = threadIdx.x % GS;
     if (u >= seq_count(vq)) return;
+    const bool rec = (u64)u - vq.n_ref >= cf.plan->n_cfg;
+    if (rec && vq.seq_len[u] == 0) return;
     const u32 r = vq.seq_region[u];
     const u32 nh = min(rh.cnt[r - rh.r0], rh.capr);
     const u32 nk = b.inner_off[r + 1] - b.inner_off[r];
@@ -338,17 +371,18 @@ __global__ void k_cfg_lost(DevBlock b, DevSeqs vq, DevConfigs cf, DevRefHits rh)
                      (i64)h.relpos + h.len <= (i64)sg[s].relpos + (i64)(sg[s + 1].out_start - sg[s].out_start);
         if (inside) continue;
         ++lost;
-        if (cf.site_raw) {
+        if (cf.site_raw && (rec || cf.cfg_sites)) {
             const u64 x = (u64)(r - rh.r0) * rh.capr + j;
             put_site(cf, (u32)c, cf.ref_pat[x], h.relpos, cf.ref_score[x], -1);
         }
+        if (rec) continue;
         const i64 hs = h.relpos, he = hs + h.len - 1;
         for (u32 k = 0; k < nk; ++k) {
             i64 is = inner[k].start - rs, ie = inner[k].end - rs;
             if ((hs >= is && hs <= ie) || (he >= is && he <= ie)) atomicSub(&col[((u64)h.pid * nk + k) * ncfg], inner[k].multiplicity);
         }
     }
-    if (lost) atomicSub(&cf.cfg_net[c], lost);
+    if (lost && !rec) atomicSub(&cf.cfg_net[c], lost);
 }
 
 __global__ void k_refhit_need(DevRefHits rh, u32 nr, DevPlan* plan) {

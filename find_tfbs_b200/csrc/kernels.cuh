@@ -12,7 +12,8 @@
 //   K3  count/rows    k_rows_*              count_matches_by_sample fan-out           (main.rs:506-531)
 //                                           + min/max filter of counts_as_genotypes   (main.rs:439-458)
 //       attribution   k_att_*               per row, the configurations that change its count (option "attribution")
-//       sites         k_site_*              per configuration, the hits it gains and loses (option "sites")
+//       sites         k_site_*              per configuration, the hits it gains and loses (option "sites"), and per record
+//                                             alone (option "record_sites")
 //
 // All arithmetic is integer; results are bit-exact by construction (scores are i32 sums, SURVEY D1).
 #pragma once

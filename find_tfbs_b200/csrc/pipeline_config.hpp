@@ -65,6 +65,8 @@ struct ConfigPipeline {
           smem_groups(fan_smem_groups(c->prop)) {}
 
     uint32_t& launches() { return slot->stats.total_launches; }
+    // option "record_sites": one virtual sequence per record of the block, behind the configurations
+    uint64_t n_rec() const { return slot->record_sites ? B.n_var : 0; }
     int scan(const uint32_t* d_in, uint64_t n_cap, const u64* n_ptr, u64* d_out) { return device_scan(ctx, L, d_in, n_cap, n_ptr, d_out, &launches()); }
     int gate(const u64* total, uint64_t add, uint64_t cap, u64* n_out, u64* need_out) {
         TFBS_LAUNCH(k_gate, 1, 1, 0, st)(total, (u64)add, (u64)cap, n_out, need_out, &plan->abort);
@@ -96,6 +98,7 @@ struct ConfigPipeline {
         if (ctx->tiny_caps) {  // testing: every growth path runs
             c = Caps{};
             c.seq = R; c.d = 1; c.cfg = 1; c.vd = 1; c.items = ref_items + 1; c.units = 1; c.dwords = 1; c.rows = 1; c.rowwords = 1; c.capr = 1; c.groups = 1; c.terms = 1; c.sites_raw = 1; c.sites = 1;
+            c.rsites = 1;
             return;
         }
         // what the previous blocks needed (+ 25 %) when there is a history, else a guess from the shape of the block; a wrong guess
@@ -105,7 +108,7 @@ struct ConfigPipeline {
         c.seq = std::max<uint64_t>(c.seq, R);
         c.d = pick(h.d, std::min<uint64_t>(2 * c.seq, ctx->scratch_bytes / 4 / 72));
         c.cfg = pick(h.cfg, 4 * n_var + R);
-        c.vd = pick(h.vd, 2 * c.cfg);
+        c.vd = pick(h.vd, 2 * c.cfg + n_rec());  // a record alone has a one-entry diff list
         c.items = ref_items + c.vd;  // the reference haplotypes in pieces, a configuration has at most one item per carried record
         c.units = std::max<uint64_t>(pick(h.units, 0), ref_units + 8 * c.cfg);
         c.dwords = pick(h.dwords, c.cfg * (n_keys / std::max<uint32_t>(1, R) + 1));
@@ -114,8 +117,9 @@ struct ConfigPipeline {
         c.capr = ctx->refhit_cap_opt ? (uint32_t)std::max<int64_t>(1, ctx->refhit_cap_opt / std::max<uint32_t>(1, R)) : (uint32_t)pick(h.capr, 512);
         c.groups = h.groups ? groups_for(h.groups) : (uint32_t)std::min<uint64_t>((uint64_t)H + 1, 2048);
         c.terms = pick(h.terms, 4 * c.rows);
-        c.sites_raw = pick(h.sites_raw, 8 * c.cfg + 1024);
+        c.sites_raw = pick(h.sites_raw, 8 * (c.cfg + n_rec()) + 1024);
         c.sites = pick(h.sites, 4 * c.cfg + 1024);
+        c.rsites = pick(h.rsites, 4 * n_rec() + 1024);
     }
     uint64_t scratch_bytes_needed() const {
         const Caps& c = slot->caps;
@@ -123,7 +127,7 @@ struct ConfigPipeline {
         while (tbl < 2 * c.d) tbl <<= 1;
         while (seg < 2 * ((uint64_t)H + 1)) seg <<= 1;
         tbl = std::max<uint64_t>(tbl, (uint64_t)R * seg);
-        return RH * 20 + tbl * 12 + c.seq * 50 + c.d * (4 + 32 + 20 + 4) + c.seq * 32 + c.cfg * 32 + (R + c.cfg) * 60 + c.vd * 36 + c.items * 28 +
+        return RH * 20 + tbl * 12 + c.seq * 50 + c.d * (4 + 32 + 20 + 4) + c.seq * 32 + c.cfg * 32 + (R + c.cfg + n_rec()) * 60 + c.vd * 36 + c.items * 28 +
                c.units * 12 + c.dwords * 4 + n_keys * 36 + (uint64_t)c.capr * R * sizeof(RefHit) + c.rows * 34 + c.rowwords * 4 + fan_vec_bytes() + attribution_bytes() + sites_bytes();
     }
     // option "attribution": scratch per diff-list entry, configuration, distinct haplotype and row, the per-slot results, the terms
@@ -131,11 +135,14 @@ struct ConfigPipeline {
         const Caps& c = slot->caps;
         return ctx->attribution ? c.d * 20 + c.cfg * 21 + c.seq * 12 + c.rows * 16 + c.terms * 8 : 0;
     }
-    // option "sites": score and pattern of every reference hit, the raw sites twice (+ flag and index), per configuration its output id,
-    // count and offsets, the per-slot results
+    // options "sites" / "record_sites": score and pattern of every reference hit, the raw sites twice (+ flag and index), per output id
+    // its count and offsets, per configuration its output id, the per-slot results (per record its flags and offsets)
     uint64_t sites_bytes() const {
         const Caps& c = slot->caps;
-        return slot->sites ? (uint64_t)c.capr * R * 8 + c.sites_raw * (2 * sizeof(RawSite) + 12) + c.cfg * 24 + c.sites * 17 : 0;
+        if (!slot->keep_sites) return 0;
+        const uint64_t ids = c.cfg + n_rec();
+        return (uint64_t)c.capr * R * 8 + c.sites_raw * (2 * sizeof(RawSite) + 12) + ids * 12 + (slot->sites ? c.cfg * 12 + c.sites * 17 : 0) +
+               (slot->record_sites ? n_rec() * 9 + c.rsites * 17 : 0);
     }
 
     // ---- fan-out: the count vectors in shared memory (k_fanout<false>, one CTA per unit) or in device memory (k_fanout<true>) ----
@@ -204,7 +211,7 @@ struct ConfigPipeline {
         RS(L.d_moff, (c.cfg + 1) * 8);
         RS(L.d_mfill, c.cfg * 4);
         RS(L.d_members, c.d * 4);
-        const uint64_t nv = R + c.cfg;
+        const uint64_t nv = R + c.cfg + n_rec();
         RS(L.d_vq_region, nv * 4);
         RS(L.d_vq_leader, nv * 4);
         RS(L.d_vq_nd, nv * 4);
@@ -262,16 +269,26 @@ struct ConfigPipeline {
             RS(slot->d_a_goff, (c.seq + 1) * 8);
             RS(slot->d_a_gcfg, c.d * 4);
         }
-        if (slot->sites) {
+        if (slot->keep_sites) {
             RS(L.d_site_refpat, (uint64_t)c.capr * R * 4);
             RS(L.d_site_refscore, (uint64_t)c.capr * R * 4);
             RS(L.d_site_raw, c.sites_raw * sizeof(RawSite));
             RS(L.d_site_bucket, c.sites_raw * sizeof(RawSite));
             RS(L.d_site_keep, c.sites_raw * 4);
             RS(L.d_site_kpos, (c.sites_raw + 1) * 8);
+            RS(L.d_site_cnt, (c.cfg + n_rec()) * 4);
+            RS(L.d_site_boff, (c.cfg + n_rec() + 1) * 8);
+        }
+        if (slot->record_sites) {
+            RS(slot->d_r_flags, n_rec());
+            RS(slot->d_r_off, (n_rec() + 1) * 8);
+            RS(slot->d_r_pat, c.rsites * 4);
+            RS(slot->d_r_start, c.rsites * 8);
+            RS(slot->d_r_score, c.rsites * 4);
+            RS(slot->d_r_change, c.rsites);
+        }
+        if (slot->sites) {
             RS(L.d_site_oid, c.cfg * 4);
-            RS(L.d_site_cnt, c.cfg * 4);
-            RS(L.d_site_boff, (c.cfg + 1) * 8);
             RS(slot->d_s_off, (c.cfg + 1) * 8);
             RS(slot->d_s_pat, c.sites * 4);
             RS(slot->d_s_start, c.sites * 8);
@@ -325,9 +342,11 @@ struct ConfigPipeline {
         slot->stats.scan_launches = 0;
         slot->stats.scan_input_bytes = 0;
         slot->res.n_rows = 0;
-        slot->res.have_dense = slot->res.have_grouped = slot->res.have_attribution = slot->res.have_sites = false;
+        slot->res.have_dense = slot->res.have_grouped = slot->res.have_attribution = slot->res.have_sites = slot->res.have_record_sites = false;
         slot->attribution = ctx->attribution != 0;
         slot->sites = slot->attribution && ctx->sites;
+        slot->record_sites = ctx->record_sites != 0;
+        slot->keep_sites = slot->sites || slot->record_sites;
         choose_caps(first_attempt);
         const Caps& c = slot->caps;
         const bool fans = n_keys && R && S;
@@ -342,9 +361,10 @@ struct ConfigPipeline {
             return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "the block needs about " + std::to_string(scratch_bytes_needed() >> 20) +
                                                             " MB of device scratch, option scratch_mb allows " + std::to_string(ctx->scratch_bytes >> 20) +
                                                             ": submit fewer regions per block");
-        if (c.seq > 0x7fffffffull || c.d > 0xfffffff0ull || R + c.cfg > 0x7fffffffull || c.items > 0xfffffff0ull ||
+        if (c.seq > 0x7fffffffull || c.d > 0xfffffff0ull || R + c.cfg + n_rec() > 0x7fffffffull || c.items > 0xfffffff0ull ||
             (fan_vec() && (uint64_t)R * fan_split() > 0xffffffffull))
             return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "block too large for 32-bit work-list indices: submit fewer regions per block");
+        if (R && !S && slot->record_sites) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "option record_sites needs a block with at least one sample");
         if ((rc = reserve())) return rc;
         dst = slot->d_status.as<DevStatus>();
         plan = slot->d_plan.as<DevPlan>();
@@ -466,11 +486,13 @@ struct ConfigPipeline {
         cf.D = L.d_D.as<u32>();
         cf.C0 = L.d_C0.as<u32>();
         cf.plan = plan;
-        if (slot->sites) {
+        if (slot->keep_sites) {
             cf.site_raw = L.d_site_raw.as<RawSite>();
             cf.site_cap = c.sites_raw;
             cf.ref_pat = L.d_site_refpat.as<u32>();
             cf.ref_score = L.d_site_refscore.as<int>();
+            cf.cfg_sites = slot->sites ? 1u : 0u;
+            cf.rec_flags = slot->d_r_flags.as<u8>();
         }
         TFBS_LAUNCH(k_cluster, R, 128, 0, st)(db, cf);
         ++launches();
@@ -487,12 +509,13 @@ struct ConfigPipeline {
         if ((rc = scan(cf.ncfg, R, nullptr, cf.cfgbase))) return rc;
         if ((rc = scan(cf.dwords, R, nullptr, cf.dbase))) return rc;
         gate(cf.cfgbase + R, 0, c.cfg, &plan->n_cfg, &plan->need_cfg);
-        gate(cf.cfgbase + R, R, R + c.cfg, &plan->n_vseq, &plan->unused);
+        gate(cf.cfgbase + R, R + n_rec(), R + c.cfg + n_rec(), &plan->n_vseq, &plan->unused);
         gate(cf.dbase + R, 0, c.dwords, &plan->n_dwords, &plan->need_dwords);
 
-        // virtual sequences: the reference haplotype of every region, then the configurations
+        // virtual sequences: the reference haplotype of every region, then the configurations, then (option "record_sites") the records
+        const uint64_t NV = R + c.cfg + n_rec();
         DevSeqs vq{};
-        vq.n_seq = (u32)(R + c.cfg);
+        vq.n_seq = (u32)NV;
         vq.n_seq_ptr = &plan->n_vseq;
         vq.abort = &plan->abort;
         vq.n_ref = R;
@@ -515,21 +538,21 @@ struct ConfigPipeline {
         vq.pk = L.d_pk.as<u64>();
         vq.nm = L.d_nm.as<u32>();
         vq.units_cap = c.units;
-        TFBS_LAUNCH(k_vseq_init, grid_for(R, 256), 256, 0, st)(R, vq);
+        TFBS_LAUNCH(k_vseq_init, grid_for(std::max<uint64_t>(R, n_rec()), 256), 256, 0, st)(db, cf, vq, (u32)n_rec());
         TFBS_LAUNCH(k_cfg_fill, grid_for(c.seq, 128), 128, 0, st)(sq, cf, vq, (u64)c.d);
         launches() += 2;
-        if ((rc = scan(vq.seq_nd, R + c.cfg, &plan->n_vseq, vq.seq_doff))) return rc;
+        if ((rc = scan(vq.seq_nd, NV, &plan->n_vseq, vq.seq_doff))) return rc;
         TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(vq.seq_doff, &plan->n_vseq, (u64)c.vd, &plan->n_vd, &plan->need_vd, &plan->abort);
         ++launches();
-        TFBS_LAUNCH(k_cfg_walk, grid_for(R + c.cfg, 128), 128, 0, st)(db, sq, cf, vq, (u64)c.vd);
+        TFBS_LAUNCH(k_cfg_walk, grid_for(NV, 128), 128, 0, st)(db, sq, cf, vq, (u64)c.vd);
         ++launches();
 
         // ---- work list, packed bases ----
-        TFBS_LAUNCH(k_vitems<false>, grid_for(R + c.cfg, 128), 128, 0, st)(vq, cp.max_len, &plan->abort);
+        TFBS_LAUNCH(k_vitems<false>, grid_for(NV, 128), 128, 0, st)(vq, cp.max_len, &plan->abort);
         ++launches();
-        if ((rc = scan(vq.seq_nitems, R + c.cfg, &plan->n_vseq, vq.item_off))) return rc;
+        if ((rc = scan(vq.seq_nitems, NV, &plan->n_vseq, vq.item_off))) return rc;
         TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(vq.item_off, &plan->n_vseq, (u64)c.items, &plan->n_items, &plan->need_items, &plan->abort);
-        TFBS_LAUNCH(k_vitems<true>, grid_for(R + c.cfg, 128), 128, 0, st)(vq, cp.max_len, &plan->abort);
+        TFBS_LAUNCH(k_vitems<true>, grid_for(NV, 128), 128, 0, st)(vq, cp.max_len, &plan->abort);
         TFBS_LAUNCH(k_vitem_units, grid_for(c.items, 256), 256, 0, st)(vq, &plan->n_items, L.d_list.as<u32>());
         launches() += 3;
         if ((rc = scan(vq.ent_units, c.items, &plan->n_items, vq.ent_uoff))) return rc;
@@ -548,8 +571,8 @@ struct ConfigPipeline {
         DevMatches dm{};
         const int smem_bytes = (int)(sizeof(CtaShared) + SCAN_WARPS * sizeof(WarpShared) + ((cp.max_chunk_bytes + 15) & ~15u));
         const bool wide = cp.fields == 2;
-        // option "sites": the kernels whose rare path also keeps the sites
-        auto kern = wide ? (slot->sites ? k_scan<2, true> : k_scan<2>) : (slot->sites ? k_scan<3, true> : k_scan<3>);
+        // options "sites" / "record_sites": the kernels whose rare path also keeps the sites
+        auto kern = wide ? (slot->keep_sites ? k_scan<2, true> : k_scan<2>) : (slot->keep_sites ? k_scan<3, true> : k_scan<3>);
         CK(raise_smem_limit(kern, ctx->device, smem_bytes));
         uint32_t scan_grid = (uint32_t)ctx->prop.multiProcessorCount;  // persistent: one CTA per SM shares one copy of the tables
         if (ctx->scan_ctas_per_sm < 0) scan_grid = (uint32_t)std::max(1, -ctx->scan_ctas_per_sm);
@@ -565,7 +588,7 @@ struct ConfigPipeline {
 
         // ---- lost reference hits, members of the configurations, counters ----
         TFBS_LAUNCH(k_refhit_need, grid_for(R, 256), 256, 0, st)(drh, R, plan);
-        TFBS_LAUNCH(k_cfg_lost, grid_for(c.cfg * 8, 256), 256, 0, st)(db, vq, cf, drh);
+        TFBS_LAUNCH(k_cfg_lost, grid_for((c.cfg + n_rec()) * 8, 256), 256, 0, st)(db, vq, cf, drh);
         launches() += 2;
         CK(cudaMemsetAsync(cf.mcount, 0, c.cfg * 4, st));
         CK(cudaMemsetAsync(cf.mfill, 0, c.cfg * 4, st));
@@ -635,11 +658,12 @@ struct ConfigPipeline {
         } else if (ctx->attribution && (rc = enqueue_attribution(sq, cf, vq, nullptr))) {
             return rc;
         }
+        if (slot->keep_sites && (rc = enqueue_sites(vq))) return rc;
         return finish_enqueue();
     }
 
     // ---- option "attribution" (k3_attribution.cuh): behind the row headers, while D, C0, the diff lists and the runs are this block's ----
-    // 6 launches, 4 more for the terms when the block has keys, and the 8 of option "sites"
+    // 6 launches, 4 more for the terms when the block has keys
     int enqueue_attribution(const DevSeqs& sq, const DevConfigs& cf, const DevSeqs& vq, const DevFan* fn) {
         const Caps& c = slot->caps;
         int rc;
@@ -684,12 +708,13 @@ struct ConfigPipeline {
             TFBS_LAUNCH(k_att_terms<true>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
             launches() += 2;
         }
-        return slot->sites ? enqueue_sites() : TFBS_OK;
+        return TFBS_OK;
     }
 
-    // ---- option "sites" (k3_sites.cuh): behind the attribution, which has written the output id of every virtual configuration ----
-    // 8 launches
-    int enqueue_sites() {
+    // ---- options "sites" / "record_sites" (k3_sites.cuh): behind the attribution, which has written the output id of every virtual
+    // configuration; the records' ids are their own ----
+    // 8 launches, whichever of the two options are on
+    int enqueue_sites(const DevSeqs& vq) {
         const Caps& c = slot->caps;
         int rc;
         DevSites s{};
@@ -697,30 +722,43 @@ struct ConfigPipeline {
         s.bucket = L.d_site_bucket.as<RawSite>();
         s.keep = L.d_site_keep.as<u32>();
         s.kpos = L.d_site_kpos.as<u64>();
-        s.oid = L.d_site_oid.as<u32>();
         s.cnt = L.d_site_cnt.as<u32>();
         s.boff = L.d_site_boff.as<u64>();
-        s.site_off = slot->d_s_off.as<u64>();
-        s.pat = slot->d_s_pat.as<u32>();
-        s.start = slot->d_s_start.as<i64>();
-        s.score = slot->d_s_score.as<int>();
-        s.change = slot->d_s_change.as<signed char>();
-        s.cfg_region = slot->d_a_creg.as<u32>();
+        s.n_cfg = &plan->n_cfg;
+        if (slot->sites) {
+            s.oid = L.d_site_oid.as<u32>();
+            s.site_off = slot->d_s_off.as<u64>();
+            s.pat = slot->d_s_pat.as<u32>();
+            s.start = slot->d_s_start.as<i64>();
+            s.score = slot->d_s_score.as<int>();
+            s.change = slot->d_s_change.as<signed char>();
+            s.cfg_region = slot->d_a_creg.as<u32>();
+        }
+        if (slot->record_sites) {
+            s.rec_off = slot->d_r_off.as<u64>();
+            s.rec_pat = slot->d_r_pat.as<u32>();
+            s.rec_start = slot->d_r_start.as<i64>();
+            s.rec_score = slot->d_r_score.as<int>();
+            s.rec_change = slot->d_r_change.as<signed char>();
+            s.vseq_region = vq.seq_region;
+            s.n_ref = vq.n_ref;
+        }
+        const uint64_t ids = c.cfg + n_rec();
         const unsigned grid = slot->stats.sm_count * 8;
         // 1. the raw sites against their capacity, grouped by output id
         gate(&plan->site_alloc, 0, c.sites_raw, &plan->n_sraw, &plan->need_sraw);
-        CK(cudaMemsetAsync(s.cnt, 0, c.cfg * 4, st));
+        CK(cudaMemsetAsync(s.cnt, 0, ids * 4, st));
         TFBS_LAUNCH(k_site_count, grid, 256, 0, st)(s, &plan->n_sraw, &plan->abort);
         ++launches();
-        if ((rc = scan(s.cnt, c.cfg, &plan->n_cfg, s.boff))) return rc;
+        if ((rc = scan(s.cnt, ids, &plan->n_sid, s.boff))) return rc;
         TFBS_LAUNCH(k_site_scatter, grid, 256, 0, st)(s, &plan->n_sraw, &plan->abort);
-        // 2. sorted per configuration, survivors flagged
-        TFBS_LAUNCH(k_site_rank, (unsigned)std::min<uint64_t>(std::max<uint64_t>(1, c.cfg), grid), SITE_THREADS, 0, st)(s, &plan->n_cfg, &plan->abort);
+        // 2. sorted per output id, survivors flagged
+        TFBS_LAUNCH(k_site_rank, (unsigned)std::min<uint64_t>(std::max<uint64_t>(1, ids), grid), SITE_THREADS, 0, st)(s, &plan->n_sid, &plan->abort);
         launches() += 2;
-        // 3. survivors numbered, checked against the result capacity, written
+        // 3. survivors numbered, checked against the result capacities, written
         if ((rc = scan(s.keep, c.sites_raw, &plan->n_sraw, s.kpos))) return rc;
-        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(s.kpos, &plan->n_sraw, (u64)c.sites, &plan->n_sites, &plan->need_sites, &plan->abort);
-        TFBS_LAUNCH(k_site_emit, grid, 256, 0, st)(db, s, &plan->n_sraw, &plan->n_cfg, &plan->abort);
+        TFBS_LAUNCH(k_site_gate, 1, 1, 0, st)(s, &plan->n_sraw, (u64)c.sites, (u64)c.rsites, plan);
+        TFBS_LAUNCH(k_site_emit, grid, 256, 0, st)(db, s, &plan->n_sraw, &plan->n_sid, &plan->abort);
         launches() += 2;
         return TFBS_OK;
     }
@@ -799,6 +837,7 @@ struct ConfigPipeline {
         g(c.terms, hp.need_terms);
         g(c.sites_raw, hp.need_sraw);
         g(c.sites, hp.need_sites);
+        g(c.rsites, hp.need_rsites);
         if (hp.need_capr > c.capr) c.capr = (uint32_t)up(hp.need_capr);
         if (hp.need_groups > c.groups) c.groups = groups_for(hp.need_groups);
     }
@@ -815,6 +854,7 @@ struct ConfigPipeline {
         h.terms = std::max<uint64_t>(h.terms, hp.need_terms);
         h.sites_raw = std::max<uint64_t>(h.sites_raw, hp.need_sraw);
         h.sites = std::max<uint64_t>(h.sites, hp.need_sites);
+        h.rsites = std::max<uint64_t>(h.rsites, hp.need_rsites);
         h.capr = std::max<uint32_t>(h.capr, hp.need_capr);
         h.groups = std::max<uint32_t>(h.groups, hp.need_groups);
     }
@@ -854,6 +894,7 @@ struct ConfigPipeline {
         slot->att_seqs = hp.n_seq;
         slot->att_terms = hp.n_terms;
         slot->n_sites = hp.n_sites;
+        slot->n_rsites = hp.n_rsites;
         slot->res.packed_words = hp.n_rowwords;
         slot->res.row_bytes = 4;
         if (ctx->rows_width == 0) slot->res.row_bytes = hs.max_count < 256 ? 1 : (hs.max_count < 65536 ? 2 : 4);
@@ -1049,6 +1090,43 @@ struct ConfigPipeline {
         CK(cudaStreamSynchronize(so));
         slot->stats.d2h_bytes += bytes;
         res.have_sites = true;
+        return TFBS_OK;
+    }
+
+    // record sites -> host (stream_out), behind the attribution and the sites: the flags and offsets first, they give the size of the
+    // rest.  Counted in d2h_bytes.
+    int fetch_record_sites() {
+        Results& res = slot->res;
+        if (res.have_record_sites) return TFBS_OK;
+        cudaStream_t so = L.stream_out;
+        const uint64_t nv = n_rec();
+        CK(res.h_r_flags.reserve(std::max<uint64_t>(1, nv), false));
+        CK(res.h_r_off.reserve((nv + 1) * 8, false));
+        uint64_t* off = res.h_r_off.as<uint64_t>();
+        uint64_t bytes = 0;
+        off[0] = 0;
+        if (nv) {  // (with no record the layout may not have run)
+            CK(cudaMemcpyAsync(res.h_r_flags.p, slot->d_r_flags.p, nv, cudaMemcpyDeviceToHost, so));
+            CK(cudaMemcpyAsync(off, slot->d_r_off.p, (nv + 1) * 8, cudaMemcpyDeviceToHost, so));
+            CK(cudaStreamSynchronize(so));
+            bytes += nv + (nv + 1) * 8;
+        }
+        const uint64_t ns = off[nv];
+        if (ns != slot->n_rsites) return fail(ctx, TFBS_ERR_INTERNAL, "record sites: the site count disagrees with the gate");
+        auto copy = [&](HostBuf& h, const DevBuf& d, uint64_t b) -> int {
+            CK(h.reserve(std::max<uint64_t>(1, b), false));
+            if (b) CK(cudaMemcpyAsync(h.p, d.p, b, cudaMemcpyDeviceToHost, so));
+            bytes += b;
+            return TFBS_OK;
+        };
+        int rc;
+        if ((rc = copy(res.h_r_pat, slot->d_r_pat, ns * 4)) || (rc = copy(res.h_r_start, slot->d_r_start, ns * 8)) ||
+            (rc = copy(res.h_r_score, slot->d_r_score, ns * 4)) || (rc = copy(res.h_r_change, slot->d_r_change, ns)))
+            return rc;
+        CK(cudaStreamSynchronize(so));
+        slot->stats.d2h_bytes += bytes;
+        slot->n_records = nv;
+        res.have_record_sites = true;
         return TFBS_OK;
     }
 

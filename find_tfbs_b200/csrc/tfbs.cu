@@ -71,43 +71,57 @@ int finish_oldest(tfbs_ctx* ctx, Slot** out) {
     return TFBS_OK;
 }
 
-// The collect that returns a block also brings its attribution to the host (option "attribution"): a later block may take the slot's
-// device buffers before tfbs_get_attribution is called.
+// The collect that returns a block also brings its attribution, sites and record sites to the host (options "attribution", "sites",
+// "record_sites"): a later block may take the slot's device buffers before tfbs_get_attribution is called.
 int take_attribution(tfbs_ctx* ctx, Slot* slot) {
-    if (slot->full_mode) { ctx->att_state = ctx->site_state = tfbs_ctx::ATT_FULL_SCAN; return TFBS_OK; }
-    ctx->site_state = tfbs_ctx::ATT_OFF;
-    if (!slot->attribution) { ctx->att_state = tfbs_ctx::ATT_OFF; return TFBS_OK; }
-    int rc = ConfigPipeline(ctx, slot).fetch_attribution();
-    if (rc) return rc;
-    if (slot->sites) {
-        if ((rc = ConfigPipeline(ctx, slot).fetch_sites())) return rc;
+    if (slot->full_mode) { ctx->att_state = ctx->site_state = ctx->rec_state = tfbs_ctx::ATT_FULL_SCAN; return TFBS_OK; }
+    ctx->att_state = ctx->site_state = ctx->rec_state = tfbs_ctx::ATT_OFF;
+    int rc;
+    if (slot->attribution) {
+        if ((rc = ConfigPipeline(ctx, slot).fetch_attribution())) return rc;
+        if (slot->sites) {
+            if ((rc = ConfigPipeline(ctx, slot).fetch_sites())) return rc;
+            const Results& res = slot->res;
+            tfbs_sites& so = ctx->site;
+            so.n_cfgs = slot->att_cfgs;
+            so.site_off = res.h_s_off.as<uint64_t>();
+            so.pattern_index = res.h_s_pat.as<uint32_t>();
+            so.start = res.h_s_start.as<int64_t>();
+            so.score = res.h_s_score.as<int32_t>();
+            so.change = res.h_s_change.as<int8_t>();
+            ctx->site_state = tfbs_ctx::ATT_READY;
+        }
         const Results& res = slot->res;
-        tfbs_sites& so = ctx->site;
-        so.n_cfgs = slot->att_cfgs;
-        so.site_off = res.h_s_off.as<uint64_t>();
-        so.pattern_index = res.h_s_pat.as<uint32_t>();
-        so.start = res.h_s_start.as<int64_t>();
-        so.score = res.h_s_score.as<int32_t>();
-        so.change = res.h_s_change.as<int8_t>();
-        ctx->site_state = tfbs_ctx::ATT_READY;
+        tfbs_attribution& out = ctx->att;
+        memset(&out, 0, sizeof out);
+        out.n_rows = res.n_rows;
+        out.ref_count = res.h_a_ref.as<uint32_t>();
+        out.term_off = res.h_a_toff.as<uint64_t>();
+        out.term_cfg = res.h_a_tcfg.as<uint32_t>();
+        out.term_diff = res.h_a_tdiff.as<int32_t>();
+        out.n_cfgs = slot->att_cfgs;
+        out.cfg_region = res.h_a_creg.as<uint32_t>();
+        out.cfg_flags = res.h_a_cflags.as<uint8_t>();
+        out.cfg_rec_off = res.h_a_croff.as<uint64_t>();
+        out.cfg_rec = res.h_a_crec.as<uint32_t>();
+        out.n_groups_total = slot->att_seqs;
+        out.group_cfg_off = res.h_a_goff.as<uint64_t>();
+        out.group_cfg = res.h_a_gcfg.as<uint32_t>();
+        ctx->att_state = tfbs_ctx::ATT_READY;
     }
-    const Results& res = slot->res;
-    tfbs_attribution& out = ctx->att;
-    memset(&out, 0, sizeof out);
-    out.n_rows = res.n_rows;
-    out.ref_count = res.h_a_ref.as<uint32_t>();
-    out.term_off = res.h_a_toff.as<uint64_t>();
-    out.term_cfg = res.h_a_tcfg.as<uint32_t>();
-    out.term_diff = res.h_a_tdiff.as<int32_t>();
-    out.n_cfgs = slot->att_cfgs;
-    out.cfg_region = res.h_a_creg.as<uint32_t>();
-    out.cfg_flags = res.h_a_cflags.as<uint8_t>();
-    out.cfg_rec_off = res.h_a_croff.as<uint64_t>();
-    out.cfg_rec = res.h_a_crec.as<uint32_t>();
-    out.n_groups_total = slot->att_seqs;
-    out.group_cfg_off = res.h_a_goff.as<uint64_t>();
-    out.group_cfg = res.h_a_gcfg.as<uint32_t>();
-    ctx->att_state = tfbs_ctx::ATT_READY;
+    if (slot->record_sites) {
+        if ((rc = ConfigPipeline(ctx, slot).fetch_record_sites())) return rc;
+        const Results& res = slot->res;
+        tfbs_record_sites& ro = ctx->rec;
+        ro.n_records = slot->n_records;
+        ro.rec_flags = res.h_r_flags.as<uint8_t>();
+        ro.site_off = res.h_r_off.as<uint64_t>();
+        ro.pattern_index = res.h_r_pat.as<uint32_t>();
+        ro.start = res.h_r_start.as<int64_t>();
+        ro.score = res.h_r_score.as<int32_t>();
+        ro.change = res.h_r_change.as<int8_t>();
+        ctx->rec_state = tfbs_ctx::ATT_READY;
+    }
     return TFBS_OK;
 }
 
@@ -285,6 +299,10 @@ int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value) {
         if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "sites must be 0 or 1");
         ctx->sites = (int)value;
     }
+    else if (k == "record_sites") {
+        if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "record_sites must be 0 or 1");
+        ctx->record_sites = (int)value;
+    }
     else if (k == "rows_width") {
         if (value != 0 && value != 32) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "rows_width must be 32 or 0 (automatic)");
         ctx->rows_width = (int)value;
@@ -342,7 +360,7 @@ int tfbs_submit_block(tfbs_ctx* ctx, const tfbs_block* block) {
 int tfbs_collect(tfbs_ctx* ctx, tfbs_rows* out) {
     if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
     CK(cudaSetDevice(ctx->device));
-    ctx->att_state = ctx->site_state = tfbs_ctx::ATT_NONE;
+    ctx->att_state = ctx->site_state = ctx->rec_state = tfbs_ctx::ATT_NONE;
     Slot* slot = nullptr;
     int rc = finish_oldest(ctx, &slot);
     if (rc) return rc;
@@ -366,12 +384,12 @@ int tfbs_collect(tfbs_ctx* ctx, tfbs_rows* out) {
 int tfbs_collect_grouped(tfbs_ctx* ctx, tfbs_grouped_rows* out) {
     if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
     CK(cudaSetDevice(ctx->device));
-    ctx->att_state = ctx->site_state = tfbs_ctx::ATT_NONE;
+    ctx->att_state = ctx->site_state = ctx->rec_state = tfbs_ctx::ATT_NONE;
     Slot* slot = nullptr;
     int rc = finish_oldest(ctx, &slot);
     if (rc) return rc;
     if (slot->full_mode) {
-        ctx->att_state = ctx->site_state = tfbs_ctx::ATT_FULL_SCAN;
+        ctx->att_state = ctx->site_state = ctx->rec_state = tfbs_ctx::ATT_FULL_SCAN;
         retire_oldest(ctx);
         return fail(ctx, TFBS_ERR_STATE, "grouped rows come from the default scoring mode (delta = 1, record_matches off): use tfbs_collect");
     }
@@ -556,6 +574,19 @@ int tfbs_get_sites(tfbs_ctx* ctx, tfbs_sites* out) {
     default: break;
     }
     *out = ctx->site;
+    return TFBS_OK;
+}
+
+int tfbs_get_record_sites(tfbs_ctx* ctx, tfbs_record_sites* out) {
+    if (!ctx || !out) return TFBS_ERR_INVALID_ARGUMENT;
+    switch (ctx->rec_state) {
+    case tfbs_ctx::ATT_NONE: return fail(ctx, TFBS_ERR_STATE, "no block has been collected yet (tfbs_collect / tfbs_collect_grouped first): no record sites");
+    case tfbs_ctx::ATT_OFF: return fail(ctx, TFBS_ERR_STATE, "option record_sites was off for the last block: set it to 1 before the run");
+    case tfbs_ctx::ATT_FULL_SCAN:
+        return fail(ctx, TFBS_ERR_STATE, "the last block was a full scan (delta = 0, record_matches or the audit): record sites come from the default path only");
+    default: break;
+    }
+    *out = ctx->rec;
     return TFBS_OK;
 }
 

@@ -268,6 +268,31 @@ typedef struct tfbs_sites {
     const int8_t* change;           /* +1 gained, -1 lost */
 } tfbs_sites;
 
+/*
+ * Binding sites of every record on its own (option "record_sites" = 1; tfbs_get_record_sites).  Let record v be
+ * tfbs_block.variants[v], in region r, and take two multisets of (pattern_index, start, score) hit triples: A, the hits of r's extended
+ * window patched with v alone, and R, the hits of the unpatched window -- the definition of tfbs_sites with the configuration replaced
+ * by the single record.  The sites of v are A - R with change +1 and R - A with change -1, ordered within a record by (pattern_index,
+ * start, score, change) ascending.  They do not depend on hash seeds, the order threads ran in, the stream the block ran on, the
+ * fan-out or on who carries v: a record no selected sample carries has its sites too.
+ * A record with a flag has no sites:
+ *   TFBS_REC_OUTSIDE        pos lies outside the region's extended window: patch_haplotype never applies it (haplotype.rs:95);
+ *   TFBS_REC_REF_MISMATCH   patch_haplotype would panic on a haplotype that carries only v: REF does not match (haplotype.rs:126-128);
+ *   TFBS_REC_MISSING_CASE   ... or a multi-base REF and ALT (haplotype.rs:141-143).
+ * A record some haplotype carries fails the block with TFBS_ERR_REF_MISMATCH / TFBS_ERR_MISSING_CASE as always, so only records nobody
+ * carries show the last two flags.  A record alone never reaches the truncation exit.
+ */
+enum { TFBS_REC_OUTSIDE = 1, TFBS_REC_REF_MISMATCH = 2, TFBS_REC_MISSING_CASE = 4 };
+typedef struct tfbs_record_sites {
+    uint64_t n_records;             /* == var_off[n_regions] of the block: every record, in tfbs_block.variants order */
+    const uint8_t* rec_flags;       /* [n_records] TFBS_REC_* */
+    const uint64_t* site_off;       /* [n_records + 1]: sites of record v are [site_off[v], site_off[v + 1]) */
+    const uint32_t* pattern_index;  /* as tfbs_sites */
+    const int64_t* start;
+    const int32_t* score;
+    const int8_t* change;
+} tfbs_record_sites;
+
 /* Row filter: which keys tfbs_collect returns. */
 enum {
     TFBS_ROWS_VARYING = 0, /* only keys with min != max, i.e. those counts_as_genotypes keeps (main.rs:456-458) */
@@ -332,7 +357,10 @@ const char* tfbs_last_error(const tfbs_ctx* ctx);
  * memory, for tests -- results are the same either way), "attribution" (0 = off, the default; 1 = the default path also keeps the
  * per-row count differences of every configuration for tfbs_get_attribution: the rows themselves do not change), "sites" (0 = off,
  * the default; 1 = the default path also keeps the hits each configuration gains and loses, with their exact scores, for
- * tfbs_get_sites; needs "attribution" = 1, else tfbs_submit_block / tfbs_run_resident fail with TFBS_ERR_INVALID_ARGUMENT), "dual_stream"
+ * tfbs_get_sites; needs "attribution" = 1, else tfbs_submit_block / tfbs_run_resident fail with TFBS_ERR_INVALID_ARGUMENT),
+ * "record_sites" (0 = off, the default; 1 = the default path also scores every record of the block alone and keeps its sites for
+ * tfbs_get_record_sites, independently of "attribution" and "sites"; a block with regions but no sample fails with
+ * TFBS_ERR_INVALID_ARGUMENT), "dual_stream"
  * (0 = off, the default; 1 = consecutive blocks of the default scoring mode alternate between two lanes, each with its own kernel
  * and copy streams and its own device scratch, so that the kernels of the two blocks in flight overlap on the device: worth it when
  * blocks are small, while a second lane doubles the scratch of large blocks; fails with TFBS_ERR_STATE while blocks are in flight). */
@@ -419,6 +447,12 @@ int tfbs_get_attribution(tfbs_ctx* ctx, tfbs_attribution* out);
  * right after its attribution.  Fails with TFBS_ERR_STATE when nothing has been collected, when option "sites" was off for that run,
  * or when the run was a full scan ("delta" = 0, "record_matches" or the audit).  Pointers stay valid as those of tfbs_rows do. */
 int tfbs_get_sites(tfbs_ctx* ctx, tfbs_sites* out);
+
+/* Record sites (see tfbs_record_sites) of the block the last tfbs_collect or tfbs_collect_grouped returned, copied to the host by that
+ * collect behind its attribution and sites.  Fails with TFBS_ERR_STATE when nothing has been collected, when option "record_sites" was
+ * off for that run, or when the run was a full scan ("delta" = 0, "record_matches" or the audit).  Pointers stay valid as those of
+ * tfbs_rows do. */
+int tfbs_get_record_sites(tfbs_ctx* ctx, tfbs_record_sites* out);
 
 /* Matches of the last run when "record_matches" was on (call after tfbs_collect). */
 int tfbs_get_matches(tfbs_ctx* ctx, tfbs_matches* out);
