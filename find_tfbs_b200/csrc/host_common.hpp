@@ -204,11 +204,13 @@ struct tfbs_ctx {
     int audit = 0;              // set by tfbs_audit_block: per-haplotype flags are kept
     int64_t tiny_caps = 0;      // testing: start the configuration path with minimal scratch so that every growth path runs
     int64_t test_reseed = 0;    // testing: the first attempt of every block is treated as a hash collision (repeated with another seed)
+    int test_sig_bits = 0;      // testing: 1..63 = the default path's first attempt keeps that many bits of each K0 signature (real collisions)
     int fan_vector = 0;         // 0: the fan-out's count vectors live in shared memory unless a region has too many groups; 1: always in device memory (testing)
     int attribution = 0;        // 1: the default path keeps the per-row configuration differences (tfbs_get_attribution)
     int sites = 0;              // 1: and the hits each configuration gains and loses (tfbs_get_sites; needs attribution = 1)
     int record_sites = 0;       // 1: the default path also scores every record of the block alone (tfbs_get_record_sites)
     int dual_stream = 0;        // 1: a block in slot 1 of the default path runs on lane 1
+    int region_tables = 1;      // 1: the default path groups a region's haplotypes in one CTA's shared memory when they fit (k_group_region); 0: never
     // attribution of the block the last tfbs_collect / tfbs_collect_grouped returned, copied to the host by that collect
     enum { ATT_NONE = 0, ATT_OFF, ATT_FULL_SCAN, ATT_READY };
     int att_state = ATT_NONE;

@@ -68,7 +68,9 @@ __device__ __forceinline__ u32 warp_transpose32(u32 a, u32 lane) {
 
 // Warp per (region, 32 consecutive haplotypes), lane = haplotype: hash of the ordered list of carried Diff classes; 0 = no diff
 // (such a haplotype stays in the reference set, main.rs:74-81,103-105).  Launch with nr * ceil(H / 32) * 32 threads.
-__global__ void k_signatures(DevBlock b, u32 r0, u32 nr, u64 seed, u64* sig, u32* nd_in) {
+// sig_mask: ~0 except under option test_sig_bits (testing), which keeps a few bits of the first attempt's signatures so that different
+// diff lists share one and the exact check must catch it.
+__global__ void k_signatures(DevBlock b, u32 r0, u32 nr, u64 seed, u64 sig_mask, u64* sig, u32* nd_in) {
     const u64 idx = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     const u32 HW = (b.H + 31) / 32, lane = threadIdx.x & 31;
     const u64 wg = idx >> 5;
@@ -105,7 +107,7 @@ __global__ void k_signatures(DevBlock b, u32 r0, u32 nr, u64 seed, u64* sig, u32
             }
     }
     if (!valid) return;
-    sig[(size_t)r * b.H + h] = carried ? (mix64(s) | 1ULL) : 0ULL;
+    sig[(size_t)r * b.H + h] = carried ? ((mix64(s) & sig_mask) | 1ULL) : 0ULL;
     nd_in[(size_t)r * b.H + h] = inw;
 }
 
@@ -214,6 +216,139 @@ __global__ void k_group_rank(u32 H, u32 r0, const u32* leader, const u32* nd_in,
         else if (l != h) hg[h] = hg[l < H ? l : h];  // leaders were written above
     }
     if (threadIdx.x == 0) { ngroups[r] = 1 + s_base; sum_nd[r] = s_nd; }
+}
+
+// ---- K0 with the region in shared memory: k_signatures + k_group_insert + k_group_lookup + k_group_rank in one CTA per region ----
+// The same signatures, leaders (smallest haplotype of a signature), collision checks and group numbers; nothing but the results
+// leaves the CTA.  Dynamic shared memory: the table (u64 key + u32 smallest haplotype per slot, `slots` a power of two > H), per
+// haplotype its slot (then its leader) and its in-window record count (then, at leaders, its group), and the masks.
+constexpr u32 GROUP_REGION_THREADS = 1024;
+constexpr u32 GROUP_REGION_BATCH = 4;  // carrier words a lane loads before it transposes them: independent loads in flight
+__host__ __device__ __forceinline__ u64 group_region_smem(u32 H, u32 slots, u32 max_words) {
+    return (u64)slots * 12 + (u64)H * 8 + (u64)H * max_words * 4;
+}
+
+// Writes hap_group, ngroups and sum_nd like k_group_rank, the masks of the leaders only (k_walk reads nothing else), and per group
+// g >= 1 its leader and in-window record count at grp_leader / grp_nd[r * H + g - 1] (k_seq_init_groups).
+__global__ void __launch_bounds__(GROUP_REGION_THREADS, 1)
+k_group_region(DevBlock b, u64 seed, u64 sig_mask, u32 slots, u32* hap_group, u32* ngroups, u32* sum_nd, u32* grp_leader, u32* grp_nd, DevStatus* st) {
+    TFBS_DYNAMIC_SHARED(smem_raw);
+    __shared__ u32 s_warp[32];
+    __shared__ u32 s_base, s_nd;
+    const u32 r = blockIdx.x, H = b.H, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, nwarp = blockDim.x >> 5;
+    const u32 v0 = b.var_off[r], v1 = b.var_off[r + 1], nw = (v1 - v0 + 31) / 32, HW = (H + 31) / 32, tmask = slots - 1;
+    u64* s_key = (u64*)smem_raw;
+    u32* s_val = (u32*)(s_key + slots);
+    u32* s_ref = s_val + slots;  // slot of the haplotype's signature (0xffffffff: no diff), then its leader
+    u32* s_cnt = s_ref + H;      // in-window records carried, then at leaders the group number
+    u32* s_mask = s_cnt + H;     // word w of haplotype h at w * H + h
+    for (u32 i = tid; i < slots; i += blockDim.x) { s_key[i] = 0; s_val[i] = 0xffffffffu; }
+    if (tid == 0) { s_base = 0; s_nd = 0; }
+    __syncthreads();
+
+    // signatures (k_signatures: warp per 32 haplotypes, lane = haplotype), inserted as soon as they are known
+    for (u32 hw = wid; hw < HW; hw += nwarp) {
+        const u32 h = hw * 32 + lane;
+        const bool valid = h < H;
+        u64 s = seed;
+        u32 carried = 0, inw = 0;
+        for (u32 w0 = 0; w0 < nw; w0 += GROUP_REGION_BATCH) {
+            u32 cw[GROUP_REGION_BATCH];
+#pragma unroll
+            for (u32 i = 0; i < GROUP_REGION_BATCH; ++i) {
+                const u32 v = v0 + (w0 + i) * 32 + lane;
+                cw[i] = (w0 + i < nw && v < v1) ? b.carriers[(size_t)b.var_row[v] * b.pitch + hw] : 0u;
+            }
+#pragma unroll
+            for (u32 i = 0; i < GROUP_REGION_BATCH; ++i) {
+                if (w0 + i >= nw) break;  // uniform across the warp
+                __syncwarp();             // the lanes leave the bit loop below at different times: all 32 meet at the transpose
+                const u32 word = warp_transpose32(cw[i], lane);
+                if (valid) {
+                    s_mask[(w0 + i) * H + h] = word;
+                    const u32 vb = v0 + (w0 + i) * 32;
+                    for (u32 m = word; m; m &= m - 1) {
+                        const u32 vv = vb + (u32)__ffs((int)m) - 1;
+                        s = mix64(s + b.var_class[vv] + 1) * 0x9e3779b97f4a7c15ULL + carried;
+                        ++carried;
+                        inw += b.var_inwin[vv];
+                    }
+                }
+            }
+        }
+        if (!valid) continue;  // no shuffle follows in this warp's last word of haplotypes
+        s_cnt[h] = inw;
+        u32 slot = 0xffffffffu;
+        if (carried) {
+            slot = table_find_or_insert(s_key, tmask, (mix64(s) & sig_mask) | 1ULL);
+            atomicMin(&s_val[slot], h);
+        }
+        s_ref[h] = slot;
+    }
+    __syncthreads();
+
+    // leaders and their exact check (k_group_lookup); a leader's mask goes out for k_walk
+    u32* gmask = b.hap_mask + b.mask_base[r];
+    for (u32 h = tid; h < H; h += blockDim.x) {
+        const u32 slot = s_ref[h];
+        const u32 ld = slot == 0xffffffffu ? 0xffffffffu : s_val[slot];
+        s_ref[h] = ld;
+        if (ld == h) {
+            for (u32 w = 0; w < nw; ++w) gmask[(u64)w * H + h] = s_mask[w * H + h];
+            continue;
+        }
+        if (ld == 0xffffffffu) continue;
+        bool same = true;
+        for (u32 w = 0; w < nw && same; ++w) same = s_mask[w * H + h] == s_mask[w * H + ld];
+        if (same) continue;
+        if (b.region_dups[r]) {  // different records may still be the same Diff values: compare the class lists
+            u32 wi = 0, wj = 0, mi = nw ? s_mask[h] : 0u, mj = nw ? s_mask[ld] : 0u;
+            for (;;) {
+                while (!mi && ++wi < nw) mi = s_mask[wi * H + h];
+                while (!mj && ++wj < nw) mj = s_mask[wj * H + ld];
+                if (!mi || !mj) { same = !mi && !mj; break; }
+                const u32 vi = v0 + wi * 32 + (u32)__ffs((int)mi) - 1, vj = v0 + wj * 32 + (u32)__ffs((int)mj) - 1;
+                if (b.var_class[vi] != b.var_class[vj]) break;
+                mi &= mi - 1;
+                mj &= mj - 1;
+            }
+        }
+        if (!same) atomicAdd(&st->sig_collision, 1u);
+    }
+    __syncthreads();
+
+    // groups numbered 1.. in order of their leader (k_group_rank)
+    u32* hg = hap_group + (size_t)r * H;
+    u32 nd_part = 0;
+    for (u32 h0 = 0; h0 < H; h0 += blockDim.x) {
+        const u32 h = h0 + tid;
+        const u32 flag = (h < H && s_ref[h] == h) ? 1u : 0u;
+        const u32 bal = __ballot_sync(0xffffffffu, flag);
+        if (lane == 0) s_warp[wid] = __popc(bal);
+        __syncthreads();
+        u32 woff = 0, tot = 0;
+        for (u32 w = 0; w < nwarp; ++w) { const u32 c = s_warp[w]; if (w < wid) woff += c; tot += c; }
+        const u32 base = s_base;
+        if (flag) {
+            const u32 g = 1 + base + woff + __popc(bal & ((1u << lane) - 1));
+            const u32 nd = s_cnt[h];
+            hg[h] = g;
+            grp_leader[(size_t)r * H + g - 1] = h;
+            grp_nd[(size_t)r * H + g - 1] = nd;
+            nd_part += nd;
+            s_cnt[h] = g;
+        }
+        __syncthreads();
+        if (tid == 0) s_base = base + tot;
+    }
+    if (nd_part) atomicAdd(&s_nd, nd_part);
+    __syncthreads();
+    for (u32 h = tid; h < H; h += blockDim.x) {
+        const u32 ld = s_ref[h];
+        if (ld == 0xffffffffu) hg[h] = 0;
+        else if (ld != h) hg[h] = s_cnt[ld];
+    }
+    if (tid == 0) { ngroups[r] = 1 + s_base; sum_nd[r] = s_nd; }
 }
 
 }  // namespace tfbs

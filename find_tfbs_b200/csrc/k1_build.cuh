@@ -90,6 +90,24 @@ __global__ void k_seq_init(u32 H, u32 r0, const u32* hap_group, const u32* leade
         }
     }
 }
+// The same from the per-group lists of k_group_region: group g >= 1 of region r at grp_leader / grp_nd[r * H + g - 1].
+__global__ void k_seq_init_groups(u32 H, const u32* ngroups, const u32* grp_leader, const u32* grp_nd, DevSeqs sq) {
+    const u32 r = blockIdx.x;
+    const u64 qb = sq.gbase[r] - sq.gbase0;
+    if (threadIdx.x == 0 && qb < sq.n_seq) {
+        sq.seq_region[qb] = r;
+        sq.seq_leader[qb] = 0xffffffffu;
+        sq.seq_nd[qb] = 0;
+    }
+    const u32 ng = ngroups[r];
+    for (u32 g = 1 + threadIdx.x; g < ng; g += blockDim.x) {
+        const u64 q = qb + g;
+        if (q >= sq.n_seq) break;  // more sequences than the scratch holds: the run is repeated (need_seq)
+        sq.seq_region[q] = r;
+        sq.seq_leader[q] = grp_leader[(size_t)r * H + g - 1];
+        sq.seq_nd[q] = grp_nd[(size_t)r * H + g - 1];
+    }
+}
 
 // derived Ord of Diff: (pos, reference, alternative), vectors lexicographic, A<C<G<T<N (types.rs:5-8,39-44)
 __device__ __forceinline__ int cmp_codes(const u8* a, u32 na, const u8* b, u32 nb) {

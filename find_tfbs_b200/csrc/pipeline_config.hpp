@@ -159,6 +159,24 @@ struct ConfigPipeline {
     uint64_t fan_vec_stride() const { return ((uint64_t)slot->caps.groups + 31) & ~31ull; }  // words of a CTA's slice, 128-byte aligned
     uint64_t fan_vec_bytes() const { return (n_keys && fan_vec()) ? (uint64_t)fan_vec_grid() * fan_vec_stride() * 4 : 0; }
 
+    // ---- K0 ----------------------------------------------------------------------------------------------------------------
+    // mask words per haplotype of the block's largest region (ceil(V / 32))
+    uint32_t max_mask_words() const {
+        uint32_t v = 0;
+        for (uint32_t r = 0; r < R; ++r) v = std::max(v, B.h_var_off[r + 1] - B.h_var_off[r]);
+        return (v + 31) / 32;
+    }
+    // Table slots of k_group_region (a power of two >= 1.25 H + 1: at most H signatures, a load factor below 0.8), or 0 when the block
+    // groups with the block-wide tables (k_signatures .. k_group_rank): option region_tables is 0, or the table, the per-haplotype
+    // words and the masks of the largest region exceed what a CTA may hold next to the kernel's static shared memory (144 bytes, ptxas).
+    uint32_t region_group_slots() const {
+        if (!ctx->region_tables) return 0;
+        uint64_t slots = 64;
+        while (slots < (uint64_t)H + H / 4 + 1) slots <<= 1;
+        if (group_region_smem(H, (uint32_t)slots, max_mask_words()) + 256 > ctx->prop.sharedMemPerBlockOptin) return 0;
+        return (uint32_t)slots;
+    }
+
     // ---- scratch -------------------------------------------------------------------------------------------------------
     int reserve() {
         const Caps& c = slot->caps;
@@ -404,14 +422,25 @@ struct ConfigPipeline {
         // the tables of K0 and of the sequence-keyed map: one segment of `seg` slots per region (L2-resident while the region is worked on)
         uint32_t seg = 64;
         while (seg < 2 * ((uint64_t)H + 1)) seg <<= 1;
-        {
+        const uint32_t group_slots = region_group_slots();
+        // option test_sig_bits (testing): the first attempt's signatures keep that many bits, so that the exact check meets collisions
+        const u64 sig_mask = (ctx->test_sig_bits && slot->attempts == 0) ? (1ull << ctx->test_sig_bits) - 1 : ~0ull;
+        if (group_slots) {
+            const int smem = (int)group_region_smem(H, group_slots, max_mask_words());
+            CK(raise_smem_limit(k_group_region, ctx->device, smem));
+            // a warp per 32 haplotypes up to GROUP_REGION_THREADS: small cohorts (configs[1]: 200 haplotypes) keep several CTAs per SM
+            const uint32_t threads = std::min<uint32_t>(GROUP_REGION_THREADS, std::max<uint32_t>(64, (H + 31) / 32 * 32));
+            TFBS_LAUNCH(k_group_region, R, threads, smem, st)(db, slot->seed, sig_mask, group_slots, hap_group, L.d_ngroups.as<u32>(), L.d_sum_nd.as<u32>(),
+                                                                          L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), dst);
+            ++launches();
+        } else {
             const uint64_t max_pairs = 1ull << 25;
             const uint32_t regions_per_super = (uint32_t)std::max<uint64_t>(1, max_pairs / std::max<uint32_t>(1, H));
             for (uint32_t r0 = 0; r0 < R; r0 += regions_per_super) {
                 const uint32_t nr = std::min(regions_per_super, R - r0);
                 const uint64_t pairs = (uint64_t)nr * H;
                 if ((rc = table_slots((uint64_t)nr * seg))) return rc;
-                TFBS_LAUNCH(k_signatures, grid_for((uint64_t)nr * ((H + 31) / 32) * 32, 256), 256, 0, st)(db, r0, nr, slot->seed, L.d_sig.as<u64>(), L.d_nd_in.as<u32>());
+                TFBS_LAUNCH(k_signatures, grid_for((uint64_t)nr * ((H + 31) / 32) * 32, 256), 256, 0, st)(db, r0, nr, slot->seed, sig_mask, L.d_sig.as<u64>(), L.d_nd_in.as<u32>());
                 TFBS_LAUNCH(k_group_insert, grid_for(pairs, 256), 256, 0, st)(H, r0, nr, L.d_sig.as<u64>(), L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg);
                 TFBS_LAUNCH(k_group_lookup, grid_for(pairs, 256), 256, 0, st)(db, r0, nr, L.d_sig.as<u64>(), L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg,
                                                                      L.d_leader.as<u32>(), dst);
@@ -443,7 +472,8 @@ struct ConfigPipeline {
         sq.seq_hash = L.d_seq_hash.as<u64>();
         sq.seq_flags = L.d_seq_flags.as<u8>();
         sq.seq_ntake = L.d_seq_ntake.as<u32>();
-        TFBS_LAUNCH(k_seq_init, R, 128, 0, st)(H, 0, hap_group, L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), sq);
+        if (group_slots) TFBS_LAUNCH(k_seq_init_groups, R, 128, 0, st)(H, L.d_ngroups.as<u32>(), L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), sq);
+        else TFBS_LAUNCH(k_seq_init, R, 128, 0, st)(H, 0, hap_group, L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), sq);
         ++launches();
         if ((rc = scan(sq.seq_nd, c.seq, &plan->n_seq, sq.seq_doff))) return rc;
         // the total sits behind the last sequence; k_gate reads it through the clamped count

@@ -156,7 +156,7 @@ private:
                 CK(L.d_vals.reserve((size_t)cap * 4));
                 CK(cudaMemsetAsync(L.d_keys.p, 0, (size_t)cap * 8, st));
                 CK(cudaMemsetAsync(L.d_vals.p, 0xff, (size_t)cap * 4, st));
-                TFBS_LAUNCH(k_signatures, grid_for((uint64_t)nr * ((H + 31) / 32) * 32, 256), 256, 0, st)(db, r0, nr, seed, L.d_sig.as<u64>(), L.d_nd_in.as<u32>());
+                TFBS_LAUNCH(k_signatures, grid_for((uint64_t)nr * ((H + 31) / 32) * 32, 256), 256, 0, st)(db, r0, nr, seed, ~0ull, L.d_sig.as<u64>(), L.d_nd_in.as<u32>());
                 TFBS_LAUNCH(k_group_insert, grid_for(pairs, 256), 256, 0, st)(H, r0, nr, L.d_sig.as<u64>(), L.d_keys.as<u64>(), L.d_vals.as<u32>(), cap - 1, 0u);
                 TFBS_LAUNCH(k_group_lookup, grid_for(pairs, 256), 256, 0, st)(db, r0, nr, L.d_sig.as<u64>(), L.d_keys.as<u64>(), L.d_vals.as<u32>(), cap - 1, 0u,
                                                                      L.d_leader.as<u32>(), dst);

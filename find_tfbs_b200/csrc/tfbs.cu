@@ -287,9 +287,17 @@ int tfbs_set_option(tfbs_ctx* ctx, const char* key, int64_t value) {
     else if (k == "refhit_cap") ctx->refhit_cap_opt = std::max<int64_t>(0, value);
     else if (k == "tiny_caps") ctx->tiny_caps = value;
     else if (k == "test_reseed") ctx->test_reseed = value;
+    else if (k == "test_sig_bits") {
+        if (value < 0 || value > 63) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "test_sig_bits must be 0 (off) .. 63");
+        ctx->test_sig_bits = (int)value;
+    }
     else if (k == "fan_vector") {
         if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "fan_vector must be 0 (automatic) or 1 (device memory)");
         ctx->fan_vector = (int)value;
+    }
+    else if (k == "region_tables") {
+        if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "region_tables must be 0 or 1");
+        ctx->region_tables = (int)value;
     }
     else if (k == "attribution") {
         if (value != 0 && value != 1) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "attribution must be 0 or 1");

@@ -354,7 +354,9 @@ const char* tfbs_last_error(const tfbs_ctx* ctx);
  * that holds every count of the block, see tfbs_rows.count_bytes -- result rows are the dominant PCIe traffic of large cohorts),
  * "fan_vector" (0 = automatic, the default: the fan-out keeps its per-group count vectors in shared memory and switches to device
  * memory when a region of the block may have more distinct haplotypes than shared memory holds, 53,120; 1 = always in device
- * memory, for tests -- results are the same either way), "attribution" (0 = off, the default; 1 = the default path also keeps the
+ * memory, for tests -- results are the same either way), "region_tables" (1 = the default: the default path groups the haplotypes
+ * of a region in one CTA's shared memory when the block's haplotypes and records per region fit there, and with the block-wide
+ * tables otherwise; 0 = always the block-wide tables, for tests and comparisons -- results are the same either way), "attribution" (0 = off, the default; 1 = the default path also keeps the
  * per-row count differences of every configuration for tfbs_get_attribution: the rows themselves do not change), "sites" (0 = off,
  * the default; 1 = the default path also keeps the hits each configuration gains and loses, with their exact scores, for
  * tfbs_get_sites; needs "attribution" = 1, else tfbs_submit_block / tfbs_run_resident fail with TFBS_ERR_INVALID_ARGUMENT),
