@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <climits>
 #include <cstdio>
 #include <cstring>
@@ -109,14 +110,9 @@ struct Results {
     bool have_record_sites = false;
 };
 
-// Capacities a run of the configuration path was enqueued with (see DevPlan): sizes that only the device learns.
-struct Caps {
-    uint64_t seq = 0, d = 0, cfg = 0, vd = 0, items = 0, units = 0, dwords = 0, rows = 0, rowwords = 0;
-    uint32_t capr = 0, groups = 0;
-    uint64_t terms = 0;  // option "attribution": non-zero (row, configuration) differences
-    uint64_t sites_raw = 0, sites = 0;  // option "sites": gained and lost hits before and after equal pairs cancel
-    uint64_t rsites = 0;                // option "record_sites": the records' hits after the cancellation
-};
+// Capacities a run of the configuration path was enqueued with, indexed by Cap (see DevPlan): sizes that only the device learns.
+using Caps = std::array<uint64_t, Cap::N>;
+const char* const CAP_NAMES[Cap::N] = {"seq", "d", "cfg", "vd", "items", "units", "dwords", "rows", "rowwords", "capr", "groups", "terms", "sites_raw", "sites", "rsites"};
 
 struct Slot {
     int state = 0;  // 0 free, 1 enqueued (nothing has been waited for), 2 finished (results final)
@@ -132,7 +128,7 @@ struct Slot {
     DevBuf d_r_flags, d_r_off, d_r_pat, d_r_start, d_r_score, d_r_change;  // record sites
     HostBuf h_status, h_plan;
     Results res;
-    Caps caps;
+    Caps caps{};
     uint64_t seed = 0;
     uint64_t n_keys = 0;
     int rows_mode = 0;
@@ -234,7 +230,7 @@ struct tfbs_ctx {
     int last = -1;                 // slot of the most recent tfbs_collect (stats, matches)
     BlockDev resident;
     BlockDev* last_block = nullptr;  // block of the most recent submit / upload (tfbs_audit_block)
-    Caps hint;                     // largest needs seen so far (+ 25 %): what the next block is given
+    Caps hint{};                   // largest needs seen so far (+ 25 %): what the next block is given
     uint8_t* arena = nullptr;      // tfbs_set_result_arena: grouped rows are copied straight into the caller's memory
     size_t arena_bytes = 0;
 
@@ -402,16 +398,26 @@ int upload_block(tfbs_ctx* ctx, const tfbs_block* b, BlockDev* B, cudaStream_t s
     return TFBS_OK;
 }
 
-// Scratch the input encoding of a block needs (shared by both pipelines).
+// Scratch the input encoding of a block needs (shared by both pipelines): visit(buffer, bytes) once per buffer.
+template <class Visit> void encoding_buffers(Lane& L, const BlockDev& B, Visit&& visit) {
+    visit(L.d_ref_codes, std::max<uint64_t>(1, B.n_ref_bytes));
+    visit(L.d_allele_codes, std::max<uint64_t>(1, B.n_allele_bytes));
+    visit(L.d_var_class, std::max<uint64_t>(1, B.n_var) * 4);
+    visit(L.d_var_inwin, std::max<uint64_t>(1, B.n_var));
+    visit(L.d_var_althash, std::max<uint64_t>(1, B.n_var) * 8);
+    visit(L.d_ref_prefix, (B.n_ref_bytes + B.R + 1) * 8);
+}
 int reserve_encoding(tfbs_ctx* ctx, Lane& L, const BlockDev& B) {
-    int rc;
-    if ((rc = grow(ctx, L.d_ref_codes, std::max<uint64_t>(1, B.n_ref_bytes)))) return rc;
-    if ((rc = grow(ctx, L.d_allele_codes, std::max<uint64_t>(1, B.n_allele_bytes)))) return rc;
-    if ((rc = grow(ctx, L.d_var_class, std::max<uint64_t>(1, B.n_var) * 4))) return rc;
-    if ((rc = grow(ctx, L.d_var_inwin, std::max<uint64_t>(1, B.n_var)))) return rc;
-    if ((rc = grow(ctx, L.d_var_althash, std::max<uint64_t>(1, B.n_var) * 8))) return rc;
-    if ((rc = grow(ctx, L.d_ref_prefix, (B.n_ref_bytes + B.R + 1) * 8))) return rc;
-    return TFBS_OK;
+    int rc = TFBS_OK;
+    encoding_buffers(L, B, [&](DevBuf& buf, uint64_t bytes) { if (!rc) rc = grow(ctx, buf, bytes); });
+    return rc;
+}
+
+// Slots of an open-addressing table for `entries` keys: a power of two >= 2 * entries, at least 1024.
+inline uint64_t table_slots_for(uint64_t entries) {
+    uint64_t slots = 1024;
+    while (slots < 2 * entries) slots <<= 1;
+    return slots;
 }
 
 // The block's arrays are only read: both lanes may run the resident block at once.  Its encoding is the lane's scratch.

@@ -73,7 +73,7 @@ __device__ __noinline__ u32 scan_on_hit(u64 hit, u32 t, u32 i, u32 item_index, C
         if (mode == 2) {  // a configuration: its column of the region's difference matrix D[key][configuration]
             const DevConfigs& cf = *env->cf;
             const u64 c = (u64)q - sq.n_ref;
-            if (SITES && c >= cf.plan->n_cfg) {  // a record alone (option "record_sites"): nothing is counted
+            if (SITES && c >= cf.plan->n[Cap::cfg]) {  // a record alone (option "record_sites"): nothing is counted
                 keep_site(env, 2, c, item_index, (u32)pi, i, L, (int)hs);
                 continue;
             }

@@ -15,23 +15,43 @@
 
 namespace tfbs {
 
+// The sizes that only the device learns, each with a capacity the host chose (Caps, DevPlan::n / need).
+struct Cap {
+    enum : int {
+        seq,        // distinct haplotypes (sequences)
+        d,          // their in-window diff-list entries
+        cfg,        // configurations
+        vd,         // diff-list entries of the virtual sequences
+        items,      // work-list items
+        units,      // units of 32 packed bases
+        dwords,     // words of the difference matrices
+        rows,       // rows
+        rowwords,   // packed row words
+        capr,       // reference hits kept per region
+        groups,     // groups a fan-out count vector holds
+        terms,      // option "attribution": non-zero (row, configuration) differences (k3_attribution.cuh)
+        sites_raw,  // options "sites" / "record_sites": raw sites, before gained / lost pairs cancel (k3_sites.cuh)
+        sites,      // option "sites": the configurations' sites after the cancellation
+        rsites,     // option "record_sites": the records' sites after the cancellation
+        N
+    };
+};
+
 // Sizes that are decided on the device.  Every stage is launched for a capacity the host chose; a gate kernel between two stages
 // publishes the real count (clamped to the capacity), records the need and raises `abort` when the capacity was too small: the host
 // then repeats the run with more scratch.  No stage ever comes back to the host.
 struct DevPlan {
-    u64 n_seq, n_d, n_cfg, n_vseq, n_vd, n_items, n_units, n_members, n_dwords, n_rows, n_rowwords;
-    u64 need_seq, need_d, need_cfg, need_vd, need_items, need_units, need_members, need_dwords, need_rows, need_rowwords;
-    u32 need_capr, need_groups;
+    u64 n[Cap::N];     // the counts, clamped to their capacity (none for capr and groups)
+    u64 need[Cap::N];  // what the run needed, 0 where an earlier overflow left it unknown
+    u64 n_vseq;        // virtual sequences: the reference haplotypes, the configurations, the records alone
+    u64 n_members;     // entries of the configurations' member lists
+    u64 n_sid;         // configurations + records alone: the virtual sequences behind the references, the ids the sites are ranked by
     u32 abort, cfg_collision;
-    u64 unused;
+    u64 unused;          // the need of the gates whose count is bounded by an earlier capacity (n_vseq, n_members)
     u64 rowwords_alloc;  // packed row words handed out by the fan-out (an atomic cursor)
     u64 fan_keys;        // keys the fan-out built a count vector for
     u64 fan_dbg[5];      // -DTFBS_FAN_STATS: pairs, member updates, groups with a non-zero difference, samples with one, keys of the dense pass
-    u64 n_terms, need_terms;  // option "attribution": non-zero (row, configuration) differences (k3_attribution.cuh)
-    u64 site_alloc;           // option "sites": raw sites handed out by the rare path and k_cfg_lost (an atomic cursor)
-    u64 n_sraw, need_sraw, n_sites, need_sites;  // raw sites, and those left after gained / lost pairs cancel (k3_sites.cuh)
-    u64 n_sid;                // configurations + records alone: the virtual sequences behind the references, the ids the sites are ranked by
-    u64 n_rsites, need_rsites;  // option "record_sites": the records' sites left after the cancellation
+    u64 site_alloc;      // options "sites" / "record_sites": raw sites handed out by the rare path and k_cfg_lost (an atomic cursor)
 };
 
 // A count becomes known: total (+ add) against the capacity its consumers were launched for.  Behind an earlier overflow nothing
@@ -213,14 +233,14 @@ __global__ void k_region_sizes(DevBlock b, DevConfigs cf) {
 // "record_sites", n_rec = the block's records) R + n_cfg + v record v alone: its diff list is [v], empty outside its region's window.
 __global__ void k_vseq_init(DevBlock b, DevConfigs cf, DevSeqs vq, u32 n_rec) {
     const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t == 0) cf.plan->n_sid = cf.plan->n_cfg + n_rec;
+    if (t == 0) cf.plan->n_sid = cf.plan->n[Cap::cfg] + n_rec;
     if (t < b.R && t < vq.n_seq) {
         vq.seq_region[t] = t;
         vq.seq_leader[t] = 0xffffffffu;
         vq.seq_nd[t] = 0;
     }
     if (t >= n_rec || cf.plan->abort) return;
-    const u64 u = (u64)vq.n_ref + cf.plan->n_cfg + t;
+    const u64 u = (u64)vq.n_ref + cf.plan->n[Cap::cfg] + t;
     if (u >= vq.n_seq) return;
     u32 lo = 0, hi = b.R;  // the region of record t: the last r with var_off[r] <= t
     while (hi - lo > 1) {
@@ -264,7 +284,7 @@ __global__ void k_cfg_walk(DevBlock b, DevSeqs sq, DevConfigs cf, DevSeqs vq, u6
     const u32 nd = vq.seq_nd[u];
     if (doff + nd > vd_cap) return;
     u32* dl = vq.dlist + doff;
-    const u64 c = (u64)u - vq.n_ref, n_cfg = cf.plan->n_cfg;
+    const u64 c = (u64)u - vq.n_ref, n_cfg = cf.plan->n[Cap::cfg];
     const bool rec = u >= vq.n_ref && c >= n_cfg;
     if (rec) {
         if (nd) dl[0] = (u32)(c - n_cfg);
@@ -349,7 +369,7 @@ __global__ void k_cfg_lost(DevBlock b, DevSeqs vq, DevConfigs cf, DevRefHits rh)
     const u32 u = vq.n_ref + (blockIdx.x * blockDim.x + threadIdx.x) / GS;
     const u32 lane = threadIdx.x % GS;
     if (u >= seq_count(vq)) return;
-    const bool rec = (u64)u - vq.n_ref >= cf.plan->n_cfg;
+    const bool rec = (u64)u - vq.n_ref >= cf.plan->n[Cap::cfg];
     if (rec && vq.seq_len[u] == 0) return;
     const u32 r = vq.seq_region[u];
     const u32 nh = min(rh.cnt[r - rh.r0], rh.capr);
@@ -390,7 +410,7 @@ __global__ void k_refhit_need(DevRefHits rh, u32 nr, DevPlan* plan) {
     if (r >= nr) return;
     const u32 n = rh.cnt[r];
     if (n > rh.capr) plan->abort = 1;
-    atomicMax(&plan->need_capr, n);
+    atomicMax(&plan->need[Cap::capr], (u64)n);
 }
 
 // Members of the configurations (thread per distinct haplotype, twice: count, then fill).  The fill pass also adds up the work

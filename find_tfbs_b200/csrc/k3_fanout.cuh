@@ -165,10 +165,10 @@ __global__ void __launch_bounds__(FAN_THREADS) k_fanout(DevBlock b, DevConfigs c
         const u32 rs = min((u32)FAN_THREADS, max(kmin, (nkeys_all + TFBS_FAN_SPLIT_NOW - 1) / TFBS_FAN_SPLIT_NOW));
         if ((u64)cy * rs >= (u64)nkeys_all) continue;  // no round for this CTA
         if (ng > fn.groups_cap) {  // more distinct haplotypes than the count vector holds: the host repeats the run
-            if (tid == 0) { atomicMax(&cf.plan->need_groups, ng); cf.plan->abort = 1; }
+            if (tid == 0) { atomicMax(&cf.plan->need[Cap::groups], (u64)ng); cf.plan->abort = 1; }
             return;
         }
-        if (tid == 0) atomicMax(&cf.plan->need_groups, ng);
+        if (tid == 0) atomicMax(&cf.plan->need[Cap::groups], (u64)ng);
         const u32 nk = b.inner_off[r + 1] - b.inner_off[r];
         const u32 nkeys = fn.n_pid * nk;
         const u64 kb = cf.kbase[r];

@@ -26,14 +26,14 @@ constexpr int SITE_THREADS = 128;
 
 struct DevSites {
     // scratch (shared by consecutive blocks)
-    RawSite* raw;       // [Caps::sites_raw] the raw sites (DevConfigs::site_raw); after the scatter, the sorted order
-    RawSite* bucket;    // [Caps::sites_raw] grouped by output id
-    u32* keep;          // [Caps::sites_raw] 1 at a surviving site of the sorted order
-    u64* kpos;          // [Caps::sites_raw + 1] exclusive scan of keep: the survivor's output index
+    RawSite* raw;       // [Cap::sites_raw] the raw sites (DevConfigs::site_raw); after the scatter, the sorted order
+    RawSite* bucket;    // [Cap::sites_raw] grouped by output id
+    u32* keep;          // [Cap::sites_raw] 1 at a surviving site of the sorted order
+    u64* kpos;          // [Cap::sites_raw + 1] exclusive scan of keep: the survivor's output index
     const u32* oid;     // [cfg] output id of each virtual configuration (DevAttr::site_oid)
     u32* cnt;           // [cfg + records] raw sites per output id
     u64* boff;          // [cfg + records + 1] exclusive scan of cnt
-    const u64* n_cfg;   // DevPlan::n_cfg: ids from n_cfg on are records
+    const u64* n_cfg;   // DevPlan::n[Cap::cfg]: ids from n_cfg on are records
     // results (per slot): option "sites" (site_off NULL when off)
     u64* site_off;      // [cfg + 1]
     u32* pat;           // [sites]
@@ -117,13 +117,13 @@ __global__ void __launch_bounds__(SITE_THREADS) k_site_rank(DevSites s, const u6
 
 // The survivors of the configurations and those of the records against their result capacities (as k_gate_at does for one count).
 __global__ void k_site_gate(DevSites s, const u64* n_raw_ptr, u64 cap_cfg, u64 cap_rec, DevPlan* plan) {
-    if (plan->abort) { plan->need_sites = plan->n_sites = plan->need_rsites = plan->n_rsites = 0; return; }
+    if (plan->abort) { plan->need[Cap::sites] = plan->n[Cap::sites] = plan->need[Cap::rsites] = plan->n[Cap::rsites] = 0; return; }
     const u64 all = s.kpos[*n_raw_ptr], in_cfg = s.kpos[s.boff[*s.n_cfg]];
-    plan->need_sites = in_cfg;
-    plan->need_rsites = all - in_cfg;
+    plan->need[Cap::sites] = in_cfg;
+    plan->need[Cap::rsites] = all - in_cfg;
     if (in_cfg > cap_cfg || all - in_cfg > cap_rec) plan->abort = 1;
-    plan->n_sites = in_cfg > cap_cfg ? cap_cfg : in_cfg;
-    plan->n_rsites = all - in_cfg > cap_rec ? cap_rec : all - in_cfg;
+    plan->n[Cap::sites] = in_cfg > cap_cfg ? cap_cfg : in_cfg;
+    plan->n[Cap::rsites] = all - in_cfg > cap_rec ? cap_rec : all - in_cfg;
 }
 
 // The survivors in sorted order behind their block-wide index (the records' behind those of the configurations), site_off[o] = the

@@ -68,10 +68,14 @@ struct ConfigPipeline {
     // option "record_sites": one virtual sequence per record of the block, behind the configurations
     uint64_t n_rec() const { return slot->record_sites ? B.n_var : 0; }
     int scan(const uint32_t* d_in, uint64_t n_cap, const u64* n_ptr, u64* d_out) { return device_scan(ctx, L, d_in, n_cap, n_ptr, d_out, &launches()); }
-    int gate(const u64* total, uint64_t add, uint64_t cap, u64* n_out, u64* need_out) {
-        TFBS_LAUNCH(k_gate, 1, 1, 0, st)(total, (u64)add, (u64)cap, n_out, need_out, &plan->abort);
+    // capacity i against its count: total (+ add), or the total of an exclusive scan behind element *n_ptr
+    void gate(int i, const u64* total, uint64_t add) {
+        TFBS_LAUNCH(k_gate, 1, 1, 0, st)(total, (u64)add, (u64)slot->caps[i], &plan->n[i], &plan->need[i], &plan->abort);
         ++launches();
-        return TFBS_OK;
+    }
+    void gate_at(int i, const u64* offsets, const u64* n_ptr) {
+        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(offsets, n_ptr, (u64)slot->caps[i], &plan->n[i], &plan->need[i], &plan->abort);
+        ++launches();
     }
 
     // ---- capacities ------------------------------------------------------------------------------------------------
@@ -96,58 +100,44 @@ struct ConfigPipeline {
         }
         if (!first_attempt) return;  // a repeated run keeps the capacities finalize() grew
         if (ctx->tiny_caps) {  // testing: every growth path runs
-            c = Caps{};
-            c.seq = R; c.d = 1; c.cfg = 1; c.vd = 1; c.items = ref_items + 1; c.units = 1; c.dwords = 1; c.rows = 1; c.rowwords = 1; c.capr = 1; c.groups = 1; c.terms = 1; c.sites_raw = 1; c.sites = 1;
-            c.rsites = 1;
+            c.fill(1);
+            c[Cap::seq] = R;
+            c[Cap::items] = ref_items + 1;
             return;
         }
         // what the previous blocks needed (+ 25 %) when there is a history, else a guess from the shape of the block; a wrong guess
         // costs one repeated run of this block, never a wrong result
-        auto pick = [](uint64_t hinted, uint64_t cold) { return hinted ? up(hinted) : cold; };
-        c.seq = std::min<uint64_t>(RH + R, pick(h.seq, std::min<uint64_t>(RH + R, std::max<uint64_t>(R, ctx->scratch_bytes / 8 / 128))));
-        c.seq = std::max<uint64_t>(c.seq, R);
-        c.d = pick(h.d, std::min<uint64_t>(2 * c.seq, ctx->scratch_bytes / 4 / 72));
-        c.cfg = pick(h.cfg, 4 * n_var + R);
-        c.vd = pick(h.vd, 2 * c.cfg + n_rec());  // a record alone has a one-entry diff list
-        c.items = ref_items + c.vd;  // the reference haplotypes in pieces, a configuration has at most one item per carried record
-        c.units = std::max<uint64_t>(pick(h.units, 0), ref_units + 8 * c.cfg);
-        c.dwords = pick(h.dwords, c.cfg * (n_keys / std::max<uint32_t>(1, R) + 1));
-        c.rows = std::min<uint64_t>(std::max<uint64_t>(1, n_keys), pick(h.rows, std::max<uint64_t>(4096, n_keys / 4)));
-        c.rowwords = pick(h.rowwords, c.rows * ((uint64_t)(H + 1) / 32 + 1));
-        c.capr = ctx->refhit_cap_opt ? (uint32_t)std::max<int64_t>(1, ctx->refhit_cap_opt / std::max<uint32_t>(1, R)) : (uint32_t)pick(h.capr, 512);
-        c.groups = h.groups ? groups_for(h.groups) : (uint32_t)std::min<uint64_t>((uint64_t)H + 1, 2048);
-        c.terms = pick(h.terms, 4 * c.rows);
-        c.sites_raw = pick(h.sites_raw, 8 * (c.cfg + n_rec()) + 1024);
-        c.sites = pick(h.sites, 4 * c.cfg + 1024);
-        c.rsites = pick(h.rsites, 4 * n_rec() + 1024);
+        for (int i = 0; i < Cap::N; ++i) c[i] = h[i] ? up(h[i]) : 0;
+        auto cold = [&c](int i, uint64_t guess) { if (!c[i]) c[i] = guess; };
+        cold(Cap::seq, std::min<uint64_t>(RH + R, std::max<uint64_t>(R, ctx->scratch_bytes / 8 / 128)));
+        c[Cap::seq] = std::max<uint64_t>(std::min<uint64_t>(c[Cap::seq], RH + R), R);
+        cold(Cap::d, std::min<uint64_t>(2 * c[Cap::seq], ctx->scratch_bytes / 4 / 72));
+        cold(Cap::cfg, 4 * n_var + R);
+        cold(Cap::vd, 2 * c[Cap::cfg] + n_rec());  // a record alone has a one-entry diff list
+        c[Cap::items] = ref_items + c[Cap::vd];  // the reference haplotypes in pieces, a configuration has at most one item per carried record
+        c[Cap::units] = std::max<uint64_t>(c[Cap::units], ref_units + 8 * c[Cap::cfg]);
+        cold(Cap::dwords, c[Cap::cfg] * (n_keys / std::max<uint32_t>(1, R) + 1));
+        cold(Cap::rows, std::max<uint64_t>(4096, n_keys / 4));
+        c[Cap::rows] = std::min<uint64_t>(std::max<uint64_t>(1, n_keys), c[Cap::rows]);
+        cold(Cap::rowwords, c[Cap::rows] * ((uint64_t)(H + 1) / 32 + 1));
+        cold(Cap::capr, 512);
+        if (ctx->refhit_cap_opt) c[Cap::capr] = (uint64_t)std::max<int64_t>(1, ctx->refhit_cap_opt / std::max<uint32_t>(1, R));
+        c[Cap::groups] = h[Cap::groups] ? groups_for(h[Cap::groups]) : std::min<uint64_t>((uint64_t)H + 1, 2048);
+        cold(Cap::terms, 4 * c[Cap::rows]);
+        cold(Cap::sites_raw, 8 * (c[Cap::cfg] + n_rec()) + 1024);
+        cold(Cap::sites, 4 * c[Cap::cfg] + 1024);
+        cold(Cap::rsites, 4 * n_rec() + 1024);
     }
-    uint64_t scratch_bytes_needed() const {
-        const Caps& c = slot->caps;
-        uint64_t tbl = 1024, seg = 64;
-        while (tbl < 2 * c.d) tbl <<= 1;
-        while (seg < 2 * ((uint64_t)H + 1)) seg <<= 1;
-        tbl = std::max<uint64_t>(tbl, (uint64_t)R * seg);
-        return RH * 20 + tbl * 12 + c.seq * 50 + c.d * (4 + 32 + 20 + 4) + c.seq * 32 + c.cfg * 32 + (R + c.cfg + n_rec()) * 60 + c.vd * 36 + c.items * 28 +
-               c.units * 12 + c.dwords * 4 + n_keys * 36 + (uint64_t)c.capr * R * sizeof(RefHit) + c.rows * 34 + c.rowwords * 4 + fan_vec_bytes() + attribution_bytes() + sites_bytes();
-    }
-    // option "attribution": scratch per diff-list entry, configuration, distinct haplotype and row, the per-slot results, the terms
-    uint64_t attribution_bytes() const {
-        const Caps& c = slot->caps;
-        return ctx->attribution ? c.d * 20 + c.cfg * 21 + c.seq * 12 + c.rows * 16 + c.terms * 8 : 0;
-    }
-    // options "sites" / "record_sites": score and pattern of every reference hit, the raw sites twice (+ flag and index), per output id
-    // its count and offsets, per configuration its output id, the per-slot results (per record its flags and offsets)
-    uint64_t sites_bytes() const {
-        const Caps& c = slot->caps;
-        if (!slot->keep_sites) return 0;
-        const uint64_t ids = c.cfg + n_rec();
-        return (uint64_t)c.capr * R * 8 + c.sites_raw * (2 * sizeof(RawSite) + 12) + ids * 12 + (slot->sites ? c.cfg * 12 + c.sites * 17 : 0) +
-               (slot->record_sites ? n_rec() * 9 + c.rsites * 17 : 0);
+    // the block's device scratch: the exact sum of what reserve() grows
+    uint64_t scratch_bytes_needed() {
+        uint64_t total = 0;
+        buffers([&](DevBuf&, uint64_t bytes) { total += bytes; });
+        return total;
     }
 
     // ---- fan-out: the count vectors in shared memory (k_fanout<false>, one CTA per unit) or in device memory (k_fanout<true>) ----
     // Device memory when a region may have more groups than shared memory holds, or when option fan_vector asks for it (testing).
-    bool fan_vec() const { return ctx->fan_vector == 1 || slot->caps.groups > smem_groups; }
+    bool fan_vec() const { return ctx->fan_vector == 1 || slot->caps[Cap::groups] > smem_groups; }
     // CTAs per region: FAN_SPLIT when there are many regions, more when few regions would leave SMs idle (sample blocks of a biobank
     // cohort: few regions, tens of thousands of groups each)
     uint32_t fan_split() const {
@@ -156,7 +146,7 @@ struct ConfigPipeline {
     uint32_t fan_vec_grid() const {
         return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)ctx->prop.multiProcessorCount * FAN_VEC_CTAS_PER_SM, (uint64_t)R * fan_split()));
     }
-    uint64_t fan_vec_stride() const { return ((uint64_t)slot->caps.groups + 31) & ~31ull; }  // words of a CTA's slice, 128-byte aligned
+    uint64_t fan_vec_stride() const { return (slot->caps[Cap::groups] + 31) & ~31ull; }  // words of a CTA's slice, 128-byte aligned
     uint64_t fan_vec_bytes() const { return (n_keys && fan_vec()) ? (uint64_t)fan_vec_grid() * fan_vec_stride() * 4 : 0; }
 
     // ---- K0 ----------------------------------------------------------------------------------------------------------------
@@ -178,166 +168,172 @@ struct ConfigPipeline {
     }
 
     // ---- scratch -------------------------------------------------------------------------------------------------------
-    int reserve() {
+    // the tables of K0 and of the sequence-keyed map: one segment of `seg` slots per region (L2-resident while the region is worked on)
+    uint64_t seg_slots() const {
+        uint64_t seg = 64;
+        while (seg < 2 * ((uint64_t)H + 1)) seg <<= 1;
+        return seg;
+    }
+    // Every device buffer a run uses, with its bytes under the run's capacities and options: reserve() grows them,
+    // scratch_bytes_needed() adds them up.  visit(buffer, bytes) once per buffer.
+    template <class Visit> void buffers(Visit&& visit) {
         const Caps& c = slot->caps;
-        int rc;
-#define RS(buf, bytes) if ((rc = grow(ctx, buf, std::max<uint64_t>(1, (uint64_t)(bytes))))) return rc
-        if ((rc = reserve_encoding(ctx, L, B))) return rc;
-        RS(slot->d_status, sizeof(DevStatus));
-        RS(slot->d_plan, sizeof(DevPlan));
-        RS(slot->d_hap_group, RH * 4);
-        RS(slot->d_gbase, (uint64_t)(R + 1) * 8);
-        RS(L.d_sig, RH * 8);
-        RS(L.d_nd_in, RH * 4);
-        RS(L.d_leader, RH * 4);
-        RS(L.d_ngroups, (uint64_t)R * 4);
-        RS(L.d_sum_nd, (uint64_t)R * 4);
-        RS(L.d_ref_used, (uint64_t)R * 4);
-        RS(L.d_kbase, (uint64_t)(R + 1) * 8);
-        {
-            uint64_t mask_words = 0;  // H * sum over the regions of ceil(V / 32)
-            for (uint32_t r = 0; r < R; ++r) mask_words += (uint64_t)H * ((B.h_var_off[r + 1] - B.h_var_off[r] + 31) / 32);
-            RS(L.d_hap_mask, mask_words * 4);
-            RS(L.d_mask_base, (uint64_t)(R + 1) * 8);
-            RS(L.d_region_dups, (uint64_t)R * 4);
-            RS(L.d_var_row, B.n_var * 4);
-        }
-        RS(L.d_seq_region, c.seq * 4);
-        RS(L.d_seq_leader, c.seq * 4);
-        RS(L.d_seq_nd, c.seq * 4);
-        RS(L.d_seq_doff, (c.seq + 1) * 8);
-        RS(L.d_seq_nseg, c.seq * 4);
-        RS(L.d_seq_len, c.seq * 4);
-        RS(L.d_seq_hash, c.seq * 8);
-        RS(L.d_seq_flags, c.seq);
-        RS(L.d_seq_ntake, c.seq * 4);
-        RS(L.d_dlist, c.d * 4);
-        RS(L.d_segs, (2 * c.d + 2 * c.seq) * sizeof(Seg));
-        RS(L.d_var_cluster, B.n_var * 4);
-        RS(L.d_var_sorted, B.n_var * 4);
-        RS(L.d_ncfg, (uint64_t)R * 4);
-        RS(L.d_dwords, (uint64_t)R * 4);
-        RS(L.d_cfgbase, (uint64_t)(R + 1) * 8);
-        RS(L.d_dbase, (uint64_t)(R + 1) * 8);
-        RS(L.d_run_len, c.d * 4);
-        RS(L.d_run_key, c.d * 8);
-        RS(L.d_run_rep, c.d * 4);
-        RS(L.d_run_cfg, c.d * 4);
-        RS(L.d_cfg_src, c.cfg * 4);
-        RS(L.d_cfg_net, c.cfg * 4);
-        RS(L.d_mcount, c.cfg * 4);
-        RS(L.d_moff, (c.cfg + 1) * 8);
-        RS(L.d_mfill, c.cfg * 4);
-        RS(L.d_members, c.d * 4);
-        const uint64_t nv = R + c.cfg + n_rec();
-        RS(L.d_vq_region, nv * 4);
-        RS(L.d_vq_leader, nv * 4);
-        RS(L.d_vq_nd, nv * 4);
-        RS(L.d_vq_doff, (nv + 1) * 8);
-        RS(L.d_vq_nseg, nv * 4);
-        RS(L.d_vq_len, nv * 4);
-        RS(L.d_vq_flags, nv);
-        RS(L.d_vq_ntake, nv * 4);
-        RS(L.d_vq_nitems, nv * 4);
-        RS(L.d_vq_item_off, (nv + 1) * 8);
-        RS(L.d_vq_dlist, c.vd * 4);
-        RS(L.d_vq_segs, (2 * c.vd + 2 * nv) * sizeof(Seg));
-        RS(L.d_items, c.items * sizeof(ScanItem));
-        RS(L.d_list, c.items * 4);
-        RS(L.d_ent_units, c.items * 4);
-        RS(L.d_ent_uoff, (c.items + 1) * 8);
-        RS(L.d_pk, c.units * 8);
-        RS(L.d_nm, c.units * 4);
-        RS(L.d_D, c.dwords * 4);
-        RS(L.d_C0, n_keys * 4);
-        RS(L.d_refhits, (uint64_t)c.capr * R * sizeof(RefHit));
-        RS(L.d_refcnt, (uint64_t)R * 4);
-        RS(L.d_vmin, n_keys * 4);
-        RS(L.d_vmax, n_keys * 4);
-        RS(L.d_flag, n_keys * 4);
-        RS(L.d_rowwords, n_keys * 4);
-        RS(L.d_kbits, n_keys);
-        RS(L.d_rowidx, (n_keys + 1) * 8);
-        RS(L.d_rowoff, (n_keys + 1) * 8);
-        RS(slot->d_o_region, c.rows * 4);
-        RS(slot->d_o_inner, c.rows * 4);
-        RS(slot->d_o_pid, c.rows * 2);
-        RS(slot->d_o_vmin, c.rows * 4);
-        RS(slot->d_o_vmax, c.rows * 4);
-        RS(slot->d_o_base, c.rows * 4);
-        RS(slot->d_o_bits, c.rows);
-        RS(slot->d_o_off, c.rows * 8);
-        RS(slot->d_o_packed, c.rowwords * 4);
-        if (fan_vec_bytes()) RS(L.d_fan_vec, fan_vec_bytes());
+        auto f = [&](DevBuf& buf, uint64_t bytes) { visit(buf, std::max<uint64_t>(1, bytes)); };
+        encoding_buffers(L, B, f);
+        f(slot->d_status, sizeof(DevStatus));
+        f(slot->d_plan, sizeof(DevPlan));
+        f(slot->d_hap_group, RH * 4);
+        f(slot->d_gbase, (uint64_t)(R + 1) * 8);
+        f(L.d_sig, RH * 8);
+        f(L.d_nd_in, RH * 4);
+        f(L.d_leader, RH * 4);
+        f(L.d_ngroups, (uint64_t)R * 4);
+        f(L.d_sum_nd, (uint64_t)R * 4);
+        f(L.d_ref_used, (uint64_t)R * 4);
+        f(L.d_kbase, (uint64_t)(R + 1) * 8);
+        uint64_t mask_words = 0;  // H * sum over the regions of ceil(V / 32)
+        for (uint32_t r = 0; r < R; ++r) mask_words += (uint64_t)H * ((B.h_var_off[r + 1] - B.h_var_off[r] + 31) / 32);
+        f(L.d_hap_mask, mask_words * 4);
+        f(L.d_mask_base, (uint64_t)(R + 1) * 8);
+        f(L.d_region_dups, (uint64_t)R * 4);
+        f(L.d_var_row, B.n_var * 4);
+        f(L.d_seq_region, c[Cap::seq] * 4);
+        f(L.d_seq_leader, c[Cap::seq] * 4);
+        f(L.d_seq_nd, c[Cap::seq] * 4);
+        f(L.d_seq_doff, (c[Cap::seq] + 1) * 8);
+        f(L.d_seq_nseg, c[Cap::seq] * 4);
+        f(L.d_seq_len, c[Cap::seq] * 4);
+        f(L.d_seq_hash, c[Cap::seq] * 8);
+        f(L.d_seq_flags, c[Cap::seq]);
+        f(L.d_seq_ntake, c[Cap::seq] * 4);
+        f(L.d_dlist, c[Cap::d] * 4);
+        f(L.d_segs, (2 * c[Cap::d] + 2 * c[Cap::seq]) * sizeof(Seg));
+        f(L.d_var_cluster, B.n_var * 4);
+        f(L.d_var_sorted, B.n_var * 4);
+        f(L.d_ncfg, (uint64_t)R * 4);
+        f(L.d_dwords, (uint64_t)R * 4);
+        f(L.d_cfgbase, (uint64_t)(R + 1) * 8);
+        f(L.d_dbase, (uint64_t)(R + 1) * 8);
+        f(L.d_run_len, c[Cap::d] * 4);
+        f(L.d_run_key, c[Cap::d] * 8);
+        f(L.d_run_rep, c[Cap::d] * 4);
+        f(L.d_run_cfg, c[Cap::d] * 4);
+        f(L.d_cfg_src, c[Cap::cfg] * 4);
+        f(L.d_cfg_net, c[Cap::cfg] * 4);
+        f(L.d_mcount, c[Cap::cfg] * 4);
+        f(L.d_moff, (c[Cap::cfg] + 1) * 8);
+        f(L.d_mfill, c[Cap::cfg] * 4);
+        f(L.d_members, c[Cap::d] * 4);
+        const uint64_t nv = R + c[Cap::cfg] + n_rec();
+        f(L.d_vq_region, nv * 4);
+        f(L.d_vq_leader, nv * 4);
+        f(L.d_vq_nd, nv * 4);
+        f(L.d_vq_doff, (nv + 1) * 8);
+        f(L.d_vq_nseg, nv * 4);
+        f(L.d_vq_len, nv * 4);
+        f(L.d_vq_flags, nv);
+        f(L.d_vq_ntake, nv * 4);
+        f(L.d_vq_nitems, nv * 4);
+        f(L.d_vq_item_off, (nv + 1) * 8);
+        f(L.d_vq_dlist, c[Cap::vd] * 4);
+        f(L.d_vq_segs, (2 * c[Cap::vd] + 2 * nv) * sizeof(Seg));
+        f(L.d_items, c[Cap::items] * sizeof(ScanItem));
+        f(L.d_list, c[Cap::items] * 4);
+        f(L.d_ent_units, c[Cap::items] * 4);
+        f(L.d_ent_uoff, (c[Cap::items] + 1) * 8);
+        f(L.d_pk, c[Cap::units] * 8);
+        f(L.d_nm, c[Cap::units] * 4);
+        f(L.d_D, c[Cap::dwords] * 4);
+        f(L.d_C0, n_keys * 4);
+        f(L.d_refhits, (uint64_t)c[Cap::capr] * R * sizeof(RefHit));
+        f(L.d_refcnt, (uint64_t)R * 4);
+        f(L.d_vmin, n_keys * 4);
+        f(L.d_vmax, n_keys * 4);
+        f(L.d_flag, n_keys * 4);
+        f(L.d_rowwords, n_keys * 4);
+        f(L.d_kbits, n_keys);
+        f(L.d_rowidx, (n_keys + 1) * 8);
+        f(L.d_rowoff, (n_keys + 1) * 8);
+        f(slot->d_o_region, c[Cap::rows] * 4);
+        f(slot->d_o_inner, c[Cap::rows] * 4);
+        f(slot->d_o_pid, c[Cap::rows] * 2);
+        f(slot->d_o_vmin, c[Cap::rows] * 4);
+        f(slot->d_o_vmax, c[Cap::rows] * 4);
+        f(slot->d_o_base, c[Cap::rows] * 4);
+        f(slot->d_o_bits, c[Cap::rows]);
+        f(slot->d_o_off, c[Cap::rows] * 8);
+        f(slot->d_o_packed, c[Cap::rowwords] * 4);
+        if (fan_vec_bytes()) f(L.d_fan_vec, fan_vec_bytes());
         if (ctx->attribution) {
-            RS(L.d_att_eflag, c.d * 4);
-            RS(L.d_att_cfgid, (c.d + 1) * 8);
-            RS(L.d_att_nrec, c.cfg * 4);
-            RS(L.d_att_col, c.cfg * 4);
-            RS(L.d_att_gn, c.seq * 4);
-            RS(L.d_att_tcnt, c.rows * 4);
-            RS(slot->d_a_ref, c.rows * 4);
-            RS(slot->d_a_toff, (c.rows + 1) * 8);
-            RS(slot->d_a_tcfg, c.terms * 4);
-            RS(slot->d_a_tdiff, c.terms * 4);
-            RS(slot->d_a_creg, c.cfg * 4);
-            RS(slot->d_a_cflags, c.cfg);
-            RS(slot->d_a_croff, (c.cfg + 1) * 8);
-            RS(slot->d_a_crec, c.d * 4);
-            RS(slot->d_a_goff, (c.seq + 1) * 8);
-            RS(slot->d_a_gcfg, c.d * 4);
+            f(L.d_att_eflag, c[Cap::d] * 4);
+            f(L.d_att_cfgid, (c[Cap::d] + 1) * 8);
+            f(L.d_att_nrec, c[Cap::cfg] * 4);
+            f(L.d_att_col, c[Cap::cfg] * 4);
+            f(L.d_att_gn, c[Cap::seq] * 4);
+            f(L.d_att_tcnt, c[Cap::rows] * 4);
+            f(slot->d_a_ref, c[Cap::rows] * 4);
+            f(slot->d_a_toff, (c[Cap::rows] + 1) * 8);
+            f(slot->d_a_tcfg, c[Cap::terms] * 4);
+            f(slot->d_a_tdiff, c[Cap::terms] * 4);
+            f(slot->d_a_creg, c[Cap::cfg] * 4);
+            f(slot->d_a_cflags, c[Cap::cfg]);
+            f(slot->d_a_croff, (c[Cap::cfg] + 1) * 8);
+            f(slot->d_a_crec, c[Cap::d] * 4);
+            f(slot->d_a_goff, (c[Cap::seq] + 1) * 8);
+            f(slot->d_a_gcfg, c[Cap::d] * 4);
         }
         if (slot->keep_sites) {
-            RS(L.d_site_refpat, (uint64_t)c.capr * R * 4);
-            RS(L.d_site_refscore, (uint64_t)c.capr * R * 4);
-            RS(L.d_site_raw, c.sites_raw * sizeof(RawSite));
-            RS(L.d_site_bucket, c.sites_raw * sizeof(RawSite));
-            RS(L.d_site_keep, c.sites_raw * 4);
-            RS(L.d_site_kpos, (c.sites_raw + 1) * 8);
-            RS(L.d_site_cnt, (c.cfg + n_rec()) * 4);
-            RS(L.d_site_boff, (c.cfg + n_rec() + 1) * 8);
+            f(L.d_site_refpat, (uint64_t)c[Cap::capr] * R * 4);
+            f(L.d_site_refscore, (uint64_t)c[Cap::capr] * R * 4);
+            f(L.d_site_raw, c[Cap::sites_raw] * sizeof(RawSite));
+            f(L.d_site_bucket, c[Cap::sites_raw] * sizeof(RawSite));
+            f(L.d_site_keep, c[Cap::sites_raw] * 4);
+            f(L.d_site_kpos, (c[Cap::sites_raw] + 1) * 8);
+            f(L.d_site_cnt, (c[Cap::cfg] + n_rec()) * 4);
+            f(L.d_site_boff, (c[Cap::cfg] + n_rec() + 1) * 8);
         }
         if (slot->record_sites) {
-            RS(slot->d_r_flags, n_rec());
-            RS(slot->d_r_off, (n_rec() + 1) * 8);
-            RS(slot->d_r_pat, c.rsites * 4);
-            RS(slot->d_r_start, c.rsites * 8);
-            RS(slot->d_r_score, c.rsites * 4);
-            RS(slot->d_r_change, c.rsites);
+            f(slot->d_r_flags, n_rec());
+            f(slot->d_r_off, (n_rec() + 1) * 8);
+            f(slot->d_r_pat, c[Cap::rsites] * 4);
+            f(slot->d_r_start, c[Cap::rsites] * 8);
+            f(slot->d_r_score, c[Cap::rsites] * 4);
+            f(slot->d_r_change, c[Cap::rsites]);
         }
         if (slot->sites) {
-            RS(L.d_site_oid, c.cfg * 4);
-            RS(slot->d_s_off, (c.cfg + 1) * 8);
-            RS(slot->d_s_pat, c.sites * 4);
-            RS(slot->d_s_start, c.sites * 8);
-            RS(slot->d_s_score, c.sites * 4);
-            RS(slot->d_s_change, c.sites);
+            f(L.d_site_oid, c[Cap::cfg] * 4);
+            f(slot->d_s_off, (c[Cap::cfg] + 1) * 8);
+            f(slot->d_s_pat, c[Cap::sites] * 4);
+            f(slot->d_s_start, c[Cap::sites] * 8);
+            f(slot->d_s_score, c[Cap::sites] * 4);
+            f(slot->d_s_change, c[Cap::sites]);
         }
-#undef RS
+        // the open-addressing table at the largest of its uses: the K0 super-batches (nr * seg slots each), the sequence-keyed map
+        // (R * seg) and the configuration runs (table_slots_for(d))
+        const uint64_t slots = std::max<uint64_t>(table_slots_for(c[Cap::d]), (uint64_t)R * seg_slots());
+        f(L.d_keys, slots * 8);
+        f(L.d_vals, slots * 4);
+    }
+    int reserve() {
+        int rc = TFBS_OK;
+        buffers([&](DevBuf& buf, uint64_t bytes) { if (!rc) rc = grow(ctx, buf, bytes); });
+        if (rc) return rc;
         CK(slot->h_status.reserve(sizeof(DevStatus), false));
         CK(slot->h_plan.reserve(sizeof(DevPlan), false));
         return TFBS_OK;
     }
 
-    int table_slots(uint64_t slots) {  // the shared open-addressing table with room for `slots` slots, emptied
-        int rc;
-        if ((rc = grow(ctx, L.d_keys, slots * 8))) return rc;
-        if ((rc = grow(ctx, L.d_vals, slots * 4))) return rc;
+    int table_slots(uint64_t slots) {  // the open-addressing table (reserve()), its first `slots` slots emptied
+        if (!L.d_keys.fits(slots * 8) || !L.d_vals.fits(slots * 4)) return fail(ctx, TFBS_ERR_INTERNAL, "the open-addressing table was reserved too small");
         CK(cudaMemsetAsync(L.d_keys.p, 0, slots * 8, st));
         CK(cudaMemsetAsync(L.d_vals.p, 0xff, slots * 4, st));
         return TFBS_OK;
     }
     int table(uint64_t entries, uint32_t* mask) {  // the same as one table of a power-of-two number of slots >= 2 * entries
-        uint64_t cap = 1024;
-        while (cap < 2 * entries) cap <<= 1;
+        const uint64_t cap = table_slots_for(entries);
         if (cap > (1ull << 31)) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "block too large for the grouping table: submit fewer regions at a time");
-        int rc;
-        if ((rc = grow(ctx, L.d_keys, cap * 8))) return rc;
-        if ((rc = grow(ctx, L.d_vals, cap * 4))) return rc;
-        CK(cudaMemsetAsync(L.d_keys.p, 0, cap * 8, st));
-        CK(cudaMemsetAsync(L.d_vals.p, 0xff, cap * 4, st));
         *mask = (uint32_t)(cap - 1);
-        return TFBS_OK;
+        return table_slots(cap);
     }
 
     // ---- the whole pipeline, enqueued ------------------------------------------------------------------------------------
@@ -368,18 +364,18 @@ struct ConfigPipeline {
         choose_caps(first_attempt);
         const Caps& c = slot->caps;
         const bool fans = n_keys && R && S;
-        slot->fan_groups_cap = fans ? c.groups : 0;
+        slot->fan_groups_cap = fans ? c[Cap::groups] : 0;
         slot->fan_ctas = fans ? (fan_vec() ? fan_vec_grid() : (uint32_t)std::min<uint64_t>(0xffffffffu, (uint64_t)R * fan_split())) : 0;
         slot->fan_in_device_memory = (fans && fan_vec()) ? 1 : 0;
         if (fan_vec_bytes() > ctx->scratch_bytes)
-            return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "the fan-out's count vectors for " + std::to_string(c.groups) + " distinct haplotypes per region need about " +
+            return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "the fan-out's count vectors for " + std::to_string(c[Cap::groups]) + " distinct haplotypes per region need about " +
                                                             std::to_string(fan_vec_bytes() >> 20) + " MB of device scratch, option scratch_mb allows " +
                                                             std::to_string(ctx->scratch_bytes >> 20));
         if (scratch_bytes_needed() > ctx->scratch_bytes)
             return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "the block needs about " + std::to_string(scratch_bytes_needed() >> 20) +
                                                             " MB of device scratch, option scratch_mb allows " + std::to_string(ctx->scratch_bytes >> 20) +
                                                             ": submit fewer regions per block");
-        if (c.seq > 0x7fffffffull || c.d > 0xfffffff0ull || R + c.cfg + n_rec() > 0x7fffffffull || c.items > 0xfffffff0ull ||
+        if (c[Cap::seq] > 0x7fffffffull || c[Cap::d] > 0xfffffff0ull || R + c[Cap::cfg] + n_rec() > 0x7fffffffull || c[Cap::items] > 0xfffffff0ull ||
             (fan_vec() && (uint64_t)R * fan_split() > 0xffffffffull))
             return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "block too large for 32-bit work-list indices: submit fewer regions per block");
         if (R && !S && slot->record_sites) return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "option record_sites needs a block with at least one sample");
@@ -419,9 +415,7 @@ struct ConfigPipeline {
 
         // ---- K0: grouping by Vec<Diff> (haplotype.rs:65-75) ----
         u32* hap_group = slot->d_hap_group.as<u32>();
-        // the tables of K0 and of the sequence-keyed map: one segment of `seg` slots per region (L2-resident while the region is worked on)
-        uint32_t seg = 64;
-        while (seg < 2 * ((uint64_t)H + 1)) seg <<= 1;
+        const uint32_t seg = (uint32_t)seg_slots();
         const uint32_t group_slots = region_group_slots();
         // option test_sig_bits (testing): the first attempt's signatures keep that many bits, so that the exact check meets collisions
         const u64 sig_mask = (ctx->test_sig_bits && slot->attempts == 0) ? (1ull << ctx->test_sig_bits) - 1 : ~0ull;
@@ -451,13 +445,13 @@ struct ConfigPipeline {
         }
         u64* gbase = slot->d_gbase.as<u64>();
         if ((rc = scan(L.d_ngroups.as<u32>(), R, nullptr, gbase))) return rc;
-        gate(gbase + R, 0, c.seq, &plan->n_seq, &plan->need_seq);
+        gate(Cap::seq, gbase + R, 0);
         CK(cudaEventRecord(slot->ev_t[1], st));
 
         // ---- K1: patch_haplotype per distinct haplotype (segments + hash), the sequence-keyed map (haplotype.rs:81-85) ----
         DevSeqs sq{};
-        sq.n_seq = (u32)c.seq;
-        sq.n_seq_ptr = &plan->n_seq;
+        sq.n_seq = (u32)c[Cap::seq];
+        sq.n_seq_ptr = &plan->n[Cap::seq];
         sq.abort = &plan->abort;
         sq.gbase = gbase;
         sq.gbase0 = 0;
@@ -475,17 +469,16 @@ struct ConfigPipeline {
         if (group_slots) TFBS_LAUNCH(k_seq_init_groups, R, 128, 0, st)(H, L.d_ngroups.as<u32>(), L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), sq);
         else TFBS_LAUNCH(k_seq_init, R, 128, 0, st)(H, 0, hap_group, L.d_leader.as<u32>(), L.d_nd_in.as<u32>(), sq);
         ++launches();
-        if ((rc = scan(sq.seq_nd, c.seq, &plan->n_seq, sq.seq_doff))) return rc;
+        if ((rc = scan(sq.seq_nd, c[Cap::seq], &plan->n[Cap::seq], sq.seq_doff))) return rc;
         // the total sits behind the last sequence; k_gate reads it through the clamped count
-        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(sq.seq_doff, &plan->n_seq, (u64)c.d, &plan->n_d, &plan->need_d, &plan->abort);
-        ++launches();
-        TFBS_LAUNCH(k_walk, grid_for(c.seq, 128), 128, 0, st)(db, sq, (u64)c.d, dst, 0u);
+        gate_at(Cap::d, sq.seq_doff, &plan->n[Cap::seq]);
+        TFBS_LAUNCH(k_walk, grid_for(c[Cap::seq], 128), 128, 0, st)(db, sq, (u64)c[Cap::d], dst, 0u);
         ++launches();
         {
             if ((rc = table_slots((uint64_t)R * seg))) return rc;  // at most H + 1 distinct haplotypes per region
             CK(cudaMemsetAsync(L.d_ref_used.p, 0, (size_t)R * 4, st));
-            TFBS_LAUNCH(k_seq_insert, grid_for(c.seq, 256), 256, 0, st)(sq, L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg, 0u);
-            TFBS_LAUNCH(k_seq_resolve, grid_for(c.seq, 128), 128, 0, st)(db, sq, L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg, 0u, dst, 0u);
+            TFBS_LAUNCH(k_seq_insert, grid_for(c[Cap::seq], 256), 256, 0, st)(sq, L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg, 0u);
+            TFBS_LAUNCH(k_seq_resolve, grid_for(c[Cap::seq], 128), 128, 0, st)(db, sq, L.d_keys.as<u64>(), L.d_vals.as<u32>(), 0u, seg, 0u, dst, 0u);
             TFBS_LAUNCH(k_redirect, grid_for(RH, 256), 256, 0, st)(H, 0, R, sq, hap_group, L.d_ref_used.as<u32>(), (u8*)nullptr, (u64*)&dst->nominal_cells,
                                                                    ctx->dpat.max_len, ctx->dpat.sum_len, (u64)ctx->dpat.sum_len_sq, ctx->dpat.n_patterns, ctx->dpat.pat_len);
             launches() += 3;
@@ -518,7 +511,7 @@ struct ConfigPipeline {
         cf.plan = plan;
         if (slot->keep_sites) {
             cf.site_raw = L.d_site_raw.as<RawSite>();
-            cf.site_cap = c.sites_raw;
+            cf.site_cap = c[Cap::sites_raw];
             cf.ref_pat = L.d_site_refpat.as<u32>();
             cf.ref_score = L.d_site_refscore.as<int>();
             cf.cfg_sites = slot->sites ? 1u : 0u;
@@ -528,22 +521,23 @@ struct ConfigPipeline {
         ++launches();
         {
             uint32_t mask;
-            if ((rc = table(c.d, &mask))) return rc;
+            if ((rc = table(c[Cap::d], &mask))) return rc;
             CK(cudaMemsetAsync(cf.ncfg, 0, (size_t)R * 4, st));
-            TFBS_LAUNCH(k_cfg_runs, grid_for(c.seq, 128), 128, 0, st)(db, sq, cf, (u64)c.d, slot->seed, L.d_keys.as<u64>(), L.d_vals.as<u32>(), mask);
-            TFBS_LAUNCH(k_cfg_resolve, grid_for(c.seq, 128), 128, 0, st)(sq, cf, (u64)c.d, L.d_keys.as<u64>(), L.d_vals.as<u32>(), mask);
+            TFBS_LAUNCH(k_cfg_runs, grid_for(c[Cap::seq], 128), 128, 0, st)(db, sq, cf, (u64)c[Cap::d], slot->seed, L.d_keys.as<u64>(), L.d_vals.as<u32>(), mask);
+            TFBS_LAUNCH(k_cfg_resolve, grid_for(c[Cap::seq], 128), 128, 0, st)(sq, cf, (u64)c[Cap::d], L.d_keys.as<u64>(), L.d_vals.as<u32>(), mask);
             launches() += 2;
         }
         TFBS_LAUNCH(k_region_sizes, grid_for(R, 256), 256, 0, st)(db, cf);
         ++launches();
         if ((rc = scan(cf.ncfg, R, nullptr, cf.cfgbase))) return rc;
         if ((rc = scan(cf.dwords, R, nullptr, cf.dbase))) return rc;
-        gate(cf.cfgbase + R, 0, c.cfg, &plan->n_cfg, &plan->need_cfg);
-        gate(cf.cfgbase + R, R + n_rec(), R + c.cfg + n_rec(), &plan->n_vseq, &plan->unused);
-        gate(cf.dbase + R, 0, c.dwords, &plan->n_dwords, &plan->need_dwords);
+        gate(Cap::cfg, cf.cfgbase + R, 0);
+        TFBS_LAUNCH(k_gate, 1, 1, 0, st)(cf.cfgbase + R, (u64)(R + n_rec()), (u64)(R + c[Cap::cfg] + n_rec()), &plan->n_vseq, &plan->unused, &plan->abort);
+        ++launches();
+        gate(Cap::dwords, cf.dbase + R, 0);
 
         // virtual sequences: the reference haplotype of every region, then the configurations, then (option "record_sites") the records
-        const uint64_t NV = R + c.cfg + n_rec();
+        const uint64_t NV = R + c[Cap::cfg] + n_rec();
         DevSeqs vq{};
         vq.n_seq = (u32)NV;
         vq.n_seq_ptr = &plan->n_vseq;
@@ -562,41 +556,40 @@ struct ConfigPipeline {
         vq.seq_nitems = L.d_vq_nitems.as<u32>();
         vq.item_off = L.d_vq_item_off.as<u64>();
         vq.items = L.d_items.as<ScanItem>();
-        vq.n_items_cap = (u32)c.items;
+        vq.n_items_cap = (u32)c[Cap::items];
         vq.ent_units = L.d_ent_units.as<u32>();
         vq.ent_uoff = L.d_ent_uoff.as<u64>();
         vq.pk = L.d_pk.as<u64>();
         vq.nm = L.d_nm.as<u32>();
-        vq.units_cap = c.units;
+        vq.units_cap = c[Cap::units];
         TFBS_LAUNCH(k_vseq_init, grid_for(std::max<uint64_t>(R, n_rec()), 256), 256, 0, st)(db, cf, vq, (u32)n_rec());
-        TFBS_LAUNCH(k_cfg_fill, grid_for(c.seq, 128), 128, 0, st)(sq, cf, vq, (u64)c.d);
+        TFBS_LAUNCH(k_cfg_fill, grid_for(c[Cap::seq], 128), 128, 0, st)(sq, cf, vq, (u64)c[Cap::d]);
         launches() += 2;
         if ((rc = scan(vq.seq_nd, NV, &plan->n_vseq, vq.seq_doff))) return rc;
-        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(vq.seq_doff, &plan->n_vseq, (u64)c.vd, &plan->n_vd, &plan->need_vd, &plan->abort);
-        ++launches();
-        TFBS_LAUNCH(k_cfg_walk, grid_for(NV, 128), 128, 0, st)(db, sq, cf, vq, (u64)c.vd);
+        gate_at(Cap::vd, vq.seq_doff, &plan->n_vseq);
+        TFBS_LAUNCH(k_cfg_walk, grid_for(NV, 128), 128, 0, st)(db, sq, cf, vq, (u64)c[Cap::vd]);
         ++launches();
 
         // ---- work list, packed bases ----
         TFBS_LAUNCH(k_vitems<false>, grid_for(NV, 128), 128, 0, st)(vq, cp.max_len, &plan->abort);
         ++launches();
         if ((rc = scan(vq.seq_nitems, NV, &plan->n_vseq, vq.item_off))) return rc;
-        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(vq.item_off, &plan->n_vseq, (u64)c.items, &plan->n_items, &plan->need_items, &plan->abort);
+        gate_at(Cap::items, vq.item_off, &plan->n_vseq);
         TFBS_LAUNCH(k_vitems<true>, grid_for(NV, 128), 128, 0, st)(vq, cp.max_len, &plan->abort);
-        TFBS_LAUNCH(k_vitem_units, grid_for(c.items, 256), 256, 0, st)(vq, &plan->n_items, L.d_list.as<u32>());
-        launches() += 3;
-        if ((rc = scan(vq.ent_units, c.items, &plan->n_items, vq.ent_uoff))) return rc;
-        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(vq.ent_uoff, &plan->n_items, (u64)c.units, &plan->n_units, &plan->need_units, &plan->abort);
-        TFBS_LAUNCH(k_emit_list, grid_for(c.items * EMIT_LANES, 256), 256, 0, st)(db, vq, L.d_list.as<u32>(), &plan->n_items);
-        TFBS_LAUNCH(k_item_stats, grid_for(c.items, 256), 256, 0, st)(vq, ctx->dpat, L.d_list.as<u32>(), &plan->n_items, dst);
-        launches() += 3;
+        TFBS_LAUNCH(k_vitem_units, grid_for(c[Cap::items], 256), 256, 0, st)(vq, &plan->n[Cap::items], L.d_list.as<u32>());
+        launches() += 2;
+        if ((rc = scan(vq.ent_units, c[Cap::items], &plan->n[Cap::items], vq.ent_uoff))) return rc;
+        gate_at(Cap::units, vq.ent_uoff, &plan->n[Cap::items]);
+        TFBS_LAUNCH(k_emit_list, grid_for(c[Cap::items] * EMIT_LANES, 256), 256, 0, st)(db, vq, L.d_list.as<u32>(), &plan->n[Cap::items]);
+        TFBS_LAUNCH(k_item_stats, grid_for(c[Cap::items], 256), 256, 0, st)(vq, ctx->dpat, L.d_list.as<u32>(), &plan->n[Cap::items], dst);
+        launches() += 2;
 
         // ---- the scan: one launch per pattern chunk ----
-        TFBS_LAUNCH(k_zero_words, slot->stats.sm_count * 8, 256, 0, st)(cf.D, &plan->n_dwords, (u64)c.dwords);
+        TFBS_LAUNCH(k_zero_words, slot->stats.sm_count * 8, 256, 0, st)(cf.D, &plan->n[Cap::dwords], (u64)c[Cap::dwords]);
         ++launches();
         if (n_keys) CK(cudaMemsetAsync(cf.C0, 0, n_keys * 4, st));
         CK(cudaMemsetAsync(L.d_refcnt.p, 0, (size_t)R * 4, st));
-        DevRefHits drh{L.d_refhits.as<RefHit>(), L.d_refcnt.as<u32>(), c.capr, 0};
+        DevRefHits drh{L.d_refhits.as<RefHit>(), L.d_refcnt.as<u32>(), (u32)c[Cap::capr], 0};
         DevCounts dc{cf.C0, cf.kbase, 0};
         DevMatches dm{};
         const int smem_bytes = (int)(sizeof(CtaShared) + SCAN_WARPS * sizeof(WarpShared) + ((cp.max_chunk_bytes + 15) & ~15u));
@@ -610,7 +603,7 @@ struct ConfigPipeline {
         CK(cudaEventRecord(slot->ev_t[3], st));
         for (uint32_t ch = 0; ch < cp.chunks.size(); ++ch) {
             CK(cudaMemsetAsync(&dst->work_counter, 0, 4, st));
-            TFBS_LAUNCH(kern, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, L.d_list.as<u32>(), &plan->n_items, (u32)SCAN_PER_GRAB, dst, ch);
+            TFBS_LAUNCH(kern, scan_grid, SCAN_CTA, smem_bytes, st)(db, vq, ctx->dpat, dc, dm, drh, cf, 1, L.d_list.as<u32>(), &plan->n[Cap::items], (u32)SCAN_PER_GRAB, dst, ch);
             ++launches();
             ++slot->stats.scan_launches;
         }
@@ -618,15 +611,15 @@ struct ConfigPipeline {
 
         // ---- lost reference hits, members of the configurations, counters ----
         TFBS_LAUNCH(k_refhit_need, grid_for(R, 256), 256, 0, st)(drh, R, plan);
-        TFBS_LAUNCH(k_cfg_lost, grid_for((c.cfg + n_rec()) * 8, 256), 256, 0, st)(db, vq, cf, drh);
+        TFBS_LAUNCH(k_cfg_lost, grid_for((c[Cap::cfg] + n_rec()) * 8, 256), 256, 0, st)(db, vq, cf, drh);
         launches() += 2;
-        CK(cudaMemsetAsync(cf.mcount, 0, c.cfg * 4, st));
-        CK(cudaMemsetAsync(cf.mfill, 0, c.cfg * 4, st));
-        TFBS_LAUNCH(k_members<false>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, drh, L.d_ref_used.as<u32>(), (u64)c.d, ctx->dpat, dst);
+        CK(cudaMemsetAsync(cf.mcount, 0, c[Cap::cfg] * 4, st));
+        CK(cudaMemsetAsync(cf.mfill, 0, c[Cap::cfg] * 4, st));
+        TFBS_LAUNCH(k_members<false>, grid_for(c[Cap::seq], 128), 128, 0, st)(sq, cf, drh, L.d_ref_used.as<u32>(), (u64)c[Cap::d], ctx->dpat, dst);
         ++launches();
-        if ((rc = scan(cf.mcount, c.cfg, &plan->n_cfg, cf.moff))) return rc;
-        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(cf.moff, &plan->n_cfg, (u64)c.d, &plan->n_members, &plan->need_members, &plan->abort);
-        TFBS_LAUNCH(k_members<true>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, drh, L.d_ref_used.as<u32>(), (u64)c.d, ctx->dpat, dst);
+        if ((rc = scan(cf.mcount, c[Cap::cfg], &plan->n[Cap::cfg], cf.moff))) return rc;
+        TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(cf.moff, &plan->n[Cap::cfg], (u64)c[Cap::d], &plan->n_members, &plan->unused, &plan->abort);
+        TFBS_LAUNCH(k_members<true>, grid_for(c[Cap::seq], 128), 128, 0, st)(sq, cf, drh, L.d_ref_used.as<u32>(), (u64)c[Cap::d], ctx->dpat, dst);
         launches() += 2;
         CK(cudaEventRecord(slot->ev_t[5], st));
 
@@ -637,7 +630,7 @@ struct ConfigPipeline {
             fn.gbase = gbase;
             fn.n_pid = n_pid;
             fn.rows_mode = ctx->rows_mode;
-            fn.groups_cap = c.groups;
+            fn.groups_cap = c[Cap::groups];
             fn.vmin = L.d_vmin.as<u32>();
             fn.vmax = L.d_vmax.as<u32>();
             fn.flag = L.d_flag.as<u32>();
@@ -645,8 +638,8 @@ struct ConfigPipeline {
             fn.k_bits = L.d_kbits.as<u8>();
             fn.k_off = L.d_rowoff.as<u64>();
             fn.rowidx = L.d_rowidx.as<u64>();
-            fn.rows_cap = c.rows;
-            fn.words_cap = c.rowwords;
+            fn.rows_cap = c[Cap::rows];
+            fn.words_cap = c[Cap::rowwords];
             fn.o_region = slot->d_o_region.as<u32>();
             fn.o_inner = slot->d_o_inner.as<u32>();
             fn.o_pid = slot->d_o_pid.as<u16>();
@@ -659,9 +652,9 @@ struct ConfigPipeline {
             fn.pid_list = ctx->d_pid_list.as<u16>();
             fn.max_count = &dst->max_count;
             // shared memory: the pairs of a round, the staged rows, (when it fits) the haplotype -> group map and, unless the count
-            // vectors are in device memory, one count vector per CTA (c.groups <= smem_groups there)
+            // vectors are in device memory, one count vector per CTA (c[Cap::groups] <= smem_groups there)
             const bool vec = fan_vec();
-            const uint32_t smem_vec_groups = vec ? 0u : c.groups;
+            const uint32_t smem_vec_groups = vec ? 0u : c[Cap::groups];
             fn.hg16 = ((uint64_t)H + 1 <= 65536 && fan_smem_bytes(smem_vec_groups, H, true) <= 64 * 1024) ? 1u : 0u;
             const size_t fan_smem = fan_smem_bytes(smem_vec_groups, H, fn.hg16 != 0);
             const uint32_t split = fan_split();
@@ -680,9 +673,9 @@ struct ConfigPipeline {
             }
             ++launches();
             if ((rc = scan(fn.flag, n_keys, nullptr, L.d_rowidx.as<u64>()))) return rc;
-            gate(L.d_rowidx.as<u64>() + n_keys, 0, c.rows, &plan->n_rows, &plan->need_rows);
-            gate(&plan->rowwords_alloc, 0, c.rowwords, &plan->n_rowwords, &plan->need_rowwords);
-            TFBS_LAUNCH(k_row_headers, R, 128, 0, st)(db, cf, fn, &plan->n_rows);
+            gate(Cap::rows, L.d_rowidx.as<u64>() + n_keys, 0);
+            gate(Cap::rowwords, &plan->rowwords_alloc, 0);
+            TFBS_LAUNCH(k_row_headers, R, 128, 0, st)(db, cf, fn, &plan->n[Cap::rows]);
             ++launches();
             if (ctx->attribution && (rc = enqueue_attribution(sq, cf, vq, &fn))) return rc;
         } else if (ctx->attribution && (rc = enqueue_attribution(sq, cf, vq, nullptr))) {
@@ -715,28 +708,28 @@ struct ConfigPipeline {
         at.term_off = slot->d_a_toff.as<u64>();
         at.term_cfg = slot->d_a_tcfg.as<u32>();
         at.term_diff = slot->d_a_tdiff.as<int>();
-        at.cfg_cap = c.cfg;
-        at.d_cap = c.d;
-        at.terms_cap = c.terms;
+        at.cfg_cap = c[Cap::cfg];
+        at.d_cap = c[Cap::d];
+        at.terms_cap = c[Cap::terms];
         // 1. output ids: the rank of the representative entries in diff-list order
-        TFBS_LAUNCH(k_att_flags, slot->stats.sm_count * 8, 256, 0, st)(cf, at, &plan->n_d);
+        TFBS_LAUNCH(k_att_flags, slot->stats.sm_count * 8, 256, 0, st)(cf, at, &plan->n[Cap::d]);
         ++launches();
-        if ((rc = scan(at.e_flag, c.d, &plan->n_d, at.cfg_id))) return rc;
+        if ((rc = scan(at.e_flag, c[Cap::d], &plan->n[Cap::d], at.cfg_id))) return rc;
         // 2. configurations and group lists: describe + count, two scans, fill
-        TFBS_LAUNCH(k_att_configs<false>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, vq, at);
+        TFBS_LAUNCH(k_att_configs<false>, grid_for(c[Cap::seq], 128), 128, 0, st)(sq, cf, vq, at);
         ++launches();
-        if ((rc = scan(at.cfg_nrec, c.cfg, &plan->n_cfg, at.cfg_rec_off))) return rc;
-        if ((rc = scan(at.glist_n, c.seq, &plan->n_seq, at.group_off))) return rc;
-        TFBS_LAUNCH(k_att_configs<true>, grid_for(c.seq, 128), 128, 0, st)(sq, cf, vq, at);
+        if ((rc = scan(at.cfg_nrec, c[Cap::cfg], &plan->n[Cap::cfg], at.cfg_rec_off))) return rc;
+        if ((rc = scan(at.glist_n, c[Cap::seq], &plan->n[Cap::seq], at.group_off))) return rc;
+        TFBS_LAUNCH(k_att_configs<true>, grid_for(c[Cap::seq], 128), 128, 0, st)(sq, cf, vq, at);
         ++launches();
         if (fn) {
             // 3. terms: count, scan, gate, fill
-            TFBS_LAUNCH(k_att_terms<false>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
+            TFBS_LAUNCH(k_att_terms<false>, R, 256, 0, st)(db, cf, *fn, at, &plan->n[Cap::rows]);
             ++launches();
-            if ((rc = scan(at.t_cnt, c.rows, &plan->n_rows, at.term_off))) return rc;
-            TFBS_LAUNCH(k_gate_at, 1, 1, 0, st)(at.term_off, &plan->n_rows, (u64)c.terms, &plan->n_terms, &plan->need_terms, &plan->abort);
-            TFBS_LAUNCH(k_att_terms<true>, R, 256, 0, st)(db, cf, *fn, at, &plan->n_rows);
-            launches() += 2;
+            if ((rc = scan(at.t_cnt, c[Cap::rows], &plan->n[Cap::rows], at.term_off))) return rc;
+            gate_at(Cap::terms, at.term_off, &plan->n[Cap::rows]);
+            TFBS_LAUNCH(k_att_terms<true>, R, 256, 0, st)(db, cf, *fn, at, &plan->n[Cap::rows]);
+            ++launches();
         }
         return TFBS_OK;
     }
@@ -754,7 +747,7 @@ struct ConfigPipeline {
         s.kpos = L.d_site_kpos.as<u64>();
         s.cnt = L.d_site_cnt.as<u32>();
         s.boff = L.d_site_boff.as<u64>();
-        s.n_cfg = &plan->n_cfg;
+        s.n_cfg = &plan->n[Cap::cfg];
         if (slot->sites) {
             s.oid = L.d_site_oid.as<u32>();
             s.site_off = slot->d_s_off.as<u64>();
@@ -773,22 +766,22 @@ struct ConfigPipeline {
             s.vseq_region = vq.seq_region;
             s.n_ref = vq.n_ref;
         }
-        const uint64_t ids = c.cfg + n_rec();
+        const uint64_t ids = c[Cap::cfg] + n_rec();
         const unsigned grid = slot->stats.sm_count * 8;
         // 1. the raw sites against their capacity, grouped by output id
-        gate(&plan->site_alloc, 0, c.sites_raw, &plan->n_sraw, &plan->need_sraw);
+        gate(Cap::sites_raw, &plan->site_alloc, 0);
         CK(cudaMemsetAsync(s.cnt, 0, ids * 4, st));
-        TFBS_LAUNCH(k_site_count, grid, 256, 0, st)(s, &plan->n_sraw, &plan->abort);
+        TFBS_LAUNCH(k_site_count, grid, 256, 0, st)(s, &plan->n[Cap::sites_raw], &plan->abort);
         ++launches();
         if ((rc = scan(s.cnt, ids, &plan->n_sid, s.boff))) return rc;
-        TFBS_LAUNCH(k_site_scatter, grid, 256, 0, st)(s, &plan->n_sraw, &plan->abort);
+        TFBS_LAUNCH(k_site_scatter, grid, 256, 0, st)(s, &plan->n[Cap::sites_raw], &plan->abort);
         // 2. sorted per output id, survivors flagged
         TFBS_LAUNCH(k_site_rank, (unsigned)std::min<uint64_t>(std::max<uint64_t>(1, ids), grid), SITE_THREADS, 0, st)(s, &plan->n_sid, &plan->abort);
         launches() += 2;
         // 3. survivors numbered, checked against the result capacities, written
-        if ((rc = scan(s.keep, c.sites_raw, &plan->n_sraw, s.kpos))) return rc;
-        TFBS_LAUNCH(k_site_gate, 1, 1, 0, st)(s, &plan->n_sraw, (u64)c.sites, (u64)c.rsites, plan);
-        TFBS_LAUNCH(k_site_emit, grid, 256, 0, st)(db, s, &plan->n_sraw, &plan->n_sid, &plan->abort);
+        if ((rc = scan(s.keep, c[Cap::sites_raw], &plan->n[Cap::sites_raw], s.kpos))) return rc;
+        TFBS_LAUNCH(k_site_gate, 1, 1, 0, st)(s, &plan->n[Cap::sites_raw], (u64)c[Cap::sites], (u64)c[Cap::rsites], plan);
+        TFBS_LAUNCH(k_site_emit, grid, 256, 0, st)(db, s, &plan->n[Cap::sites_raw], &plan->n_sid, &plan->abort);
         launches() += 2;
         return TFBS_OK;
     }
@@ -834,13 +827,14 @@ struct ConfigPipeline {
             }
             // repeat the block: a hash collision with another seed, an overflow with the capacities the device asked for
             if (++slot->attempts > 16) return fail(ctx, TFBS_ERR_INTERNAL, "the block did not fit after 16 attempts to grow the scratch");
-            if (getenv("TFBS_DEBUG"))
-                fprintf(stderr, "tfbs: block repeated (attempt %d): collided %d, need seq %llu d %llu cfg %llu vd %llu items %llu units %llu dwords %llu rows %llu rowwords %llu capr %u groups %u | caps seq %llu d %llu cfg %llu vd %llu items %llu units %llu dwords %llu rows %llu rowwords %llu capr %u groups %u\n",
-                        slot->attempts, (int)collided, (unsigned long long)hp.need_seq, (unsigned long long)hp.need_d, (unsigned long long)hp.need_cfg, (unsigned long long)hp.need_vd,
-                        (unsigned long long)hp.need_items, (unsigned long long)hp.need_units, (unsigned long long)hp.need_dwords, (unsigned long long)hp.need_rows,
-                        (unsigned long long)hp.need_rowwords, hp.need_capr, hp.need_groups, (unsigned long long)slot->caps.seq, (unsigned long long)slot->caps.d,
-                        (unsigned long long)slot->caps.cfg, (unsigned long long)slot->caps.vd, (unsigned long long)slot->caps.items, (unsigned long long)slot->caps.units,
-                        (unsigned long long)slot->caps.dwords, (unsigned long long)slot->caps.rows, (unsigned long long)slot->caps.rowwords, slot->caps.capr, slot->caps.groups);
+            if (getenv("TFBS_DEBUG")) {
+                std::string need, caps;
+                for (int i = 0; i < Cap::N; ++i) {
+                    need += std::string(" ") + CAP_NAMES[i] + " " + std::to_string(hp.need[i]);
+                    caps += std::string(" ") + CAP_NAMES[i] + " " + std::to_string(slot->caps[i]);
+                }
+                fprintf(stderr, "tfbs: block repeated (attempt %d): collided %d, need%s | caps%s\n", slot->attempts, (int)collided, need.c_str(), caps.c_str());
+            }
             if (collided) slot->seed = slot->seed * 0x9e3779b97f4a7c15ull + 0x7f4a7c15ull;
             int rc = quiesce(ctx);
             if (rc) return rc;
@@ -853,40 +847,15 @@ struct ConfigPipeline {
     void grow_caps(const DevPlan& hp) {
         Caps& c = slot->caps;
         choose_caps(false);  // ref_items of this block
-        auto g = [](uint64_t& cap, uint64_t need) { if (need > cap) cap = up(need); };
-        g(c.seq, hp.need_seq);
-        g(c.d, hp.need_d);
-        g(c.cfg, hp.need_cfg);
-        g(c.vd, hp.need_vd);
-        c.items = std::max<uint64_t>(c.items, ref_items + c.vd);
-        g(c.items, hp.need_items);
-        g(c.units, hp.need_units);
-        g(c.dwords, hp.need_dwords);
-        g(c.rows, hp.need_rows);
-        g(c.rowwords, hp.need_rowwords);
-        g(c.terms, hp.need_terms);
-        g(c.sites_raw, hp.need_sraw);
-        g(c.sites, hp.need_sites);
-        g(c.rsites, hp.need_rsites);
-        if (hp.need_capr > c.capr) c.capr = (uint32_t)up(hp.need_capr);
-        if (hp.need_groups > c.groups) c.groups = groups_for(hp.need_groups);
+        for (int i = 0; i < Cap::N; ++i)
+            if (i != Cap::items && i != Cap::groups && hp.need[i] > c[i]) c[i] = up(hp.need[i]);
+        c[Cap::items] = std::max<uint64_t>(c[Cap::items], ref_items + c[Cap::vd]);
+        if (hp.need[Cap::items] > c[Cap::items]) c[Cap::items] = up(hp.need[Cap::items]);
+        if (hp.need[Cap::groups] > c[Cap::groups]) c[Cap::groups] = groups_for(hp.need[Cap::groups]);
     }
     void note_needs(const DevPlan& hp) {
-        Caps& h = ctx->hint;
-        h.seq = std::max<uint64_t>(h.seq, hp.need_seq);
-        h.d = std::max<uint64_t>(h.d, hp.need_d);
-        h.cfg = std::max<uint64_t>(h.cfg, hp.need_cfg);
-        h.vd = std::max<uint64_t>(h.vd, hp.need_vd);
-        h.units = std::max<uint64_t>(h.units, hp.need_units);
-        h.dwords = std::max<uint64_t>(h.dwords, hp.need_dwords);
-        h.rows = std::max<uint64_t>(h.rows, hp.need_rows);
-        h.rowwords = std::max<uint64_t>(h.rowwords, hp.need_rowwords);
-        h.terms = std::max<uint64_t>(h.terms, hp.need_terms);
-        h.sites_raw = std::max<uint64_t>(h.sites_raw, hp.need_sraw);
-        h.sites = std::max<uint64_t>(h.sites, hp.need_sites);
-        h.rsites = std::max<uint64_t>(h.rsites, hp.need_rsites);
-        h.capr = std::max<uint32_t>(h.capr, hp.need_capr);
-        h.groups = std::max<uint32_t>(h.groups, hp.need_groups);
+        for (int i = 0; i < Cap::N; ++i)
+            if (i != Cap::items) ctx->hint[i] = std::max<uint64_t>(ctx->hint[i], hp.need[i]);  // items follow vd (choose_caps)
     }
 
     int publish(const DevStatus& hs, const DevPlan& hp) {
@@ -906,9 +875,9 @@ struct ConfigPipeline {
         s.nominal_cells = hs.nominal_cells;
         s.n_hits = hs.n_hits;
         s.n_keys = n_keys;
-        s.n_rows = hp.n_rows;
+        s.n_rows = hp.n[Cap::rows];
         s.evaluated_cells = hs.evaluated_cells;
-        s.n_scan_items = hp.n_items;
+        s.n_scan_items = hp.n[Cap::items];
         s.n_dropped = hs.n_dropped;
         s.n_truncated = hs.n_truncated;
         s.reserved = (uint32_t)std::min<uint64_t>(hp.fan_keys, 0xffffffffu);
@@ -918,14 +887,14 @@ struct ConfigPipeline {
                     (unsigned long long)hp.fan_dbg[3], (unsigned long long)hp.fan_dbg[4]);
         uint64_t table_bytes = 0;
         for (const ChunkDesc& cd : ctx->cp.chunks) table_bytes += (uint64_t)cd.tbl_words * 8 * s.scan_ctas;
-        s.scan_input_bytes = (R && S) ? hp.n_units * 12 * ctx->cp.chunks.size() + table_bytes : 0;
-        slot->res.n_rows = hp.n_rows;
-        slot->att_cfgs = hp.n_cfg;
-        slot->att_seqs = hp.n_seq;
-        slot->att_terms = hp.n_terms;
-        slot->n_sites = hp.n_sites;
-        slot->n_rsites = hp.n_rsites;
-        slot->res.packed_words = hp.n_rowwords;
+        s.scan_input_bytes = (R && S) ? hp.n[Cap::units] * 12 * ctx->cp.chunks.size() + table_bytes : 0;
+        slot->res.n_rows = hp.n[Cap::rows];
+        slot->att_cfgs = hp.n[Cap::cfg];
+        slot->att_seqs = hp.n[Cap::seq];
+        slot->att_terms = hp.n[Cap::terms];
+        slot->n_sites = hp.n[Cap::sites];
+        slot->n_rsites = hp.n[Cap::rsites];
+        slot->res.packed_words = hp.n[Cap::rowwords];
         slot->res.row_bytes = 4;
         if (ctx->rows_width == 0) slot->res.row_bytes = hs.max_count < 256 ? 1 : (hs.max_count < 65536 ? 2 : 4);
         slot->state = 2;
@@ -1176,7 +1145,7 @@ struct ConfigPipeline {
             if ((rc = grow(ctx, slot->d_left, n * S * eb))) return rc;
             if ((rc = grow(ctx, slot->d_right, n * S * eb))) return rc;
             DevDenseRows out{slot->d_left.p, slot->d_right.p};
-            const u64* n_rows_ptr = &slot->d_plan.as<DevPlan>()->n_rows;
+            const u64* n_rows_ptr = &slot->d_plan.as<DevPlan>()->n[Cap::rows];
 #define TFBS_EXPAND(T)                                                                                                                     \
     TFBS_LAUNCH(k_rows_expand<T>, grid_for(n * 32, 256), 256, 0, so)(S, H, slot->d_hap_group.as<u32>(), n_rows_ptr, slot->d_o_region.as<u32>(), \
                                                                       slot->d_o_base.as<u32>(), slot->d_o_bits.as<u8>(), slot->d_o_off.as<u64>(),  \

@@ -150,8 +150,7 @@ private:
             for (uint32_t r0 = 0; r0 < R; r0 += regions_per_super) {
                 uint32_t nr = std::min(regions_per_super, R - r0);
                 uint64_t pairs = (uint64_t)nr * H;
-                uint32_t cap = 1024;
-                while (cap < 2 * pairs) cap <<= 1;
+                const uint32_t cap = (uint32_t)table_slots_for(pairs);
                 CK(L.d_keys.reserve((size_t)cap * 8));
                 CK(L.d_vals.reserve((size_t)cap * 4));
                 CK(cudaMemsetAsync(L.d_keys.p, 0, (size_t)cap * 8, st));
@@ -232,69 +231,74 @@ private:
     }
 
     // ---- phase 2: batches under the scratch budget ---------------------------------------------------
-    void region_cost(uint32_t r, uint64_t* n_seq, uint64_t* n_d, uint64_t* n_units, uint64_t* n_c, uint64_t* n_keys) const {
-        uint64_t g = ctx->h_ngroups[r];
-        uint64_t W = (uint64_t)(B.h_region_end[r] - B.h_region_start[r] + 1) + B.h_ins_extra[r];
-        uint64_t nk = B.h_inner_off[r + 1] - B.h_inner_off[r];
-        *n_seq = g;
-        *n_d = ctx->h_sum_nd[r];
-        *n_units = g * ((W + 31) / 32 + 3);
-        *n_c = g * n_pid * nk;
-        *n_keys = (uint64_t)n_pid * nk;
+    // region r joins the batch
+    void add_region(Batch* b, uint32_t r) const {
+        const uint64_t g = ctx->h_ngroups[r];
+        const uint64_t W = (uint64_t)(B.h_region_end[r] - B.h_region_start[r] + 1) + B.h_ins_extra[r];
+        const uint64_t nk = B.h_inner_off[r + 1] - B.h_inner_off[r];
+        b->n_seq += g;
+        b->n_d += ctx->h_sum_nd[r];
+        b->n_units += g * ((W + 31) / 32 + 3);
+        b->n_c += g * n_pid * nk;
+        b->n_keys += (uint64_t)n_pid * nk;
+        b->r1 = r + 1;
+        b->nr = b->r1 - b->r0;
     }
-    static uint64_t bytes_of(uint64_t n_seq, uint64_t n_d, uint64_t n_units, uint64_t n_c, uint64_t n_keys) {
-        // sequences (with one work-list item each), diff lists + segments, packed bases, counts, keys, the sequence-keyed map
-        return n_seq * (4 * 7 + 8 * 3 + 1 + 32 + 40) + n_d * (4 + 32) + n_units * 12 + n_c * 4 + n_keys * 24 + n_seq * 2 * 12;
+    // Every scratch buffer of a batch with its bytes: reserve_batch() grows them, plan_batch() adds them up.  visit(buffer, bytes)
+    // once per buffer.  (The rows of fetch_rows are sized by the batch's count pass.)
+    template <class Visit> void batch_buffers(const Batch& b, Visit&& visit) {
+        const uint64_t n_seq = b.n_seq, n_d = b.n_d, n_c = b.n_c, n_keys = b.n_keys;
+        const uint64_t ic = std::max<uint64_t>(1, n_seq);  // at most one item per sequence
+        const uint64_t slots = table_slots_for(n_seq);     // the sequence-keyed map
+        visit(L.d_seq_region, n_seq * 4);
+        visit(L.d_seq_leader, n_seq * 4);
+        visit(L.d_seq_nd, n_seq * 4);
+        visit(L.d_seq_doff, (n_seq + 1) * 8);
+        visit(L.d_dlist, std::max<uint64_t>(1, n_d) * 4);
+        visit(L.d_segs, (2 * n_d + 2 * n_seq) * sizeof(Seg));
+        visit(L.d_seq_nseg, n_seq * 4);
+        visit(L.d_seq_len, n_seq * 4);
+        visit(L.d_seq_hash, n_seq * 8);
+        visit(L.d_seq_flags, n_seq);
+        visit(L.d_seq_ntake, n_seq * 4);
+        visit(L.d_C, std::max<uint64_t>(1, n_c) * 4);
+        visit(L.d_vmin, std::max<uint64_t>(1, n_keys) * 4);
+        visit(L.d_vmax, std::max<uint64_t>(1, n_keys) * 4);
+        visit(L.d_flag, std::max<uint64_t>(1, n_keys) * 4);
+        visit(L.d_rowidx, (n_keys + 1) * 8);
+        visit(L.d_refcnt, (uint64_t)b.nr * 4);
+        visit(L.d_seq_nitems, n_seq * 4);
+        visit(L.d_item_off, (n_seq + 1) * 8);
+        visit(L.d_items, ic * sizeof(ScanItem));
+        visit(L.d_list, ic * 4);
+        visit(L.d_ent_units, ic * 4);
+        visit(L.d_ent_uoff, (ic + 1) * 8);
+        visit(L.d_pk, std::max<uint64_t>(1, b.n_units) * 8);
+        visit(L.d_nm, std::max<uint64_t>(1, b.n_units) * 4);
+        visit(L.d_keys, slots * 8);
+        visit(L.d_vals, slots * 4);
     }
 
     int plan_batch(uint32_t r0, Batch* b) {
-        b->r0 = r0;
-        uint32_t r1 = r0;
-        while (r1 < R) {
-            uint64_t a, b2, c2, d2, e2;
-            region_cost(r1, &a, &b2, &c2, &d2, &e2);
-            if (r1 > r0 && (bytes_of(b->n_seq + a, b->n_d + b2, b->n_units + c2, b->n_c + d2, b->n_keys + e2) > ctx->scratch_bytes ||
-                            b->n_seq + a > 0x7fffffffull || b->n_seq + a + b->n_d + b2 > (1ull << 30)))
-                break;
-            b->n_seq += a; b->n_d += b2; b->n_units += c2; b->n_c += d2; b->n_keys += e2;
-            ++r1;
+        b->r0 = b->r1 = r0;
+        while (b->r1 < R) {
+            Batch t = *b;
+            add_region(&t, b->r1);
+            uint64_t bytes = 0;
+            batch_buffers(t, [&](DevBuf&, uint64_t n) { bytes += n; });
+            if (t.nr > 1 && (bytes > ctx->scratch_bytes || t.n_seq > 0x7fffffffull || t.n_seq + t.n_d > (1ull << 30))) break;
+            *b = t;
         }
-        b->r1 = r1;
-        b->nr = r1 - r0;
         if (b->n_seq > 0x7fffffffull || b->n_seq + b->n_d > (1ull << 30))
             return fail(ctx, TFBS_ERR_INVALID_ARGUMENT, "a single region has more haplotype groups / carried variants than one batch can hold");
         return TFBS_OK;
     }
 
     int reserve_batch(Batch* b) {
-        const uint64_t n_seq = b->n_seq, n_d = b->n_d, n_c = b->n_c, n_keys = b->n_keys;
-        const uint64_t ic = std::max<uint64_t>(1, n_seq);  // at most one item per sequence
-        CK(L.d_seq_region.reserve(n_seq * 4));
-        CK(L.d_seq_leader.reserve(n_seq * 4));
-        CK(L.d_seq_nd.reserve(n_seq * 4));
-        CK(L.d_seq_doff.reserve((n_seq + 1) * 8));
-        CK(L.d_dlist.reserve(std::max<uint64_t>(1, n_d) * 4));
-        CK(L.d_segs.reserve((2 * n_d + 2 * n_seq) * sizeof(Seg)));
-        CK(L.d_seq_nseg.reserve(n_seq * 4));
-        CK(L.d_seq_len.reserve(n_seq * 4));
-        CK(L.d_seq_hash.reserve(n_seq * 8));
-        CK(L.d_seq_flags.reserve(n_seq));
-        CK(L.d_seq_ntake.reserve(n_seq * 4));
-        CK(L.d_C.reserve(std::max<uint64_t>(1, n_c) * 4));
-        CK(L.d_vmin.reserve(std::max<uint64_t>(1, n_keys) * 4));
-        CK(L.d_vmax.reserve(std::max<uint64_t>(1, n_keys) * 4));
-        CK(L.d_flag.reserve(std::max<uint64_t>(1, n_keys) * 4));
-        CK(L.d_rowidx.reserve((n_keys + 1) * 8));
-        CK(L.d_refcnt.reserve((size_t)b->nr * 4));
-        CK(L.d_seq_nitems.reserve(n_seq * 4));
-        CK(L.d_item_off.reserve((n_seq + 1) * 8));
-        CK(L.d_items.reserve(ic * sizeof(ScanItem)));
-        CK(L.d_list.reserve(ic * 4));
-        CK(L.d_ent_units.reserve(ic * 4));
-        CK(L.d_ent_uoff.reserve((ic + 1) * 8));
-        CK(L.d_pk.reserve(std::max<uint64_t>(1, b->n_units) * 8));
-        CK(L.d_nm.reserve(std::max<uint64_t>(1, b->n_units) * 4));
-
+        cudaError_t e = cudaSuccess;
+        batch_buffers(*b, [&](DevBuf& buf, uint64_t bytes) { if (e == cudaSuccess) e = buf.reserve(bytes); });
+        CK(e);
+        const uint64_t n_seq = b->n_seq, ic = std::max<uint64_t>(1, n_seq);
         DevSeqs& sq = b->sq;
         sq = DevSeqs{};
         sq.n_seq = (u32)n_seq;
@@ -337,10 +341,7 @@ private:
         if ((rc = scan(b.sq.seq_nd, n_seq, b.sq.seq_doff))) return rc;
         TFBS_LAUNCH(k_walk, grid_for(n_seq, 128), 128, 0, st)(db, b.sq, ~0ull, dst, 1u);
         ++launches();
-        uint32_t cap = 1024;
-        while (cap < 2 * n_seq) cap <<= 1;
-        CK(L.d_keys.reserve((size_t)cap * 8));
-        CK(L.d_vals.reserve((size_t)cap * 4));
+        const uint32_t cap = (uint32_t)table_slots_for(n_seq);  // reserved by reserve_batch
         CK(cudaMemsetAsync(L.d_keys.p, 0, (size_t)cap * 8, st));
         CK(cudaMemsetAsync(L.d_vals.p, 0xff, (size_t)cap * 4, st));
         CK(cudaMemsetAsync(L.d_ref_used.as<u32>() + b.r0, 0, (size_t)b.nr * 4, st));

@@ -48,7 +48,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--min-seconds", type=float, default=0.5, help="and at least this much timed work per arm")
     ap.add_argument("--scratch-mb", type=int, default=65536, help="option scratch_mb of both arms (the one block's scratch estimate is "
-                    "25.6 GB, more than the default 24 GB)")
+                    "30.9 GB, more than the default 24 GB)")
     ap.add_argument("--out", default="", help="also write the JSON here")
     args = ap.parse_args()
 
